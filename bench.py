@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N ...            # the reference's CPU update step (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as .npy files
 
 A "step" is ONE `SAC_exp._update` for EVERY agent of the population resident on a GPU (gather ->
 critics -> actor (+expert term) -> temperature -> Polyak).  Weak scaling: every rank holds
@@ -43,7 +44,12 @@ def parse():
     p.add_argument("--no-fork", action="store_true", help="whole update on one stream")
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--cpu-seconds", type=float, default=16.0)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last of them computed to DIR/<name>.npy (see dump_outputs)")
+    a = p.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        p.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
+    return a
 
 
 def workload_name(a):
@@ -305,6 +311,34 @@ def measure(pop, a, world, barrier, steps, warmup, torch, dist):
     return float(t.item()), pop.launches - l0
 
 
+DUMP_BYTES = 64 * 10**6      # --dump-outputs writes at most this much (plus the .npy headers)
+DUMP_AGENTS = 16             # agents whose parameter and optimiser tables are written
+DUMP_PER_AGENT = ("losses", "alpha", "alpha_m", "alpha_v")
+DUMP_TABLES = (("actor", "na"), ("actor_m", "na"), ("actor_v", "na"),
+               ("q", "nc"), ("q_m", "nc"), ("q_v", "nc"), ("qt", "nc"))
+
+
+def dump_outputs(pop, out_dir):
+    """Writes the state one timed `pop.update` leaves behind, so that two builds run with the same arguments can be
+    compared array for array: the per-agent losses the call returns and the temperature with its Adam moments, for every
+    agent; the actor, both critics, both targets and their Adam moments (trimmed to the real parameter count, stride
+    padding dropped) for a fixed sample of agents, drawn with numpy.random.default_rng(0), as many as fit DUMP_BYTES
+    up to DUMP_AGENTS.  All float32."""
+    import numpy as np
+    import torch
+    L, n = pop.L, pop.spec.n_agents
+    out = {name: pop.losses if name == "losses" else pop.t[name] for name in DUMP_PER_AGENT}
+    fixed = sum(v.numel() * 4 for v in out.values())
+    per_agent = sum(pop.t[name][0, ..., :getattr(L, width)].numel() * 4 for name, width in DUMP_TABLES)
+    count = min(n, DUMP_AGENTS, (DUMP_BYTES - fixed) // per_agent)
+    agents = np.sort(np.random.default_rng(0).choice(n, size=count, replace=False))
+    sel = torch.as_tensor(agents, device=pop.dev)
+    out.update({name: pop.t[name][sel, ..., :getattr(L, width)] for name, width in DUMP_TABLES})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.float().cpu().numpy())
+
+
 def run_b200(a):
     import numpy as np
     import torch
@@ -353,6 +387,8 @@ def run_b200(a):
     losses = pop.losses.cpu().numpy()
     if not np.isfinite(losses).all():
         raise RuntimeError("non-finite losses after the timed region")
+    if a.dump_outputs and rank == 0:     # before the end-to-end section below updates the same population again
+        dump_outputs(pop, a.dump_outputs)
     value = n_global * a.steps / (ms * 1e-3)
 
     # ---- end-to-end through the host-buffer API ("e2e") -------------------------------------
