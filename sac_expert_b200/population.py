@@ -10,7 +10,7 @@ what the class mirrors in ``sac_expert_b200/sac_eo`` use.
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, replace
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -214,6 +214,7 @@ class Population:
         _l.check(self.lib.saceo_create(C.byref(self.cfg), C.byref(self.ctx)))
         self._bind()
         self.losses = z(n, L.n_losses)
+        self.model_batch = None          # set by fit_bind
         self._pin_idx = None
         self._pin_exp = None
         self._pin_loss = None
@@ -395,6 +396,11 @@ class Population:
     def set_expert(self, agent: int, sE, spE):
         self.t["expert_s"][agent].copy_(torch.from_numpy(np.asarray(sE, np.float32)))
         self.t["expert_sp"][agent].copy_(torch.from_numpy(np.asarray(spE, np.float32)))
+
+    def set_expert_all(self, sE, spE):
+        """``set_expert`` for EVERY agent in one copy per table: ``sE, spE`` [n_agents, E, S]."""
+        self.t["expert_s"].copy_(torch.from_numpy(np.asarray(sE, np.float32)))
+        self.t["expert_sp"].copy_(torch.from_numpy(np.asarray(spE, np.float32)))
 
     # ------------------------------------------------------------------ hot path
     def gather(self, idx: torch.Tensor):
@@ -800,3 +806,20 @@ class Population:
                 logs[i].update(mse=float(extra[0][i]), norm_pg=float(extra[1][i, 6]), norm_MSE=float(extra[1][i, 7]))
         return logs
 
+
+
+class SharedPopulation:
+    """One ``n_agents`` population shared by objects that each describe a single agent: the first ``get(spec)``
+    creates it from the one-agent ``spec`` with ``n_agents`` replaced, every later call must describe the same
+    population.  Lets R algorithm objects built one after the other bind to agents 0 .. R-1 of one population."""
+
+    def __init__(self, n_agents: int):
+        self.n_agents, self.pop = int(n_agents), None
+
+    def get(self, spec: PopulationSpec) -> Population:
+        spec = replace(spec, n_agents=self.n_agents)
+        if self.pop is None:
+            self.pop = Population(spec)
+        elif spec != self.pop.spec:
+            raise ValueError(f"a shared population needs one spec for every agent: {spec} != {self.pop.spec}")
+        return self.pop

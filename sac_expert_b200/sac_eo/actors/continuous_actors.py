@@ -11,6 +11,7 @@ import numpy as np
 import torch
 
 from ..common.device_net import DeviceNet
+from ..common.lockstep import Request, inline, np_random
 from ..common.nn_utils import broadcast_activations, check_two_hidden, create_nn_weights
 from ..envs.synthetic import flatdim
 
@@ -69,16 +70,21 @@ class SquashedGaussianActor(DeviceNet):
         return pop.actor_forward(obs, nz, want_neglogp=want_nlp), x.shape[0]
 
     # ---- reference interface -------------------------------------------------------------
-    def sample(self, s, deterministic=False):
-        n = self._as_rows(s, self.s_dim).shape[0]
-        u = None if deterministic else np.random.normal(size=(n, self.a_dim))      # :297
-        act, n = self._run(s, u, False)
-        act = self._host(act[0])
+    def _sample_steps(self, s, deterministic=False):
+        x = self._as_rows(s, self.s_dim)
+        n = x.shape[0]
+        u = None if deterministic else np_random().normal(size=(n, self.a_dim))    # :297
+        pop = self._need_device()
+        self._sync_rms()
+        act = yield Request("act", pop, self._agent, (n, u is None), obs=x,
+                            noise=None if u is None else np.asarray(u, np.float32).reshape(n, self.a_dim))
         return act[0] if n == 1 else act                                           # squeeze like :302-303
+
+    sample = inline(_sample_steps)
 
     def evaluate(self, s):
         n = self._as_rows(s, self.s_dim).shape[0]
-        u = np.random.normal(size=(n, self.a_dim))                                 # :350
+        u = np_random().normal(size=(n, self.a_dim))                               # :350
         (act, nlp), n = self._run(s, u, True)
         act, nlp = self._host(act[0]), self._host(nlp[0])
         return (act[0], nlp[0]) if n == 1 else (act, nlp)

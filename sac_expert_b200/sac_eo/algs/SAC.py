@@ -16,9 +16,10 @@ import torch
 from ... import lib as _l
 from ...population import Population, PopulationSpec
 from ..common.buffers import TrajectoryBuffer
+from ..common.lockstep import Request, inline, np_random
 from ..common.logger import Logger
 from ..common.normalizer import RunningNormalizers
-from ..common.samplers import trajectory_sampler
+from ..common.samplers import trajectory_sampler_steps
 from ..envs.synthetic import flatdim
 
 _DEFAULTS = dict(gamma=0.995, lam=0.97, init_temperature=0.1, q_crit_lr=3e-4, mbpo_actor_lr=1e-4, mbpo_alpha_lr=1e-4,
@@ -35,7 +36,8 @@ _DEFAULTS = dict(gamma=0.995, lam=0.97, init_temperature=0.1, q_crit_lr=3e-4, mb
 class SAC:
     _expert_term = False
 
-    def __init__(self, idx, env, env_eval, actor, critics, q_targets, q_critics, models, alg_kwargs, mf_update_kwargs):
+    def __init__(self, idx, env, env_eval, actor, critics, q_targets, q_critics, models, alg_kwargs, mf_update_kwargs,
+                 population=None, agent=0):
         self.env, self.env_eval = env, env_eval
         self.actor, self.critics, self.q_targets, self.q_critics, self.models = actor, critics, q_targets, q_critics, models
         self.s_dim, self.a_dim = flatdim(env.observation_space), flatdim(env.action_space)
@@ -47,7 +49,7 @@ class SAC:
         self.model_normalizer = RunningNormalizers(self.s_dim, self.a_dim, self.gamma, self.init_rms_stats)
         self.env_data = TrajectoryBuffer(self.s_dim, self.a_dim, self.gamma, self.lam, self.env_buffer_size)
         self.target_entropy = -len(env.action_space.sample())              # SAC_expert.py:46
-        self._build_population()
+        self._build_population(population, agent)
         self._set_rms()
 
     # ------------------------------------------------------------------ setup
@@ -84,7 +86,9 @@ class SAC:
     def _expert_rows(self):
         return 0
 
-    def _build_population(self):
+    def _build_population(self, population=None, agent=0):
+        """Binds the networks, the replay buffer and the per-agent records to agent ``agent`` of a device population:
+        a new one-agent ``Population`` by default, or the population a ``SharedPopulation`` holds for several runs."""
         a, q, kw = self.actor, self.q_critics[0], self.alg_kwargs
         nm = self._n_models()
         m = self.models[0] if nm else None
@@ -99,18 +103,18 @@ class SAC:
             delta_clip_pred=(m.delta_clip_pred or 0.0) if m else 0.0, B=self.sac_batch_size, E=max(self._expert_rows(), 2),
             target_update_int=self.target_update_int, replay_capacity=cap, std_mult=a.std_mult,
             gemm_mode=kw["gemm_mode"], device=kw["device"])
-        self.pop = Population(spec)
-        pop = self.pop
-        a._bind(pop, 0, "actor")
+        self.pop = pop = Population(spec) if population is None else population.get(spec)
+        self.agent = agent
+        a._bind(pop, agent, "actor")
         for k, (live, tgt) in enumerate(zip(self.q_critics, self.q_targets)):
-            live._bind(pop, 0, "q%d" % (k + 1))
-            tgt._bind(pop, 0, "t%d" % (k + 1))
+            live._bind(pop, agent, "q%d" % (k + 1))
+            tgt._bind(pop, agent, "t%d" % (k + 1))
         for k in range(nm):
-            self.models[k]._bind(pop, 0, "m%d" % (k + 1))
-        pop.t["alpha"][0] = float(np.log(self.init_temperature))          # raw, log-initialised (SAC_expert.py:106)
-        pop.set_hyper(0, gamma=self.gamma, tau=self.soft_tau, lr_q=self.mbpo_lr, lr_pi=self.mbpo_actor_lr,
+            self.models[k]._bind(pop, agent, "m%d" % (k + 1))
+        pop.t["alpha"][agent] = float(np.log(self.init_temperature))      # raw, log-initialised (SAC_expert.py:106)
+        pop.set_hyper(agent, gamma=self.gamma, tau=self.soft_tau, lr_q=self.mbpo_lr, lr_pi=self.mbpo_actor_lr,
                       lr_alpha=self.mbpo_alpha_lr, eps=self.epsilon, target_entropy=float(self.target_entropy))
-        self.env_data.attach(pop, 0)
+        self.env_data.attach(pop, agent)
 
     def _set_rms(self):
         """Shares the normalisers with all networks (SAC_expert.py:135-153)."""
@@ -122,14 +126,15 @@ class SAC:
 
     @property
     def alpha(self):
-        return float(self.pop.t["alpha"][0])
+        return float(self.pop.t["alpha"][self.agent])
 
     # ------------------------------------------------------------------ the hot path
     def _draw(self, expert_reg=None):
         """Host draws in the reference's consumption order (SURVEY.md App. A)."""
         B, A = self.sac_batch_size, self.a_dim
-        idx = np.random.randint(self.env_data.current_size, size=B)        # buffers.py:135
-        u1 = np.random.normal(size=(B, A))                                 # evaluate(sp), continuous_actors.py:350
+        rand = np_random()
+        idx = rand.randint(self.env_data.current_size, size=B)        # buffers.py:135
+        u1 = rand.normal(size=(B, A))                                 # evaluate(sp), continuous_actors.py:350
         perm, u_exp = None, []
         if expert_reg is not None:
             E = len(expert_reg[0])
@@ -142,14 +147,14 @@ class SAC:
                 if len(sections[0]) != len(sections[1]):
                     raise ValueError("two-model expert term needs an even number of expert rows (SAC_expert.py:329-332)")
                 perm = np.concatenate(sections[:2])
-        u2 = np.random.normal(size=(B, A))                                 # evaluate(s)
+        u2 = rand.normal(size=(B, A))                                 # evaluate(s)
         if expert_reg is not None:
             if self._n_models() == 1:
-                u_exp = [np.random.normal(size=(len(perm), A))]
+                u_exp = [rand.normal(size=(len(perm), A))]
             else:
                 h = len(perm) // 2
-                u_exp = [np.random.normal(size=(h, A)), np.random.normal(size=(h, A))]   # sample(s_E_one/two)
-        u5 = np.random.normal(size=(B, A))                                 # evaluate(s) for the alpha step
+                u_exp = [rand.normal(size=(h, A)), rand.normal(size=(h, A))]   # sample(s_E_one/two)
+        u5 = rand.normal(size=(B, A))                                 # evaluate(s) for the alpha step
         noise = np.concatenate([u1, u2] + u_exp + [u5], 0).astype(np.float32)
         return idx.astype(np.int64), noise, perm
 
@@ -159,29 +164,37 @@ class SAC:
         for net in [self.actor] + list(self.q_critics) + list(self.q_targets) + list(self.models[: self._n_models()]):
             net._sync_rms()
 
-    def _device_update(self, num_timesteps, expert_reg=None):
+    def _device_update_steps(self, num_timesteps, expert_reg=None, expert=None, eps=None):
+        """One update of this agent; ``expert`` = (s_E, sp_E) rows and ``eps`` (None: unchanged) are uploaded first."""
         self._sync_rms()
         idx, noise, perm = self._draw(expert_reg)
         self.last_idx = idx
-        self.pop.set_draws(idx[None], noise[None], None if perm is None else perm[None].astype(np.int32))
-        losses = self.pop.update(1, num_timesteps=int(num_timesteps), use_device_rng=False).cpu().numpy()[0]
+        perm = None if perm is None else perm.astype(np.int32)
+        losses = yield Request("update", self.pop, self.agent,
+                               ("update", int(num_timesteps), idx.shape, noise.shape, None if perm is None else perm.shape),
+                               bc=False, num_timesteps=int(num_timesteps), idx=idx, noise=noise, perm=perm, expert=expert,
+                               eps=eps)
         return dict(q1_loss=losses[0], q2_loss=losses[1], pi_loss=losses[2], mse_loss=losses[3], p_loss=losses[4],
                     alpha_loss=losses[5], alpha=losses[6], epsilon=losses[7])
 
-    def _update(self, num_timesteps):
+    def _update_steps(self, num_timesteps):
         """``SAC._update`` (SAC.py:236-250)."""
-        self.last_losses = self._device_update(num_timesteps)
+        self.last_losses = yield from self._device_update_steps(num_timesteps)
+
+    _update = inline(_update_steps)
 
     def _update_q_target(self):
         """Polyak averaging is fused into the critic Adam kernel, gated on
         ``num_timesteps % target_update_int == 0`` like SAC.py:246-248; nothing to do here."""
 
     # ------------------------------------------------------------------ environment loop (host; callers of the hot path)
-    def _evaluate(self, num_timesteps):
+    def _evaluate_steps(self, num_timesteps):
         """``_evaluate`` (base_onpolicy_alg.py:174-197)."""
         t0 = time.time()
-        J = [trajectory_sampler(self.env_eval, self.actor, self.env_horizon, eval=True, deterministic=True)[-1]
-             for _ in range(self.eval_num_traj)]
+        J = []
+        for _ in range(self.eval_num_traj):
+            J.append((yield from trajectory_sampler_steps(self.env_eval, self.actor, self.env_horizon, eval=True,
+                                                          deterministic=True))[-1])
         self.logger.log_train({"J_tot_eval": np.mean(J), "steps_eval": num_timesteps - self.last_eval,
                                "time_eval": time.time() - t0})
         self.last_eval = num_timesteps
@@ -189,7 +202,7 @@ class SAC:
     def _data_sinks(self):
         return [self.env_data]
 
-    def _collect_env_data(self, num_timesteps, update_normalizers=True, only_model_normalizer=False):
+    def _collect_env_data_steps(self, num_timesteps, update_normalizers=True, only_model_normalizer=False):
         """``_collect_env_data`` (SAC_expert.py:625-683 / SAC.py): whole rollouts with the current actor before the
         per-step loop starts."""
         t0 = time.time()
@@ -198,11 +211,12 @@ class SAC:
         cur, J_all = 0, []
         while cur < batch_size:
             horizon = min(batch_size - cur, self.env_horizon) if self.env_batch_type == "steps" else self.env_horizon
-            s, a, r, sp, d, J = trajectory_sampler(self.env, self.actor, horizon, eval=True, corruptor=self.corruptor)
+            s, a, r, sp, d, J = yield from trajectory_sampler_steps(self.env, self.actor, horizon, eval=True,
+                                                                    corruptor=self.corruptor)
             if update_normalizers:
                 (self.model_normalizer if only_model_normalizer else self.normalizer).update_rms(s, a, r, sp)
             for sink in self._data_sinks():
-                sink.add(s, a, r, sp, d)
+                yield from sink._add_steps(s, a, r, sp, d)
             if horizon == self.env_horizon:
                 J_all.append(J)
             cur = (self.env_data.steps_total - steps_start) if self.env_batch_type == "steps" \
@@ -213,12 +227,13 @@ class SAC:
                                "traj": self.env_data.traj_total - traj_start, "time_env_data": time.time() - t0})
         return steps_new
 
-    def _episode_start(self):
+    def _episode_start_steps(self):
         """Per-episode work before the first step (SAC_exp: model fitting + adaptive expert weight)."""
         return None
+        yield
 
-    def _step_update(self, num_timesteps, episode_ctx):
-        self._update(num_timesteps)
+    def _step_update_steps(self, num_timesteps, episode_ctx):
+        yield from self._update_steps(num_timesteps)
 
     def _dump_and_save(self, params):
         """``_dump_and_save`` (base_onpolicy_alg.py:366-374)."""
@@ -227,15 +242,17 @@ class SAC:
         self.logger.dump_and_save(self.save_path, self.checkpoint_name)
         self.logger.reset()
 
-    def _train_prologue(self):
+    def _train_prologue_steps(self):
         self._set_rms()
+        return
+        yield
 
-    def train(self, total_timesteps, params):
+    def train_steps(self, total_timesteps, params):
         """The reference's training loop (SAC_expert.py:685-824; SAC.py:254-385): initial data collection, then one
         environment step + one ``_update`` per iteration, per-episode bookkeeping, evaluation and checkpoints.  Host
-        Python; every network call inside is a device call.  Returns the checkpoint name."""
+        Python; every network call inside is a device request (``common/lockstep.py``).  Returns the checkpoint name."""
         total_timesteps = int(total_timesteps)
-        self._train_prologue()
+        yield from self._train_prologue_steps()
         pts = lambda f: np.concatenate((np.arange(0, total_timesteps, f)[1:], [total_timesteps]))
         checkpoints = np.array([total_timesteps]) if self.save_freq is None else pts(self.save_freq)
         evaluate = self.eval_freq is not None
@@ -243,8 +260,8 @@ class SAC:
         checkpt_idx = eval_idx = 0
         num_timesteps = 0
         if evaluate:
-            self._evaluate(num_timesteps)
-        num_timesteps += self._collect_env_data(num_timesteps, update_normalizers=self.update_normalizers,
+            yield from self._evaluate_steps(num_timesteps)
+        num_timesteps += yield from self._collect_env_data_steps(num_timesteps, update_normalizers=self.update_normalizers,
                                                 only_model_normalizer=self.only_model_normalizer)
         new_traj = TrajectoryBuffer(self.s_dim, self.a_dim, self.gamma, self.lam)
         episode_step, episode, episode_reward, done = 0, 0, 0.0, True
@@ -267,29 +284,31 @@ class SAC:
                 obs = self.env.reset()
                 done, episode_reward, episode_step = False, 0.0, 0
                 episode += 1
-                ctx = self._episode_start()
+                ctx = yield from self._episode_start_steps()
                 t0 = time.time()
-            a = np.asarray(self.actor.sample(obs, deterministic=not self.random_act).numpy())      # SAC_expert.py:779
-            self._step_update(num_timesteps, ctx)
+            a = np.asarray((yield from self.actor._sample_steps(obs, deterministic=not self.random_act)).numpy())   # :779
+            yield from self._step_update_steps(num_timesteps, ctx)
             next_obs, r, done, _ = self.env.step(self.actor.clip(a))
             done_no_max = False if episode_step + 1 == self._max_episode_steps else done
             episode_reward += r
             row = (np.array([obs]), np.array([a]), np.array([r]), np.array([next_obs]), np.array([done_no_max]))
             for sink in self._data_sinks():
-                sink.add(*row)
+                yield from sink._add_steps(*row)
             if self.update_normalizers:
                 new_traj.add(*row)
             obs = next_obs
             episode_step += 1
             num_timesteps += 1
             if evaluate and num_timesteps >= eval_points[eval_idx]:
-                self._evaluate(num_timesteps)
+                yield from self._evaluate_steps(num_timesteps)
                 eval_idx += 1
             if num_timesteps >= checkpoints[checkpt_idx]:
                 self._dump_and_save(params)
                 checkpt_idx += 1
         self._dump_and_save(params)
         return self.checkpoint_name
+
+    train = inline(train_steps)
 
     def _dump_stats(self):
         """{'actor_weights','critic_weights','rms_stats'} checkpoint payload (base_onpolicy_alg.py:351-364)."""

@@ -7,6 +7,7 @@ import numpy as np
 import torch
 
 from ...lib import SaceoError
+from .lockstep import Request, inline, np_random
 
 
 class TrajectoryBuffer:
@@ -58,7 +59,7 @@ class TrajectoryBuffer:
         if self.current_size:
             pop.append_rows(agent, self.s_all, self.a_all, self.r_all, self.sp_all, self.d_all)
 
-    def add(self, s_traj, a_traj, r_traj, sp_traj, d_traj):
+    def _add_steps(self, s_traj, a_traj, r_traj, sp_traj, d_traj):
         s_traj = np.asarray(s_traj).reshape(-1, self.s_dim)
         a_traj = np.asarray(a_traj).reshape(-1, self.a_dim)
         r_traj, d_traj = np.atleast_1d(np.asarray(r_traj)), np.atleast_1d(np.asarray(d_traj))
@@ -82,7 +83,9 @@ class TrajectoryBuffer:
         if self._pop is not None:
             if not self.buffer_size and self.current_size > self._pop.spec.replay_capacity:
                 raise SaceoError("unbounded TrajectoryBuffer outgrew the device replay_capacity")
-            self._pop.append_rows(self._agent, s_traj, a_traj, r_traj, sp_traj, d_traj)
+            yield Request("append", self._pop, self._agent, (k,), rows=(s_traj, a_traj, r_traj, sp_traj, d_traj))
+
+    add = inline(_add_steps)
 
     def _device_gather(self, idx):
         if self._pop is None:
@@ -96,7 +99,7 @@ class TrajectoryBuffer:
 
     def get_offmodel_info(self, batch_size=None):
         if batch_size:
-            idx = np.random.randint(self.current_size, size=batch_size)
+            idx = np_random().randint(self.current_size, size=batch_size)
             self.last_idx = idx
             s, a, sp, r, d = self._device_gather(idx)
             return s, a, sp, r, d
@@ -104,7 +107,7 @@ class TrajectoryBuffer:
 
     def get_model_info(self, batch_size=None):
         if batch_size:
-            idx = np.random.randint(self.current_size, size=batch_size)
+            idx = np_random().randint(self.current_size, size=batch_size)
             if self._pop is not None and batch_size == self._pop.spec.B:
                 s, a, sp, r, _ = self._device_gather(idx)
                 return s, a, sp, r

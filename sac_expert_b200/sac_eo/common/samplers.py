@@ -3,14 +3,25 @@
 per-step ``actor.sample`` is the batched device forward (``saceo_actor_forward``)."""
 import numpy as np
 
+from .lockstep import run_inline
+
 
 def trajectory_sampler(env, actor, horizon, s_init=None, eval=False, deterministic=False, corruptor=None):
+    return run_inline(trajectory_sampler_steps(env, actor, horizon, s_init, eval, deterministic, corruptor))
+
+
+def trajectory_sampler_steps(env, actor, horizon, s_init=None, eval=False, deterministic=False, corruptor=None):
+    """``trajectory_sampler`` as a generator of its device requests (``common/lockstep.py``); an actor without
+    ``_sample_steps`` (any object with the reference's ``sample``) is called directly."""
+    sample_steps = getattr(actor, "_sample_steps", None)
     s_traj, a_traj, r_traj, sp_traj, d_traj = [], [], [], [], []
     J_tot = 0.0
     s = env.reset(s_init) if s_init is not None else env.reset()
     for t in range(int(horizon)):
         s_old = s
-        a = np.asarray(actor.sample(s_old, deterministic=deterministic).numpy())
+        a = (yield from sample_steps(s_old, deterministic=deterministic)) if sample_steps is not None \
+            else actor.sample(s_old, deterministic=deterministic)
+        a = np.asarray(a.numpy())
         s_true, r, d, _ = env.step(actor.clip(a))
         if corruptor is not None:
             s_store = corruptor.corrupt_samples(s_true)

@@ -4,6 +4,8 @@ The simulators are out of scope (SURVEY.md §2 row 16); this class only supplies
 ``action_space`` and a cheap linear-dynamics ``step`` for smoke runs."""
 import numpy as np
 
+from ..common.lockstep import np_random
+
 
 class Box:
     def __init__(self, low, high, shape):
@@ -12,7 +14,7 @@ class Box:
         self.high = np.full(self.shape, high, np.float32)
 
     def sample(self):
-        return np.random.uniform(self.low, self.high).astype(np.float32)
+        return np_random().uniform(self.low, self.high).astype(np.float32)
 
 
 def flatdim(space) -> int:

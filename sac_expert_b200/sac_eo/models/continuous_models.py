@@ -7,6 +7,7 @@ import numpy as np
 import torch
 
 from ..common.device_net import DeviceNet
+from ..common.lockstep import Request, inline
 from ..common.nn_utils import broadcast_activations, check_two_hidden, create_nn_weights
 from ..envs.synthetic import flatdim
 
@@ -90,16 +91,18 @@ class MSEModel(DeviceNet):
             if name is not None:
                 self._pop.set_net(self._agent, name, self._reward_weights)
 
-    def sample(self, s, a, deterministic=True):
+    def _sample_steps(self, s, a, deterministic=True):
         if self.gaussian and not deterministic:
             raise NotImplementedError("stochastic GaussianModel rollouts are not on the SAC-EO update path")
         pop = self._need_device()
         self._sync_rms()
         net = int(self._table[1]) - 1
         s_, a_ = self._as_rows(s, self.s_dim), self._as_rows(np.asarray(a), self.a_dim)
-        sp = pop.model_eval(torch.from_numpy(s_)[None], torch.from_numpy(a_)[None])
-        out = self._host(sp[0, net])
+        sp = yield Request("model", pop, self._agent, (s_.shape[0],), obs=s_, act=a_)
+        out = sp[net]
         return out[0] if out.shape[0] == 1 else out
+
+    sample = inline(_sample_steps)
 
     def get_loss(self, s, sp, a, r):
         raise NotImplementedError("per-model losses are evaluated inside the joint device step: use "

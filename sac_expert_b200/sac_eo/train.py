@@ -21,15 +21,15 @@ from .envs import init_env
 from .models.init_world_models import init_world_models
 
 
-def train(inputs_dict):
-    """Training on given seed (train.py:33-107)."""
+def build_run(inputs_dict, population=None, agent=0):
+    """Seeds, environments, networks and algorithm of one run (train.py:33-106), in the reference's order, so the run
+    consumes the global NumPy stream like the reference.  ``population`` / ``agent``: see ``init_alg``."""
     setup = inputs_dict["setup_kwargs"]
     idx = setup["idx"]
     inputs_dict["alg_kwargs"]["alg_seed"] = setup["algorithm_seed"]
     env_kwargs, actor_kwargs = inputs_dict["env_kwargs"], inputs_dict["actor_kwargs"]
     critic_kwargs, model_kwargs = inputs_dict["critic_kwargs"], inputs_dict["model_kwargs"]
     alg_kwargs, mf_update_kwargs = inputs_dict["alg_kwargs"], inputs_dict["mf_update_kwargs"]
-    total_timesteps = alg_kwargs["total_timesteps"]
 
     init_seeds(setup["setup_seed"])
     env, env_eval, env_expert = init_env(**env_kwargs), init_env(**env_kwargs), init_env(**env_kwargs)
@@ -52,9 +52,14 @@ def train(inputs_dict):
     init_seeds(setup["eval_seed"], env_eval)
     init_seeds(setup["sim_seed"], env)
     init_seeds(setup["expert_seed"], env_expert)
-    alg = init_alg(idx, env, env_eval, env_expert, actor, critics, q_targets, q_critics, models, alg_kwargs,
-                   mf_update_kwargs, expert, init_expert_rms_stats)
-    return alg.train(total_timesteps, inputs_dict)
+    return init_alg(idx, env, env_eval, env_expert, actor, critics, q_targets, q_critics, models, alg_kwargs,
+                    mf_update_kwargs, expert, init_expert_rms_stats, population, agent)
+
+
+def train(inputs_dict):
+    """Training on given seed (train.py:33-107)."""
+    total_timesteps = inputs_dict["alg_kwargs"]["total_timesteps"]
+    return build_run(inputs_dict).train(total_timesteps, inputs_dict)
 
 
 def build_inputs(args):
@@ -75,11 +80,8 @@ def build_inputs(args):
     return out
 
 
-def main(argv=None):
-    start = datetime.now()
-    args = create_train_parser().parse_args(argv)
-    inputs_list = build_inputs(args)
-    log_names = [train(inp) for inp in inputs_list]
+def save_outputs(args, log_names):
+    """Aggregates the per-run checkpoint files into one pickle and removes them (train.py:159-194); returns its path."""
     outputs = []
     os.makedirs(args.save_path, exist_ok=True)
     for name in log_names:                           # aggregate the per-run checkpoint files (train.py:159-168)
@@ -97,6 +99,14 @@ def main(argv=None):
         fn = os.path.join(args.save_path, name)
         if os.path.exists(fn):
             os.remove(fn)
+    return save_filefull
+
+
+def main(argv=None):
+    start = datetime.now()
+    args = create_train_parser().parse_args(argv)
+    inputs_list = build_inputs(args)
+    save_filefull = save_outputs(args, [train(inp) for inp in inputs_list])
     end = datetime.now()
     print("Time Elapsed: %s" % (end - start))
     return save_filefull
