@@ -342,6 +342,33 @@ int saceo_trpo_eval(saceo_ctx *ctx, const float *act, const float *adv, const fl
  * tables.actor[agent] = theta_ref[agent] + scale[agent] * dir[agent]; theta_ref, dir [n, na_stride], scale [n]. */
 int saceo_actor_step(saceo_ctx *ctx, const float *theta_ref, const float *dir, const float *scale, void *stream);
 
+/* ---- policy acting for any depth (expert policies) ------------------------------------------------
+ * An expert is only ever rolled out, never trained: SAC_exp._collect_expert_data (sac_eo/algs/SAC_expert.py:156-209)
+ * calls expert.sample(s, deterministic=True) through trajectory_sampler (common/samplers.py:31).  The reference loads
+ * that expert with --expert_file (train.py:65-83); it is a GaussianActor (actors/continuous_actors.py:9-234) or a
+ * SquashedGaussianActor (:237-415) of any depth.  These entry points act for a set of n_policies independent policies
+ * in one launch, in exact fp32 on CUDA cores, without a context and without the two-hidden-layer training engine. */
+#define SACEO_POLICY_MAX_HIDDEN 8
+typedef struct saceo_policy_config {
+  int32_t abi_version, device, n_policies, S, A;
+  int32_t n_hidden, hidden[SACEO_POLICY_MAX_HIDDEN], act[SACEO_POLICY_MAX_HIDDEN];   /* widths 1..1024, SACEO_ACT_* */
+  int32_t squash, per_state_std;   /* head; per_state_std: output 2A, else A outputs + logstd variable [A] */
+  float   std_mult;                /* GaussianActor only */
+} saceo_policy_config;
+
+/* Host arithmetic, no GPU: parameter count, per-policy stride (padded to 32 words), normaliser record stride.  Any
+ * output pointer may be NULL. */
+int saceo_policy_layout(const saceo_policy_config *cfg, int64_t *n_params, int64_t *param_stride, int32_t *norm_stride);
+
+/* expert.sample(s, deterministic) for every policy of the set: GaussianActor._forward + .sample (squash = 0,
+ * continuous_actors.py:74-123) or SquashedGaussianActor.sample (squash = 1, :270-306), observations normalised with the
+ * policy's own statistics (normalizer.py:26-41).
+ * params [P, param_stride] flat Keras order [W0|b0|...|Wn|bn|(logstd)]; norm [P, norm_stride] = s_mean | s_std | act_limit;
+ * obs [P, rows, S]; noise [P, rows, A] or NULL (deterministic); act_out [P, rows, A].  All device pointers on cfg->device.
+ * Stream-ordered, no context; one kernel launch.  Policy i's actions are bit-identical whatever the other policies are. */
+int saceo_policy_act(const saceo_policy_config *cfg, const float *params, const float *norm, const float *obs,
+                     int32_t rows, const float *noise, float *act_out, void *stream);
+
 /* Test / inspection surface: device pointer of a named workspace buffer (e.g. "g_q", "g_actor",
  * "y", "losses", "idx", "noise") and its size in bytes; NULL if unknown. */
 void *saceo_debug_ptr(saceo_ctx *ctx, const char *name, int64_t *bytes_out);

@@ -19,6 +19,7 @@
 #include "mlp_ws.cuh"
 #include "model_term.cuh"
 #include "model_fit.cuh"
+#include "policy.cuh"
 
 using namespace saceo;
 
@@ -1515,6 +1516,113 @@ extern "C" int saceo_actor_step(saceo_ctx* x, const float* theta_ref, const floa
   LAUNCH(x, k_actor_step, dim3(cdiv(x->L.na, 256), k.n_agents), 256, 0, st, k, theta_ref, dir, scale);
   x->planes_dirty |= 1;        // theta written outside k_adam: the weight planes are rebuilt before their next use
   return check_launch();
+}
+
+// ------------------------------------------------------------------------------------------
+// policy acting for any depth (policy.cuh)
+// ------------------------------------------------------------------------------------------
+static int policy_validate(const saceo_policy_config* c) {
+  if (!c) return fail(SACEO_E_INVALID, "null policy config");
+  if (c->abi_version != SACEO_ABI_VERSION) return fail(SACEO_E_INVALID, "abi_version %d != %d", c->abi_version, SACEO_ABI_VERSION);
+  if (c->n_policies < 1 || c->n_policies > 65535) return fail(SACEO_E_INVALID, "n_policies must be in [1, 65535]");
+  if (c->S < 1 || c->A < 1) return fail(SACEO_E_INVALID, "S and A must be positive");
+  if (c->n_hidden < 1 || c->n_hidden > SACEO_POLICY_MAX_HIDDEN)
+    return fail(SACEO_E_INVALID, "n_hidden must be in [1, %d] (got %d)", SACEO_POLICY_MAX_HIDDEN, c->n_hidden);
+  for (int l = 0; l < c->n_hidden; ++l) {
+    if (c->hidden[l] < 1 || c->hidden[l] > POL_MAX_WIDTH)
+      return fail(SACEO_E_INVALID, "hidden width %d of layer %d outside [1, %d]", c->hidden[l], l, POL_MAX_WIDTH);
+    if (c->act[l] < SACEO_ACT_RELU || c->act[l] > SACEO_ACT_ELU)
+      return fail(SACEO_E_INVALID, "activations must be tanh, relu or elu (layer %d: %d)", l, c->act[l]);
+  }
+  if (!(c->std_mult > 0.f)) return fail(SACEO_E_INVALID, "std_mult must be positive");
+  return 0;
+}
+
+static void policy_layout(const saceo_policy_config* c, long long* n, long long* stride, int* nstride, long long* off) {
+  const int Ao = c->per_state_std ? 2 * c->A : c->A;
+  long long o = 0; int in = c->S;
+  for (int l = 0; l <= c->n_hidden; ++l) {
+    const int outw = l < c->n_hidden ? c->hidden[l] : Ao;
+    if (off) off[l] = o;
+    o += (long long)in * outw + outw;
+    in = outw;
+  }
+  if (off) off[c->n_hidden + 1] = o;
+  if (!c->per_state_std) o += c->A;          // logstd variable (continuous_actors.py:56-57)
+  *n = o; *stride = rup(o, 32); *nstride = (int)rup(2LL * c->S + c->A, 4);
+}
+
+extern "C" int saceo_policy_layout(const saceo_policy_config* cfg, int64_t* n_params, int64_t* param_stride,
+                                   int32_t* norm_stride) {
+  int rc = policy_validate(cfg); if (rc) return rc;
+  long long n, s; int ns;
+  policy_layout(cfg, &n, &s, &ns, nullptr);
+  if (n_params) *n_params = n;
+  if (param_stride) *param_stride = s;
+  if (norm_stride) *norm_stride = ns;
+  return 0;
+}
+
+static constexpr int kPolMaxSmem = 200 * 1024;
+static int policy_device_ready(int dev) {      // sm_100 check + shared-memory opt-in, once per device
+  static int ready[64] = {0};
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+    cudaGetLastError();
+    return fail(SACEO_E_NODEVICE, "no CUDA device: libsaceo has no CPU fallback");
+  }
+  if (dev < 0 || dev >= ndev || dev >= 64) return fail(SACEO_E_INVALID, "device %d out of range", dev);
+  if (ready[dev]) return 0;
+  int major = 0, minor = 0;
+  CU(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
+  CU(cudaDeviceGetAttribute(&minor, cudaDevAttrComputeCapabilityMinor, dev));
+  if (major != 10) return fail(SACEO_E_NODEVICE, "device %d is sm_%d%d; libsaceo is built for sm_100a only", dev, major, minor);
+  int prev = 0;
+  CU(cudaGetDevice(&prev));
+  if (prev != dev) CU(cudaSetDevice(dev));
+  const cudaError_t e = cudaFuncSetAttribute(k_policy_forward, cudaFuncAttributeMaxDynamicSharedMemorySize, kPolMaxSmem);
+  if (prev != dev) cudaSetDevice(prev);
+  CU(e);
+  ready[dev] = 1;
+  return 0;
+}
+
+extern "C" int saceo_policy_act(const saceo_policy_config* cfg, const float* params, const float* norm, const float* obs,
+                                int32_t rows, const float* noise, float* act_out, void* stream) {
+  int rc = policy_validate(cfg); if (rc) return rc;
+  if (rows < 1) return fail(SACEO_E_INVALID, "rows must be positive");
+  if (!params || !norm || !obs || !act_out) return fail(SACEO_E_INVALID, "null argument");
+  PolicyP p{};
+  long long n; int ns;
+  policy_layout(cfg, &n, &p.pstride, &ns, p.off);
+  p.params = params; p.norm = norm; p.obs = obs; p.noise = noise; p.out = act_out;
+  p.nstride = ns; p.rows = rows; p.S = cfg->S; p.A = cfg->A; p.Ao = cfg->per_state_std ? 2 * cfg->A : cfg->A;
+  p.nl = cfg->n_hidden + 1;
+  p.width[0] = cfg->S;
+  int w = cfg->S > p.Ao ? cfg->S : p.Ao;
+  for (int l = 0; l < cfg->n_hidden; ++l) {
+    p.width[l + 1] = cfg->hidden[l]; p.act[l] = cfg->act[l];
+    if (cfg->hidden[l] > w) w = cfg->hidden[l];
+  }
+  p.width[p.nl] = p.Ao; p.act[cfg->n_hidden] = ACT_LINEAR;
+  p.squash = cfg->squash != 0; p.per_state_std = cfg->per_state_std != 0;
+  p.ls_add = cfg->per_state_std ? (float)(log((double)cfg->std_mult) - log(log(2.0))) : (float)log((double)cfg->std_mult);
+  p.ld = (int)rup(w, 4);
+  // row tile: as many rows as ~96 KB of ping-pong buffers hold (weight reuse), at least one 4-row block
+  int rt = (96 * 1024 / 4) / (2 * p.ld);
+  rt = rt < POL_RB ? POL_RB : rt > 32 ? 32 : rt / POL_RB * POL_RB;
+  if (rt > rup(rows, POL_RB)) rt = (int)rup(rows, POL_RB);
+  p.rt = rt;
+  const size_t smem = (size_t)2 * rt * p.ld * sizeof(float);
+  if (smem > (size_t)kPolMaxSmem) return fail(SACEO_E_INVALID, "S = %d too wide for the shared-memory activation buffers", cfg->S);
+  rc = policy_device_ready(cfg->device); if (rc) return rc;
+  int prev = 0;
+  CU(cudaGetDevice(&prev));
+  if (prev != cfg->device) CU(cudaSetDevice(cfg->device));
+  k_policy_forward<<<dim3(cdiv(rows, rt), cfg->n_policies), POL_THREADS, smem, (cudaStream_t)stream>>>(p);
+  rc = check_launch();
+  if (prev != cfg->device) cudaSetDevice(prev);
+  return rc;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -71,6 +71,18 @@ class FitTables(C.Structure):
                 "reward", "reward_m", "reward_v")
 
 
+POLICY_MAX_HIDDEN = 8
+
+
+class PolicyConfig(C.Structure):
+    """saceo_policy_config (include/saceo.h): a set of policies of any depth, acted by ``saceo_policy_act``."""
+    _fields_ = [
+        ("abi_version", C.c_int32), ("device", C.c_int32), ("n_policies", C.c_int32), ("S", C.c_int32), ("A", C.c_int32),
+        ("n_hidden", C.c_int32), ("hidden", C.c_int32 * POLICY_MAX_HIDDEN), ("act", C.c_int32 * POLICY_MAX_HIDDEN),
+        ("squash", C.c_int32), ("per_state_std", C.c_int32), ("std_mult", C.c_float),
+    ]
+
+
 FIT_HYPER = 8
 FIT_HYPER_NAMES = ("model_lr", "reward_loss_coef", "delta_clip_loss", "reward_clip_loss", "model_max_grad_norm",
                    "r_mean", "r_std", "scale_model_loss")
@@ -83,6 +95,7 @@ EXPORTS = [
     "saceo_set_draws", "saceo_update", "saceo_update_host", "saceo_update_host_async", "saceo_update_phase", "saceo_bc_update", "saceo_profile_step",
     "saceo_actor_forward", "saceo_critic_forward", "saceo_model_eval", "saceo_fvp", "saceo_cg_solve",
     "saceo_fit_bind", "saceo_model_fit", "saceo_trpo_grad", "saceo_trpo_eval", "saceo_actor_step", "saceo_ppo_grad", "saceo_actor_adam", "saceo_onpolicy_expert_grad", "saceo_grad_blend",
+    "saceo_policy_layout", "saceo_policy_act",
     "saceo_debug_ptr", "saceo_launch_count", "saceo_test_gemm", "saceo_last_error", "saceo_abi_version",
 ]
 
@@ -127,6 +140,8 @@ def load() -> C.CDLL:
         "saceo_actor_adam": (C.c_int, [vp, vp, vp]),
         "saceo_onpolicy_expert_grad": (C.c_int, [vp, C.c_int32, C.c_int32, vp, vp, vp]),
         "saceo_grad_blend": (C.c_int, [vp, vp, vp, vp, f32, vp, vp, vp]),
+        "saceo_policy_layout": (C.c_int, [C.POINTER(PolicyConfig), C.POINTER(i64), C.POINTER(i64), C.POINTER(i32)]),
+        "saceo_policy_act": (C.c_int, [C.POINTER(PolicyConfig), vp, vp, vp, i32, vp, vp, vp]),
         "saceo_debug_ptr": (vp, [vp, C.c_char_p, C.POINTER(i64)]),
         "saceo_launch_count": (i64, [vp]),
         "saceo_test_gemm": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp]),

@@ -17,6 +17,7 @@ import numpy as np
 import torch
 
 from . import lib as _l
+from .policy import PolicySet, PolicySpec
 
 LOSS_NAMES = ("q1_loss", "q2_loss", "pi_loss", "mse_loss", "p_loss", "alpha_loss", "alpha", "epsilon")
 HYPER_NAMES = ("gamma", "tau", "lr_q", "lr_pi", "lr_alpha", "eps", "target_entropy", "damp")
@@ -811,15 +812,16 @@ class Population:
 class SharedPopulation:
     """One ``n_agents`` population shared by objects that each describe a single agent: the first ``get(spec)``
     creates it from the one-agent ``spec`` with ``n_agents`` replaced, every later call must describe the same
-    population.  Lets R algorithm objects built one after the other bind to agents 0 .. R-1 of one population."""
+    population.  Lets R algorithm objects built one after the other bind to agents 0 .. R-1 of one population.
+    A ``PolicySpec`` (expert policies, ``policy.py``) makes it a ``PolicySet`` of ``n_agents`` policies instead."""
 
     def __init__(self, n_agents: int):
         self.n_agents, self.pop = int(n_agents), None
 
-    def get(self, spec: PopulationSpec) -> Population:
+    def get(self, spec):
         spec = replace(spec, n_agents=self.n_agents)
         if self.pop is None:
-            self.pop = Population(spec)
+            self.pop = PolicySet(spec) if isinstance(spec, PolicySpec) else Population(spec)
         elif spec != self.pop.spec:
             raise ValueError(f"a shared population needs one spec for every agent: {spec} != {self.pop.spec}")
         return self.pop

@@ -18,6 +18,7 @@ from ...population import Population, PopulationSpec
 from ..common.buffers import TrajectoryBuffer
 from ..common.lockstep import Request, inline, np_random
 from ..common.logger import Logger
+from ..common.nn_utils import check_two_hidden
 from ..common.normalizer import RunningNormalizers
 from ..common.samplers import trajectory_sampler_steps
 from ..envs.synthetic import flatdim
@@ -90,6 +91,7 @@ class SAC:
         """Binds the networks, the replay buffer and the per-agent records to agent ``agent`` of a device population:
         a new one-agent ``Population`` by default, or the population a ``SharedPopulation`` holds for several runs."""
         a, q, kw = self.actor, self.q_critics[0], self.alg_kwargs
+        check_two_hidden(a.layers)           # the training engine's actor: two hidden layers (DESIGN.md §8)
         nm = self._n_models()
         m = self.models[0] if nm else None
         cap = self.env_buffer_size or int(kw["device_replay_capacity"])

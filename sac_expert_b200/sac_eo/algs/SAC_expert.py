@@ -74,16 +74,27 @@ class SAC_exp(SAC):
     def _bind_expert(self, population=None, agent=0):
         """The expert policy is only ever rolled out (never updated): it gets a single-agent device population of its
         own for its forward passes, with its own normaliser statistics (``init_expert_rms_stats``, :128-133), or agent
-        ``agent`` of the population a ``SharedPopulation`` holds for the experts of several runs."""
+        ``agent`` of the population a ``SharedPopulation`` holds for the experts of several runs.  A two-hidden-layer
+        ``SquashedGaussianActor`` goes on the training engine's ``Population``; every other expert (a ``GaussianActor``,
+        any depth) on a ``PolicySet``, which acts policies of any depth in one launch."""
         if self.expert is None or getattr(self.expert, "_pop", None) is not None:
             return
         from ...population import Population, PopulationSpec
+        from ...policy import PolicySet, PolicySpec
+        from ..actors.continuous_actors import SquashedGaussianActor
         e = self.expert
-        spec = PopulationSpec(n_agents=1, S=self.s_dim, A=self.a_dim, actor_hidden=e.layers, critic_hidden=(8, 8),
-                              model_hidden=(8, 8), actor_acts=e.activations, per_state_std=e.per_state_std, num_models=0,
-                              B=self.sac_batch_size, E=2, replay_capacity=16, std_mult=e.std_mult,
-                              gemm_mode=self.alg_kwargs["gemm_mode"], device=self.alg_kwargs["device"])
-        self._expert_pop = Population(spec) if population is None else population.get(spec)
+        if isinstance(e, SquashedGaussianActor) and len(e.layers) == 2:
+            spec = PopulationSpec(n_agents=1, S=self.s_dim, A=self.a_dim, actor_hidden=e.layers, critic_hidden=(8, 8),
+                                  model_hidden=(8, 8), actor_acts=e.activations, per_state_std=e.per_state_std, num_models=0,
+                                  B=self.sac_batch_size, E=2, replay_capacity=16, std_mult=e.std_mult,
+                                  gemm_mode=self.alg_kwargs["gemm_mode"], device=self.alg_kwargs["device"])
+            make = Population
+        else:
+            spec = PolicySpec(n_agents=1, S=self.s_dim, A=self.a_dim, hidden=e.layers, acts=e.activations,
+                              squash=isinstance(e, SquashedGaussianActor), per_state_std=e.per_state_std,
+                              std_mult=e.std_mult, device=self.alg_kwargs["device"])
+            make = PolicySet
+        self._expert_pop = make(spec) if population is None else population.get(spec)
         e._bind(self._expert_pop, agent, "actor")
         e.set_rms(self.expert_normalizer)
 

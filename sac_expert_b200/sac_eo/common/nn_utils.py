@@ -1,7 +1,8 @@
 """Weight-list conventions of the reference networks (``/root/reference/sac_eo/common/nn_utils.py``):
 Keras ``Sequential`` of ``Dense`` layers, ``y = x @ W + b``, ``W: [in, out]``, ``get_weights()`` order
 ``[W0, b0, W1, b1, W2, b2]``; orthogonal(sqrt 2) hidden / orthogonal(gain) final initialisation, zero biases.
-Two hidden layers are supported (every BASELINE config is 2x256 / 2x512)."""
+The networks this project trains have two hidden layers (every BASELINE config is 2x256 / 2x512); weight lists of any
+depth are built for actors that are only acted (expert policies)."""
 import math
 
 import numpy as np
@@ -40,11 +41,11 @@ def _orthogonal(rng, rows, cols, gain):
 def create_nn_weights(in_dim, out_dim, layers, gain, init_type="orthogonal", rng=None):
     """Initial weight list of ``create_nn`` (nn_utils.py:86-138)."""
     rng = rng if rng is not None else np.random.default_rng(np.random.randint(2 ** 31))
-    dims = [in_dim, layers[0], layers[1], out_dim]
+    dims = [in_dim] + list(layers) + [out_dim]
     ws = []
-    for l in range(3):
+    for l in range(len(layers) + 1):
         rows, cols = dims[l], dims[l + 1]
-        last = l == 2
+        last = l == len(layers)
         if init_type == "orthogonal":
             w = _orthogonal(rng, rows, cols, gain if (last and gain) else math.sqrt(2.0))
         elif init_type == "var":          # VarianceScaling(uniform, fan_out)

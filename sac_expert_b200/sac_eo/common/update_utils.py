@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 from ...population import Population, PopulationSpec
+from .nn_utils import check_two_hidden
 
 
 class _DeviceF:
@@ -70,7 +71,8 @@ class _DeviceF:
 
 
 def make_F(actor, s_all, trust_sub=1, trust_damp=0.01, **kw):
-    """``TRPO._make_F`` (trpo.py:200-227) for a (Squashed)GaussianActor."""
+    """``TRPO._make_F`` (trpo.py:200-227) for a (Squashed)GaussianActor of two hidden layers (the training engine's)."""
+    check_two_hidden(actor.layers)
     return _DeviceF(actor, s_all, trust_sub, trust_damp, **kw)
 
 
