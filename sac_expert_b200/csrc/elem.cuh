@@ -514,7 +514,7 @@ __global__ void __launch_bounds__(256, 4) k_adam(float* __restrict__ theta, floa
                        const float* __restrict__ g, float* __restrict__ target,
                        const float* __restrict__ lrt, const float* __restrict__ hyper, int hyper_stride,
                        int opt0, long long n, long long stride, int nnet, int do_polyak,
-                       uint8_t* __restrict__ planes, uint8_t* __restrict__ tplanes, int K0) {
+                       uint8_t* __restrict__ planes, uint8_t* __restrict__ tplanes, int K0, int nout) {
   // planes / tplanes (nullable): fp16 hi/lo weight-plane images of theta / target (planes.cuh), one image per
   // (agent, net), kept current here so that no forward / backward pass ever converts a weight again
   // one float4 (4 consecutive parameters) per thread: every table row is 128-byte aligned (strides are multiples of 32)
@@ -548,9 +548,9 @@ __global__ void __launch_bounds__(256, 4) k_adam(float* __restrict__ theta, floa
   *reinterpret_cast<float4*>(theta + o) = make_float4(th[0], th[1], th[2], th[3]);
   if (do_polyak) *reinterpret_cast<float4*>(target + o) = make_float4(tg[0], tg[1], tg[2], tg[3]);
   if (planes) {
-    const long long ib = ((long long)agent * nnet + net) * ws_image_bytes(K0);
-    ws_planes_store4(planes + ib, K0, i4, th);
-    if (do_polyak && tplanes) ws_planes_store4(tplanes + ib, K0, i4, tg);
+    const long long ib = ((long long)agent * nnet + net) * ws_image_bytes(K0, nout);
+    ws_planes_store4(planes + ib, K0, nout, i4, th);
+    if (do_polyak && tplanes) ws_planes_store4(tplanes + ib, K0, nout, i4, tg);
   }
 }
 

@@ -18,10 +18,16 @@
 //     the accumulator of layer l lives in one half of TMEM, the fp16 hi/lo A operand of layer l+1 is written IN PLACE
 //     over it (32 fp32 columns -> 16 hi + 16 lo columns), the next accumulator goes to the other half, so the MMAs of
 //     layer l+1 start on the first 64-wide k group while the epilogue still converts the rest.
-//   * SKINNY LAYERS ON CUDA CORES, EXACT FP32.  The output layer (N = 1 / A / 2A), the first backward step
-//     (dOut W2^T, K = N_out) and the action-column input gradient (N = A) are dot products against a few weight rows:
+//   * OUTPUT LAYER OF THE ACTOR ON THE TENSOR CORE.  Nets with more than one output append W2^T to their plane image
+//     (planes.cuh); epilogue 1 writes h2 as fp16 hi/lo in place over its accumulator, exactly as epilogue 0 does for
+//     h1, and the MMA thread forms out = h2 W2 (N = 16 ceil(nout / 16), 48 MMAs with A in TMEM) into the dead layer-0
+//     half.  Nothing is converted or reduced across warps on the way: one TMEM read per row, plus b2.  The backward
+//     kernel reads the same W2 bytes as an MN-major B operand for its first step dOut W2^T (K = 16 ceil(k_out / 16)),
+//     with the dOut rows as a scaled fp16 hi/lo A operand in TMEM.
+//   * SKINNY LAYERS ON CUDA CORES, EXACT FP32.  The critics' single-output layer and first backward step (an outer
+//     product) and the action-column input gradient (N = A) are dot products against a few weight rows:
 //     they are formed inside the epilogues from the row each thread already holds (weights broadcast from shared
-//     memory), instead of 48 latency-bound N=16 MMAs behind a register-staged conversion.
+//     memory).
 //   * Backward operands: tcgen05 kind::f16 rejects mixed A/B formats (bf16 x fp16 traps, tools/umma_probe.cu), so the
 //     gradient tile uses fp16 hi/lo planes too, with a per-row power-of-two scale (chosen from a bound on the row's
 //     magnitude, removed exactly in the next epilogue): 22 significant bits relative to the row maximum.
@@ -34,14 +40,14 @@ namespace saceo {
 constexpr int WS_NEW = 16;                    // conversion / epilogue warps: 4 TMEM lane quarters x 4 column groups of 64
 constexpr int WS_NEPI = WS_NEW * 32, WS_NT = WS_NEPI + 64;    // + TMA producer warp + MMA / TMEM-allocator warp
 constexpr int WS_NST = 3, WS_RING = WS_NST * WS_STAGE;
-constexpr int WS_AUX = 49152;                 // [0, WS_RED): X planes (fwd layer 0) | fp32 skinny weights; [WS_RED, ..): reductions / column sums
+constexpr int WS_AUX = 49152;                 // [0, WS_RED): X planes (fwd layer 0) | fp32 skinny weights (bwd); [WS_RED, ..): reductions / column sums
 constexpr int WS_PATCH1 = 32 * 32 * 4;        // warp-private 32 x 32 float transposition patch, 16-byte chunks XOR (row & 7)
 constexpr int WS_PATCH = WS_NEW * WS_PATCH1;
 constexpr int WS_MAIN = WS_RING + WS_AUX + WS_PATCH;
 constexpr int WS_BYTES = WS_MAIN + 1024 + 256;
 constexpr int WS_RED = 40960;                 // offset inside AUX of the 8 KB reduction / column-sum scratch
 constexpr int WS_MAXOUT = 36;                 // skinny dims (n_out, k_out) supported: fp32 [256][<=36] fits below WS_RED
-enum { WB_FULL = 0, WB_EMPTY = WS_NST, WB_XFULL = 2 * WS_NST, WB_XEMPTY, WB_D0, WB_D1, WB_AP /* 4 */ };
+enum { WB_FULL = 0, WB_EMPTY = WS_NST, WB_XFULL = 2 * WS_NST, WB_XEMPTY, WB_D0, WB_D1, WB_AP /* 4 */, WB_D2 = WB_AP + 4 };
 
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
@@ -57,9 +63,10 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 512;" ::: "memory"); }   // the 16 epilogue warps only
-// MN-major SWIZZLE_128B descriptor of a weight-plane stage: LBO = 4096 (next 64-wide n atom), SBO = 1024 (next 8 k rows)
-__device__ __forceinline__ uint64_t umma_desc_mn(uint32_t saddr) {
-  return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)(4096 >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) |
+// MN-major SWIZZLE_128B descriptor of a weight-plane stage: LBO = next 64-wide n atom (4096 in the W0 / W1 stages),
+// SBO = 1024 (next 8 k rows)
+__device__ __forceinline__ uint64_t umma_desc_mn(uint32_t saddr, uint32_t lbo = 4096) {
+  return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) |
          ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
 }
 constexpr uint32_t WS_IDESC_FWD = (1u << 4) | (1u << 16) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);  // fp16, B MN-major, N 256
@@ -69,13 +76,26 @@ constexpr uint32_t WS_IDESC_BWD = (1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((u
 // plane image maintenance
 // ------------------------------------------------------------------------------------------
 // Builds the images of `nets` nets from their fp32 tables.  grid: (ceil(items/256), nets), item = one 16-byte chunk.
-__global__ void k_planes_build(const float* __restrict__ theta, long long stride, uint8_t* __restrict__ img, int K0) {
-  const int n0 = (K0 + 31) / 32, rows = n0 * 32 + 256;
+__global__ void k_planes_build(const float* __restrict__ theta, long long stride, uint8_t* __restrict__ img, int K0, int nout) {
+  const int n0 = (K0 + 31) / 32, N2 = ws_w2_rows(nout), rows = n0 * 32 + 256 + N2;
   const int item = blockIdx.x * blockDim.x + threadIdx.x;
   if (item >= rows * 32) return;
   const int row = item >> 5, c8 = item & 31;
   const float* th = theta + (long long)blockIdx.y * stride;
+  uint8_t* net_img = img + (long long)blockIdx.y * ws_image_bytes(K0, nout);
   float x[8];
+  if (row >= n0 * 32 + 256) {       // W2 section: row n of W2^T = column n of W2 [256][nout] (zero for n >= nout)
+    const int n = row - n0 * 32 - 256;
+    const long long o = (long long)K0 * 256 + 256 + 65536 + 256 + (long long)(c8 * 8) * nout + n;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) x[j] = n < nout ? th[o + (long long)j * nout] * WS_W2_SCALE : 0.f;
+    uint4 hi, lo;
+    split8<true>(x, hi, lo);
+    uint8_t* dst = net_img + (long long)(n0 + 8) * WS_STAGE + ws_w2_off(N2, n, c8);
+    *reinterpret_cast<uint4*>(dst) = hi;
+    *reinterpret_cast<uint4*>(dst + N2 * 128) = lo;
+    return;
+  }
   if (row < n0 * 32) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) x[j] = row < K0 ? th[(long long)row * 256 + c8 * 8 + j] : 0.f;
@@ -86,7 +106,7 @@ __global__ void k_planes_build(const float* __restrict__ theta, long long stride
   }
   uint4 hi, lo;
   split8<true>(x, hi, lo);
-  uint8_t* dst = img + (long long)blockIdx.y * ws_image_bytes(K0) + ws_image_off(row, c8);
+  uint8_t* dst = net_img + ws_image_off(row, c8);
   *reinterpret_cast<uint4*>(dst) = hi;
   *reinterpret_cast<uint4*>(dst + 16384) = lo;
 }
@@ -307,12 +327,6 @@ __device__ __forceinline__ void ws_load_wrow(const float* __restrict__ W, int j,
     for (int c = 0; c < NR; ++c) w[c] = c < n ? __ldg(r + c) : 0.f;
   }
 }
-template <int NR>
-__device__ __forceinline__ void ws_store_wrow(uint32_t dst, int j, int np, const float (&w)[NR]) {
-#pragma unroll
-  for (int c4 = 0; c4 < NR / 4; ++c4)
-    if (c4 * 4 < np) sts128f(dst + (uint32_t)(j * np + 4 * c4) * 4, w[4 * c4], w[4 * c4 + 1], w[4 * c4 + 2], w[4 * c4 + 3]);
-}
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
@@ -410,7 +424,8 @@ __device__ __forceinline__ float ws_row_scale(float bound) {
 
 // ==========================================================================================
 // forward:  h1 = act0(X W0 + b0);  h2 = act1(h1 W1 + b1);  out = h2 W2 + b2        (nn_utils.py:101-136)
-// grid (row tiles, agents * nnet), 576 threads.  NG = ceil(nout / 16) accumulator groups of the output layer.
+// grid (row tiles, agents * nnet), 576 threads.  Multi-output nets (the actor) form the output layer on the tensor core
+// from the W2 section of the plane image (N = N2 = 16 ceil(nout / 16)); single-output nets (the critics) on CUDA cores.
 // Epilogue warp w: TMEM lane quarter q = w & 3 (rows 32q..32q+31 of the tile), column group cg = w >> 2 (columns
 // 64cg..64cg+63 = the k group cg of the next layer).
 // ==========================================================================================
@@ -426,7 +441,6 @@ struct FwdW {
 };
 #define WS_STAMP(i) do { if (f.dbg && lane == 0) f.dbg[(size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 16 + (i)] = gtime(); } while (0)
 
-template <int NG>
 __global__ void __launch_bounds__(WS_NT, 1) k_mlp_fwd_ws(FwdW f) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sb = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -436,11 +450,13 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_fwd_ws(FwdW f) {
   const int row0 = blockIdx.x * TC_BM;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n0 = (f.K0 + 31) >> 5, nk64 = (f.K0 + 63) >> 6;
+  const int N2 = ws_w2_rows(f.nout);            // 0: single output, formed on CUDA cores
+  const uint32_t idesc_out = (1u << 4) | ((uint32_t)(N2 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);   // fp16, K-major, N = N2
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < 2 * WS_NST; ++s) mbar_init(bar(s), 1);
     mbar_init(bar(WB_XFULL), WS_NEW); mbar_init(bar(WB_XEMPTY), 1);
-    mbar_init(bar(WB_D0), 1); mbar_init(bar(WB_D1), 1);
+    mbar_init(bar(WB_D0), 1); mbar_init(bar(WB_D1), 1); mbar_init(bar(WB_D2), 1);
     for (int g = 0; g < 4; ++g) mbar_init(bar(WB_AP + g), 8);     // 4 lane quarters x the 2 warps converting the group's two chunks
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -458,14 +474,18 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_fwd_ws(FwdW f) {
     // ------------------------------ TMA producer ------------------------------
     if (lane == 0) {
       const uint8_t* img = f.planes + agent * f.sPa + net * f.sPn;
-      const int total = n0 + 8;
+      // W0 stages, W1 stages, then (multi-output nets) the W2 section as two items of two 64-wide j atoms each
+      const int total = n0 + 8 + (N2 ? 2 : 0);
+      const uint32_t w2_item = (uint32_t)N2 * 512;
+      auto item_src = [&](int it) { return it < n0 + 8 ? img + (long long)it * WS_STAGE : img + (long long)(n0 + 8) * WS_STAGE + (it - n0 - 8) * w2_item; };
       for (int it = 0; it < total; ++it) {
         const int s = it % WS_NST;
+        const uint32_t bytes = it < n0 + 8 ? (uint32_t)WS_STAGE : w2_item;
         mbar_wait(bar(WB_EMPTY + s), (uint32_t)(((it / WS_NST) & 1) ^ 1));
-        mbar_expect_tx(bar(WB_FULL + s), WS_STAGE);
-        bulk_g2s(ring + s * WS_STAGE, img + (long long)it * WS_STAGE, WS_STAGE, bar(WB_FULL + s));
+        mbar_expect_tx(bar(WB_FULL + s), bytes);
+        bulk_g2s(ring + s * WS_STAGE, item_src(it), bytes, bar(WB_FULL + s));
         if (it == WS_NST - 1)      // ring primed: pull the rest of the image into L2 so that the refills are L2 hits
-          for (int j = WS_NST; j < total; ++j) bulk_prefetch_l2(img + (long long)j * WS_STAGE, WS_STAGE);
+          for (int j = WS_NST; j < total; ++j) bulk_prefetch_l2(item_src(j), j < n0 + 8 ? (uint32_t)WS_STAGE : w2_item);
       }
       WS_STAMP(11);
     }
@@ -515,6 +535,28 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_fwd_ws(FwdW f) {
       }
       umma_commit(bar(WB_D1));
       WS_STAMP(10);
+      if (N2) {                                    // output layer: D2 (tP[0, N2)) = h2 . W2, A = h2 hi/lo written in place over D1
+        for (int w = 0; w < 2; ++w, ++it) {        // ring item w holds the W2 atoms (k groups) 2w, 2w+1
+          const int s = it % WS_NST;
+          mbar_wait(bar(WB_FULL + s), (uint32_t)((it / WS_NST) & 1));
+          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          for (int gg = 0; gg < 2; ++gg) {
+            const int g = 2 * w + gg;
+            mbar_wait(bar(WB_AP + g), 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const uint32_t bh = ring + s * WS_STAGE + (uint32_t)(gg * N2 * 256), bl = bh + (uint32_t)N2 * 128;
+#pragma unroll
+            for (int kk = 0; kk < 4; ++kk) {
+              const uint32_t ta_hi = tQ + 64 * g + 32 * (kk >> 1) + 8 * (kk & 1), ta_lo = ta_hi + 16, kb = (uint32_t)kk * 32;
+              umma_f16_ts(tP, ta_hi, umma_desc(bh + kb), idesc_out, (g | kk) ? 1u : 0u);
+              umma_f16_ts(tP, ta_hi, umma_desc(bl + kb), idesc_out, 1u);
+              umma_f16_ts(tP, ta_lo, umma_desc(bh + kb), idesc_out, 1u);
+            }
+          }
+          umma_commit(bar(WB_EMPTY + s));
+        }
+        umma_commit(bar(WB_D2));
+      }
     }
   } else {
     // ------------------------------ conversion + epilogue warps ------------------------------
@@ -530,7 +572,6 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_fwd_ws(FwdW f) {
     float* H2 = f.H2 ? f.H2 + agent * f.sHa + net * f.sHn : nullptr;
     float* Out = f.Out + agent * f.sOa + net * f.sOn;
     if (warp == 0) WS_STAMP(0);
-    const int np = (f.nout + 3) & ~3;
     // per-CTA constants -> shared memory: b0 | b1 | w2 (single-output nets) | b2
     const uint32_t cb0 = aux + WS_RED + 2048, cb1 = cb0 + 1024, cw2 = cb1 + 1024, cb2 = cw2 + 1024;
     if (threadIdx.x < FW_H) {
@@ -583,90 +624,68 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_fwd_ws(FwdW f) {
       } else if (H1) { ws_store_rows(patch, v, H1, rbase, f.rows, col, lane); __syncwarp(); }
     }
     if (warp == 0) WS_STAMP(3);
-    // ---- output-layer weights as fp32 [256][np] in AUX (the X planes are dead: every layer-0 MMA has retired); the
-    //      loads fly while layer 1 runs
-    if (f.nout > 1 && threadIdx.x < FW_H) {
-      float w2r[NG * 16];
-      ws_load_wrow<NG * 16>(th + oW2, threadIdx.x, f.nout, w2r);
-      ws_store_wrow<NG * 16>(aux, threadIdx.x, np, w2r);
-    }
-    epi_bar();
     if (warp == 0) WS_STAMP(4);
-    // ---- epilogue 1: h2 = act1(D1 + b1) [+ saved h2]; out = h2 . W2 + b2 on CUDA cores (exact fp32)
     mbar_wait(bar(WB_D1), 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     if (warp == 0) WS_STAMP(5);
-    float acc[NG * 16];
+    if (N2) {
+      // ---- epilogue 1: h2 = act1(D1 + b1) -> fp16 hi/lo in place (A operand of the output layer) [+ saved h2], k groups in
+      //      the order of epilogue 0, so that the output-layer MMAs of groups 0 / 1 start after half of it
+#pragma unroll 1
+      for (int c = 0; c < 2; ++c) {
+        const int kg = 2 * c + (cg >> 1), col = kg * 64 + (cg & 1) * 32;
+        uint32_t v[32];
+        tmem_ld32(tQ + lane_addr + (uint32_t)col, v);
+        ws_bias_act_rt(f.act1, v, cb1 + col * 4);
+        ws_split_store(tQ + lane_addr + (uint32_t)col, v, 1.f);
+        {
+          asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+          __syncwarp();
+          if (lane == 0) mbar_arrive(bar(WB_AP + kg));      // second phase of the k-group barrier: output-layer MMAs of group kg
+        }
+        if (H2) { ws_store_rows(patch, v, H2, rbase, f.rows, col, lane); __syncwarp(); }
+      }
+      if (warp == 0) WS_STAMP(6);
+      // ---- out = D2 / WS_W2_SCALE + b2: column group 0 reads its rows' N2 accumulator columns
+      if (cg == 0) {
+        mbar_wait(bar(WB_D2), 0);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        for (int r0 = 0; r0 < N2; r0 += 32) {
+          uint32_t v[32];
+          tmem_ld32(tP + lane_addr + (uint32_t)r0, v);
+          if (grow < f.rows) {
 #pragma unroll
-    for (int i = 0; i < NG * 16; ++i) acc[i] = 0.f;
-    float qacc = 0.f;
-    auto head_chunk = [&](uint32_t (&v)[32], int col) {       // out += h2[row, col..col+31] . W2[col..col+31, :]
-      if (f.nout == 1) {
+            for (int cc = 0; cc < 32; ++cc)
+              if (r0 + cc < f.nout) Out[(long long)grow * f.ldo + r0 + cc] = __uint_as_float(v[cc]) * (1.f / WS_W2_SCALE) + lds32(cb2 + (uint32_t)(r0 + cc) * 4);
+          }
+        }
+      }
+    } else {
+      // ---- epilogue 1: h2 = act1(D1 + b1) [+ saved h2]; out = h2 . w2 + b2 on CUDA cores (exact fp32), fixed-order sum of
+      //      the four column groups
+      float qacc = 0.f;
+#pragma unroll 1
+      for (int c = 0; c < 2; ++c) {
+        const int col = cg * 64 + c * 32;
+        uint32_t v[32];
+        tmem_ld32(tQ + lane_addr + (uint32_t)col, v);
+        ws_bias_act_rt(f.act1, v, cb1 + col * 4);
+        if (H2) { ws_store_rows(patch, v, H2, rbase, f.rows, col, lane); __syncwarp(); }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const float4 t4 = lds128(cw2 + (uint32_t)(col + 4 * j) * 4);
           qacc = fmaf(__uint_as_float(v[4 * j]), t4.x, qacc); qacc = fmaf(__uint_as_float(v[4 * j + 1]), t4.y, qacc);
           qacc = fmaf(__uint_as_float(v[4 * j + 2]), t4.z, qacc); qacc = fmaf(__uint_as_float(v[4 * j + 3]), t4.w, qacc);
         }
-      } else {
-#pragma unroll
-        for (int jj = 0; jj < 32; ++jj) {
-          const float h = __uint_as_float(v[jj]);
-          const uint32_t wrow = aux + (uint32_t)((col + jj) * np) * 4;
-#pragma unroll
-          for (int g4 = 0; g4 < NG * 4; ++g4) {
-            if (g4 * 4 < np) {
-              const float4 w = lds128(wrow + g4 * 16);
-              acc[4 * g4] = fmaf(h, w.x, acc[4 * g4]); acc[4 * g4 + 1] = fmaf(h, w.y, acc[4 * g4 + 1]);
-              acc[4 * g4 + 2] = fmaf(h, w.z, acc[4 * g4 + 2]); acc[4 * g4 + 3] = fmaf(h, w.w, acc[4 * g4 + 3]);
-            }
-          }
-        }
       }
-    };
-#pragma unroll 1
-    for (int c = 0; c < 2; ++c) {
-      const int col = cg * 64 + c * 32;
-      uint32_t v[32];
-      tmem_ld32(tQ + lane_addr + (uint32_t)col, v);
-      ws_bias_act_rt(f.act1, v, cb1 + col * 4);
-      if (H2) { ws_store_rows(patch, v, H2, rbase, f.rows, col, lane); __syncwarp(); }
-      head_chunk(v, col);
-    }
-    if (warp == 0) WS_STAMP(6);
-    // ---- fixed-order sum of the four column groups + bias -> Out
-    const uint32_t red = aux + WS_RED;               // [3 groups][128 rows] scratch (one output column at a time is enough for q)
-    if (f.nout == 1) {
+      if (warp == 0) WS_STAMP(6);
+      const uint32_t red = aux + WS_RED;             // [3 groups][128 rows] scratch
       if (cg > 0) asm volatile("st.shared.f32 [%0], %1;" ::"r"(red + (uint32_t)((cg - 1) * TC_BM + q * 32 + lane) * 4), "f"(qacc) : "memory");
       epi_bar();
       if (cg == 0 && grow < f.rows) {
         const uint32_t r = red + (uint32_t)(q * 32 + lane) * 4;
         Out[(long long)grow * f.ldo] = ((qacc + lds32(r)) + (lds32(r + TC_BM * 4) + lds32(r + 2 * TC_BM * 4))) + lds32(cb2);
-      }
-    } else {
-      // groups 1..3 park their partial rows in their patch (column index rotated by the lane: conflict-free), group 0 adds
-#pragma unroll
-      for (int r0 = 0; r0 < NG * 16; r0 += 32) {
-        if (r0 < f.nout) {
-          if (cg > 0) {
-#pragma unroll
-            for (int cc = 0; cc < 32; ++cc)
-              if (r0 + cc < NG * 16) asm volatile("st.shared.f32 [%0], %1;" ::"r"(patch + (uint32_t)(lane * 32 + ((cc + lane) & 31)) * 4), "f"(acc[(r0 + cc) < NG * 16 ? r0 + cc : 0]) : "memory");
-          }
-          epi_bar();
-          if (cg == 0 && grow < f.rows) {
-#pragma unroll
-            for (int cc = 0; cc < 32; ++cc) {
-              if (r0 + cc < NG * 16 && r0 + cc < f.nout) {
-                const uint32_t o = (uint32_t)(lane * 32 + ((cc + lane) & 31)) * 4;
-                const float p1 = lds32(patch_base + (uint32_t)(warp + 4) * WS_PATCH1 + o), p2 = lds32(patch_base + (uint32_t)(warp + 8) * WS_PATCH1 + o),
-                            p3 = lds32(patch_base + (uint32_t)(warp + 12) * WS_PATCH1 + o);
-                Out[(long long)grow * f.ldo + r0 + cc] = ((acc[(r0 + cc) < NG * 16 ? r0 + cc : 0] + p1) + (p2 + p3)) + lds32(cb2 + (uint32_t)(r0 + cc) * 4);
-              }
-            }
-          }
-          if (r0 + 32 < f.nout) epi_bar();
-        }
       }
     }
     if (warp == 0) WS_STAMP(7);
@@ -717,6 +736,7 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_bwd_ws(BwdW f) {
     for (int s = 0; s < 2 * WS_NST; ++s) mbar_init(bar(s), 1);
     mbar_init(bar(WB_D0), 1); mbar_init(bar(WB_D1), 1);                 // accumulator halves 0 / 1
     for (int g = 0; g < 4; ++g) mbar_init(bar(WB_AP + g), 8);     // 4 lane quarters x the 2 warps converting the group's two chunks
+    mbar_init(bar(WB_XFULL), 4); mbar_init(bar(WB_XEMPTY), 1);    // NG > 0: dOut operand written (4 lane quarters) / dOut W2^T formed
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("st.shared.u32 [%0], %1;" ::"r"(aux + WS_RED - 256), "r"(0u) : "memory");     // max |W2| accumulator
   }
@@ -734,8 +754,18 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_bwd_ws(BwdW f) {
     // TMA producer: stage (h, s) = rows i in [128h, 128h+128) of the 64-wide j slab s, K-major: 4 KB pieces (t, plane, s)
     if (lane == 0) {
       const uint8_t* w1 = f.planes + agent * f.sPa + net * f.sPn + (long long)n0 * WS_STAGE;
-      for (int it = 0; it < 8; ++it) {
-        const int h = it >> 2, sj = it & 3, s = it % WS_NST;
+      if (NG > 0) {   // multi-output nets: first the W2 section (planes.cuh), ring item 0 = its hi plane, item 1 = its lo plane,
+                      // each compacted to [s][n][64 j] (the 64-wide j atoms N2 * 128 bytes apart)
+        const int N2 = ws_w2_rows(f.nout);
+        const uint8_t* w2 = w1 + 8LL * WS_STAGE;
+        for (int pl = 0; pl < 2; ++pl) {
+          mbar_expect_tx(bar(WB_FULL + pl), (uint32_t)N2 * 512);
+          for (int sj = 0; sj < 4; ++sj)
+            bulk_g2s(ring + pl * WS_STAGE + sj * N2 * 128, w2 + (sj * 2 + pl) * N2 * 128, (uint32_t)N2 * 128, bar(WB_FULL + pl));
+        }
+      }
+      for (int i = 0; i < 8; ++i) {
+        const int it = i + (NG > 0 ? 2 : 0), h = i >> 2, sj = i & 3, s = it % WS_NST;
         mbar_wait(bar(WB_EMPTY + s), (uint32_t)(((it / WS_NST) & 1) ^ 1));
         mbar_expect_tx(bar(WB_FULL + s), WS_STAGE);
         for (int pl = 0; pl < 2; ++pl)
@@ -748,8 +778,25 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_bwd_ws(BwdW f) {
     }
   } else if (warp == WS_NEW + 1) {
     if (lane == 0) {
-      for (int it = 0; it < 8; ++it) {          // D1[:, 128h..] (tQ) = dH2' . W1^T, contraction over the j slab sj
-        const int h = it >> 2, sj = it & 3, s = it % WS_NST;
+      if (NG > 0) {     // D0 (tP) = dOut' . W2^T: A = the scaled dOut rows as fp16 hi/lo in tQ, B = the W2 planes read MN-major
+        const uint32_t lbo = (uint32_t)ws_w2_rows(f.nout) * 128;
+        mbar_wait(bar(WB_XFULL), 0);
+        mbar_wait(bar(WB_FULL + 0), 0);
+        mbar_wait(bar(WB_FULL + 1), 0);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#pragma unroll
+        for (int ks = 0; ks < NG; ++ks) {
+          const uint32_t ta_hi = tQ + 16 * ks, ta_lo = ta_hi + 8, kb = (uint32_t)ks * 2048;
+          umma_f16_ts(tP, ta_hi, umma_desc_mn(ring + kb, lbo), WS_IDESC_FWD, ks ? 1u : 0u);
+          umma_f16_ts(tP, ta_hi, umma_desc_mn(ring + WS_STAGE + kb, lbo), WS_IDESC_FWD, 1u);
+          umma_f16_ts(tP, ta_lo, umma_desc_mn(ring + kb, lbo), WS_IDESC_FWD, 1u);
+        }
+        umma_commit(bar(WB_EMPTY + 0));
+        umma_commit(bar(WB_EMPTY + 1));
+        umma_commit(bar(WB_XEMPTY));
+      }
+      for (int i = 0; i < 8; ++i) {             // D1[:, 128h..] (tQ) = dH2' . W1^T, contraction over the j slab sj
+        const int it = i + (NG > 0 ? 2 : 0), h = i >> 2, sj = i & 3, s = it % WS_NST;
         if (h == 0) {
           mbar_wait(bar(WB_AP + sj), 0);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -785,40 +832,73 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_bwd_ws(BwdW f) {
     const bool pH1 = MODE != 0 || f.H1p != nullptr;
     const bool pdH2 = MODE == 1 || (MODE == 0 && f.dH2p != nullptr), pdH1 = MODE == 1 || (MODE == 0 && f.dH1p != nullptr);
     const bool want_cs = f.dbpart && (dH2 || pdH2) && (dH1 || pdH1);
-    const int kp = (f.kout + 3) & ~3;
-    const uint32_t wmax_s = aux + WS_RED - 256;            // max |W2| over the staged block (int bit pattern)
+    const uint32_t wmax_s = aux + WS_RED - 256;            // max |W2[:, :kout]| (int bit pattern)
 
     if (warp == 0) WS_STAMP(0);
     // chunk order of epilogue 0 by k group (as in the forward kernel): step c converts the j slabs 2c and 2c+1
     const int col0_0 = (cg >> 1) * 64 + (cg & 1) * 32, col0_1 = (2 + (cg >> 1)) * 64 + (cg & 1) * 32;
     ws_rows_prefetch(H2, rbase, f.rows, col0_0, lane);      // saved activations of both chunks -> L2 while W2 is staged
     ws_rows_prefetch(H2, rbase, f.rows, col0_1, lane);
-    // ---- stage W2[:, :kout] as fp32 [256][kp]; max |W2| over the block bounds every row of dOut . W2^T (row scale)
-    constexpr int ND = NG > 0 ? NG * 16 : 1;               // NG == 0: single output (critics), the first step is an outer product
-    float d[ND];
+    const float* __restrict__ drow = dOut + (long long)grow * f.ldd;
+    // max |W2[:, :kout]| bounds every row of dOut . W2^T (row scale of the dH2 operand)
+    float d0 = 0.f, bound = 0.f, inv_d = 1.f;
+    if (NG == 0) {       // single output (critics): the first step is an outer product with w2 staged as fp32 in AUX
+      d0 = rvalid ? __ldg(drow) : 0.f;
+      bound = fabsf(d0);
+      if (threadIdx.x < FW_H) {
+        float wr[4];
+        ws_load_wrow<4>(th + oW2, threadIdx.x, f.nout, wr);          // hidden unit j = threadIdx.x
+        float m = fabsf(wr[0]);
+        asm volatile("st.shared.f32 [%0], %1;" ::"r"(aux + threadIdx.x * 4), "f"(wr[0]) : "memory");
+        for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+        if (lane == 0) atomicMax(reinterpret_cast<int*>(smem_raw + (wmax_s - smem_u32(smem_raw))), __float_as_int(m));
+      }
+    } else {
+      // multi-output nets (actor): dOut . W2^T on the tensor core.  The dOut row goes in as fp16 hi/lo scaled by a power of
+      // two that puts its largest element in [512, 1024); the accumulator then holds dH2 * dscale * WS_W2_SCALE
+      float dmax = 0.f;
+      for (int cc = 0; cc < f.kout; ++cc) {
+        const float x = rvalid ? fabsf(__ldg(drow + cc)) : 0.f;
+        bound += x; dmax = fmaxf(dmax, x);
+      }
+      const float dscale = ws_row_scale(dmax);
+      inv_d = (1.f / dscale) * (1.f / WS_W2_SCALE);
+      if (cg == 0) {     // one warp per lane quarter writes the A operand: K = 16 NG columns, [8 hi | 8 lo] per 16-wide k step
 #pragma unroll
-    for (int cc = 0; cc < ND; ++cc) d[cc] = (rvalid && cc < f.kout) ? __ldg(dOut + (long long)grow * f.ldd + cc) : 0.f;
-    if (threadIdx.x < FW_H) {
-      float wr[NG > 0 ? NG * 16 : 4];
-      ws_load_wrow<(NG > 0 ? NG * 16 : 4)>(th + oW2, threadIdx.x, f.nout, wr);          // hidden unit j = threadIdx.x
-      float m = 0.f;
+        for (int ks = 0; ks < NG; ++ks) {
+          uint32_t hi[8], lo[8];
 #pragma unroll
-      for (int cc = 0; cc < (NG > 0 ? NG * 16 : 4); ++cc) { if (cc >= f.kout) wr[cc] = 0.f; m = fmaxf(m, fabsf(wr[cc])); }
-      if (NG > 0) ws_store_wrow<(NG > 0 ? NG * 16 : 4)>(aux, threadIdx.x, kp, wr);
-      else asm volatile("st.shared.f32 [%0], %1;" ::"r"(aux + threadIdx.x * 4), "f"(wr[0]) : "memory");
-      for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-      if (lane == 0) atomicMax(reinterpret_cast<int*>(smem_raw + (wmax_s - smem_u32(smem_raw))), __float_as_int(m));
+          for (int j = 0; j < 8; ++j) {
+            const int c0 = 16 * ks + 2 * j;
+            const float x0 = (rvalid && c0 < f.kout) ? __ldg(drow + c0) * dscale : 0.f;
+            const float x1 = (rvalid && c0 + 1 < f.kout) ? __ldg(drow + c0 + 1) * dscale : 0.f;
+            asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi[j]) : "f"(x1), "f"(x0));
+            const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hi[j]));
+            asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo[j]) : "f"(x1 - hf.y), "f"(x0 - hf.x));
+          }
+          tmem_st8(tQ + lane_addr + 16 * ks, hi);
+          tmem_st8(tQ + lane_addr + 16 * ks + 8, lo);
+        }
+        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncwarp();
+        if (lane == 0) mbar_arrive(bar(WB_XFULL));
+      }
+      if (threadIdx.x < FW_H) {
+        float m = 0.f;
+        const float* wr = th + oW2 + (long long)threadIdx.x * f.nout;
+        for (int cc = 0; cc < f.kout; ++cc) m = fmaxf(m, fabsf(__ldg(wr + cc)));
+        for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+        if (lane == 0) atomicMax(reinterpret_cast<int*>(smem_raw + (wmax_s - smem_u32(smem_raw))), __float_as_int(m));
+      }
     }
     epi_bar();
-    // this row's upstream gradient and its scale: |dH2[row, j]| <= sum_c |dOut[row, c]| * max |W2|
-    float bound = 0.f;
-#pragma unroll
-    for (int cc = 0; cc < ND; ++cc) bound += fabsf(d[cc]);
+    // this row's scale: |dH2[row, j]| <= sum_c |dOut[row, c]| * max |W2|
     bound *= __int_as_float((int)lds_u32(wmax_s));
     const float scale = ws_row_scale(bound), inv_scale = 1.f / scale;
     if (warp == 0) WS_STAMP(1);
 
-    // ---- epilogue 0: dH2 = (dOut . W2^T) * act1'(H2) on CUDA cores -> scaled fp16 hi/lo A operand (tP) [+ saved dH2, column sums]
+    // ---- epilogue 0: dH2 = (dOut . W2^T) * act1'(H2) -> scaled fp16 hi/lo A operand in place (tP) [+ saved dH2, column sums]
 #pragma unroll 1
     for (int c = 0; c < 2; ++c) {
       const int col = c ? col0_1 : col0_0, kg = 2 * c + (cg >> 1);
@@ -836,26 +916,17 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_bwd_ws(BwdW f) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const float4 t4 = lds128(aux + (uint32_t)(col + 4 * j) * 4);
-          v[4 * j] = __float_as_uint(d[0] * t4.x); v[4 * j + 1] = __float_as_uint(d[0] * t4.y);
-          v[4 * j + 2] = __float_as_uint(d[0] * t4.z); v[4 * j + 3] = __float_as_uint(d[0] * t4.w);
+          v[4 * j] = __float_as_uint(d0 * t4.x); v[4 * j + 1] = __float_as_uint(d0 * t4.y);
+          v[4 * j + 2] = __float_as_uint(d0 * t4.z); v[4 * j + 3] = __float_as_uint(d0 * t4.w);
         }
       } else {
-#pragma unroll
-        for (int jj = 0; jj < 32; ++jj) {
-          float a = 0.f;
-          const uint32_t wrow = aux + (uint32_t)((col + jj) * kp) * 4;
-#pragma unroll
-          for (int g4 = 0; g4 < NG * 4; ++g4) {
-            if (g4 * 4 < kp) {
-              const float4 w = lds128(wrow + g4 * 16);
-              a = fmaf(d[(4 * g4) % ND], w.x, a); a = fmaf(d[(4 * g4 + 1) % ND], w.y, a);
-              a = fmaf(d[(4 * g4 + 2) % ND], w.z, a); a = fmaf(d[(4 * g4 + 3) % ND], w.w, a);
-            }
-          }
-          v[jj] = __float_as_uint(a);
+        if (c == 0) {
+          mbar_wait(bar(WB_XEMPTY), 0);
+          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         }
+        tmem_ld32(tP + lane_addr + (uint32_t)col, v);
       }
-      ws_mul_dact_p_rt(f.act1, v, patch, lane, 1.f);
+      ws_mul_dact_p_rt(f.act1, v, patch, lane, inv_d);
       ws_split_store(tP + lane_addr + (uint32_t)col, v, scale);
       {
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
@@ -1212,7 +1283,7 @@ static inline cudaError_t mlp_ws_init() {
   if (done) return cudaSuccess;
   cudaError_t e;
 #define WS_ATTR(K) e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_BYTES); if (e) return e;
-  WS_ATTR(k_mlp_fwd_ws<1>) WS_ATTR(k_mlp_fwd_ws<2>) WS_ATTR(k_mlp_fwd_ws<3>)
+  WS_ATTR(k_mlp_fwd_ws)
   WS_ATTR((k_mlp_bwd_ws<0, 0, 0>)) WS_ATTR((k_mlp_bwd_ws<0, 1, 0>)) WS_ATTR((k_mlp_bwd_ws<0, 2, 0>))
   WS_ATTR((k_mlp_bwd_ws<1, 0, 0>)) WS_ATTR((k_mlp_bwd_ws<2, 0, 0>)) WS_ATTR((k_mlp_bwd_ws<3, 0, 0>))
   WS_ATTR((k_mlp_bwd_ws<0, 0, 1>)) WS_ATTR((k_mlp_bwd_ws<1, 0, 1>)) WS_ATTR((k_mlp_bwd_ws<0, 1, 2>))
@@ -1228,9 +1299,7 @@ static inline bool mlp_fwd_ws_eligible(int h1, int h2, int nout, int K0, const f
 }
 static inline cudaError_t mlp_fwd_ws_launch(const FwdW& f, int nagents, cudaStream_t st) {
   dim3 grid((f.rows + TC_BM - 1) / TC_BM, nagents * f.nnet);
-  if (f.nout <= 16) k_mlp_fwd_ws<1><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (f.nout <= 32) k_mlp_fwd_ws<2><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else k_mlp_fwd_ws<3><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  k_mlp_fwd_ws<<<grid, WS_NT, WS_BYTES, st>>>(f);
   return cudaPeekAtLastError();
 }
 // the backward variants that exist: single-output nets (critics) with 0 / 1 / 2 action groups, multi-output nets

@@ -231,13 +231,13 @@ static void carve(saceo_ctx* x, char* base) {
   x->a_img = (long long)(R / 32) * WS_STAGE; x->c_img = (long long)(rup(B, 32) / 32) * WS_STAGE;
   if (c.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && c.reserved[5] == 0) {
     if (c.actor_hidden[0] == FW_H && c.actor_hidden[1] == FW_H) {
-      x->pl_actor = b.get<uint8_t>("pl_actor", n * ws_image_bytes(S));
+      x->pl_actor = b.get<uint8_t>("pl_actor", n * ws_image_bytes(S, L.Ao));
       x->aH1p = b.get<uint8_t>("aH1p", n * x->a_img); x->adH2p = b.get<uint8_t>("adH2p", n * x->a_img);
       x->adH1p = b.get<uint8_t>("adH1p", n * x->a_img);
     }
     if (c.critic_hidden[0] == FW_H && c.critic_hidden[1] == FW_H) {
-      x->pl_q = b.get<uint8_t>("pl_q", n * 2 * ws_image_bytes(SA));
-      x->pl_qt = b.get<uint8_t>("pl_qt", n * 2 * ws_image_bytes(SA));
+      x->pl_q = b.get<uint8_t>("pl_q", n * 2 * ws_image_bytes(SA, 1));
+      x->pl_qt = b.get<uint8_t>("pl_qt", n * 2 * ws_image_bytes(SA, 1));
       x->cH1p = b.get<uint8_t>("cH1p", n * 2 * x->c_img); x->cdH2p = b.get<uint8_t>("cdH2p", n * 2 * x->c_img);
       x->cdH1p = b.get<uint8_t>("cdH1p", n * 2 * x->c_img);
     }
@@ -402,13 +402,13 @@ extern "C" int saceo_weights_changed(saceo_ctx* x) {
 static int ensure_planes(saceo_ctx* x, cudaStream_t st) {
   if (!x->planes_dirty || !x->bound) return 0;
   const saceo_config& c = x->cfg; const int n = c.n_agents;
-  auto items = [](int K0) { return (((K0 + 31) / 32) * 32 + 256) * 32; };
+  auto items = [](int K0, int nout) { return (((K0 + 31) / 32) * 32 + 256 + ws_w2_rows(nout)) * 32; };
   if (x->pl_actor && (x->planes_dirty & 1)) {
-    k_planes_build<<<dim3(cdiv(items(c.S), 256), n), 256, 0, st>>>(x->k.T.actor, x->L.na_stride, x->pl_actor, c.S);   // maintenance: not counted as a launch of the step
+    k_planes_build<<<dim3(cdiv(items(c.S, x->L.Ao), 256), n), 256, 0, st>>>(x->k.T.actor, x->L.na_stride, x->pl_actor, c.S, x->L.Ao);   // maintenance: not counted as a launch of the step
   }
   if (x->pl_q && (x->planes_dirty & 2)) {
-    k_planes_build<<<dim3(cdiv(items(c.S + c.A), 256), 2 * n), 256, 0, st>>>(x->k.T.q, x->L.nc_stride, x->pl_q, c.S + c.A);
-    k_planes_build<<<dim3(cdiv(items(c.S + c.A), 256), 2 * n), 256, 0, st>>>(x->k.T.qt, x->L.nc_stride, x->pl_qt, c.S + c.A);
+    k_planes_build<<<dim3(cdiv(items(c.S + c.A, 1), 256), 2 * n), 256, 0, st>>>(x->k.T.q, x->L.nc_stride, x->pl_q, c.S + c.A, 1);
+    k_planes_build<<<dim3(cdiv(items(c.S + c.A, 1), 256), 2 * n), 256, 0, st>>>(x->k.T.qt, x->L.nc_stride, x->pl_qt, c.S + c.A, 1);
   }
   x->planes_dirty = 0;
   cudaError_t e = cudaPeekAtLastError();
@@ -697,14 +697,14 @@ static NetD actor_net(const saceo_ctx* x) {
   const saceo_config& c = x->cfg;
   NetD d{x->k.T.actor, x->L.na_stride, 0, 1, c.S, c.actor_hidden[0], c.actor_hidden[1], x->L.Ao,
          c.actor_act[0], c.actor_act[1]};
-  d.planes = x->pl_actor; d.pa = ws_image_bytes(c.S); d.pn = 0;
+  d.planes = x->pl_actor; d.pa = ws_image_bytes(c.S, x->L.Ao); d.pn = 0;
   return d;
 }
 static NetD critic_net(const saceo_ctx* x, bool target) {
   const saceo_config& c = x->cfg;
   NetD d{target ? x->k.T.qt : x->k.T.q, 2 * x->L.nc_stride, x->L.nc_stride, 2, c.S + c.A,
          c.critic_hidden[0], c.critic_hidden[1], 1, c.critic_act[0], c.critic_act[1]};
-  d.planes = target ? x->pl_qt : x->pl_q; d.pn = ws_image_bytes(c.S + c.A); d.pa = 2 * d.pn;
+  d.planes = target ? x->pl_qt : x->pl_q; d.pn = ws_image_bytes(c.S + c.A, 1); d.pa = 2 * d.pn;
   return d;
 }
 static NetD model_net(const saceo_ctx* x, int nnet) {
@@ -755,7 +755,7 @@ static int phase_critic_grads(saceo_ctx* x, cudaStream_t st) {
 static int phase_critic_apply(saceo_ctx* x, int do_polyak, cudaStream_t st) {
   const KCtx& k = x->k;
   LAUNCH(x, k_adam, dim3(cdiv(cdiv(x->L.nc, 4), 256), 2, k.n_agents), 256, 0, st, k.T.q, k.T.q_m, k.T.q_v, k.g_q, k.T.qt,
-         k.lrt, k.T.hyper, x->L.hyper_stride, 0, x->L.nc, x->L.nc_stride, 2, do_polyak, x->pl_q, x->pl_qt, k.S + k.A);
+         k.lrt, k.T.hyper, x->L.hyper_stride, 0, x->L.nc, x->L.nc_stride, 2, do_polyak, x->pl_q, x->pl_qt, k.S + k.A, 1);
   return check_launch();
 }
 
@@ -880,7 +880,7 @@ static int phase_actor_apply(saceo_ctx* x, cudaStream_t st) {
   const KCtx& k = x->k;
   LAUNCH(x, k_adam, dim3(cdiv(cdiv(x->L.na, 4), 256), 1, k.n_agents), 256, 0, st, k.T.actor, k.T.actor_m, k.T.actor_v,
          k.g_actor, (float*)nullptr, k.lrt, k.T.hyper, x->L.hyper_stride, 2, x->L.na, x->L.na_stride, 1, 0,
-         x->pl_actor, (uint8_t*)nullptr, k.S);
+         x->pl_actor, (uint8_t*)nullptr, k.S, k.Ao);
   return check_launch();
 }
 
@@ -1493,7 +1493,7 @@ extern "C" int saceo_actor_adam(saceo_ctx* x, const float* grad, void* stream) {
   LAUNCH(x, k_bc_begin, dim3(cdiv(k.n_agents, 128)), 128, 0, st, k, 0);
   LAUNCH(x, k_adam, dim3(cdiv(cdiv(x->L.na, 4), 256), 1, k.n_agents), 256, 0, st, k.T.actor, k.T.actor_m, k.T.actor_v,
          grad, (float*)nullptr, k.lrt, k.T.hyper, x->L.hyper_stride, 2, x->L.na, x->L.na_stride, 1, 0,
-         x->pl_actor, (uint8_t*)nullptr, k.S);
+         x->pl_actor, (uint8_t*)nullptr, k.S, k.Ao);
   return check_launch();
 }
 
