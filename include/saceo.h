@@ -84,12 +84,10 @@ typedef struct saceo_config {
   int32_t use_graph;          /* capture one update into a CUDA graph and replay it */
   int32_t reserved[8];        /* tuning switches, 0 = default: [0] tcgen05 tile variant (0: 128x256 tile, 1: 128x128 2 CTAs/SM,
                                  2: force the register-staged kernel); [1] != 0 disables the fused 3-layer forward kernel;
-                                 [2] != 0 disables the fused backward-chain kernel; [3] != 0 disables the fused model-term kernel;
-                                 [4] != 0 keeps the hidden-layer bias gradients on the ones-row GEMM path;
+                                 [2] != 0 disables the fused backward-chain kernel;
                                  [5] != 0 disables the warp-specialised TMA-fed fused kernels and their weight planes
                                  (round-1 fused kernels are used instead); [6] != 0 keeps the whole update on one stream (no
-                                 concurrent actor-phase branch); [7] expert-term kernel: 0 = hidden layer on mma.sync fp16 hi/lo x3 (default where the
-                                 shape allows), 1 = column-blocked CUDA-core kernel, 2 = round-1 CUDA-core kernel */
+                                 concurrent actor-phase branch); [3], [4], [7] must be 0 (SACEO_E_INVALID otherwise) */
 } saceo_config;
 
 /* Strides/offsets (in 4-byte words unless stated) derived from a config. */

@@ -217,268 +217,6 @@ __global__ void __launch_bounds__(MT_THREADS, 2) k_model_term(KCtx c, float* __r
   }
 }
 
-// Column-blocked variant (round 2 experiment, opt-in through reserved[7]): every thread owns MT4_CPT hidden columns, so
-// that one broadcast float4 of the row activations feeds 4 x MT4_CPT FMAs instead of 4.  ncu of the round-1 kernel:
-// L1/TEX 90 % busy with 62 M shared-memory wavefronts + 66 M global sectors per launch (profiles/r2_model_term_ncu.txt).
-// Measured on the 256-agent step: 4 columns x 128 threads 571 us (shared wavefronts 62 M -> 22 M, but 16 warps per SM
-// leave the FMAs waiting on LDS: short-scoreboard stalls dominate), 2 columns x 256 threads 465 us, round-1 kernel
-// 467 us.  Not a win; kept for the record and for small hidden sizes.
-constexpr int MT4_THREADS = 256, MT4_CPT = 2;
-template <int MS>
-__global__ void __launch_bounds__(MT4_THREADS, 3) k_model_term4(KCtx c, float* __restrict__ mse_part) {
-  extern __shared__ float msm[];
-  const int net = blockIdx.x, agent = blockIdx.y;
-  const int S = c.S, A = c.A, SA = S + A, H1 = c.mh1, H2 = c.mh2, mo = c.mo, E = c.E;
-  const int half = c.nmod == 2 ? E / 2 : E;             // rows handled by this model
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nwarp = MT4_THREADS / 32;
-  float* xs = msm;                      // [MS][SA]
-  float* h1 = xs + MS * SA;             // [MS][H1]   (later dh1)
-  float* h2 = h1 + MS * H1;             // [MS][H2]   (later dh2)
-  float* ob = h2 + MS * H2;             // [MS][mo]   model output
-  float* dd = ob + MS * mo;             // [MS][S]    d(eps*MSE)/d(delta)
-  __shared__ float red[32];
-  const float* th = c.T.model + ((long long)agent * 2 + net) * c.L.nm_stride;
-  const float* W0 = th; const float* b0 = W0 + (long long)SA * H1;
-  const float* W1 = b0 + H1; const float* b1 = W1 + (long long)H1 * H2;
-  const float* W2 = b1 + H2; const float* b2 = W2 + (long long)H2 * mo;
-  const float* nr = c.T.norm + (long long)agent * c.L.norm_stride;
-  const float* Xm = c.Xm + ((long long)agent * 2 + net) * E * SA;
-
-  for (int e = tid; e < MS * SA; e += MT4_THREADS) { const int r = e / SA; xs[e] = r < half ? Xm[e] : 0.f; }
-  __syncthreads();
-
-  // ---- layer 0: thread t owns output columns t + 128 c --------------------------------------------
-  for (int jb = tid; jb < H1; jb += MT4_THREADS * MT4_CPT) {
-    float acc[MT4_CPT][MS];
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc) {
-      const int j = jb + cc * MT4_THREADS;
-      const float bj = j < H1 ? __ldg(b0 + j) : 0.f;
-#pragma unroll
-      for (int r = 0; r < MS; ++r) acc[cc][r] = bj;
-    }
-    for (int k = 0; k < SA; k += 4) {
-      float w[4][MT4_CPT];
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-#pragma unroll
-        for (int cc = 0; cc < MT4_CPT; ++cc)
-          w[u][cc] = (k + u < SA && jb + cc * MT4_THREADS < H1) ? __ldg(W0 + (long long)(k + u) * H1 + jb + cc * MT4_THREADS) : 0.f;
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        if (k + u < SA) {
-#pragma unroll
-          for (int r = 0; r < MS; ++r) {
-            const float xv = xs[r * SA + k + u];
-#pragma unroll
-            for (int cc = 0; cc < MT4_CPT; ++cc) acc[cc][r] = fmaf(xv, w[u][cc], acc[cc][r]);
-          }
-        }
-      }
-    }
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc) {
-      const int j = jb + cc * MT4_THREADS;
-      if (j < H1) {
-#pragma unroll
-        for (int r = 0; r < MS; ++r) h1[r * H1 + j] = apply_act(c.mact0, acc[cc][r]);
-      }
-    }
-  }
-  __syncthreads();
-  // ---- layer 1 ---------------------------------------------------------------------------------
-  for (int jb = tid; jb < H2; jb += MT4_THREADS * MT4_CPT) {
-    float acc[MT4_CPT][MS];
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc) {
-      const int j = jb + cc * MT4_THREADS;
-      const float bj = j < H2 ? __ldg(b1 + j) : 0.f;
-#pragma unroll
-      for (int r = 0; r < MS; ++r) acc[cc][r] = bj;
-    }
-    float wn[4][MT4_CPT];
-#pragma unroll
-    for (int u = 0; u < 4; ++u)
-#pragma unroll
-      for (int cc = 0; cc < MT4_CPT; ++cc)
-        wn[u][cc] = (jb + cc * MT4_THREADS < H2) ? __ldg(W1 + (long long)u * H2 + jb + cc * MT4_THREADS) : 0.f;
-    for (int k = 0; k < H1; k += 4) {
-      float w[4][MT4_CPT];
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-#pragma unroll
-        for (int cc = 0; cc < MT4_CPT; ++cc) w[u][cc] = wn[u][cc];
-      if (k + 4 < H1) {
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-#pragma unroll
-          for (int cc = 0; cc < MT4_CPT; ++cc)
-            wn[u][cc] = (jb + cc * MT4_THREADS < H2) ? __ldg(W1 + (long long)(k + 4 + u) * H2 + jb + cc * MT4_THREADS) : 0.f;   // next group flies during the FMAs
-      }
-#pragma unroll
-      for (int r = 0; r < MS; ++r) {
-        const float4 a = *reinterpret_cast<const float4*>(h1 + r * H1 + k);            // broadcast: 16 FMAs per LDS.128
-#pragma unroll
-        for (int cc = 0; cc < MT4_CPT; ++cc) {
-          acc[cc][r] = fmaf(a.x, w[0][cc], acc[cc][r]); acc[cc][r] = fmaf(a.y, w[1][cc], acc[cc][r]);
-          acc[cc][r] = fmaf(a.z, w[2][cc], acc[cc][r]); acc[cc][r] = fmaf(a.w, w[3][cc], acc[cc][r]);
-        }
-      }
-    }
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc) {
-      const int j = jb + cc * MT4_THREADS;
-      if (j < H2) {
-#pragma unroll
-        for (int r = 0; r < MS; ++r) h2[r * H2 + j] = apply_act(c.mact1, acc[cc][r]);
-      }
-    }
-  }
-  __syncthreads();
-  // ---- layer 2: one warp per output column, lanes walk k ------------------------------------
-  for (int col = warp; col < mo; col += nwarp) {
-    float acc[MS];
-#pragma unroll
-    for (int r = 0; r < MS; ++r) acc[r] = 0.f;
-    for (int k0 = lane; k0 < H2; k0 += 256) {
-      float w[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) w[u] = (k0 + 32 * u < H2) ? __ldg(W2 + (long long)(k0 + 32 * u) * mo + col) : 0.f;
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (k0 + 32 * u < H2) {
-#pragma unroll
-          for (int r = 0; r < MS; ++r) acc[r] = fmaf(h2[r * H2 + k0 + 32 * u], w[u], acc[r]);
-        }
-      }
-    }
-#pragma unroll
-    for (int r = 0; r < MS; ++r) {
-      float v = acc[r];
-      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (lane == 0) ob[r * mo + col] = v + __ldg(b2 + col);
-    }
-  }
-  __syncthreads();
-  // ---- loss and d(eps * MSE)/d(delta) -----------------------------------------------------------
-  const float eps = agent_eps(c, agent);
-  const float inv = 1.f / (float)half;
-  float part = 0.f;
-  for (int e = tid; e < MS * S; e += MT4_THREADS) {
-    const int i = e / S, j = e - i * S;
-    float g = 0.f;
-    if (i < half) {
-      const int src = c.perm[(long long)agent * E + net * half + i];
-      float delta = ob[i * mo + j];
-      float cm = 1.f;
-      if (c.delta_clip > 0.f) {
-        cm = (delta >= -c.delta_clip && delta <= c.delta_clip) ? 1.f : 0.f;
-        delta = fminf(fmaxf(delta, -c.delta_clip), c.delta_clip);
-      }
-      const float sd = nstd(nr[c.L.off_m_d_std + j]);
-      const float pred = c.expert_s[((long long)agent * E + src) * S + j] + (delta * sd + nr[c.L.off_m_d_mean + j]);
-      const float err = c.expert_sp[((long long)agent * E + src) * S + j] - pred;
-      part += 0.5f * err * err;
-      g = (-err * inv * eps) * sd * cm;
-    }
-    dd[e] = g;
-  }
-  part = block_sum(part, red);
-  if (tid == 0) mse_part[agent * 2 + net] = part * inv;
-  __syncthreads();
-  // ---- layer 2 transposed: thread j reads its own (contiguous) row of W2 ----------------------
-  for (int j = tid; j < H2; j += MT4_THREADS) {
-    float acc[MS];
-#pragma unroll
-    for (int r = 0; r < MS; ++r) acc[r] = 0.f;
-    for (int cc = 0; cc < S; cc += 8) {
-      float w[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) w[u] = (cc + u < S) ? __ldg(W2 + (long long)j * mo + cc + u) : 0.f;
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (cc + u < S) {
-#pragma unroll
-          for (int r = 0; r < MS; ++r) acc[r] = fmaf(dd[r * S + cc + u], w[u], acc[r]);
-        }
-      }
-    }
-#pragma unroll
-    for (int r = 0; r < MS; ++r) h2[r * H2 + j] = acc[r] * dact_from_out(c.mact1, h2[r * H2 + j]);   // own column only
-  }
-  __syncthreads();
-  // ---- layer 1 transposed: thread t owns input indices t + 128 c and streams THEIR contiguous W1 rows (16-byte pieces);
-  // the dz2 rows are broadcast from shared memory, one float4 feeding 16 FMAs
-  for (int ib = tid; ib < H1; ib += MT4_THREADS * MT4_CPT) {
-    float acc[MT4_CPT][MS];
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc)
-#pragma unroll
-      for (int r = 0; r < MS; ++r) acc[cc][r] = 0.f;
-    const float4* wrow[MT4_CPT];
-    float4 wn[MT4_CPT];
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc) {
-      const int i = ib + cc * MT4_THREADS;
-      wrow[cc] = reinterpret_cast<const float4*>(W1 + (long long)(i < H1 ? i : 0) * H2);
-      wn[cc] = __ldg(wrow[cc]);
-    }
-    for (int j = 0; j < H2; j += 4) {
-      float4 w[MT4_CPT];
-#pragma unroll
-      for (int cc = 0; cc < MT4_CPT; ++cc) w[cc] = wn[cc];
-      if (j + 4 < H2) {
-#pragma unroll
-        for (int cc = 0; cc < MT4_CPT; ++cc) wn[cc] = __ldg(wrow[cc] + ((j + 4) >> 2));
-      }
-#pragma unroll
-      for (int r = 0; r < MS; ++r) {
-        const float4 a = *reinterpret_cast<const float4*>(h2 + r * H2 + j);            // broadcast
-#pragma unroll
-        for (int cc = 0; cc < MT4_CPT; ++cc) {
-          acc[cc][r] = fmaf(a.x, w[cc].x, acc[cc][r]); acc[cc][r] = fmaf(a.y, w[cc].y, acc[cc][r]);
-          acc[cc][r] = fmaf(a.z, w[cc].z, acc[cc][r]); acc[cc][r] = fmaf(a.w, w[cc].w, acc[cc][r]);
-        }
-      }
-    }
-#pragma unroll
-    for (int cc = 0; cc < MT4_CPT; ++cc) {
-      const int i = ib + cc * MT4_THREADS;
-      if (i < H1) {
-#pragma unroll
-        for (int r = 0; r < MS; ++r) h1[r * H1 + i] = acc[cc][r] * dact_from_out(c.mact0, h1[r * H1 + i]);   // own columns only
-      }
-    }
-  }
-  __syncthreads();
-  // ---- layer 0 transposed, action rows only: one warp per action ------------------------------
-  float* out = c.mdXa + ((long long)agent * 2 + net) * E * A;
-  for (int a = warp; a < A; a += nwarp) {
-    float acc[MS];
-#pragma unroll
-    for (int r = 0; r < MS; ++r) acc[r] = 0.f;
-    const float* wrow = W0 + (long long)(S + a) * H1;
-    for (int j0 = lane; j0 < H1; j0 += 256) {
-      float w[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) w[u] = (j0 + 32 * u < H1) ? __ldg(wrow + j0 + 32 * u) : 0.f;
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (j0 + 32 * u < H1) {
-#pragma unroll
-          for (int r = 0; r < MS; ++r) acc[r] = fmaf(h1[r * H1 + j0 + 32 * u], w[u], acc[r]);
-        }
-      }
-    }
-#pragma unroll
-    for (int r = 0; r < MS; ++r) {
-      float v = acc[r];
-      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (lane == 0 && r < half) out[r * A + a] = v;
-    }
-  }
-}
-
 static inline int model_term_ms(const KCtx& c) {
   const int half = c.nmod == 2 ? c.E / 2 : c.E;
   return half <= 4 ? 4 : half <= 8 ? 8 : half <= 12 ? 12 : half <= 16 ? 16 : 32;
@@ -499,9 +237,6 @@ static inline cudaError_t model_term_init() {
 #define MT_ATTR(MSV) e = cudaFuncSetAttribute(k_model_term<MSV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); if (e) return e;
   MT_ATTR(4) MT_ATTR(8) MT_ATTR(12) MT_ATTR(16) MT_ATTR(32)
 #undef MT_ATTR
-#define MT_ATTR(MSV) e = cudaFuncSetAttribute(k_model_term4<MSV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); if (e) return e;
-  MT_ATTR(4) MT_ATTR(8) MT_ATTR(12) MT_ATTR(16)
-#undef MT_ATTR
 #define MT_ATTR(MSV) e = cudaFuncSetAttribute(k_model_term_mma<MSV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024); if (e) return e;
   MT_ATTR(4) MT_ATTR(8) MT_ATTR(12) MT_ATTR(16)
 #undef MT_ATTR
@@ -511,17 +246,18 @@ static inline cudaError_t model_term_init() {
 static inline size_t model_term_smem(const KCtx& c, int ms) {
   return (size_t)ms * (c.S + c.A + c.mh1 + c.mh2 + c.mo + c.S) * sizeof(float);
 }
-// variant 0: hidden layer on the tensor cores (k_model_term_mma) where the shape allows, else the round-1 kernel;
-// 1: column-blocked CUDA-core kernel; 2: round-1 kernel.
 static inline bool model_term_mma_ok(const KCtx& c) {
   const int half = c.nmod == 2 ? c.E / 2 : c.E;
   return half <= 16 && (c.mh1 % 32) == 0 && (c.mh2 % 32) == 0 && ((c.L.nm_stride % 4) == 0) &&
          (((long long)(c.S + c.A) * c.mh1 + c.mh1) % 4) == 0 && c.mo <= 32 && model_term_mma_smem(c, 16) <= 224 * 1024;
 }
-static inline cudaError_t model_term_launch(const KCtx& c, float* mse_part, cudaStream_t st, int variant = 0) {
+static bool g_mt_fp32 = false;      // test-only: k_model_term even where k_model_term_mma applies (saceo_test_set_mt_fp32)
+// For shapes model_term_eligible accepts: the hidden layer on the tensor cores (k_model_term_mma) where the shape allows,
+// else the fp32 CUDA-core kernel.
+static inline cudaError_t model_term_launch(const KCtx& c, float* mse_part, cudaStream_t st) {
   const int half = c.nmod == 2 ? c.E / 2 : c.E;
   dim3 grid(c.nmod, c.n_agents);
-  if (variant == 0 && model_term_mma_ok(c)) {
+  if (!g_mt_fp32 && model_term_mma_ok(c)) {
     const int nthr = MTM_THREADS;
 #define MT_GOM(MSV) do { k_model_term_mma<MSV><<<grid, nthr, model_term_mma_smem(c, MSV), st>>>(c, mse_part, g_mt_dbg); } while (0)
     if (half <= 4) MT_GOM(4);
@@ -529,15 +265,6 @@ static inline cudaError_t model_term_launch(const KCtx& c, float* mse_part, cuda
     else if (half <= 12) MT_GOM(12);
     else MT_GOM(16);
 #undef MT_GOM
-    return cudaPeekAtLastError();
-  }
-  if (variant == 1 && half <= 16) {      // column-blocked kernel (4 hidden columns per thread)
-#define MT_GO4(MSV) do { k_model_term4<MSV><<<grid, MT4_THREADS, model_term_smem(c, MSV), st>>>(c, mse_part); } while (0)
-    if (half <= 4) MT_GO4(4);
-    else if (half <= 8) MT_GO4(8);
-    else if (half <= 12) MT_GO4(12);
-    else MT_GO4(16);
-#undef MT_GO4
     return cudaPeekAtLastError();
   }
 #define MT_GO(MSV) do { k_model_term<MSV><<<grid, MT_THREADS, model_term_smem(c, MSV), st>>>(c, mse_part); } while (0)

@@ -133,6 +133,7 @@ static int validate(const saceo_config* c) {
   if (c->replay_capacity < 1) return fail(SACEO_E_INVALID, "replay_capacity must be >= 1");
   if (c->gemm_mode != SACEO_GEMM_FP32_SIMT && c->gemm_mode != SACEO_GEMM_TCGEN05_BF16X3)
     return fail(SACEO_E_INVALID, "unknown gemm_mode");
+  if (c->reserved[3] || c->reserved[4] || c->reserved[7]) return fail(SACEO_E_INVALID, "reserved[3], [4] and [7] must be 0");
   return 0;
 }
 
@@ -461,24 +462,39 @@ static int gemm(saceo_ctx* x, bool TA, bool TB, bool ONES, const GemmP& p, int n
   return 0;
 }
 
+// One pass of one net population: what its forward and its backward call share.  The plane images are set only
+// when the backward pass takes the plane path (fused chain + column-sum biases + k_dw_planes); the forward pass then
+// writes h1 ONLY as a plane image, so both calls must see the same pass.
+struct Pass {
+  NetD n;
+  const float* X; int ldx; long long sXa, sXn;        // input rows
+  int rows; long long rowsAllocH;                      // rows of the pass / rows per net allocated in H1, H2
+  float *H1, *H2;                                      // saved activations
+  uint8_t *H1p = nullptr, *dH2p = nullptr, *dH1p = nullptr;   // bf16 hi/lo plane images of h1 / dH2 / dH1
+  long long sQa = 0, sQn = 0;                          // their bytes per agent / net
+  // the caller guarantees that rows [rows, rowsAllocH) of X, H1, H2, dOut, dH2, dH1 are zero, so the
+  // weight-gradient contractions may run over a row count rounded up to the 32-row slabs of the streaming kernel
+  bool kpad = false;
+};
+
 // forward through one population of 3-layer MLPs (nn_utils.py:101-136), rows [row0, rows), unfused: three GEMMs
-static int mlp_forward_unfused(saceo_ctx* x, const NetD& n, const float* X, int ldx, long long sXa, long long sXn,
-                               int row0, int rows, float* H1, float* H2, long long rowsAllocH, float* Out, int ldo,
-                               long long sOa, long long sOn, cudaStream_t st) {
+static int mlp_forward_unfused(saceo_ctx* x, const Pass& ps, int row0, float* Out, int ldo, long long sOa, long long sOn,
+                               cudaStream_t st) {
+  const NetD& n = ps.n;
   const int na = x->cfg.n_agents;
   GemmP p{}; p.nnet = n.nnet; p.f16 = 1;     // forward operands are O(1): fp16 planes (tc_gemm.cuh split8)
-  const int M = rows - row0;
+  const int M = ps.rows - row0;
   // layer 0
-  p.A = X + (long long)row0 * ldx; p.lda = ldx; p.sAa = sXa; p.sAn = sXn;
+  p.A = ps.X + (long long)row0 * ps.ldx; p.lda = ps.ldx; p.sAa = ps.sXa; p.sAn = ps.sXn;
   p.B = n.theta + n.oW0(); p.ldb = n.h1; p.sBa = n.sa; p.sBn = n.sn;
   p.bias = n.theta + n.ob0(); p.sba = n.sa; p.sbn = n.sn;
-  p.C = H1 + (long long)row0 * n.h1; p.ldc = n.h1; p.sCa = (long long)n.nnet * rowsAllocH * n.h1; p.sCn = rowsAllocH * n.h1;
+  p.C = ps.H1 + (long long)row0 * n.h1; p.ldc = n.h1; p.sCa = (long long)n.nnet * ps.rowsAllocH * n.h1; p.sCn = ps.rowsAllocH * n.h1;
   p.M = M; p.N = n.h1; p.K = n.in; p.epi = EPI_ACT; p.act = n.act0;
   int rc = gemm(x, false, false, false, p, na, st); if (rc) return rc;
   // layer 1
   p.A = p.C; p.lda = n.h1; p.sAa = p.sCa; p.sAn = p.sCn;
   p.B = n.theta + n.oW1(); p.ldb = n.h2; p.bias = n.theta + n.ob1();
-  p.C = H2 + (long long)row0 * n.h2; p.ldc = n.h2; p.sCa = (long long)n.nnet * rowsAllocH * n.h2; p.sCn = rowsAllocH * n.h2;
+  p.C = ps.H2 + (long long)row0 * n.h2; p.ldc = n.h2; p.sCa = (long long)n.nnet * ps.rowsAllocH * n.h2; p.sCn = ps.rowsAllocH * n.h2;
   p.M = M; p.N = n.h2; p.K = n.h1; p.act = n.act1;
   rc = gemm(x, false, false, false, p, na, st); if (rc) return rc;
   // layer 2 (linear)
@@ -491,20 +507,20 @@ static int mlp_forward_unfused(saceo_ctx* x, const NetD& n, const float* X, int 
 
 // Forward pass dispatcher: full 128-row tiles of 2x256 nets go through the fused tcgen05 kernel (activations
 // stay in TMEM between layers; h1/h2 reach HBM only when save_h), leftover rows through the GEMM chain.
-static int mlp_forward(saceo_ctx* x, const NetD& n, const float* X, int ldx, long long sXa, long long sXn,
-                       int rows, float* H1, float* H2, long long rowsAllocH, float* Out, int ldo,
-                       long long sOa, long long sOn, cudaStream_t st, bool save_h = true,
-                       uint8_t* H1p = nullptr, long long sQa = 0, long long sQn = 0) {
+static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long long sOa, long long sOn, cudaStream_t st,
+                       bool save_h = true) {
+  const NetD& n = ps.n;
+  const int rows = ps.rows;
   int row0 = 0;
   if (n.planes && x->cfg.reserved[1] == 0 && mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) {
     // warp-specialised kernel on the TMA-fed weight planes: every row (partial tiles are masked)
     FwdW f{};
-    f.X = X; f.ldx = ldx; f.sXa = sXa; f.sXn = sXn;
+    f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
     f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
-    f.H1 = save_h ? H1 : nullptr; f.H2 = save_h ? H2 : nullptr;
-    f.sHa = (long long)n.nnet * rowsAllocH * n.h1; f.sHn = rowsAllocH * n.h1;
-    f.H1p = save_h ? H1p : nullptr; f.sQa = sQa; f.sQn = sQn;
+    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr;
+    f.sHa = (long long)n.nnet * ps.rowsAllocH * n.h1; f.sHn = ps.rowsAllocH * n.h1;
+    f.H1p = save_h ? ps.H1p : nullptr; f.sQa = ps.sQa; f.sQn = ps.sQn;
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
     f.rows = rows; f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1;
     f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
@@ -517,10 +533,10 @@ static int mlp_forward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lon
     int tiles = rows / TC_BM;
     if (rows % TC_BM >= 16) tiles += 1;
     FwdP f{};
-    f.X = X; f.ldx = ldx; f.sXa = sXa; f.sXn = sXn;
+    f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
-    f.H1 = save_h ? H1 : nullptr; f.H2 = save_h ? H2 : nullptr;
-    f.sHa = (long long)n.nnet * rowsAllocH * n.h1; f.sHn = rowsAllocH * n.h1;
+    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr;
+    f.sHa = (long long)n.nnet * ps.rowsAllocH * n.h1; f.sHn = ps.rowsAllocH * n.h1;
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
     f.rows = tiles * TC_BM < rows ? tiles * TC_BM : rows;
     f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1; f.dbg = g_tc_dbg;
@@ -530,22 +546,19 @@ static int mlp_forward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lon
     row0 = f.rows;
     if (row0 >= rows) return 0;
   }
-  return mlp_forward_unfused(x, n, X, ldx, sXa, sXn, row0, rows, H1, H2, rowsAllocH, Out, ldo, sOa, sOn, st);
+  return mlp_forward_unfused(x, ps, row0, Out, ldo, sOa, sOn, st);
 }
 
-// backward through the same MLPs.  grads (nullable): flat [W|b] blocks via the ones-row trick.
-// dXa (nullable): gradient w.r.t. the ACTION columns of the input only (rows S.. of W0).
-static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, long long sXa, long long sXn,
-                        int rows, const float* H1, const float* H2, long long rowsAllocH,
-                        const float* dOut, int ldd, long long sDa, long long sDn, int out_cols,
-                        float* dH2, float* dH1, float* grads, long long sGa, long long sGn,
-                        float* dXa, int S_cols, int A_cols, long long sXaA, long long sXaN, cudaStream_t st,
-                        bool kpad = false, const uint8_t* H1p = nullptr, uint8_t* dH2p = nullptr, long long sQa = 0,
-                        long long sQn = 0, uint8_t* dH1p = nullptr) {
-  const int na = x->cfg.n_agents;
-  // kpad: the caller guarantees that rows [rows, rowsAllocH) of X, H1, H2, dOut, dH2, dH1 are zero, so the
-  // weight-gradient contractions may run over a row count rounded up to the 32-row slabs of the streaming kernel
-  const int krows = (kpad && rup(rows, 32) <= rowsAllocH) ? (int)rup(rows, 32) : rows;
+// backward through the same MLPs.  grads (nullable): flat [W|b] blocks in the layout of theta, via the ones-row trick.
+// dXa (nullable): gradient w.r.t. the last A_cols (action) columns of the input only (their rows of W0).
+static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd, long long sDa, long long sDn,
+                        float* dH2, float* dH1, float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN,
+                        cudaStream_t st) {
+  const NetD& n = ps.n;
+  const int na = x->cfg.n_agents, rows = ps.rows, S_cols = n.in - A_cols;
+  const float *H1 = ps.H1, *H2 = ps.H2;
+  const long long rowsAllocH = ps.rowsAllocH, sGa = n.sa, sGn = n.sn;
+  const int krows = (ps.kpad && rup(rows, 32) <= rowsAllocH) ? (int)rup(rows, 32) : rows;
   const long long sH1a = (long long)n.nnet * rowsAllocH * n.h1, sH1n = rowsAllocH * n.h1;
   const long long sH2a = (long long)n.nnet * rowsAllocH * n.h2, sH2n = rowsAllocH * n.h2;
   int rc;
@@ -553,9 +566,9 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
   // fused gradient chain (dH2, dH1, dXa) on tensor cores with the tile resident in TMEM
   bool fused = false, bias_done = false, dw1_planes = false, dw0_planes = false;
   if (n.planes && x->cfg.reserved[2] == 0 &&
-      mlp_bwd_ws_eligible(n.h1, n.h2, out_cols, n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn)) {
+      mlp_bwd_ws_eligible(n.h1, n.h2, n.out, n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn)) {
     BwdW f{};
-    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = out_cols;
+    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = n.out;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
     f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
     f.H1 = H1; f.H2 = H2; f.sHa = sH1a; f.sHn = sH1n;
@@ -564,13 +577,13 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
     f.rows = rows; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1;
     const int tiles = (rows + TC_BM - 1) / TC_BM;
     const bool db_fits = (long long)na * n.nnet * tiles * 2 * FW_H <= x->dbpart_cap;
-    f.dbpart = (grads && x->dbpart && db_fits && x->cfg.reserved[4] == 0) ? x->dbpart : nullptr;
+    f.dbpart = (grads && x->dbpart && db_fits) ? x->dbpart : nullptr;
     // hidden-to-hidden weight gradient from bf16 plane images (k_dw_planes): dH2 then leaves the kernel as planes only
-    dw1_planes = grads && f.dbpart && H1p && dH2p;
-    if (dw1_planes) { f.dH2 = nullptr; f.dH2p = dH2p; f.H1p = H1p; f.sQa = sQa; f.sQn = sQn; }
+    dw1_planes = grads && f.dbpart && ps.H1p;
+    if (dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
     // first-layer weight gradient from the dH1 plane image (k_dw0_planes): dH1 then leaves the kernel as planes only
-    dw0_planes = dw1_planes && dH1p && dw0_planes_eligible(n.in, rows, ldx, X, sXa, sXn);
-    if (dw0_planes) { f.dH1 = nullptr; f.dH1p = dH1p; }
+    dw0_planes = dw1_planes && ps.dH1p && dw0_planes_eligible(n.in, rows, ps.ldx, ps.X, ps.sXa, ps.sXn);
+    if (dw0_planes) { f.dH1 = nullptr; f.dH1p = ps.dH1p; }
     f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
     if (mlp_bwd_ws_launch(f, na, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused backward launch failed");
     count_launch(x, "k_mlp_bwd_ws", st);
@@ -580,12 +593,10 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
       count_launch(x, "k_bias_finish", st);
       bias_done = true;
     }
-  } else
-  if (x->cfg.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && x->cfg.reserved[2] == 0 && n.h1 == FW_H && n.h2 == FW_H &&
-      out_cols >= 1 && out_cols <= 64 && rows >= TC_BM && (rows % TC_BM == 0 || rows % TC_BM >= 16) &&
-      (!dXa || A_cols <= 32) && ((reinterpret_cast<uintptr_t>(n.theta) & 15) == 0) && ((n.sa & 3) == 0) && ((n.sn & 3) == 0)) {
+  } else if (x->cfg.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && x->cfg.reserved[2] == 0 &&
+             mlp_bwd_tc_eligible(n.h1, n.h2, n.out, rows, dXa != nullptr, A_cols, n.theta, n.sa, n.sn)) {
     BwdP f{};
-    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = out_cols;
+    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = n.out;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
     f.H1 = H1; f.H2 = H2; f.sHa = sH1a; f.sHn = sH1n;
     f.dH2 = grads ? dH2 : nullptr; f.dH1 = grads ? dH1 : nullptr;
@@ -595,7 +606,7 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
     // the kernel indexes dbpart as [agent*nnet+net][tile][2][256]: callers with more row tiles than the workspace was
     // sized for (e.g. model fitting with 256-wide models and a large minibatch) take the ones-row bias path instead
     const bool db_fits = (long long)na * n.nnet * grid.x * 2 * FW_H <= x->dbpart_cap;
-    f.dbpart = (grads && x->dbpart && db_fits && x->cfg.reserved[4] == 0) ? x->dbpart : nullptr;
+    f.dbpart = (grads && x->dbpart && db_fits) ? x->dbpart : nullptr;
     k_mlp_bwd_tc<<<grid, FW_NT, FW_BYTES, st>>>(f);
     count_launch(x, "k_mlp_bwd_tc", st);
     fused = true;
@@ -623,17 +634,17 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
     rc = gemm(x, true, false, true, p, na, st2); if (rc) return rc;
   }
   if (!fused) {
-  // dH2 = (dOut . W2[:, :out_cols]^T) * act1'(H2)
+  // dH2 = (dOut . W2^T) * act1'(H2)
   p = GemmP{}; p.nnet = n.nnet;
   p.A = dOut; p.lda = ldd; p.sAa = sDa; p.sAn = sDn;
   p.B = n.theta + n.oW2(); p.ldb = n.out; p.sBa = n.sa; p.sBn = n.sn;
   p.C = dH2; p.ldc = n.h2; p.sCa = sH2a; p.sCn = sH2n; p.aux = H2;
-  p.M = rows; p.N = n.h2; p.K = out_cols; p.epi = EPI_MUL_DACT; p.act = n.act1;
+  p.M = rows; p.N = n.h2; p.K = n.out; p.epi = EPI_MUL_DACT; p.act = n.act1;
   rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
   }
   if (grads && dw1_planes) {   // dW1 = H1^T . dH2 from the plane images (db1 came from the kernel's column sums)
     DwP d{};
-    d.Ap = H1p; d.sAa = sQa; d.sAn = sQn; d.Bp = dH2p; d.sBa = sQa; d.sBn = sQn;
+    d.Ap = ps.H1p; d.sAa = ps.sQa; d.sAn = ps.sQn; d.Bp = ps.dH2p; d.sBa = ps.sQa; d.sBn = ps.sQn;
     d.G = grads + n.oW1(); d.sGa = sGa; d.sGn = sGn; d.rows = rows; d.nnet = n.nnet;
     k_dw_planes<<<na * n.nnet, WS_NT, DW_BYTES, st>>>(d);
     count_launch(x, "k_dw_planes", st);
@@ -656,13 +667,13 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
   }
   if (grads && dw0_planes) {   // dW0 = X^T . dH1 from the plane image (db0 came from the kernel's column sums)
     Dw0P d{};
-    d.X = X; d.ldx = ldx; d.sXa = sXa; d.sXn = sXn; d.Bp = dH1p; d.sBa = sQa; d.sBn = sQn;
+    d.X = ps.X; d.ldx = ps.ldx; d.sXa = ps.sXa; d.sXn = ps.sXn; d.Bp = ps.dH1p; d.sBa = ps.sQa; d.sBn = ps.sQn;
     d.G = grads + n.oW0(); d.sGa = sGa; d.sGn = sGn; d.rows = rows; d.in = n.in; d.nnet = n.nnet;
     k_dw0_planes<<<na * n.nnet, WS_NT, DW0_BYTES, st0>>>(d);
     count_launch(x, "k_dw0_planes", st0);
   } else if (grads) {   // [dW0; db0] = [X,1]^T . dH1
     p = GemmP{}; p.nnet = n.nnet;
-    p.A = X; p.lda = ldx; p.sAa = sXa; p.sAn = sXn;
+    p.A = ps.X; p.lda = ps.ldx; p.sAa = ps.sXa; p.sAn = ps.sXn;
     p.B = dH1; p.ldb = n.h1; p.sBa = sH1a; p.sBn = sH1n;
     p.C = grads + n.oW0(); p.ldc = n.h1; p.sCa = sGa; p.sCn = sGn;
     p.M = bias_done ? n.in : n.in + 1; p.N = n.h1; p.K = krows; p.epi = EPI_NONE;
@@ -681,16 +692,6 @@ static int mlp_backward(saceo_ctx* x, const NetD& n, const float* X, int ldx, lo
     rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
   }
   return 0;
-}
-
-// Will mlp_backward(grads) of this net on `rows` rows take the plane path (fused chain + column-sum biases + k_dw_planes)?
-// The forward pass that saves the activations asks the same question: it then writes h1 ONLY as a plane image.
-static bool dw_planes_ok(const saceo_ctx* x, const NetD& n, int rows, int out_cols, const uint8_t* H1p, const uint8_t* dH2p) {
-  if (!n.planes || x->cfg.reserved[2] != 0 || x->cfg.reserved[1] != 0 || x->cfg.reserved[4] != 0 || !H1p || !dH2p || !x->dbpart) return false;
-  if (!mlp_bwd_ws_eligible(n.h1, n.h2, out_cols, n.out, false, 0, n.theta, n.sa, n.sn)) return false;
-  if (!mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) return false;
-  const int tiles = (rows + TC_BM - 1) / TC_BM;
-  return (long long)x->cfg.n_agents * n.nnet * tiles * 2 * FW_H <= x->dbpart_cap;
 }
 
 static NetD actor_net(const saceo_ctx* x) {
@@ -713,6 +714,57 @@ static NetD model_net(const saceo_ctx* x, int nnet) {
               c.model_hidden[1], x->L.model_out, c.model_act[0], c.model_act[1]};
 }
 
+// Gives a pass the plane images if mlp_backward(grads) of it takes the plane path (fused chain + column-sum biases +
+// k_dw_planes); decided once, so that its forward and backward calls cannot disagree.
+static void plane_path(const saceo_ctx* x, Pass& ps, uint8_t* H1p, uint8_t* dH2p, uint8_t* dH1p, long long sQa, long long sQn) {
+  const NetD& n = ps.n;
+  if (!n.planes || x->cfg.reserved[2] != 0 || x->cfg.reserved[1] != 0 || !H1p || !dH2p || !x->dbpart) return;
+  if (!mlp_bwd_ws_eligible(n.h1, n.h2, n.out, n.out, false, 0, n.theta, n.sa, n.sn)) return;
+  if (!mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) return;
+  const int tiles = (ps.rows + TC_BM - 1) / TC_BM;
+  if ((long long)x->cfg.n_agents * n.nnet * tiles * 2 * FW_H > x->dbpart_cap) return;
+  ps.H1p = H1p; ps.dH2p = dH2p; ps.dH1p = dH1p; ps.sQa = sQa; ps.sQn = sQn;
+}
+
+// the actor on the staged observation rows Xpi of view k: <= B rows (TD target, temperature, acting) or the E expert
+// rows of the on-policy expert gradient
+static Pass actor_pass(const saceo_ctx* x, const KCtx& k, int rows) {
+  return Pass{actor_net(x), k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, rows, k.Rs, k.aH1, k.aH2};
+}
+// the actor update over its R = B + E rows
+static Pass actor_update_pass(const saceo_ctx* x, const KCtx& k) {
+  Pass ps = actor_pass(x, k, k.R);
+  ps.kpad = true;
+  plane_path(x, ps, x->aH1p, x->adH2p, x->adH1p, x->a_img, 0);
+  return ps;
+}
+// twin critics (or their targets) on the first `rows` of B critic input rows X (Xc, Xc2 or Xc3)
+static Pass critic_pass(const saceo_ctx* x, bool target, const float* X, int rows) {
+  const KCtx& k = x->k;
+  return Pass{critic_net(x, target), X, k.ldXc, (long long)k.B * k.ldXc, 0, rows, k.B, k.cH1, k.cH2};
+}
+// the critic update over the B minibatch rows
+static Pass critic_update_pass(const saceo_ctx* x) {
+  Pass ps = critic_pass(x, false, x->k.Xc2, x->k.B);
+  plane_path(x, ps, x->cH1p, x->cdH2p, x->cdH1p, 2 * x->c_img, x->c_img);
+  return ps;
+}
+// the actor on the fvp_rows states (Fisher-vector product, CG, TRPO / PPO surrogate)
+static Pass fvp_pass(const saceo_ctx* x) {
+  const KCtx& k = x->k; const FvpWs& f = x->f;
+  return Pass{actor_net(x), f.X, k.S, (long long)f.N * k.S, 0, f.N, f.N, f.H1, f.H2};
+}
+// the models on the first `rows` of the E staged rows of Xm; every model reads net 0's block (zero net stride)
+static Pass model_eval_pass(const saceo_ctx* x, int rows) {
+  const KCtx& k = x->k; const int SA = k.S + k.A;
+  return Pass{model_net(x, k.nmod), k.Xm, SA, 2LL * k.E * SA, 0, rows, k.E, k.mH1, k.mH2};
+}
+// a model or reward net being fitted on the staged minibatch rows
+static Pass fit_pass(const saceo_ctx* x, const NetD& n, float* H1, float* H2) {
+  const FitCtx& f = x->fit; const int SA = x->cfg.S + x->cfg.A;
+  return Pass{n, f.X, SA, 2LL * f.mbs * SA, (long long)f.mbs * SA, f.mb, f.mbs, H1, H2};
+}
+
 // ------------------------------------------------------------------------------------------
 // update phases
 // ------------------------------------------------------------------------------------------
@@ -733,21 +785,16 @@ static int phase_gather(saceo_ctx* x, cudaStream_t st) {
 static int phase_critic_grads(saceo_ctx* x, cudaStream_t st) {
   const KCtx& k = x->k; const int n = k.n_agents, B = k.B, A = k.A;
   int rc;
-  NetD an = actor_net(x), tn = critic_net(x, true), qn = critic_net(x, false);
   // inputs were staged by the gather: Xpi = N_s(sp), Xc = [N_s(sp) | .], Xc2 = [N_s(s) | N_a(a)]
-  rc = mlp_forward(x, an, k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, B, k.aH1, k.aH2, k.Rs, k.aOut, k.Ao,
-                   (long long)k.Rs * k.Ao, 0, st, false); if (rc) return rc;
+  rc = mlp_forward(x, actor_pass(x, k, B), k.aOut, k.Ao, (long long)k.Rs * k.Ao, 0, st, false); if (rc) return rc;
   LAUNCH(x, k_head_fwd, dim3(cdiv(B, 128), n), 128, 0, st, k, B, B, k.noise, (3LL * B + k.E) * A, 0, 1,
          (float*)nullptr, (float*)nullptr, 0LL, 0);
-  rc = mlp_forward(x, tn, k.Xc, k.ldXc, (long long)B * k.ldXc, 0, B, k.cH1, k.cH2, B, k.cQ, 1, 2LL * B, B, st, false); if (rc) return rc;
+  rc = mlp_forward(x, critic_pass(x, true, k.Xc, B), k.cQ, 1, 2LL * B, B, st, false); if (rc) return rc;
   LAUNCH(x, k_td_target, dim3(cdiv(B, 128), n), 128, 0, st, k);
-  const bool cpl = dw_planes_ok(x, qn, B, 1, x->cH1p, x->cdH2p);
-  rc = mlp_forward(x, qn, k.Xc2, k.ldXc, (long long)B * k.ldXc, 0, B, k.cH1, k.cH2, B, k.cQ, 1, 2LL * B, B, st, true,
-                   cpl ? x->cH1p : nullptr, 2 * x->c_img, x->c_img); if (rc) return rc;
+  const Pass qp = critic_update_pass(x);
+  rc = mlp_forward(x, qp, k.cQ, 1, 2LL * B, B, st); if (rc) return rc;
   LAUNCH(x, k_critic_loss, dim3(2, n), 256, 0, st, k);
-  rc = mlp_backward(x, qn, k.Xc2, k.ldXc, (long long)B * k.ldXc, 0, B, k.cH1, k.cH2, B, k.cdQ, 1, 2LL * B, B, 1,
-                    k.cdH2, k.cdH1, k.g_q, 2 * x->L.nc_stride, x->L.nc_stride, nullptr, 0, 0, 0, 0, st, false,
-                    cpl ? x->cH1p : nullptr, cpl ? x->cdH2p : nullptr, 2 * x->c_img, x->c_img, cpl ? x->cdH1p : nullptr);
+  rc = mlp_backward(x, qp, k.cdQ, 1, 2LL * B, B, k.cdH2, k.cdH1, k.g_q, nullptr, 0, 0, 0, st);
   if (rc) return rc;
   return check_launch();
 }
@@ -774,9 +821,9 @@ static KCtx actor_view(const saceo_ctx* x, bool bc = false) {
 static int model_term_phase(saceo_ctx* x, const KCtx& k, cudaStream_t st) {
   const int n = k.n_agents, S = k.S, A = k.A, SA = S + A, E = k.E;
   int rc;
-  if (k.nmod > 0 && x->cfg.reserved[3] == 0 && model_term_eligible(k)) {
+  if (k.nmod > 0 && model_term_eligible(k)) {
     // fused expert-observation term: model forward, MSE, backward to the action columns in one kernel
-    if (model_term_launch(k, k.mse_part, st, x->cfg.reserved[7]) != cudaSuccess) return fail(SACEO_E_CUDA, "model-term launch failed");
+    if (model_term_launch(k, k.mse_part, st) != cudaSuccess) return fail(SACEO_E_CUDA, "model-term launch failed");
     count_launch(x, "k_model_term", st);
   } else if (k.nmod > 0) {
     const int half = k.nmod == 2 ? E / 2 : E;
@@ -831,13 +878,10 @@ static int model_term_phase(saceo_ctx* x, const KCtx& k, cudaStream_t st) {
 // phase 2a: everything of the actor step that does not depend on the critics
 static int phase_actor_pre(saceo_ctx* x, cudaStream_t st, bool bc = false) {
   const KCtx kk = actor_view(x, bc);
-  const KCtx& k = kk; const int n = k.n_agents, B = k.B, S = k.S, A = k.A, SA = S + A, R = k.R, E = k.E, Rs = k.Rs;
+  const KCtx& k = kk; const int n = k.n_agents, B = k.B, S = k.S, A = k.A, R = k.R, E = k.E;
   int rc;
-  NetD an = actor_net(x);
   LAUNCH(x, k_stage, dim3(cdiv((long long)R * S, 256), n), 256, 0, st, k);
-  rc = mlp_forward(x, an, k.Xpi, k.ldXp, (long long)Rs * k.ldXp, 0, R, k.aH1, k.aH2, Rs, k.aOut, k.Ao, (long long)Rs * k.Ao, 0, st, true,
-                   dw_planes_ok(x, an, R, k.Ao, x->aH1p, x->adH2p) ? x->aH1p : nullptr, x->a_img, 0);
-  if (rc) return rc;
+  rc = mlp_forward(x, actor_update_pass(x, k), k.aOut, k.Ao, (long long)k.Rs * k.Ao, 0, st); if (rc) return rc;
   LAUNCH(x, k_head_fwd, dim3(cdiv(R, 128), n), 128, 0, st, k, R, B, k.noise, (3LL * B + E) * A, B, 2,
          (float*)nullptr, (float*)nullptr, 0LL, 0);      // pi(s) -> the action columns of Xc3
   rc = model_term_phase(x, k, st); if (rc) return rc;
@@ -849,24 +893,20 @@ static int phase_actor_pre(saceo_ctx* x, cudaStream_t st, bool bc = false) {
 // backward-to-action on the B minibatch rows) is skipped: those rows then carry exactly-zero output gradients.
 static int phase_actor_post(saceo_ctx* x, cudaStream_t st, bool bc = false) {
   const KCtx kk = actor_view(x, bc);
-  const KCtx& k = kk; const int n = k.n_agents, B = k.B, S = k.S, A = k.A, R = k.R, Rs = k.Rs;
+  const KCtx& k = kk; const int n = k.n_agents, B = k.B, A = k.A, R = k.R;
   int rc;
-  NetD an = actor_net(x), qn = critic_net(x, false);
   if (!bc) {
-    rc = mlp_forward(x, qn, k.Xc2, k.ldXc, (long long)B * k.ldXc, 0, B, k.cH1, k.cH2, B, k.cQ, 1, 2LL * B, B, st); if (rc) return rc;
+    const Pass qp = critic_pass(x, false, k.Xc2, B);
+    rc = mlp_forward(x, qp, k.cQ, 1, 2LL * B, B, st); if (rc) return rc;
     LAUNCH(x, k_actor_q, dim3(n), 256, 0, st, k);
-    rc = mlp_backward(x, qn, k.Xc2, k.ldXc, (long long)B * k.ldXc, 0, B, k.cH1, k.cH2, B, k.cdQ, 1, 2LL * B, B, 1,
-                      k.cdH2, k.cdH1, nullptr, 0, 0, k.cdXa, S, A, 2LL * B * A, (long long)B * A, st);
+    rc = mlp_backward(x, qp, k.cdQ, 1, 2LL * B, B, k.cdH2, k.cdH1, nullptr, k.cdXa, A, 2LL * B * A, (long long)B * A, st);
     if (rc) return rc;
   } else {
     CU(cudaMemsetAsync(k.cdXa, 0, sizeof(float) * (size_t)n * 2 * B * A, st));
   }
   LAUNCH(x, k_head_bwd, dim3(cdiv(R, 128), n), 128, 0, st, k, R);
-  rc = mlp_backward(x, an, k.Xpi, k.ldXp, (long long)Rs * k.ldXp, 0, R, k.aH1, k.aH2, Rs, k.daOut, k.Ao, (long long)Rs * k.Ao, 0,
-                    k.Ao, k.daH2, k.daH1, k.g_actor, x->L.na_stride, 0, nullptr, 0, 0, 0, 0, st, true,
-                    dw_planes_ok(x, an, R, k.Ao, x->aH1p, x->adH2p) ? x->aH1p : nullptr,
-                    dw_planes_ok(x, an, R, k.Ao, x->aH1p, x->adH2p) ? x->adH2p : nullptr, x->a_img, 0,
-                    dw_planes_ok(x, an, R, k.Ao, x->aH1p, x->adH2p) ? x->adH1p : nullptr);
+  rc = mlp_backward(x, actor_update_pass(x, k), k.daOut, k.Ao, (long long)k.Rs * k.Ao, 0, k.daH2, k.daH1, k.g_actor,
+                    nullptr, 0, 0, 0, st);
   if (rc) return rc;
   if (!k.per_state_std) LAUNCH(x, k_lsv_reduce, dim3(n), 32 * cdiv(A, 32), 0, st, k, R);
   return check_launch();
@@ -888,9 +928,7 @@ static int phase_actor_apply(saceo_ctx* x, cudaStream_t st) {
 static int phase_alpha(saceo_ctx* x, int apply, cudaStream_t st) {
   const KCtx kk = actor_view(x);          // Xpi2 still holds N_s(s) from the actor phase
   const KCtx& k = kk; const int n = k.n_agents, B = k.B, A = k.A;
-  NetD an = actor_net(x);
-  int rc = mlp_forward(x, an, k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, B, k.aH1, k.aH2, k.Rs, k.aOut, k.Ao,
-                       (long long)k.Rs * k.Ao, 0, st, false); if (rc) return rc;
+  int rc = mlp_forward(x, actor_pass(x, k, B), k.aOut, k.Ao, (long long)k.Rs * k.Ao, 0, st, false); if (rc) return rc;
   LAUNCH(x, k_head_fwd, dim3(cdiv(B, 128), n), 128, 0, st, k, B, B, k.noise, (3LL * B + k.E) * A, 2 * B + k.E, 0,
          (float*)nullptr, (float*)nullptr, 0LL, 0);
   LAUNCH(x, k_alpha_step, dim3(n), 256, 0, st, k, apply);
@@ -1152,14 +1190,12 @@ extern "C" int saceo_actor_forward(saceo_ctx* x, const float* obs, int32_t rows,
   if (!x->bound) return fail(SACEO_E_UNBOUND, "saceo_bind() has not been called");
   cudaStream_t st = (cudaStream_t)stream; const KCtx& k = x->k; const int n = k.n_agents;
   { int rcp = ensure_planes(x, st); if (rcp) return rcp; }
-  NetD an = actor_net(x);
   // expert rows would be routed to the model input: use only the first B ("main") rows per chunk
   for (int r0 = 0; r0 < rows; r0 += k.B) {
     const int nr = rows - r0 < k.B ? rows - r0 : k.B;
     LAUNCH(x, k_stage_obs, dim3(cdiv((long long)nr * k.S, 256), n), 256, 0, st, k, obs, rows, r0, nr, k.Xpi, k.ldXp,
            (long long)k.Rs * k.ldXp, 0);
-    int rc = mlp_forward(x, an, k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, nr, k.aH1, k.aH2, k.Rs, k.aOut, k.Ao,
-                         (long long)k.Rs * k.Ao, 0, st, false); if (rc) return rc;
+    int rc = mlp_forward(x, actor_pass(x, k, nr), k.aOut, k.Ao, (long long)k.Rs * k.Ao, 0, st, false); if (rc) return rc;
     LAUNCH(x, k_head_fwd, dim3(cdiv(nr, 128), n), 128, 0, st, k, nr, nr, noise, (long long)rows * k.A, r0, 0,
            act_out, neglogp_out, (long long)rows, r0);
   }
@@ -1172,15 +1208,13 @@ extern "C" int saceo_critic_forward(saceo_ctx* x, int32_t which, const float* ob
   if (!x->bound) return fail(SACEO_E_UNBOUND, "saceo_bind() has not been called");
   cudaStream_t st = (cudaStream_t)stream; const KCtx& k = x->k; const int n = k.n_agents;
   { int rcp = ensure_planes(x, st); if (rcp) return rcp; }
-  NetD qn = critic_net(x, which != 0);
   for (int r0 = 0; r0 < rows; r0 += k.B) {
     const int nr = rows - r0 < k.B ? rows - r0 : k.B;
     LAUNCH(x, k_stage_obs, dim3(cdiv((long long)nr * k.S, 256), n), 256, 0, st, k, obs, rows, r0, nr, k.Xc, k.ldXc,
            (long long)k.B * k.ldXc, 0);
     LAUNCH(x, k_stage_act, dim3(cdiv((long long)nr * k.A, 256), n), 256, 0, st, k, act, rows, r0, nr, k.Xc, k.ldXc,
            (long long)k.B * k.ldXc, 0);
-    int rc = mlp_forward(x, qn, k.Xc, k.ldXc, (long long)k.B * k.ldXc, 0, nr, k.cH1, k.cH2, k.B, q_out + r0, 1,
-                         2LL * rows, rows, st, false); if (rc) return rc;
+    int rc = mlp_forward(x, critic_pass(x, which != 0, k.Xc, nr), q_out + r0, 1, 2LL * rows, rows, st, false); if (rc) return rc;
   }
   if (scale_ret) LAUNCH(x, k_scale_ret, dim3(cdiv(2LL * rows, 256), n), 256, 0, st, k, q_out, rows);
   return check_launch();
@@ -1192,7 +1226,6 @@ extern "C" int saceo_model_eval(saceo_ctx* x, const float* obs, const float* act
   if (!x->bound) return fail(SACEO_E_UNBOUND, "saceo_bind() has not been called");
   if (x->cfg.num_models < 1) return fail(SACEO_E_INVALID, "no models configured");
   cudaStream_t st = (cudaStream_t)stream; const KCtx& k = x->k; const int n = k.n_agents, SA = k.S + k.A, E = k.E;
-  NetD mn = model_net(x, k.nmod);
   for (int r0 = 0; r0 < rows; r0 += E) {
     const int nr = rows - r0 < E ? rows - r0 : E;
     // every model sees the same rows: stage them into net 0's block and read it with a zero net stride
@@ -1200,8 +1233,8 @@ extern "C" int saceo_model_eval(saceo_ctx* x, const float* obs, const float* act
            2LL * E * SA, 1);
     LAUNCH(x, k_stage_act, dim3(cdiv((long long)nr * k.A, 256), n), 256, 0, st, k, act, rows, r0, nr, k.Xm, SA,
            2LL * E * SA, 1);
-    int rc = mlp_forward(x, mn, k.Xm, SA, 2LL * E * SA, 0, nr, k.mH1, k.mH2, E, k.mOut, mn.out,
-                         2LL * E * mn.out, (long long)E * mn.out, st); if (rc) return rc;
+    const int mo = x->L.model_out;
+    int rc = mlp_forward(x, model_eval_pass(x, nr), k.mOut, mo, 2LL * E * mo, (long long)E * mo, st); if (rc) return rc;
     LAUNCH(x, k_model_out, dim3(cdiv((long long)nr * k.S, 256), n, k.nmod), 256, 0, st, k, obs, rows, r0, nr, sp_out);
   }
   return check_launch();
@@ -1284,31 +1317,27 @@ extern "C" int saceo_model_fit(saceo_ctx* x, int32_t n_steps, const int64_t* idx
   cudaStream_t st = (cudaStream_t)stream;
   const KCtx& k = x->k; const FitCtx& f = x->fit;
   const int n = k.n_agents, mb = f.mb, ms = f.mbs, SA = k.S + k.A, mo = x->L.model_out;
-  NetD net{f.model, 2 * x->L.nm_stride, x->L.nm_stride, f.nmod, SA, x->cfg.model_hidden[0], x->cfg.model_hidden[1], mo,
-           x->cfg.model_act[0], x->cfg.model_act[1]};
+  const Pass mp = fit_pass(x, NetD{f.model, 2 * x->L.nm_stride, x->L.nm_stride, f.nmod, SA, x->cfg.model_hidden[0],
+                                   x->cfg.model_hidden[1], mo, x->cfg.model_act[0], x->cfg.model_act[1]}, f.H1, f.H2);
+  const Pass rp = fit_pass(x, NetD{f.rw, 2 * f.nr_stride, f.nr_stride, f.nmod, SA, f.rh1, f.rh2, 1, f.ract0, f.ract1},
+                           f.rH1, f.rH2);
   for (int s = 0; s < n_steps; ++s) {
     const long long* ix = reinterpret_cast<const long long*>(idx) + (long long)s * n * f.nmod * mb;
     LAUNCH(x, k_fit_begin, cdiv(n, 128), 128, 0, st, f, n);
     LAUNCH(x, k_fit_stage, dim3(cdiv((long long)mb * (SA + k.S + 1), 256), f.nmod, n), 256, 0, st, k, f, ix);
-    int rc = mlp_forward(x, net, f.X, SA, 2LL * ms * SA, (long long)ms * SA, mb, f.H1, f.H2, ms, f.Out, mo,
-                         2LL * ms * mo, (long long)ms * mo, st, true);
+    int rc = mlp_forward(x, mp, f.Out, mo, 2LL * ms * mo, (long long)ms * mo, st);
     if (rc) return rc;
-    NetD rnet{f.rw, 2 * f.nr_stride, f.nr_stride, f.nmod, SA, f.rh1, f.rh2, 1, f.ract0, f.ract1};
     if (f.rw) {      // the reward network sees the same normalised input (base_world_model.py:72-74)
-      rc = mlp_forward(x, rnet, f.X, SA, 2LL * ms * SA, (long long)ms * SA, mb, f.rH1, f.rH2, ms, f.rOut, 1,
-                       2LL * ms, (long long)ms, st, true);
+      rc = mlp_forward(x, rp, f.rOut, 1, 2LL * ms, (long long)ms, st);
       if (rc) return rc;
     }
     LAUNCH(x, k_fit_loss, dim3(f.nmod, n), 256, 0, st, k, f,
            losses_out ? losses_out + (long long)s * n * f.nmod : (float*)nullptr);
-    rc = mlp_backward(x, net, f.X, SA, 2LL * ms * SA, (long long)ms * SA, mb, f.H1, f.H2, ms, f.dOut, mo,
-                      2LL * ms * mo, (long long)ms * mo, mo, f.dH2, f.dH1, f.g, 2 * x->L.nm_stride, x->L.nm_stride,
-                      nullptr, 0, 0, 0, 0, st, false);    // K = 200 on the register-staged kernel beats K = 224 streamed (measured)
+    // no kpad: K = 200 on the register-staged kernel beats K = 224 streamed (measured)
+    rc = mlp_backward(x, mp, f.dOut, mo, 2LL * ms * mo, (long long)ms * mo, f.dH2, f.dH1, f.g, nullptr, 0, 0, 0, st);
     if (rc) return rc;
     if (f.rw) {
-      rc = mlp_backward(x, rnet, f.X, SA, 2LL * ms * SA, (long long)ms * SA, mb, f.rH1, f.rH2, ms, f.rdOut, 1,
-                        2LL * ms, (long long)ms, 1, f.rdH2, f.rdH1, f.g_r, 2 * f.nr_stride, f.nr_stride,
-                        nullptr, 0, 0, 0, 0, st, false);
+      rc = mlp_backward(x, rp, f.rdOut, 1, 2LL * ms, (long long)ms, f.rdH2, f.rdH1, f.g_r, nullptr, 0, 0, 0, st);
       if (rc) return rc;
     }
     if (f.use_clip) LAUNCH(x, k_fit_gnorm, n, 1024, 0, st, f);
@@ -1324,10 +1353,9 @@ extern "C" int saceo_model_fit(saceo_ctx* x, int32_t n_steps, const int64_t* idx
 static int fvp_prepare(saceo_ctx* x, cudaStream_t st) {
   { int rcp = ensure_planes(x, st); if (rcp) return rcp; }
   const KCtx& k = x->k; const FvpWs& f = x->f; const int n = k.n_agents, N = f.N;
-  NetD an = actor_net(x);
   LAUNCH(x, k_stage_obs, dim3(cdiv((long long)N * k.S, 256), n), 256, 0, st, k, k.T.fvp_states, N, 0, N, f.X, k.S,
          (long long)N * k.S, 0);
-  return mlp_forward(x, an, f.X, k.S, (long long)N * k.S, 0, N, f.H1, f.H2, N, f.Out, k.Ao, (long long)N * k.Ao, 0, st);
+  return mlp_forward(x, fvp_pass(x), f.Out, k.Ao, (long long)N * k.Ao, 0, st);
 }
 
 // Fx = J^T M J x / N + damp x, with the activations of fvp_prepare() resident
@@ -1361,8 +1389,7 @@ static int fvp_apply(saceo_ctx* x, const float* xin, float damp, float* Fx, cuda
   // metric: G = M . J x / N   (per row), plus per-row logstd_var contribution
   LAUNCH(x, k_fvp_metric, dim3(cdiv(N, 128), n), 128, 0, st, k, f, xin, x->cfg.std_mult);
   // J^T G  -> Fx (flat layout), then + damp x
-  rc = mlp_backward(x, an, f.X, k.S, (long long)N * k.S, 0, N, f.H1, f.H2, N, f.G, k.Ao, sO, 0, k.Ao, f.dH2, f.dH1,
-                    Fx, x->L.na_stride, 0, nullptr, 0, 0, 0, 0, st); if (rc) return rc;
+  rc = mlp_backward(x, fvp_pass(x), f.G, k.Ao, sO, 0, f.dH2, f.dH1, Fx, nullptr, 0, 0, 0, st); if (rc) return rc;
   LAUNCH(x, k_fvp_finish, dim3(cdiv(x->L.na, 256), n), 256, 0, st, k, f, xin, damp, Fx);
   return check_launch();
 }
@@ -1411,13 +1438,12 @@ static int surrogate_grad(saceo_ctx* x, const float* act, const float* adv, cons
   int rc = trpo_check(x); if (rc) return rc;
   if (!act || !adv || !grad_out) return fail(SACEO_E_INVALID, "act, adv and grad_out are required");
   const KCtx& k = x->k; const FvpWs& f = x->f; const int n = k.n_agents, N = f.N;
-  NetD an = actor_net(x);
   rc = fvp_prepare(x, st); if (rc) return rc;
   LAUNCH(x, k_trpo_rows, dim3(cdiv(N, 128), n), 128, 0, st, k, f, act, adv, nlp_old, (const float*)nullptr, alpha,
          x->cfg.std_mult, 1, clip_eps, (float*)nullptr, (float*)nullptr);
   if (stats_out) LAUNCH(x, k_trpo_reduce, dim3(n), 256, 0, st, f, stats_out);
-  rc = mlp_backward(x, an, f.X, k.S, (long long)N * k.S, 0, N, f.H1, f.H2, N, f.G, k.Ao, (long long)N * k.Ao, 0, k.Ao,
-                    f.dH2, f.dH1, grad_out, x->L.na_stride, 0, nullptr, 0, 0, 0, 0, st); if (rc) return rc;
+  rc = mlp_backward(x, fvp_pass(x), f.G, k.Ao, (long long)N * k.Ao, 0, f.dH2, f.dH1, grad_out, nullptr, 0, 0, 0, st);
+  if (rc) return rc;
   // logstd-variable entries = fixed-order column sums of the per-row terms (damp 0: the x operand is only a finite filler)
   LAUNCH(x, k_fvp_finish, dim3(cdiv(x->L.na, 256), n), 256, 0, st, k, f, (const float*)k.T.actor, 0.f, grad_out);
   if (want_norm) LAUNCH(x, k_grad_clip, dim3(n), 256, 0, st, k, grad_out, max_grad_norm, stats_out);
@@ -1450,17 +1476,16 @@ extern "C" int saceo_onpolicy_expert_grad(saceo_ctx* x, int32_t n_models, int32_
   KCtx kk = actor_view(x, true);            // expert weight forced to 1: the blend is applied by saceo_grad_blend
   kk.nmod = n_models; kk.g_actor = grad_out;
   const KCtx& k = kk; const int n = k.n_agents, E = k.E, Rs = k.Rs;
-  NetD an = actor_net(x);
+  const Pass ap = actor_pass(x, k, E);
   int rc;
   CU(cudaMemsetAsync(grad_out, 0, sizeof(float) * (size_t)n * x->L.na_stride, st));
   LAUNCH(x, k_exp_stage, dim3(cdiv((long long)E * k.S, 256), n), 256, 0, st, k);
-  rc = mlp_forward(x, an, k.Xpi, k.ldXp, (long long)Rs * k.ldXp, 0, E, k.aH1, k.aH2, Rs, k.aOut, k.Ao, (long long)Rs * k.Ao, 0, st, true);
+  rc = mlp_forward(x, ap, k.aOut, k.Ao, (long long)Rs * k.Ao, 0, st);
   if (rc) return rc;
   LAUNCH(x, k_ghead, dim3(cdiv(E, 128), n), 128, 0, st, k, x->cfg.std_mult, clip_actions, 0);
   rc = model_term_phase(x, k, st); if (rc) return rc;
   LAUNCH(x, k_ghead, dim3(cdiv(E, 128), n), 128, 0, st, k, x->cfg.std_mult, clip_actions, 1);
-  rc = mlp_backward(x, an, k.Xpi, k.ldXp, (long long)Rs * k.ldXp, 0, E, k.aH1, k.aH2, Rs, k.daOut, k.Ao, (long long)Rs * k.Ao, 0,
-                    k.Ao, k.daH2, k.daH1, grad_out, x->L.na_stride, 0, nullptr, 0, 0, 0, 0, st);
+  rc = mlp_backward(x, ap, k.daOut, k.Ao, (long long)Rs * k.Ao, 0, k.daH2, k.daH1, grad_out, nullptr, 0, 0, 0, st);
   if (rc) return rc;
   if (!k.per_state_std) LAUNCH(x, k_lsv_reduce, dim3(n), 32 * cdiv(k.A, 32), 0, st, k, E);
   if (stats_out) LAUNCH(x, k_exp_stats, dim3(cdiv(n, 128)), 128, 0, st, k, stats_out);
@@ -1632,6 +1657,8 @@ extern "C" int saceo_policy_act(const saceo_policy_config* cfg, const float* par
 extern "C" int saceo_test_set_tc_debug(void* dbg) { g_tc_dbg = (unsigned long long*)dbg; return 0; }
 // test-only: 8 phase stamps per CTA of the tensor-core expert-term kernel
 extern "C" int saceo_test_set_mt_debug(void* dbg) { g_mt_dbg = (unsigned long long*)dbg; return 0; }
+// test-only: on != 0 runs the expert term on the fp32 CUDA-core kernel (k_model_term) wherever it is eligible
+extern "C" int saceo_test_set_mt_fp32(int32_t on) { g_mt_fp32 = on != 0; return 0; }
 // test-only: the sel-th warp-specialised fused launch from now on writes 16 phase stamps per CTA into dbg
 extern "C" int saceo_test_set_ws_debug(void* dbg, int32_t sel) { g_ws_dbg = (unsigned long long*)dbg; g_ws_sel = sel; g_ws_count = 0; return 0; }
 

@@ -1208,6 +1208,11 @@ static inline bool mlp_fwd_tc_eligible(int h1, int h2, int nout, int rows, const
   return h1 == FW_H && h2 == FW_H && nout >= 1 && nout <= 64 && rows >= TC_BM && K0 >= 1 &&
          ((reinterpret_cast<uintptr_t>(theta) & 15) == 0) && ((sTa & 3) == 0) && ((sTn & 3) == 0);
 }
+static inline bool mlp_bwd_tc_eligible(int h1, int h2, int kout, int rows, bool want_dxa, int a_cols, const float* theta,
+                                       long long sTa, long long sTn) {
+  return h1 == FW_H && h2 == FW_H && kout >= 1 && kout <= 64 && rows >= TC_BM && (rows % TC_BM == 0 || rows % TC_BM >= 16) &&
+         (!want_dxa || a_cols <= 32) && ((reinterpret_cast<uintptr_t>(theta) & 15) == 0) && ((sTa & 3) == 0) && ((sTn & 3) == 0);
+}
 static inline cudaError_t mlp_fwd_tc_init() {
   static bool done_dev[64] = {};
   int dev_ = 0; cudaGetDevice(&dev_);

@@ -50,11 +50,9 @@ class PopulationSpec:
     tc_variant: int = 0            # tcgen05 tile variant (0: 128x256 1 CTA/SM, 1: 128x128 2 CTAs/SM)
     fuse_forward: bool = True      # fused 3-layer tcgen05 forward (activations resident in TMEM)
     fuse_backward: bool = True     # fused tcgen05 gradient chain dOut -> dH2 -> dH1 -> dXa
-    fuse_model: bool = True        # fused expert-observation term (model forward + MSE + backward to action)
     use_graph: bool = True         # one update = one CUDA-graph replay
     ws_kernels: bool = True        # warp-specialised TMA-fed fused kernels on optimiser-maintained weight planes (round 2)
     fork_actor: bool = True        # critic-independent half of the actor phase on a second stream (needs ws_kernels)
-    model_variant: int = 0         # expert-term kernel: 0 hidden layer on mma.sync tf32 hi/lo (default), 1 column-blocked CUDA-core, 2 round-1 CUDA-core
     device: int = 0
 
     def to_config(self) -> _l.Config:
@@ -86,10 +84,8 @@ class PopulationSpec:
         c.reserved[0] = self.tc_variant
         c.reserved[1] = 0 if self.fuse_forward else 1
         c.reserved[2] = 0 if self.fuse_backward else 1
-        c.reserved[3] = 0 if self.fuse_model else 1
         c.reserved[5] = 0 if self.ws_kernels else 1
         c.reserved[6] = 0 if self.fork_actor else 1
-        c.reserved[7] = int(self.model_variant)
         return c
 
 

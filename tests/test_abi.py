@@ -57,6 +57,10 @@ def test_config_validation_mirrors_reference_errors(lib):
         PopulationSpec(n_agents=1, S=4, A=2, actor_acts=("gelu", "relu")).to_config()
     three = PopulationSpec(n_agents=1, S=4, A=2, num_models=3).to_config()
     assert lib.saceo_query_layout(C.byref(three), C.byref(lay)) == -1
+    for slot in (3, 4, 7):          # switches without a meaning: only 0 is accepted
+        cfg = PopulationSpec(n_agents=1, S=4, A=2).to_config()
+        cfg.reserved[slot] = 1
+        assert lib.saceo_query_layout(C.byref(cfg), C.byref(lay)) == -1
 
 
 def test_create_refuses_without_device(lib):

@@ -1,6 +1,8 @@
 """GPU: engine-level consistency - fused tcgen05 kernels vs the unfused GEMM chain vs the exact fp32 engine,
 the Humanoid-shaped wide-input case, and statistical checks of the in-kernel Philox draws (the reference's
 NumPy streams cannot be reproduced on device, SURVEY.md §4 tier 4)."""
+import contextlib
+
 import numpy as np
 import pytest
 import torch
@@ -15,6 +17,18 @@ pytestmark = pytest.mark.gpu
 TOL = 1e-3
 
 
+@contextlib.contextmanager
+def fp32_expert_term(on=True):
+    """Populations updated inside the block run the expert term on the fp32 CUDA-core kernel (k_model_term) where the
+    tensor-core kernel (k_model_term_mma) would run by default."""
+    lib = L.load()
+    L.check(lib.saceo_test_set_mt_fp32(int(on)))
+    try:
+        yield
+    finally:
+        L.check(lib.saceo_test_set_mt_fp32(0))
+
+
 def _run(cfg, **kw):
     pop, probs = build(cfg, n_agents=2, B=256, E=20, N=1500, seed=31, **kw)
     pop.update(1, num_timesteps=0, use_device_rng=False)
@@ -26,11 +40,11 @@ def _run(cfg, **kw):
     return out
 
 
-def test_fused_vs_unfused_vs_fp32_engine():
+def test_fused_vs_unfused_mlp_vs_fp32_engine():
     cfg = NetCfg(S=27, A=8)       # Ant-shaped, 2x256 nets, 2x512 models
     ref = _run(cfg, gemm_mode=L.GEMM_FP32_SIMT)
     fused = _run(cfg, gemm_mode=L.GEMM_TCGEN05_BF16X3)
-    plain = _run(cfg, gemm_mode=L.GEMM_TCGEN05_BF16X3, fuse_forward=False, fuse_backward=False, fuse_model=False)
+    plain = _run(cfg, gemm_mode=L.GEMM_TCGEN05_BF16X3, fuse_forward=False, fuse_backward=False)
     for name, got in (("fused", fused), ("unfused", plain)):
         # north_star tolerance (1e-3); the actor gradient runs through min(Q1,Q2) and tanh, which amplify the ~1e-5
         # per-GEMM error of the bf16x3 engine
@@ -80,23 +94,24 @@ def test_device_rng_statistics():
 
 @pytest.mark.parametrize("seed", [5, 31, 77])
 @pytest.mark.parametrize("fuse", [True, False])
-def test_relu_mask_stability_tcgen05(seed, fuse):
+def test_relu_mask_stability_operand_planes(seed, fuse):
     """ReLU nets on the tensor-core engine: forward passes use fp16 hi/lo planes so that activation masks and the
     min(Q1,Q2) selection agree with the fp32 oracle; with bf16 planes these seeds gave g_actor errors of 6e-3.
     Gradients are held to 2e-4 here (5x tighter than the 1e-3 bar) to catch a regression of the plane format."""
     cfg = NetCfg(S=27, A=8)
-    # seed 31 holds an exact tie in a frozen MODEL (test_model_relu_tie_is_confined below): the fp32 CUDA-core expert
+    # seed 31 holds an exact tie in a frozen MODEL (test_model_relu_tie_confined_to_one_row below): the fp32 CUDA-core expert
     # term keeps this test about the actor / critic operand planes
-    pop, probs = build(cfg, n_agents=2, B=256, E=20, N=2000, seed=seed, gemm_mode=L.GEMM_TCGEN05_BF16X3,
-                       fuse_forward=fuse, fuse_backward=fuse, model_variant=2 if seed == 31 else 0)
-    w = compare_update(pop, cfg, probs)
+    with fp32_expert_term(seed == 31):
+        pop, probs = build(cfg, n_agents=2, B=256, E=20, N=2000, seed=seed, gemm_mode=L.GEMM_TCGEN05_BF16X3,
+                           fuse_forward=fuse, fuse_backward=fuse)
+        w = compare_update(pop, cfg, probs)
     pop.close()
     for k in ("g_q1", "g_q2", "g_actor", "y", "L_pi"):
         assert w[k] < 2e-4, (k, w[k])
     assert max(w.values()) < TOL, w
 
 
-def test_model_relu_tie_is_confined():
+def test_model_relu_tie_confined_to_one_row():
     """Seed 31 of the test above: one hidden pre-activation of one 2x512 ReLU model sits at 4.6e-8 of the magnitude of
     its summed terms - below fp32 epsilon, so the summation order alone decides the ReLU branch (the oracle, the fp32
     CUDA-core kernel and the tensor-core kernel are three orders).  The tensor-core expert term may take the other
@@ -105,16 +120,17 @@ def test_model_relu_tie_is_confined():
     cfg = NetCfg(S=27, A=8)
     n, E, SA, H = 2, 20, 35, 512
     outs = {}
-    for variant in (0, 2):
-        pop, probs = build(cfg, n_agents=n, B=256, E=E, N=2000, seed=31, gemm_mode=L.GEMM_TCGEN05_BF16X3, model_variant=variant)
-        pop.update(1, num_timesteps=0, use_device_rng=False)
-        torch.cuda.synchronize()
-        outs[variant] = pop.debug("mdXa").cpu().numpy().reshape(n, 2, E, cfg.A)[:, :, :E // 2].copy()
-        if variant == 0:
+    for kernel in ("mma", "fp32"):
+        with fp32_expert_term(kernel == "fp32"):
+            pop, probs = build(cfg, n_agents=n, B=256, E=E, N=2000, seed=31, gemm_mode=L.GEMM_TCGEN05_BF16X3)
+            pop.update(1, num_timesteps=0, use_device_rng=False)
+            torch.cuda.synchronize()
+        outs[kernel] = pop.debug("mdXa").cpu().numpy().reshape(n, 2, E, cfg.A)[:, :, :E // 2].copy()
+        if kernel == "mma":
             Xm = pop.debug("Xm").cpu().numpy().reshape(n, 2, E, SA)[:, :, :E // 2].astype(np.float64)
             th = pop.t["model"].cpu().numpy().astype(np.float64).reshape(n, 2, -1)
         pop.close()
-    d = np.abs(outs[0] - outs[2]).max(-1) / (np.abs(outs[2]).max(-1) + 1e-30)       # [agent, model, row]
+    d = np.abs(outs["mma"] - outs["fp32"]).max(-1) / (np.abs(outs["fp32"]).max(-1) + 1e-30)       # [agent, model, row]
     bad = np.argwhere(d > 1e-5)
     assert len(bad) <= 1, d
     for a, m, r in bad:
@@ -186,25 +202,25 @@ def test_profile_step_reports_every_launch():
 @pytest.mark.parametrize("hidden,acts,E,nm", [((512, 512), ("relu", "relu"), 20, 2), ((512, 512), ("tanh", "tanh"), 20, 2),
                                                ((64, 96), ("relu", "tanh"), 8, 2), ((96, 32), ("tanh", "relu"), 16, 1),
                                                ((256, 256), ("relu", "relu"), 32, 2), ((64, 64), ("relu", "relu"), 6, 2)])
-def test_model_term_tensor_core_hidden_layer(hidden, acts, E, nm):
-    """Expert term, hidden layer on mma.sync tf32 hi/lo x3 (model_variant 0, the default) against the fp32 CUDA-core
-    kernels (variants 1, 2): the gradient w.r.t. the expert actions (mdXa) and the per-model MSE agree to fp32 rounding,
-    and the whole update agrees with the oracle (compare_update)."""
+def test_model_term_mma_matches_fp32_kernel(hidden, acts, E, nm):
+    """Expert term, hidden layer on mma.sync tf32 hi/lo x3 (the default) against the fp32 CUDA-core kernel: the gradient
+    w.r.t. the expert actions (mdXa) and the per-model MSE agree to fp32 rounding, and the whole update agrees with the
+    oracle (compare_update)."""
     cfg = NetCfg(S=11, A=3, actor_hidden=(32, 32), critic_hidden=(32, 32), model_hidden=hidden, model_acts=acts, num_models=nm,
                  delta_clip_pred=3.0)
     outs = {}
-    for variant in (0, 1, 2):
-        pop, probs = build(cfg, n_agents=3, B=64, E=E, N=600, seed=13, model_variant=variant)
-        if variant == 0:
-            w = compare_update(pop, cfg, probs)
-            assert max(v for k, v in w.items() if not k.startswith("oracle32")) < TOL, w
-        else:
-            pop.update(1, num_timesteps=0, use_device_rng=False)
-        torch.cuda.synchronize()
-        outs[variant] = (pop.debug("mdXa").cpu().numpy().copy(), pop.debug("mse_part").cpu().numpy().copy(),
-                         pop.t["actor"].cpu().numpy().copy())
+    for kernel in ("mma", "fp32"):
+        with fp32_expert_term(kernel == "fp32"):
+            pop, probs = build(cfg, n_agents=3, B=64, E=E, N=600, seed=13)
+            if kernel == "mma":
+                w = compare_update(pop, cfg, probs)
+                assert max(v for k, v in w.items() if not k.startswith("oracle32")) < TOL, w
+            else:
+                pop.update(1, num_timesteps=0, use_device_rng=False)
+            torch.cuda.synchronize()
+        outs[kernel] = (pop.debug("mdXa").cpu().numpy().copy(), pop.debug("mse_part").cpu().numpy().copy(),
+                        pop.t["actor"].cpu().numpy().copy())
         pop.close()
-    for variant in (1, 2):
-        assert rel(outs[0][0], outs[variant][0]) < 1e-5, (variant, rel(outs[0][0], outs[variant][0]), rel(outs[1][0], outs[2][0]))
-        assert np.allclose(outs[0][1], outs[variant][1], rtol=1e-5, atol=1e-9)
-        assert rel(outs[0][2], outs[variant][2]) < 1e-5
+    assert rel(outs["mma"][0], outs["fp32"][0]) < 1e-5, rel(outs["mma"][0], outs["fp32"][0])
+    assert np.allclose(outs["mma"][1], outs["fp32"][1], rtol=1e-5, atol=1e-9)
+    assert rel(outs["mma"][2], outs["fp32"][2]) < 1e-5

@@ -58,6 +58,9 @@ RAGGED = {
                                               critic_acts=("tanh", "tanh")), 129, 20),
     "B144_plain_sac": (NetCfg(S=27, A=8, num_models=0, actor_acts=("elu", "elu"), critic_acts=("elu", "elu")), 144, 0),
     "B512_E32_A1": (NetCfg(S=3, A=1, actor_acts=("tanh", "tanh"), critic_acts=("tanh", "tanh"), model_hidden=(256, 256)), 512, 32),
+    # 40 expert rows per model, more than the fused expert-term kernels take: the term runs as the GEMM chain
+    "B160_E80_expert_term_gemms": (NetCfg(S=11, A=3, actor_acts=("tanh", "tanh"), critic_acts=("tanh", "tanh"),
+                                          model_hidden=(64, 64), model_acts=("tanh", "tanh")), 160, 80),
 }
 
 

@@ -7,7 +7,7 @@ accumulator groups, and W2 rows that straddle the float4 groups of k_adam when 2
   * after several graph-replayed updates, the tensor-core actor forward agrees with an exact-fp32 population holding
     the same weights - a stale or misplaced W2 plane element shows up here;
   * one update's actor gradients (dOut W2^T on the tensor core) agree with the fp32 oracle to 2e-4, the bound
-    test_relu_mask_stability_tcgen05 uses.
+    test_relu_mask_stability_operand_planes uses.
 """
 import pytest
 import torch

@@ -9,7 +9,7 @@ for acts in (("tanh", "tanh"), ("relu", "relu")):
     worst = {}
     for seed in (5, 31, 77):
         pop, probs = build(cfg, n_agents=2, B=256, E=20, N=2000, seed=seed, gemm_mode=L.GEMM_TCGEN05_BF16X3,
-                           fuse_forward=fuse, fuse_backward=fuse, fuse_model=fuse)
+                           fuse_forward=fuse, fuse_backward=fuse)
         w = compare_update(pop, cfg, probs)
         for k, v in w.items():
             worst[k] = max(worst.get(k, 0), v)
