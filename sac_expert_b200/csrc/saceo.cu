@@ -44,16 +44,22 @@ struct NetD {            // one (population of) MLP(s) in the flat Keras layout
   const float* theta; long long sa, sn; int nnet;
   int in, h1, h2, out, act0, act1;
   const uint8_t* planes = nullptr; long long pa = 0, pn = 0;   // fp16 hi/lo weight-plane images (mlp_ws.cuh), bytes per agent / net
-  long long oW0() const { return 0; }
-  long long ob0() const { return (long long)in * h1; }
-  long long oW1() const { return ob0() + h1; }
-  long long ob1() const { return oW1() + (long long)h1 * h2; }
-  long long oW2() const { return ob1() + h2; }
-  long long ob2() const { return oW2() + (long long)h2 * out; }
+  // layer l in {0, 1, 2}: fan-in, width, activation, and the offsets of its weight [K x N] and bias [N] in theta
+  int K(int l) const { return l == 0 ? in : l == 1 ? h1 : h2; }
+  int N(int l) const { return l == 0 ? h1 : l == 1 ? h2 : out; }
+  int act(int l) const { return l == 0 ? act0 : l == 1 ? act1 : ACT_LINEAR; }
+  long long oW(int l) const { return l == 0 ? 0 : ob(l - 1) + N(l - 1); }
+  long long ob(int l) const { return oW(l) + (long long)K(l) * N(l); }
 };
 
 struct saceo_ctx {
   saceo_config cfg;
+  // engine switches, decoded once from cfg.gemm_mode and the cfg.reserved tuning switches (include/saceo.h)
+  bool tc = false;                     // tcgen05 bf16x3 GEMM engine
+  int tc_variant = 0;                  // its tile variant
+  bool fuse_fwd = false, fuse_bwd = false;   // fused 3-layer forward / backward-chain kernels (tcgen05 engine only)
+  bool ws_kernels = false;             // warp-specialised TMA-fed fused kernels and their weight planes (tcgen05 engine only)
+  bool fork = false;                   // side streams: the concurrent actor-phase branch and the weight-gradient fan-out
   saceo_layout L;
   KCtx k;                 // device-visible view (tables + workspace)
   FvpWs f;
@@ -179,6 +185,16 @@ static void fill_layout(const saceo_config* c, saceo_layout* L) {
   L->n_losses = 8;
 }
 
+static void decode_switches(saceo_ctx* x) {
+  const saceo_config& c = x->cfg;
+  x->tc = c.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3;
+  x->tc_variant = c.reserved[0];
+  x->fuse_fwd = x->tc && c.reserved[1] == 0;
+  x->fuse_bwd = x->tc && c.reserved[2] == 0;
+  x->ws_kernels = x->tc && c.reserved[5] == 0;
+  x->fork = c.reserved[6] == 0;
+}
+
 static void carve(saceo_ctx* x, char* base) {
   const saceo_config& c = x->cfg; const saceo_layout& L = x->L;
   KCtx& k = x->k;
@@ -230,7 +246,7 @@ static void carve(saceo_ctx* x, char* base) {
   x->pl_actor = x->pl_q = x->pl_qt = nullptr;
   x->aH1p = x->adH2p = x->cH1p = x->cdH2p = x->adH1p = x->cdH1p = nullptr;
   x->a_img = (long long)(R / 32) * WS_STAGE; x->c_img = (long long)(rup(B, 32) / 32) * WS_STAGE;
-  if (c.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && c.reserved[5] == 0) {
+  if (x->ws_kernels) {
     if (c.actor_hidden[0] == FW_H && c.actor_hidden[1] == FW_H) {
       x->pl_actor = b.get<uint8_t>("pl_actor", n * ws_image_bytes(S, L.Ao));
       x->aH1p = b.get<uint8_t>("aH1p", n * x->a_img); x->adH2p = b.get<uint8_t>("adH2p", n * x->a_img);
@@ -270,6 +286,7 @@ extern "C" int saceo_query_layout(const saceo_config* cfg, saceo_layout* out) {
   if (!out) return fail(SACEO_E_INVALID, "null out");
   fill_layout(cfg, out);
   saceo_ctx tmp; tmp.cfg = *cfg; tmp.L = *out;
+  decode_switches(&tmp);
   carve(&tmp, nullptr);
   out->workspace_bytes = tmp.ws_bytes;
   return 0;
@@ -303,6 +320,7 @@ extern "C" int saceo_create(const saceo_config* cfg, saceo_ctx** out) {
 
 static int create_fill(saceo_ctx* x, const saceo_config* cfg) {
   x->cfg = *cfg;
+  decode_switches(x);
   fill_layout(cfg, &x->L);
   memset(&x->k, 0, sizeof(KCtx)); memset(&x->f, 0, sizeof(FvpWs)); memset(&x->fit, 0, sizeof(FitCtx));
   carve(x, nullptr);
@@ -437,8 +455,8 @@ static void simt_launch(bool TA, bool TB, bool ONES, const GemmP& p, int nagents
 static int gemm(saceo_ctx* x, bool TA, bool TB, bool ONES, const GemmP& p, int nagents, cudaStream_t st) {
   if (p.M <= 0 || p.N <= 0 || p.K <= 0) return 0;
   int row0 = 0;
-  if (x->cfg.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && tc_gemm_eligible(TA, TB, ONES, p)) {
-    if (tc_gemm_launch(TA, TB, ONES, p, nagents, x->cfg.reserved[0], st) < 0) return fail(SACEO_E_CUDA, "tcgen05 gemm launch failed");
+  if (x->tc && tc_gemm_eligible(TA, TB, ONES, p)) {
+    if (tc_gemm_launch(TA, TB, ONES, p, nagents, x->tc_variant, st) < 0) return fail(SACEO_E_CUDA, "tcgen05 gemm launch failed");
     count_launch(x, "k_gemm_tc", st);
     row0 = tc_rows(ONES, p);
     if (row0 >= p.M) return 0;
@@ -475,34 +493,33 @@ struct Pass {
   // the caller guarantees that rows [rows, rowsAllocH) of X, H1, H2, dOut, dH2, dH1 are zero, so the
   // weight-gradient contractions may run over a row count rounded up to the 32-row slabs of the streaming kernel
   bool kpad = false;
+  int hnets = 0;        // nets per agent the activation buffers H1, H2, dH2, dH1 are laid out for (0: n.nnet)
+  int dout_cols = 0;    // columns of dOut that flow back into dH2 (0: n.out)
+  bool fwd_f16 = true;  // forward operands are O(1): the GEMM chain splits them into fp16 planes (tc_gemm.cuh split8), else bf16
+  long long sHa(int w) const { return (long long)(hnets ? hnets : n.nnet) * rowsAllocH * w; }   // agent / net strides of
+  long long sHn(int w) const { return rowsAllocH * w; }                                          // a w-wide activation
+  int kout() const { return dout_cols ? dout_cols : n.out; }
 };
 
-// forward through one population of 3-layer MLPs (nn_utils.py:101-136), rows [row0, rows), unfused: three GEMMs
+// forward through one population of 3-layer MLPs (nn_utils.py:101-136), rows [row0, rows), unfused: one GEMM per layer
 static int mlp_forward_unfused(saceo_ctx* x, const Pass& ps, int row0, float* Out, int ldo, long long sOa, long long sOn,
                                cudaStream_t st) {
   const NetD& n = ps.n;
-  const int na = x->cfg.n_agents;
-  GemmP p{}; p.nnet = n.nnet; p.f16 = 1;     // forward operands are O(1): fp16 planes (tc_gemm.cuh split8)
-  const int M = ps.rows - row0;
-  // layer 0
-  p.A = ps.X + (long long)row0 * ps.ldx; p.lda = ps.ldx; p.sAa = ps.sXa; p.sAn = ps.sXn;
-  p.B = n.theta + n.oW0(); p.ldb = n.h1; p.sBa = n.sa; p.sBn = n.sn;
-  p.bias = n.theta + n.ob0(); p.sba = n.sa; p.sbn = n.sn;
-  p.C = ps.H1 + (long long)row0 * n.h1; p.ldc = n.h1; p.sCa = (long long)n.nnet * ps.rowsAllocH * n.h1; p.sCn = ps.rowsAllocH * n.h1;
-  p.M = M; p.N = n.h1; p.K = n.in; p.epi = EPI_ACT; p.act = n.act0;
-  int rc = gemm(x, false, false, false, p, na, st); if (rc) return rc;
-  // layer 1
-  p.A = p.C; p.lda = n.h1; p.sAa = p.sCa; p.sAn = p.sCn;
-  p.B = n.theta + n.oW1(); p.ldb = n.h2; p.bias = n.theta + n.ob1();
-  p.C = ps.H2 + (long long)row0 * n.h2; p.ldc = n.h2; p.sCa = (long long)n.nnet * ps.rowsAllocH * n.h2; p.sCn = ps.rowsAllocH * n.h2;
-  p.M = M; p.N = n.h2; p.K = n.h1; p.act = n.act1;
-  rc = gemm(x, false, false, false, p, na, st); if (rc) return rc;
-  // layer 2 (linear)
-  p.A = p.C; p.lda = n.h2; p.sAa = p.sCa; p.sAn = p.sCn;
-  p.B = n.theta + n.oW2(); p.ldb = n.out; p.bias = n.theta + n.ob2();
-  p.C = Out + (long long)row0 * ldo; p.ldc = ldo; p.sCa = sOa; p.sCn = sOn;
-  p.M = M; p.N = n.out; p.K = n.h2; p.epi = EPI_NONE; p.act = ACT_LINEAR;
-  return gemm(x, false, false, false, p, na, st);
+  float* const H[2] = {ps.H1, ps.H2};
+  const float* A = ps.X + (long long)row0 * ps.ldx; int lda = ps.ldx; long long sAa = ps.sXa, sAn = ps.sXn;
+  for (int l = 0; l < 3; ++l) {
+    GemmP p{}; p.nnet = n.nnet; p.f16 = ps.fwd_f16;
+    p.A = A; p.lda = lda; p.sAa = sAa; p.sAn = sAn;
+    p.B = n.theta + n.oW(l); p.ldb = n.N(l); p.sBa = n.sa; p.sBn = n.sn;
+    p.bias = n.theta + n.ob(l); p.sba = n.sa; p.sbn = n.sn;
+    if (l < 2) { p.C = H[l]; p.ldc = n.N(l); p.sCa = ps.sHa(n.N(l)); p.sCn = ps.sHn(n.N(l)); }
+    else { p.C = Out; p.ldc = ldo; p.sCa = sOa; p.sCn = sOn; }
+    p.C += (long long)row0 * p.ldc;
+    p.M = ps.rows - row0; p.N = n.N(l); p.K = n.K(l); p.epi = l < 2 ? EPI_ACT : EPI_NONE; p.act = n.act(l);
+    int rc = gemm(x, false, false, false, p, x->cfg.n_agents, st); if (rc) return rc;
+    A = p.C; lda = p.ldc; sAa = p.sCa; sAn = p.sCn;
+  }
+  return 0;
 }
 
 // Forward pass dispatcher: full 128-row tiles of 2x256 nets go through the fused tcgen05 kernel (activations
@@ -512,14 +529,13 @@ static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long l
   const NetD& n = ps.n;
   const int rows = ps.rows;
   int row0 = 0;
-  if (n.planes && x->cfg.reserved[1] == 0 && mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) {
+  if (n.planes && x->fuse_fwd && mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) {
     // warp-specialised kernel on the TMA-fed weight planes: every row (partial tiles are masked)
     FwdW f{};
     f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
     f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
-    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr;
-    f.sHa = (long long)n.nnet * ps.rowsAllocH * n.h1; f.sHn = ps.rowsAllocH * n.h1;
+    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr; f.sHa = ps.sHa(n.h1); f.sHn = ps.sHn(n.h1);
     f.H1p = save_h ? ps.H1p : nullptr; f.sQa = ps.sQa; f.sQn = ps.sQn;
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
     f.rows = rows; f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1;
@@ -528,15 +544,13 @@ static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long l
     count_launch(x, "k_mlp_fwd_ws", st);
     return 0;
   }
-  if (x->cfg.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && x->cfg.reserved[1] == 0 &&
-      mlp_fwd_tc_eligible(n.h1, n.h2, n.out, rows, n.theta, n.sa, n.sn, n.in)) {
+  if (x->fuse_fwd && mlp_fwd_tc_eligible(n.h1, n.h2, n.out, rows, n.theta, n.sa, n.sn, n.in)) {
     int tiles = rows / TC_BM;
     if (rows % TC_BM >= 16) tiles += 1;
     FwdP f{};
     f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
-    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr;
-    f.sHa = (long long)n.nnet * ps.rowsAllocH * n.h1; f.sHn = ps.rowsAllocH * n.h1;
+    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr; f.sHa = ps.sHa(n.h1); f.sHn = ps.sHn(n.h1);
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
     f.rows = tiles * TC_BM < rows ? tiles * TC_BM : rows;
     f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1; f.dbg = g_tc_dbg;
@@ -549,149 +563,135 @@ static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long l
   return mlp_forward_unfused(x, ps, row0, Out, ldo, sOa, sOn, st);
 }
 
+// The fused backward kernels index dbpart as [agent*nnet+net][tile][2][256]: callers with more row tiles than the
+// workspace was sized for (e.g. model fitting with 256-wide models and a large minibatch) take the ones-row bias path.
+static bool dbpart_fits(const saceo_ctx* x, const NetD& n, int rows) {
+  return x->dbpart && (long long)x->cfg.n_agents * n.nnet * cdiv(rows, TC_BM) * 2 * FW_H <= x->dbpart_cap;
+}
+
+// What a fused backward kernel has done before the per-layer loop runs.
+struct BwdFused {
+  bool chain = false;        // dH2, dH1 and dXa
+  bool bias = false;         // db1 and db0, from the kernel's column sums (k_bias_finish)
+  bool dw1_planes = false;   // dH2 left as planes only: dW1 from the plane images (k_dw_planes)
+  bool dw0_planes = false;   // dH1 left as planes only: dW0 from the dH1 plane image (k_dw0_planes)
+};
+
+// Backward through the layers, from layer 2 down to layer 0, of whatever the fused chain left: per layer the weight
+// gradient (grads) and, without the fused chain, the input gradient (dH2, dH1, then the dXa columns).
+static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd, long long sDa, long long sDn,
+                               float* dH2, float* dH1, float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN,
+                               const BwdFused& fz, cudaStream_t st) {
+  const NetD& n = ps.n;
+  const int na = x->cfg.n_agents;
+  const int krows = (ps.kpad && rup(ps.rows, 32) <= ps.rowsAllocH) ? (int)rup(ps.rows, 32) : ps.rows;
+  // activation i (X, H1, H2) and its gradient D[i] (dH1, dH2, dOut for i = 1, 2, 3); H_i and dH_i share ld and strides
+  const float* Act[3] = {ps.X, ps.H1, ps.H2};
+  const float* D[4] = {nullptr, dH1, dH2, dOut};
+  float* const dH[3] = {nullptr, dH1, dH2};
+  const int ld[4] = {ps.ldx, n.h1, n.h2, ldd};
+  const long long sa[4] = {ps.sXa, ps.sHa(n.h1), ps.sHa(n.h2), sDa}, sn[4] = {ps.sXn, ps.sHn(n.h1), ps.sHn(n.h2), sDn};
+  // the three weight-gradient GEMMs are independent of each other: with the fused chain they fan out over three streams
+  // (captured into the graph as parallel branches) - at small populations each is one under-filled, latency-bound wave
+  const bool fan = fz.chain && grads && x->fork && !x->prof && x->s3 && x->s4;
+  cudaStream_t wst[3] = {st, st, st};    // streams of dW0, dW1, dW2
+  if (fan) {
+    CU(cudaEventRecord(x->ev_g, st));
+    CU(cudaStreamWaitEvent(x->s3, x->ev_g, 0)); CU(cudaStreamWaitEvent(x->s4, x->ev_g, 0));
+    wst[2] = x->s3; wst[0] = x->s4;
+  }
+  int rc;
+  for (int l = 2; l >= 0; --l) {
+    if (grads && l == 1 && fz.dw1_planes) {   // dW1 = H1^T . dH2 from the plane images
+      DwP d{};
+      d.Ap = ps.H1p; d.sAa = ps.sQa; d.sAn = ps.sQn; d.Bp = ps.dH2p; d.sBa = ps.sQa; d.sBn = ps.sQn;
+      d.G = grads + n.oW(1); d.sGa = n.sa; d.sGn = n.sn; d.rows = ps.rows; d.nnet = n.nnet;
+      k_dw_planes<<<na * n.nnet, WS_NT, DW_BYTES, wst[1]>>>(d);
+      count_launch(x, "k_dw_planes", wst[1]);
+    } else if (grads && l == 0 && fz.dw0_planes) {   // dW0 = X^T . dH1 from the plane image
+      Dw0P d{};
+      d.X = ps.X; d.ldx = ps.ldx; d.sXa = ps.sXa; d.sXn = ps.sXn; d.Bp = ps.dH1p; d.sBa = ps.sQa; d.sBn = ps.sQn;
+      d.G = grads + n.oW(0); d.sGa = n.sa; d.sGn = n.sn; d.rows = ps.rows; d.in = n.in; d.nnet = n.nnet;
+      k_dw0_planes<<<na * n.nnet, WS_NT, DW0_BYTES, wst[0]>>>(d);
+      count_launch(x, "k_dw0_planes", wst[0]);
+    } else if (grads) {   // [dW_l; db_l] = [Act_l, 1]^T . D_l+1, without the ones row where the fused kernel formed db_l
+      const bool ones = l == 2 || !fz.bias;
+      GemmP p{}; p.nnet = n.nnet;
+      p.A = Act[l]; p.lda = ld[l]; p.sAa = sa[l]; p.sAn = sn[l];
+      p.B = D[l + 1]; p.ldb = ld[l + 1]; p.sBa = sa[l + 1]; p.sBn = sn[l + 1];
+      p.C = grads + n.oW(l); p.ldc = n.N(l); p.sCa = n.sa; p.sCn = n.sn;
+      p.M = ones ? n.K(l) + 1 : n.K(l); p.N = n.N(l); p.K = krows; p.epi = EPI_NONE;
+      rc = gemm(x, true, false, ones, p, na, wst[l]); if (rc) return rc;
+    }
+    if (l == 0 && fan) {
+      CU(cudaEventRecord(x->ev_g3, x->s3)); CU(cudaEventRecord(x->ev_g4, x->s4));
+      CU(cudaStreamWaitEvent(st, x->ev_g3, 0)); CU(cudaStreamWaitEvent(st, x->ev_g4, 0));
+    }
+    if (fz.chain || (l == 0 && !dXa)) continue;
+    // l > 0: dH_l = (D_l+1 . W_l^T) * act_l-1'(H_l);  l = 0: dX[:, S:S+A] = dH1 . W0[S:S+A, :]^T
+    GemmP p{}; p.nnet = n.nnet;
+    p.A = D[l + 1]; p.lda = ld[l + 1]; p.sAa = sa[l + 1]; p.sAn = sn[l + 1];
+    p.B = n.theta + n.oW(l); p.ldb = n.N(l); p.sBa = n.sa; p.sBn = n.sn;
+    if (l > 0) {
+      p.C = dH[l]; p.ldc = ld[l]; p.sCa = sa[l]; p.sCn = sn[l]; p.aux = Act[l];
+      p.N = n.K(l); p.epi = EPI_MUL_DACT; p.act = n.act(l - 1);
+    } else {
+      p.B += (long long)(n.in - A_cols) * n.h1;
+      p.C = dXa; p.ldc = A_cols; p.sCa = sXaA; p.sCn = sXaN; p.N = A_cols; p.epi = EPI_NONE;
+    }
+    p.M = ps.rows; p.K = l == 2 ? ps.kout() : n.N(l);
+    rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
+  }
+  return 0;
+}
+
 // backward through the same MLPs.  grads (nullable): flat [W|b] blocks in the layout of theta, via the ones-row trick.
 // dXa (nullable): gradient w.r.t. the last A_cols (action) columns of the input only (their rows of W0).
+// The fused gradient chain (dH2, dH1, dXa) runs on tensor cores with the tile resident in TMEM where a kernel takes the
+// pass; the per-layer loop does the rest.
 static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd, long long sDa, long long sDn,
                         float* dH2, float* dH1, float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN,
                         cudaStream_t st) {
   const NetD& n = ps.n;
-  const int na = x->cfg.n_agents, rows = ps.rows, S_cols = n.in - A_cols;
-  const float *H1 = ps.H1, *H2 = ps.H2;
-  const long long rowsAllocH = ps.rowsAllocH, sGa = n.sa, sGn = n.sn;
-  const int krows = (ps.kpad && rup(rows, 32) <= rowsAllocH) ? (int)rup(rows, 32) : rows;
-  const long long sH1a = (long long)n.nnet * rowsAllocH * n.h1, sH1n = rowsAllocH * n.h1;
-  const long long sH2a = (long long)n.nnet * rowsAllocH * n.h2, sH2n = rowsAllocH * n.h2;
-  int rc;
-  GemmP p{};
-  // fused gradient chain (dH2, dH1, dXa) on tensor cores with the tile resident in TMEM
-  bool fused = false, bias_done = false, dw1_planes = false, dw0_planes = false;
-  if (n.planes && x->cfg.reserved[2] == 0 &&
-      mlp_bwd_ws_eligible(n.h1, n.h2, n.out, n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn)) {
-    BwdW f{};
-    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = n.out;
-    f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
-    f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
-    f.H1 = H1; f.H2 = H2; f.sHa = sH1a; f.sHn = sH1n;
-    f.dH2 = grads ? dH2 : nullptr; f.dH1 = grads ? dH1 : nullptr;
-    f.dXa = dXa; f.s_cols = S_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
-    f.rows = rows; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1;
-    const int tiles = (rows + TC_BM - 1) / TC_BM;
-    const bool db_fits = (long long)na * n.nnet * tiles * 2 * FW_H <= x->dbpart_cap;
-    f.dbpart = (grads && x->dbpart && db_fits) ? x->dbpart : nullptr;
-    // hidden-to-hidden weight gradient from bf16 plane images (k_dw_planes): dH2 then leaves the kernel as planes only
-    dw1_planes = grads && f.dbpart && ps.H1p;
-    if (dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
-    // first-layer weight gradient from the dH1 plane image (k_dw0_planes): dH1 then leaves the kernel as planes only
-    dw0_planes = dw1_planes && ps.dH1p && dw0_planes_eligible(n.in, rows, ps.ldx, ps.X, ps.sXa, ps.sXn);
-    if (dw0_planes) { f.dH1 = nullptr; f.dH1p = ps.dH1p; }
-    f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
-    if (mlp_bwd_ws_launch(f, na, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused backward launch failed");
-    count_launch(x, "k_mlp_bwd_ws", st);
-    fused = true;
-    if (f.dbpart) {
-      k_bias_finish<<<na * n.nnet, 2 * FW_H, 0, st>>>(f.dbpart, tiles, grads, sGa, sGn, n.nnet, n.ob1(), n.ob0());
-      count_launch(x, "k_bias_finish", st);
-      bias_done = true;
+  const int na = x->cfg.n_agents, rows = ps.rows, tiles = cdiv(rows, TC_BM);
+  BwdFused fz;
+  const bool ws = n.planes && x->fuse_bwd &&
+                  mlp_bwd_ws_eligible(n.h1, n.h2, ps.kout(), n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn);
+  if (ws || (x->fuse_bwd && mlp_bwd_tc_eligible(n.h1, n.h2, n.out, rows, dXa != nullptr, A_cols, n.theta, n.sa, n.sn))) {
+    float* dbpart = grads && dbpart_fits(x, n, rows) ? x->dbpart : nullptr;
+    auto chain = [&](auto& f) {    // the fields BwdW and BwdP share
+      f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = ps.kout();
+      f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
+      f.H1 = ps.H1; f.H2 = ps.H2; f.sHa = ps.sHa(n.h1); f.sHn = ps.sHn(n.h1);
+      f.dH2 = grads ? dH2 : nullptr; f.dH1 = grads ? dH1 : nullptr;
+      f.dXa = dXa; f.s_cols = n.in - A_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
+      f.rows = rows; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1; f.dbpart = dbpart;
+    };
+    if (ws) {
+      BwdW f{}; chain(f);
+      f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
+      // hidden-to-hidden weight gradient from bf16 plane images (k_dw_planes): dH2 then leaves the kernel as planes only
+      fz.dw1_planes = dbpart && ps.H1p;
+      if (fz.dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
+      // first-layer weight gradient from the dH1 plane image (k_dw0_planes): dH1 then leaves the kernel as planes only
+      fz.dw0_planes = fz.dw1_planes && ps.dH1p && dw0_planes_eligible(n.in, rows, ps.ldx, ps.X, ps.sXa, ps.sXn);
+      if (fz.dw0_planes) { f.dH1 = nullptr; f.dH1p = ps.dH1p; }
+      f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
+      if (mlp_bwd_ws_launch(f, na, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused backward launch failed");
+      count_launch(x, "k_mlp_bwd_ws", st);
+    } else {
+      BwdP f{}; chain(f);
+      k_mlp_bwd_tc<<<dim3(tiles, na * n.nnet), FW_NT, FW_BYTES, st>>>(f);
+      count_launch(x, "k_mlp_bwd_tc", st);
     }
-  } else if (x->cfg.gemm_mode == SACEO_GEMM_TCGEN05_BF16X3 && x->cfg.reserved[2] == 0 &&
-             mlp_bwd_tc_eligible(n.h1, n.h2, n.out, rows, dXa != nullptr, A_cols, n.theta, n.sa, n.sn)) {
-    BwdP f{};
-    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = n.out;
-    f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
-    f.H1 = H1; f.H2 = H2; f.sHa = sH1a; f.sHn = sH1n;
-    f.dH2 = grads ? dH2 : nullptr; f.dH1 = grads ? dH1 : nullptr;
-    f.dXa = dXa; f.s_cols = S_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
-    f.rows = rows; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1;
-    dim3 grid((rows + TC_BM - 1) / TC_BM, na * n.nnet);
-    // the kernel indexes dbpart as [agent*nnet+net][tile][2][256]: callers with more row tiles than the workspace was
-    // sized for (e.g. model fitting with 256-wide models and a large minibatch) take the ones-row bias path instead
-    const bool db_fits = (long long)na * n.nnet * grid.x * 2 * FW_H <= x->dbpart_cap;
-    f.dbpart = (grads && x->dbpart && db_fits) ? x->dbpart : nullptr;
-    k_mlp_bwd_tc<<<grid, FW_NT, FW_BYTES, st>>>(f);
-    count_launch(x, "k_mlp_bwd_tc", st);
-    fused = true;
-    if (f.dbpart) {     // bias gradients of the two hidden layers come from the kernel's column sums
-      k_bias_finish<<<na * n.nnet, 2 * FW_H, 0, st>>>(f.dbpart, (int)grid.x, grads, sGa, sGn, n.nnet, n.ob1(), n.ob0());
+    fz.chain = true;
+    if (dbpart) {     // bias gradients of the two hidden layers come from the kernel's column sums
+      k_bias_finish<<<na * n.nnet, 2 * FW_H, 0, st>>>(dbpart, tiles, grads, n.sa, n.sn, n.nnet, n.ob(1), n.ob(0));
       count_launch(x, "k_bias_finish", st);
-      bias_done = true;
+      fz.bias = true;
     }
   }
-  // the three weight-gradient GEMMs are independent of each other: with the fused chain they fan out over three streams
-  // (captured into the graph as parallel branches) - at small populations each is one under-filled, latency-bound wave
-  const bool fan = fused && grads && x->cfg.reserved[6] == 0 && !x->prof && x->s3 && x->s4;
-  cudaStream_t st2 = st, st0 = st;
-  if (fan) {
-    CU(cudaEventRecord(x->ev_g, st));
-    CU(cudaStreamWaitEvent(x->s3, x->ev_g, 0)); CU(cudaStreamWaitEvent(x->s4, x->ev_g, 0));
-    st2 = x->s3; st0 = x->s4;
-  }
-  if (grads) {   // [dW2; db2] = [H2,1]^T . dOut
-    p = GemmP{}; p.nnet = n.nnet;
-    p.A = H2; p.lda = n.h2; p.sAa = sH2a; p.sAn = sH2n;
-    p.B = dOut; p.ldb = ldd; p.sBa = sDa; p.sBn = sDn;
-    p.C = grads + n.oW2(); p.ldc = n.out; p.sCa = sGa; p.sCn = sGn;
-    p.M = n.h2 + 1; p.N = n.out; p.K = krows; p.epi = EPI_NONE;
-    rc = gemm(x, true, false, true, p, na, st2); if (rc) return rc;
-  }
-  if (!fused) {
-  // dH2 = (dOut . W2^T) * act1'(H2)
-  p = GemmP{}; p.nnet = n.nnet;
-  p.A = dOut; p.lda = ldd; p.sAa = sDa; p.sAn = sDn;
-  p.B = n.theta + n.oW2(); p.ldb = n.out; p.sBa = n.sa; p.sBn = n.sn;
-  p.C = dH2; p.ldc = n.h2; p.sCa = sH2a; p.sCn = sH2n; p.aux = H2;
-  p.M = rows; p.N = n.h2; p.K = n.out; p.epi = EPI_MUL_DACT; p.act = n.act1;
-  rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
-  }
-  if (grads && dw1_planes) {   // dW1 = H1^T . dH2 from the plane images (db1 came from the kernel's column sums)
-    DwP d{};
-    d.Ap = ps.H1p; d.sAa = ps.sQa; d.sAn = ps.sQn; d.Bp = ps.dH2p; d.sBa = ps.sQa; d.sBn = ps.sQn;
-    d.G = grads + n.oW1(); d.sGa = sGa; d.sGn = sGn; d.rows = rows; d.nnet = n.nnet;
-    k_dw_planes<<<na * n.nnet, WS_NT, DW_BYTES, st>>>(d);
-    count_launch(x, "k_dw_planes", st);
-  } else if (grads) {   // [dW1; db1] = [H1,1]^T . dH2
-    p = GemmP{}; p.nnet = n.nnet;
-    p.A = H1; p.lda = n.h1; p.sAa = sH1a; p.sAn = sH1n;
-    p.B = dH2; p.ldb = n.h2; p.sBa = sH2a; p.sBn = sH2n;
-    p.C = grads + n.oW1(); p.ldc = n.h2; p.sCa = sGa; p.sCn = sGn;
-    p.M = bias_done ? n.h1 : n.h1 + 1; p.N = n.h2; p.K = krows; p.epi = EPI_NONE;
-    rc = gemm(x, true, false, !bias_done, p, na, st); if (rc) return rc;
-  }
-  if (!fused) {
-  // dH1 = (dH2 . W1^T) * act0'(H1)
-  p = GemmP{}; p.nnet = n.nnet;
-  p.A = dH2; p.lda = n.h2; p.sAa = sH2a; p.sAn = sH2n;
-  p.B = n.theta + n.oW1(); p.ldb = n.h2; p.sBa = n.sa; p.sBn = n.sn;
-  p.C = dH1; p.ldc = n.h1; p.sCa = sH1a; p.sCn = sH1n; p.aux = H1;
-  p.M = rows; p.N = n.h1; p.K = n.h2; p.epi = EPI_MUL_DACT; p.act = n.act0;
-  rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
-  }
-  if (grads && dw0_planes) {   // dW0 = X^T . dH1 from the plane image (db0 came from the kernel's column sums)
-    Dw0P d{};
-    d.X = ps.X; d.ldx = ps.ldx; d.sXa = ps.sXa; d.sXn = ps.sXn; d.Bp = ps.dH1p; d.sBa = ps.sQa; d.sBn = ps.sQn;
-    d.G = grads + n.oW0(); d.sGa = sGa; d.sGn = sGn; d.rows = rows; d.in = n.in; d.nnet = n.nnet;
-    k_dw0_planes<<<na * n.nnet, WS_NT, DW0_BYTES, st0>>>(d);
-    count_launch(x, "k_dw0_planes", st0);
-  } else if (grads) {   // [dW0; db0] = [X,1]^T . dH1
-    p = GemmP{}; p.nnet = n.nnet;
-    p.A = ps.X; p.lda = ps.ldx; p.sAa = ps.sXa; p.sAn = ps.sXn;
-    p.B = dH1; p.ldb = n.h1; p.sBa = sH1a; p.sBn = sH1n;
-    p.C = grads + n.oW0(); p.ldc = n.h1; p.sCa = sGa; p.sCn = sGn;
-    p.M = bias_done ? n.in : n.in + 1; p.N = n.h1; p.K = krows; p.epi = EPI_NONE;
-    rc = gemm(x, true, false, !bias_done, p, na, st0); if (rc) return rc;
-  }
-  if (fan) {
-    CU(cudaEventRecord(x->ev_g3, x->s3)); CU(cudaEventRecord(x->ev_g4, x->s4));
-    CU(cudaStreamWaitEvent(st, x->ev_g3, 0)); CU(cudaStreamWaitEvent(st, x->ev_g4, 0));
-  }
-  if (dXa && !fused) {     // dX[:, S:S+A] = dH1 . W0[S:S+A, :]^T
-    p = GemmP{}; p.nnet = n.nnet;
-    p.A = dH1; p.lda = n.h1; p.sAa = sH1a; p.sAn = sH1n;
-    p.B = n.theta + n.oW0() + (long long)S_cols * n.h1; p.ldb = n.h1; p.sBa = n.sa; p.sBn = n.sn;
-    p.C = dXa; p.ldc = A_cols; p.sCa = sXaA; p.sCn = sXaN;
-    p.M = rows; p.N = A_cols; p.K = n.h1; p.epi = EPI_NONE;
-    rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
-  }
-  return 0;
+  return mlp_backward_layers(x, ps, dOut, ldd, sDa, sDn, dH2, dH1, grads, dXa, A_cols, sXaA, sXaN, fz, st);
 }
 
 static NetD actor_net(const saceo_ctx* x) {
@@ -718,11 +718,9 @@ static NetD model_net(const saceo_ctx* x, int nnet) {
 // k_dw_planes); decided once, so that its forward and backward calls cannot disagree.
 static void plane_path(const saceo_ctx* x, Pass& ps, uint8_t* H1p, uint8_t* dH2p, uint8_t* dH1p, long long sQa, long long sQn) {
   const NetD& n = ps.n;
-  if (!n.planes || x->cfg.reserved[2] != 0 || x->cfg.reserved[1] != 0 || !H1p || !dH2p || !x->dbpart) return;
-  if (!mlp_bwd_ws_eligible(n.h1, n.h2, n.out, n.out, false, 0, n.theta, n.sa, n.sn)) return;
+  if (!n.planes || !x->fuse_bwd || !x->fuse_fwd || !H1p || !dH2p || !dbpart_fits(x, n, ps.rows)) return;
+  if (!mlp_bwd_ws_eligible(n.h1, n.h2, ps.kout(), n.out, false, 0, n.theta, n.sa, n.sn)) return;
   if (!mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) return;
-  const int tiles = (ps.rows + TC_BM - 1) / TC_BM;
-  if ((long long)x->cfg.n_agents * n.nnet * tiles * 2 * FW_H > x->dbpart_cap) return;
   ps.H1p = H1p; ps.dH2p = dH2p; ps.dH1p = dH1p; ps.sQa = sQa; ps.sQn = sQn;
 }
 
@@ -758,6 +756,15 @@ static Pass fvp_pass(const saceo_ctx* x) {
 static Pass model_eval_pass(const saceo_ctx* x, int rows) {
   const KCtx& k = x->k; const int SA = k.S + k.A;
   return Pass{model_net(x, k.nmod), k.Xm, SA, 2LL * k.E * SA, 0, rows, k.E, k.mH1, k.mH2};
+}
+// the k.nmod frozen models of view k, each on its share of the E staged expert rows of Xm (expert-observation term)
+static Pass model_term_pass(const saceo_ctx* x, const KCtx& k) {
+  const int SA = k.S + k.A;
+  Pass ps{model_net(x, k.nmod), k.Xm, SA, 2LL * k.E * SA, (long long)k.E * SA, k.nmod == 2 ? k.E / 2 : k.E, k.E, k.mH1, k.mH2};
+  ps.hnets = 2;         // the model buffers are carved [agent][2][E rows] whatever nmod, as k_model_loss reads mOut / mdOut
+  ps.dout_cols = k.S;   // k_model_loss writes the S state columns of mdOut: the reward output column gets no gradient
+  ps.fwd_f16 = false;   // the expert term's forward keeps the bf16 planes it has always used and been tested with
+  return ps;
 }
 // a model or reward net being fitted on the staged minibatch rows
 static Pass fit_pass(const saceo_ctx* x, const NetD& n, float* H1, float* H2) {
@@ -819,60 +826,22 @@ static KCtx actor_view(const saceo_ctx* x, bool bc = false) {
 // Expert-observation term on the staged model inputs Xm: forward through the frozen model(s), MSE against s'E, backward
 // to the action columns (mdXa, mse_part).  Shared by the SAC-EO / BC actor phase and the on-policy expert gradient.
 static int model_term_phase(saceo_ctx* x, const KCtx& k, cudaStream_t st) {
-  const int n = k.n_agents, S = k.S, A = k.A, SA = S + A, E = k.E;
-  int rc;
-  if (k.nmod > 0 && model_term_eligible(k)) {
+  const int n = k.n_agents, S = k.S, A = k.A, E = k.E, mo = x->L.model_out;
+  if (k.nmod == 0) return 0;
+  if (model_term_eligible(k)) {
     // fused expert-observation term: model forward, MSE, backward to the action columns in one kernel
     if (model_term_launch(k, k.mse_part, st) != cudaSuccess) return fail(SACEO_E_CUDA, "model-term launch failed");
     count_launch(x, "k_model_term", st);
-  } else if (k.nmod > 0) {
-    const int half = k.nmod == 2 ? E / 2 : E;
-    NetD mn = model_net(x, k.nmod);
-    // model buffers are laid out [agent][2][E rows]; net strides are fixed at E rows regardless of nmod
-    // forward
-    {
-      GemmP p{}; p.nnet = mn.nnet;
-      p.A = k.Xm; p.lda = SA; p.sAa = 2LL * E * SA; p.sAn = (long long)E * SA;
-      p.B = mn.theta + mn.oW0(); p.ldb = mn.h1; p.sBa = mn.sa; p.sBn = mn.sn;
-      p.bias = mn.theta + mn.ob0(); p.sba = mn.sa; p.sbn = mn.sn;
-      p.C = k.mH1; p.ldc = mn.h1; p.sCa = 2LL * E * mn.h1; p.sCn = (long long)E * mn.h1;
-      p.M = half; p.N = mn.h1; p.K = SA; p.epi = EPI_ACT; p.act = mn.act0;
-      rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-      p.A = k.mH1; p.lda = mn.h1; p.sAa = p.sCa; p.sAn = p.sCn;
-      p.B = mn.theta + mn.oW1(); p.ldb = mn.h2; p.bias = mn.theta + mn.ob1();
-      p.C = k.mH2; p.ldc = mn.h2; p.sCa = 2LL * E * mn.h2; p.sCn = (long long)E * mn.h2;
-      p.N = mn.h2; p.K = mn.h1; p.act = mn.act1;
-      rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-      p.A = k.mH2; p.lda = mn.h2; p.sAa = p.sCa; p.sAn = p.sCn;
-      p.B = mn.theta + mn.oW2(); p.ldb = mn.out; p.bias = mn.theta + mn.ob2();
-      p.C = k.mOut; p.ldc = mn.out; p.sCa = 2LL * E * mn.out; p.sCn = (long long)E * mn.out;
-      p.N = mn.out; p.K = mn.h2; p.epi = EPI_NONE; p.act = ACT_LINEAR;
-      rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-    }
-    LAUNCH(x, k_model_loss, dim3(n), 256, 0, st, k);
-    // backward to the action columns (weights frozen)
-    {
-      GemmP p{}; p.nnet = mn.nnet;
-      p.A = k.mdOut; p.lda = S; p.sAa = 2LL * E * S; p.sAn = (long long)E * S;
-      p.B = mn.theta + mn.oW2(); p.ldb = mn.out; p.sBa = mn.sa; p.sBn = mn.sn;
-      p.C = k.mdH2; p.ldc = mn.h2; p.sCa = 2LL * E * mn.h2; p.sCn = (long long)E * mn.h2; p.aux = k.mH2;
-      p.M = half; p.N = mn.h2; p.K = S; p.epi = EPI_MUL_DACT; p.act = mn.act1;
-      rc = gemm(x, false, true, false, p, n, st); if (rc) return rc;
-      p = GemmP{}; p.nnet = mn.nnet;
-      p.A = k.mdH2; p.lda = mn.h2; p.sAa = 2LL * E * mn.h2; p.sAn = (long long)E * mn.h2;
-      p.B = mn.theta + mn.oW1(); p.ldb = mn.h2; p.sBa = mn.sa; p.sBn = mn.sn;
-      p.C = k.mdH1; p.ldc = mn.h1; p.sCa = 2LL * E * mn.h1; p.sCn = (long long)E * mn.h1; p.aux = k.mH1;
-      p.M = half; p.N = mn.h1; p.K = mn.h2; p.epi = EPI_MUL_DACT; p.act = mn.act0;
-      rc = gemm(x, false, true, false, p, n, st); if (rc) return rc;
-      p = GemmP{}; p.nnet = mn.nnet;
-      p.A = k.mdH1; p.lda = mn.h1; p.sAa = 2LL * E * mn.h1; p.sAn = (long long)E * mn.h1;
-      p.B = mn.theta + mn.oW0() + (long long)S * mn.h1; p.ldb = mn.h1; p.sBa = mn.sa; p.sBn = mn.sn;
-      p.C = k.mdXa; p.ldc = A; p.sCa = 2LL * E * A; p.sCn = (long long)E * A;
-      p.M = half; p.N = A; p.K = mn.h1; p.epi = EPI_NONE;
-      rc = gemm(x, false, true, false, p, n, st); if (rc) return rc;
-    }
+    return 0;
   }
-  return 0;
+  // the GEMM chain directly, not the mlp_forward / mlp_backward dispatchers: 256-wide models with >= 128 rows per
+  // model would take the fused MLP kernels, which this term has never run on
+  const Pass mp = model_term_pass(x, k);
+  int rc = mlp_forward_unfused(x, mp, 0, k.mOut, mo, 2LL * E * mo, (long long)E * mo, st); if (rc) return rc;
+  LAUNCH(x, k_model_loss, dim3(n), 256, 0, st, k);
+  // backward to the action columns (weights frozen)
+  return mlp_backward_layers(x, mp, k.mdOut, S, 2LL * E * S, (long long)E * S, k.mdH2, k.mdH1, nullptr, k.mdXa, A,
+                             2LL * E * A, (long long)E * A, BwdFused{}, st);
 }
 
 // phase 2a: everything of the actor step that does not depend on the critics
@@ -916,10 +885,11 @@ static int phase_actor_grads(saceo_ctx* x, cudaStream_t st, bool bc = false) {
   return phase_actor_post(x, st, bc);
 }
 
-static int phase_actor_apply(saceo_ctx* x, cudaStream_t st) {
+// one Keras-Adam step of the actor optimiser with gradient g; k_adam also keeps the actor's weight planes current
+static int actor_adam(saceo_ctx* x, const float* g, cudaStream_t st) {
   const KCtx& k = x->k;
   LAUNCH(x, k_adam, dim3(cdiv(cdiv(x->L.na, 4), 256), 1, k.n_agents), 256, 0, st, k.T.actor, k.T.actor_m, k.T.actor_v,
-         k.g_actor, (float*)nullptr, k.lrt, k.T.hyper, x->L.hyper_stride, 2, x->L.na, x->L.na_stride, 1, 0,
+         g, (float*)nullptr, k.lrt, k.T.hyper, x->L.hyper_stride, 2, x->L.na, x->L.na_stride, 1, 0,
          x->pl_actor, (uint8_t*)nullptr, k.S, k.Ao);
   return check_launch();
 }
@@ -945,11 +915,10 @@ static int step_once(saceo_ctx* x, int use_rng, int do_polyak, cudaStream_t st) 
   }
   if ((rc = phase_gather(x, st))) return rc;
   // fork: the critic-independent half of the actor phase on the second stream (captured into the same graph).
-  // reserved[6]: 0 = on, 1 = off (single stream; also used by the per-kernel profile)
+  // Off on a single-stream context and in the per-kernel profile.
   // Only with the warp-specialised fused kernels: the fallback engines write their hidden activations of the
   // TD-target actor pass into the buffers the actor phase saves into.
-  const bool fork = x->cfg.reserved[6] == 0 && !x->prof && x->s2 != nullptr && x->pl_actor != nullptr && x->pl_q != nullptr &&
-                    x->cfg.reserved[1] == 0;
+  const bool fork = x->fork && !x->prof && x->s2 != nullptr && x->pl_actor != nullptr && x->pl_q != nullptr && x->fuse_fwd;
   if (fork) {
     CU(cudaEventRecord(x->ev_fork, st));
     CU(cudaStreamWaitEvent(x->s2, x->ev_fork, 0));
@@ -961,7 +930,7 @@ static int step_once(saceo_ctx* x, int use_rng, int do_polyak, cudaStream_t st) 
   if (fork) { CU(cudaStreamWaitEvent(st, x->ev_join, 0)); }
   else if ((rc = phase_actor_pre(x, st))) return rc;
   if ((rc = phase_actor_post(x, st))) return rc;
-  if ((rc = phase_actor_apply(x, st))) return rc;
+  if ((rc = actor_adam(x, x->k.g_actor, st))) return rc;
   if ((rc = phase_alpha(x, 1, st))) return rc;
   return 0;
 }
@@ -1030,7 +999,7 @@ extern "C" int saceo_bc_update(saceo_ctx* x, int32_t n_steps, int32_t use_device
       LAUNCH(x, k_rng_fill, dim3(cdiv(items > k.B ? items : k.B, 256), k.n_agents), 256, 0, st, k, 1);
     }
     int rc = phase_actor_grads(x, st, true); if (rc) return rc;
-    if ((rc = phase_actor_apply(x, st))) return rc;
+    if ((rc = actor_adam(x, x->k.g_actor, st))) return rc;
     LAUNCH(x, k_bc_loss, cdiv(k.n_agents, 128), 128, 0, st, k);
   }
   if (losses_out)
@@ -1147,7 +1116,7 @@ extern "C" int saceo_update_phase(saceo_ctx* x, int32_t phase, int64_t num_times
       return phase_critic_grads(x, st);
     case 1: return phase_critic_apply(x, (num_timesteps % x->cfg.target_update_int) == 0 ? 1 : 0, st);
     case 2: return phase_actor_grads(x, st);
-    case 3: return phase_actor_apply(x, st);
+    case 3: return actor_adam(x, x->k.g_actor, st);
     case 4: return phase_alpha(x, 0, st);
     case 5: LAUNCH(x, k_alpha_apply, dim3(cdiv(k.n_agents, 128)), 128, 0, st, k); return check_launch();
     default: return fail(SACEO_E_INVALID, "phase must be 0..5");
@@ -1367,23 +1336,23 @@ static int fvp_apply(saceo_ctx* x, const float* xin, float damp, float* Fx, cuda
   int rc; GemmP p{};
   // T1 = (X.P0 + c0) * act0'(H1)
   p = GemmP{}; p.nnet = 1; p.A = f.X; p.lda = k.S; p.sAa = (long long)N * k.S;
-  p.B = tn.theta + tn.oW0(); p.ldb = an.h1; p.sBa = an.sa; p.bias = tn.theta + tn.ob0(); p.sba = an.sa;
+  p.B = tn.theta + tn.oW(0); p.ldb = an.h1; p.sBa = an.sa; p.bias = tn.theta + tn.ob(0); p.sba = an.sa;
   p.C = f.T1; p.ldc = an.h1; p.sCa = sH1; p.aux = f.H1; p.M = N; p.N = an.h1; p.K = k.S; p.epi = EPI_MUL_DACT; p.act = an.act0;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
   // Tmp = T1.W1 ;  T2 = (H1.P1 + c1 + Tmp) * act1'(H2)
-  p = GemmP{}; p.nnet = 1; p.A = f.T1; p.lda = an.h1; p.sAa = sH1; p.B = an.theta + an.oW1(); p.ldb = an.h2; p.sBa = an.sa;
+  p = GemmP{}; p.nnet = 1; p.A = f.T1; p.lda = an.h1; p.sAa = sH1; p.B = an.theta + an.oW(1); p.ldb = an.h2; p.sBa = an.sa;
   p.C = f.Tmp; p.ldc = an.h2; p.sCa = sH2; p.M = N; p.N = an.h2; p.K = an.h1; p.epi = EPI_NONE;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  p = GemmP{}; p.nnet = 1; p.A = f.H1; p.lda = an.h1; p.sAa = sH1; p.B = tn.theta + tn.oW1(); p.ldb = an.h2; p.sBa = an.sa;
-  p.bias = tn.theta + tn.ob1(); p.sba = an.sa; p.addend = f.Tmp; p.aux = f.H2;
+  p = GemmP{}; p.nnet = 1; p.A = f.H1; p.lda = an.h1; p.sAa = sH1; p.B = tn.theta + tn.oW(1); p.ldb = an.h2; p.sBa = an.sa;
+  p.bias = tn.theta + tn.ob(1); p.sba = an.sa; p.addend = f.Tmp; p.aux = f.H2;
   p.C = f.T2; p.ldc = an.h2; p.sCa = sH2; p.M = N; p.N = an.h2; p.K = an.h1; p.epi = EPI_MUL_DACT; p.act = an.act1;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
   // Tmp = T2.W2 ; TOut = H2.P2 + c2 + Tmp
-  p = GemmP{}; p.nnet = 1; p.A = f.T2; p.lda = an.h2; p.sAa = sH2; p.B = an.theta + an.oW2(); p.ldb = k.Ao; p.sBa = an.sa;
+  p = GemmP{}; p.nnet = 1; p.A = f.T2; p.lda = an.h2; p.sAa = sH2; p.B = an.theta + an.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
   p.C = f.Tmp; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.h2; p.epi = EPI_NONE;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  p = GemmP{}; p.nnet = 1; p.A = f.H2; p.lda = an.h2; p.sAa = sH2; p.B = tn.theta + tn.oW2(); p.ldb = k.Ao; p.sBa = an.sa;
-  p.bias = tn.theta + tn.ob2(); p.sba = an.sa; p.addend = f.Tmp;
+  p = GemmP{}; p.nnet = 1; p.A = f.H2; p.lda = an.h2; p.sAa = sH2; p.B = tn.theta + tn.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
+  p.bias = tn.theta + tn.ob(2); p.sba = an.sa; p.addend = f.Tmp;
   p.C = f.TOut; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.h2; p.epi = EPI_NONE;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
   // metric: G = M . J x / N   (per row), plus per-row logstd_var contribution
@@ -1500,7 +1469,7 @@ extern "C" int saceo_grad_blend(saceo_ctx* x, const float* neg_pg, const float* 
   cudaStream_t st = (cudaStream_t)stream; const KCtx& k = x->k;
   NetD an = actor_net(x);
   BlendSeg sg{};
-  const long long bnd[8] = {0, an.ob0(), an.oW1(), an.ob1(), an.oW2(), an.ob2(), an.ob2() + an.out, x->L.na};
+  const long long bnd[8] = {0, an.ob(0), an.oW(1), an.ob(1), an.oW(2), an.ob(2), an.ob(2) + an.out, x->L.na};
   sg.nseg = (x->L.na > bnd[6]) ? 7 : 6;           // + the state-independent logstd variable
   for (int i = 0; i < 8; ++i) sg.b[i] = bnd[i];
   LAUNCH(x, k_grad_blend, dim3(k.n_agents), 256, 0, st, k, sg, neg_pg, mse_grad, eps, out, stats_out);
@@ -1516,10 +1485,7 @@ extern "C" int saceo_actor_adam(saceo_ctx* x, const float* grad, void* stream) {
   if (reinterpret_cast<uintptr_t>(grad) & 15) return fail(SACEO_E_INVALID, "grad must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream; const KCtx& k = x->k;
   LAUNCH(x, k_bc_begin, dim3(cdiv(k.n_agents, 128)), 128, 0, st, k, 0);
-  LAUNCH(x, k_adam, dim3(cdiv(cdiv(x->L.na, 4), 256), 1, k.n_agents), 256, 0, st, k.T.actor, k.T.actor_m, k.T.actor_v,
-         grad, (float*)nullptr, k.lrt, k.T.hyper, x->L.hyper_stride, 2, x->L.na, x->L.na_stride, 1, 0,
-         x->pl_actor, (uint8_t*)nullptr, k.S, k.Ao);
-  return check_launch();
+  return actor_adam(x, grad, st);
 }
 
 extern "C" int saceo_trpo_eval(saceo_ctx* x, const float* act, const float* adv, const float* nlp_old, const float* kl_ref,
@@ -1668,8 +1634,8 @@ extern "C" int saceo_test_gemm(int32_t gemm_mode, int32_t batch, int32_t M, int3
   GemmP p{}; p.nnet = 1; p.A = A; p.B = Bm; p.C = C; p.M = M; p.N = N; p.K = K;
   p.lda = transA ? M : K; p.ldb = transB ? K : N; p.ldc = N;
   p.sAa = (long long)M * K; p.sBa = (long long)K * N; p.sCa = (long long)M * N; p.epi = EPI_NONE;
-  saceo_ctx tmp; memset(&tmp.cfg, 0, sizeof(tmp.cfg)); tmp.cfg.gemm_mode = gemm_mode & 0xff; tmp.cfg.reserved[0] = (gemm_mode >> 8) & 0xff; tmp.cfg.n_agents = batch;
-  if ((gemm_mode & 0xff) == SACEO_GEMM_TCGEN05_BF16X3) {
+  saceo_ctx tmp; tmp.tc = (gemm_mode & 0xff) == SACEO_GEMM_TCGEN05_BF16X3; tmp.tc_variant = (gemm_mode >> 8) & 0xff;
+  if (tmp.tc) {
     CU(tc_gemm_init());
     if (!tc_gemm_eligible(transA != 0, transB != 0, false, p))
       return fail(SACEO_E_INVALID, "shape not eligible for the tcgen05 engine");

@@ -573,7 +573,6 @@ static inline cudaError_t tc_gemm_init() {
   e = cudaFuncSetAttribute(k_gemm_tc_stream<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TS_BYTES); if (e) return e;
   e = cudaFuncSetAttribute(k_gemm_tc_stream<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TS_BYTES); if (e) return e;
   e = cudaFuncSetAttribute(k_gemm_tc_stream<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TS_BYTES); if (e) return e;
-  e = cudaFuncSetAttribute(k_gemm_tc_stream<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TS_BYTES); if (e) return e;
   done = true;
   return cudaSuccess;
 }
@@ -614,8 +613,7 @@ static inline int tc_gemm_launch(bool TA, bool TB, bool ONES, const GemmP& p, in
   if (variant != 2 && aligned && !both_kc && (p.K % TS_BK) == 0 && (p.N % TS_BN) == 0) {
     dim3 grid(p.N / TS_BN, mt, nagents * p.nnet);
     const bool akc = (q.a_sk == 1), bkc = (q.b_sk == 1);
-    if (akc && bkc) k_gemm_tc_stream<true, true><<<grid, TS_NT, TS_BYTES, st>>>(q);
-    else if (akc) k_gemm_tc_stream<true, false><<<grid, TS_NT, TS_BYTES, st>>>(q);
+    if (akc) k_gemm_tc_stream<true, false><<<grid, TS_NT, TS_BYTES, st>>>(q);
     else if (bkc) k_gemm_tc_stream<false, true><<<grid, TS_NT, TS_BYTES, st>>>(q);
     else k_gemm_tc_stream<false, false><<<grid, TS_NT, TS_BYTES, st>>>(q);
   } else if (variant == 1) {

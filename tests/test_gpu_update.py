@@ -61,6 +61,14 @@ RAGGED = {
     # 40 expert rows per model, more than the fused expert-term kernels take: the term runs as the GEMM chain
     "B160_E80_expert_term_gemms": (NetCfg(S=11, A=3, actor_acts=("tanh", "tanh"), critic_acts=("tanh", "tanh"),
                                           model_hidden=(64, 64), model_acts=("tanh", "tanh")), 160, 80),
+    # the same with one model: its activations keep the two-model row stride of the model buffers
+    "B160_E40_one_model_expert_term_gemms": (NetCfg(S=11, A=3, num_models=1, actor_acts=("tanh", "tanh"),
+                                                    critic_acts=("tanh", "tanh"), model_hidden=(64, 64),
+                                                    model_acts=("tanh", "tanh")), 160, 40),
+    # 512-wide models: the chain's hidden-layer GEMMs run on the tensor cores (S = 17, A = 6: at S = 11, A = 3 one agent's
+    # policy loss cancels to 2e-5 against terms of about 7, too close to zero for a relative tolerance)
+    "B160_E80_expert_term_gemms_512": (NetCfg(S=17, A=6, actor_acts=("tanh", "tanh"), critic_acts=("tanh", "tanh"),
+                                              model_acts=("tanh", "tanh")), 160, 80),
 }
 
 
