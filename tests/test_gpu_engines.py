@@ -1,8 +1,6 @@
 """GPU: engine-level consistency - fused tcgen05 kernels vs the unfused GEMM chain vs the exact fp32 engine,
 the Humanoid-shaped wide-input case, and statistical checks of the in-kernel Philox draws (the reference's
 NumPy streams cannot be reproduced on device, SURVEY.md §4 tier 4)."""
-import contextlib
-
 import numpy as np
 import pytest
 import torch
@@ -11,22 +9,10 @@ from oracle.sac_eo_oracle import NetCfg
 from sac_expert_b200 import lib as L
 from sac_expert_b200.population import Population, PopulationSpec
 from sac_expert_b200.synth import fill_synthetic
-from tests.helpers import build, compare_update, rel
+from tests.helpers import build, compare_update, fp32_expert_term, rel
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-3
-
-
-@contextlib.contextmanager
-def fp32_expert_term(on=True):
-    """Populations updated inside the block run the expert term on the fp32 CUDA-core kernel (k_model_term) where the
-    tensor-core kernel (k_model_term_mma) would run by default."""
-    lib = L.load()
-    L.check(lib.saceo_test_set_mt_fp32(int(on)))
-    try:
-        yield
-    finally:
-        L.check(lib.saceo_test_set_mt_fp32(0))
 
 
 def _run(cfg, **kw):
