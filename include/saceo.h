@@ -28,6 +28,8 @@
  * sac_eo/common/nn_utils.py:86-138,162-182; actor: sac_eo/actors/continuous_actors.py:201-209):
  *     [ W0 (in x h1) | b0 (h1) | W1 (h1 x h2) | b1 (h2) | W2 (h2 x out) | b2 (out) | logstd (A)* ]
  *     (*) only for a state-independent-std actor.  W is [in, out], y = x @ W + b.
+ * Actors, critics and reward networks have two hidden layers.  A dynamics model has model_layers of them (1..8):
+ *     [ W0 (in x h1) | b0 (h1) | ... | W_L (h_L x out) | b_L (out) ],  L = model_layers.
  */
 #ifndef SACEO_H_
 #define SACEO_H_
@@ -38,7 +40,10 @@
 extern "C" {
 #endif
 
-#define SACEO_ABI_VERSION 1
+#define SACEO_ABI_VERSION 2
+
+/* Most hidden layers of a dynamics model (saceo_config.model_layers) and of an acted policy (saceo_policy_config). */
+#define SACEO_POLICY_MAX_HIDDEN 8
 
 enum {
   SACEO_OK = 0,
@@ -68,8 +73,11 @@ typedef struct saceo_config {
   int32_t device;             /* CUDA device ordinal */
   int32_t n_agents;
   int32_t S, A;               /* observation / action dims */
-  int32_t actor_hidden[2], critic_hidden[2], model_hidden[2];
-  int32_t actor_act[2], critic_act[2], model_act[2];   /* SACEO_ACT_* per hidden layer */
+  int32_t actor_hidden[2], critic_hidden[2];
+  int32_t actor_act[2], critic_act[2];                 /* SACEO_ACT_* per hidden layer */
+  int32_t model_layers;                                /* hidden layers of every dynamics model, 1..SACEO_POLICY_MAX_HIDDEN */
+  int32_t model_hidden[SACEO_POLICY_MAX_HIDDEN];       /* their widths (>= 1); entries from model_layers on are ignored */
+  int32_t model_act[SACEO_POLICY_MAX_HIDDEN];          /* their SACEO_ACT_* activations */
   int32_t per_state_std;      /* actor outputs 2A (mean, logstd) instead of A */
   int32_t separate_reward_nn; /* model outputs S instead of S+1 */
   int32_t num_models;         /* 0 = plain SAC (SAC.py), 1 / 2 = SAC-EO branches (SAC_expert.py:271,299) */
@@ -92,7 +100,7 @@ typedef struct saceo_config {
 
 /* Strides/offsets (in 4-byte words unless stated) derived from a config. */
 typedef struct saceo_layout {
-  int64_t na, nc, nm;                 /* parameter counts actor / one critic / one model */
+  int64_t na, nc, nm;                 /* parameter counts actor / one critic / one model (sum over its layers of K*N + N) */
   int64_t na_stride, nc_stride, nm_stride;   /* padded per-agent (per-net) strides */
   int32_t Ao, model_out;
   /* device replay row (AoS, 16-byte aligned): [ s(S) | a(A) | sp(S) | r | pad | d (f64, 2 words) | pad ] */
@@ -346,7 +354,6 @@ int saceo_actor_step(saceo_ctx *ctx, const float *theta_ref, const float *dir, c
  * that expert with --expert_file (train.py:65-83); it is a GaussianActor (actors/continuous_actors.py:9-234) or a
  * SquashedGaussianActor (:237-415) of any depth.  These entry points act for a set of n_policies independent policies
  * in one launch, in exact fp32 on CUDA cores, without a context and without the two-hidden-layer training engine. */
-#define SACEO_POLICY_MAX_HIDDEN 8
 typedef struct saceo_policy_config {
   int32_t abi_version, device, n_policies, S, A;
   int32_t n_hidden, hidden[SACEO_POLICY_MAX_HIDDEN], act[SACEO_POLICY_MAX_HIDDEN];   /* widths 1..1024, SACEO_ACT_* */

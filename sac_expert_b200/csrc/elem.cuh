@@ -19,6 +19,7 @@ struct KCtx {
   int Rs;   // row stride of the per-agent [R rows] actor buffers (R rounded up to 32; the pad rows stay zero)
   int ah1, ah2, ch1, ch2, mh1, mh2;
   int aact0, aact1, cact0, cact1, mact0, mact1;
+  int mnh;           // hidden layers of the models; mh1 / mh2 / mact0 / mact1 describe them only when mnh == 2
   float delta_clip;
   int cap;
   saceo_layout L;
@@ -30,7 +31,7 @@ struct KCtx {
   float *Xc, *cH1, *cH2, *cQ, *cdQ, *cdH2, *cdH1, *cdXa;
   float *Xc2;        // live-critic input [N_s(s) | N_a(a)] (Xc holds the target-critic input [N_s(sp) | N_a(a')])
   float *Xc3;        // actor-phase critic input [N_s(s) | N_a(pi(s))]: state columns written by the gather, action columns by the head
-  float *Xm, *mH1, *mH2, *mOut, *mdOut, *mdH2, *mdH1, *mdXa;
+  float *Xm, *mOut, *mdOut, *mdXa;
   float *y, *nlp;
   float *g_q, *g_actor;
   float *lrt, *losses, *mse_part;

@@ -19,7 +19,8 @@ struct FitCtx {
   float *ls, *ls_m, *ls_v;   // GaussianModel.logstd [n_agents, 2, S] and its Adam slots (NULL: MSEModel loss)
   float *g_ls;               // workspace: gradient of logstd [n_agents, 2, S]
   // workspace, all [n_agents, 2, ...]
-  float *X, *T, *H1, *H2, *Out, *dOut, *dH2, *dH1, *g;
+  float *X, *T, *Out, *dOut, *g;
+  float *H[SACEO_POLICY_MAX_HIDDEN], *dH[SACEO_POLICY_MAX_HIDDEN];   // per hidden layer of the model: activation, gradient
   float *loss_part;      // [n_agents, 2]
   float *gscale;         // [n_agents] gradient scale of clip_by_global_norm (1 when clipping is off)
   float *gnorm;          // [n_agents] global gradient norm (diagnostic)

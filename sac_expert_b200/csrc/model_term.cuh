@@ -224,7 +224,7 @@ static inline int model_term_ms(const KCtx& c) {
 static inline size_t model_term_smem(const KCtx& c, int ms);
 static inline bool model_term_eligible(const KCtx& c) {
   const int half = c.nmod == 2 ? c.E / 2 : c.E;
-  return c.nmod > 0 && half <= 32 && (c.mh1 % 8) == 0 && (c.mh2 % 8) == 0 && ((c.L.nm_stride % 4) == 0) &&
+  return c.nmod > 0 && c.mnh == 2 && half <= 32 && (c.mh1 % 8) == 0 && (c.mh2 % 8) == 0 && ((c.L.nm_stride % 4) == 0) &&
          (((long long)(c.S + c.A) * c.mh1) % 4) == 0 &&
          model_term_smem(c, model_term_ms(c)) <= 200 * 1024;
 }

@@ -40,17 +40,28 @@ static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b)
 // ------------------------------------------------------------------------------------------
 // context
 // ------------------------------------------------------------------------------------------
-struct NetD {            // one (population of) MLP(s) in the flat Keras layout
+constexpr int MAXH = SACEO_POLICY_MAX_HIDDEN;
+
+struct NetD {            // one (population of) MLP(s) in the flat Keras layout: nh hidden layers, then the linear output layer
   const float* theta; long long sa, sn; int nnet;
-  int in, h1, h2, out, act0, act1;
+  int in, out, nh;
+  int hw[MAXH], ha[MAXH];  // width and activation of each hidden layer
   const uint8_t* planes = nullptr; long long pa = 0, pn = 0;   // fp16 hi/lo weight-plane images (mlp_ws.cuh), bytes per agent / net
-  // layer l in {0, 1, 2}: fan-in, width, activation, and the offsets of its weight [K x N] and bias [N] in theta
-  int K(int l) const { return l == 0 ? in : l == 1 ? h1 : h2; }
-  int N(int l) const { return l == 0 ? h1 : l == 1 ? h2 : out; }
-  int act(int l) const { return l == 0 ? act0 : l == 1 ? act1 : ACT_LINEAR; }
+  // layer l in [0, nh]: fan-in, width, activation, and the offsets of its weight [K x N] and bias [N] in theta
+  int K(int l) const { return l == 0 ? in : hw[l - 1]; }
+  int N(int l) const { return l == nh ? out : hw[l]; }
+  int act(int l) const { return l == nh ? ACT_LINEAR : ha[l]; }
   long long oW(int l) const { return l == 0 ? 0 : ob(l - 1) + N(l - 1); }
   long long ob(int l) const { return oW(l) + (long long)K(l) * N(l); }
+  // the fused kernels (mlp_ws.cuh, k_mlp_fwd_tc / k_mlp_bwd_tc, k_bias_finish) take only nets of two hidden layers
+  bool two_hidden() const { return nh == 2; }
 };
+static NetD net_desc(const float* theta, long long sa, long long sn, int nnet, int in, int out, int nh, const int* hw,
+                     const int* ha) {
+  NetD d{theta, sa, sn, nnet, in, out, nh};
+  for (int l = 0; l < nh; ++l) { d.hw[l] = hw[l]; d.ha[l] = ha[l]; }
+  return d;
+}
 
 struct saceo_ctx {
   saceo_config cfg;
@@ -79,6 +90,8 @@ struct saceo_ctx {
   // bf16 hi/lo plane images of h1 / dH2 (actor: Rs rows, critics: B rows per net): operands of k_dw_planes
   uint8_t *aH1p = nullptr, *adH2p = nullptr, *cH1p = nullptr, *cdH2p = nullptr, *adH1p = nullptr, *cdH1p = nullptr;
   long long a_img = 0, c_img = 0;      // bytes per (agent, net) image
+  // model activations of each hidden layer and their gradients, [agent][2][E rows][width] (evaluation, expert term)
+  float *mH[MAXH] = {}, *mdH[MAXH] = {};
   cudaStream_t s2 = nullptr, s3 = nullptr, s4 = nullptr;      // s3 / s4: the three independent weight-gradient GEMMs of a backward pass side by side
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_g = nullptr, ev_g3 = nullptr, ev_g4 = nullptr;
   // saceo_update_host_async: the H2D copies of step t+1 ride a copy stream into one of two device staging sets while step
@@ -123,17 +136,21 @@ static int validate(const saceo_config* c) {
   if (c->abi_version != SACEO_ABI_VERSION) return fail(SACEO_E_INVALID, "abi_version %d != %d", c->abi_version, SACEO_ABI_VERSION);
   if (c->n_agents < 1 || c->n_agents > 32000) return fail(SACEO_E_INVALID, "n_agents out of range");
   if (c->S < 1 || c->A < 1 || c->B < 1) return fail(SACEO_E_INVALID, "S, A, B must be positive");
+  if (c->model_layers < 1 || c->model_layers > MAXH)
+    return fail(SACEO_E_INVALID, "model_layers must be in [1, %d] (got %d)", MAXH, c->model_layers);
   for (int i = 0; i < 2; ++i) {
     if (c->actor_hidden[i] < 1 || c->critic_hidden[i] < 1) return fail(SACEO_E_INVALID, "hidden sizes must be positive");
-    if (c->actor_act[i] < 0 || c->actor_act[i] > 2 || c->critic_act[i] < 0 || c->critic_act[i] > 2 ||
-        c->model_act[i] < 0 || c->model_act[i] > 2)
+    if (c->actor_act[i] < 0 || c->actor_act[i] > 2 || c->critic_act[i] < 0 || c->critic_act[i] > 2)
       return fail(SACEO_E_INVALID, "activations must be tanh, relu or elu");   // nn_utils.py:18
   }
+  for (int i = 0; i < c->model_layers; ++i)
+    if (c->model_act[i] < 0 || c->model_act[i] > 2) return fail(SACEO_E_INVALID, "activations must be tanh, relu or elu");
   if (c->num_models < 0 || c->num_models > 2) return fail(SACEO_E_INVALID, "num_models must be 0, 1 or 2 (only models[0..1] are used, SAC_expert.py:325-326)");
   if (c->num_models > 0) {
     if (c->E < 1) return fail(SACEO_E_INVALID, "E must be positive for SAC-EO");
     if (c->num_models == 2 && (c->E & 1)) return fail(SACEO_E_INVALID, "E must be even with two models (unequal array_split halves cannot be added, SAC_expert.py:329-332)");
-    if (c->model_hidden[0] < 1 || c->model_hidden[1] < 1) return fail(SACEO_E_INVALID, "model hidden sizes must be positive");
+    for (int i = 0; i < c->model_layers; ++i)
+      if (c->model_hidden[i] < 1) return fail(SACEO_E_INVALID, "model hidden sizes must be positive (layer %d: %d)", i, c->model_hidden[i]);
   }
   if (c->target_update_int < 1) return fail(SACEO_E_INVALID, "target_update_int must be >= 1");
   if (c->replay_capacity < 1) return fail(SACEO_E_INVALID, "replay_capacity must be >= 1");
@@ -165,7 +182,12 @@ static void fill_layout(const saceo_config* c, saceo_layout* L) {
     return in * h1 + h1 + h1 * h2 + h2 + h2 * out + out; };
   L->na = cnt(S, c->actor_hidden[0], c->actor_hidden[1], L->Ao) + (c->per_state_std ? 0 : A);
   L->nc = cnt(S + A, c->critic_hidden[0], c->critic_hidden[1], 1);
-  L->nm = c->num_models > 0 ? cnt(S + A, c->model_hidden[0], c->model_hidden[1], L->model_out) : 0;
+  L->nm = 0;
+  for (int l = 0, in = S + A; c->num_models > 0 && l <= c->model_layers; ++l) {
+    const int w = l < c->model_layers ? c->model_hidden[l] : L->model_out;
+    L->nm += (long long)in * w + w;
+    in = w;
+  }
   L->na_stride = rup(L->na + 1, 32);   // last padded word carries g_alpha in the grad buffer
   L->nc_stride = rup(L->nc, 32);
   L->nm_stride = rup(L->nm > 0 ? L->nm : 1, 32);
@@ -224,11 +246,13 @@ static void carve(saceo_ctx* x, char* base) {
   k.cdH2 = b.get<float>("cdH2", n * 2 * B * c.critic_hidden[1]); k.cdH1 = b.get<float>("cdH1", n * 2 * B * c.critic_hidden[0]);
   k.cdXa = b.get<float>("cdXa", n * 2 * B * A);
   const long long e1 = E > 0 ? E : 1;
-  const int mh1 = c.num_models > 0 ? c.model_hidden[0] : 1, mh2 = c.num_models > 0 ? c.model_hidden[1] : 1;
+  const int mnh = c.model_layers;
+  auto mh = [&](int l) -> long long { return c.num_models > 0 ? c.model_hidden[l] : 1; };
+  char nm[24];
   k.Xm = b.get<float>("Xm", n * 2 * e1 * SA);
-  k.mH1 = b.get<float>("mH1", n * 2 * e1 * mh1);   k.mH2 = b.get<float>("mH2", n * 2 * e1 * mh2);
+  for (int l = 0; l < mnh; ++l) { snprintf(nm, sizeof(nm), "mH%d", l + 1); x->mH[l] = b.get<float>(nm, n * 2 * e1 * mh(l)); }
   k.mOut = b.get<float>("mOut", n * 2 * e1 * L.model_out); k.mdOut = b.get<float>("mdOut", n * 2 * e1 * S);
-  k.mdH2 = b.get<float>("mdH2", n * 2 * e1 * mh2); k.mdH1 = b.get<float>("mdH1", n * 2 * e1 * mh1);
+  for (int l = mnh - 1; l >= 0; --l) { snprintf(nm, sizeof(nm), "mdH%d", l + 1); x->mdH[l] = b.get<float>(nm, n * 2 * e1 * mh(l)); }
   k.mdXa = b.get<float>("mdXa", n * 2 * e1 * A);
   k.y = b.get<float>("y", n * B);  k.nlp = b.get<float>("nlp", n * R);
   k.g_q = b.get<float>("g_q", n * 2 * L.nc_stride);
@@ -338,7 +362,7 @@ static int create_fill(saceo_ctx* x, const saceo_config* cfg) {
   k.per_state_std = cfg->per_state_std; k.sep_reward = cfg->separate_reward_nn;
   k.ah1 = cfg->actor_hidden[0]; k.ah2 = cfg->actor_hidden[1];
   k.ch1 = cfg->critic_hidden[0]; k.ch2 = cfg->critic_hidden[1];
-  k.mh1 = cfg->model_hidden[0]; k.mh2 = cfg->model_hidden[1];
+  k.mnh = cfg->model_layers; k.mh1 = cfg->model_hidden[0]; k.mh2 = cfg->model_hidden[1];
   k.aact0 = cfg->actor_act[0]; k.aact1 = cfg->actor_act[1];
   k.cact0 = cfg->critic_act[0]; k.cact1 = cfg->critic_act[1];
   k.mact0 = cfg->model_act[0]; k.mact1 = cfg->model_act[1];
@@ -486,36 +510,36 @@ static int gemm(saceo_ctx* x, bool TA, bool TB, bool ONES, const GemmP& p, int n
 struct Pass {
   NetD n;
   const float* X; int ldx; long long sXa, sXn;        // input rows
-  int rows; long long rowsAllocH;                      // rows of the pass / rows per net allocated in H1, H2
-  float *H1, *H2;                                      // saved activations
+  int rows; long long rowsAllocH;                      // rows of the pass / rows per net allocated in H, dH
+  float* H[MAXH];                                      // saved activation of each hidden layer
+  float* dH[MAXH];                                     // its gradient (backward)
   uint8_t *H1p = nullptr, *dH2p = nullptr, *dH1p = nullptr;   // bf16 hi/lo plane images of h1 / dH2 / dH1
   long long sQa = 0, sQn = 0;                          // their bytes per agent / net
-  // the caller guarantees that rows [rows, rowsAllocH) of X, H1, H2, dOut, dH2, dH1 are zero, so the
+  // the caller guarantees that rows [rows, rowsAllocH) of X, H, dOut, dH are zero, so the
   // weight-gradient contractions may run over a row count rounded up to the 32-row slabs of the streaming kernel
   bool kpad = false;
-  int hnets = 0;        // nets per agent the activation buffers H1, H2, dH2, dH1 are laid out for (0: n.nnet)
-  int dout_cols = 0;    // columns of dOut that flow back into dH2 (0: n.out)
+  int hnets = 0;        // nets per agent the activation buffers H, dH are laid out for (0: n.nnet)
+  int dout_cols = 0;    // columns of dOut that flow back into the last hidden layer's dH (0: n.out)
   bool fwd_f16 = true;  // forward operands are O(1): the GEMM chain splits them into fp16 planes (tc_gemm.cuh split8), else bf16
   long long sHa(int w) const { return (long long)(hnets ? hnets : n.nnet) * rowsAllocH * w; }   // agent / net strides of
   long long sHn(int w) const { return rowsAllocH * w; }                                          // a w-wide activation
   int kout() const { return dout_cols ? dout_cols : n.out; }
 };
 
-// forward through one population of 3-layer MLPs (nn_utils.py:101-136), rows [row0, rows), unfused: one GEMM per layer
+// forward through one population of MLPs (nn_utils.py:101-136), rows [row0, rows), unfused: one GEMM per layer
 static int mlp_forward_unfused(saceo_ctx* x, const Pass& ps, int row0, float* Out, int ldo, long long sOa, long long sOn,
                                cudaStream_t st) {
   const NetD& n = ps.n;
-  float* const H[2] = {ps.H1, ps.H2};
   const float* A = ps.X + (long long)row0 * ps.ldx; int lda = ps.ldx; long long sAa = ps.sXa, sAn = ps.sXn;
-  for (int l = 0; l < 3; ++l) {
+  for (int l = 0; l <= n.nh; ++l) {
     GemmP p{}; p.nnet = n.nnet; p.f16 = ps.fwd_f16;
     p.A = A; p.lda = lda; p.sAa = sAa; p.sAn = sAn;
     p.B = n.theta + n.oW(l); p.ldb = n.N(l); p.sBa = n.sa; p.sBn = n.sn;
     p.bias = n.theta + n.ob(l); p.sba = n.sa; p.sbn = n.sn;
-    if (l < 2) { p.C = H[l]; p.ldc = n.N(l); p.sCa = ps.sHa(n.N(l)); p.sCn = ps.sHn(n.N(l)); }
+    if (l < n.nh) { p.C = ps.H[l]; p.ldc = n.N(l); p.sCa = ps.sHa(n.N(l)); p.sCn = ps.sHn(n.N(l)); }
     else { p.C = Out; p.ldc = ldo; p.sCa = sOa; p.sCn = sOn; }
     p.C += (long long)row0 * p.ldc;
-    p.M = ps.rows - row0; p.N = n.N(l); p.K = n.K(l); p.epi = l < 2 ? EPI_ACT : EPI_NONE; p.act = n.act(l);
+    p.M = ps.rows - row0; p.N = n.N(l); p.K = n.K(l); p.epi = l < n.nh ? EPI_ACT : EPI_NONE; p.act = n.act(l);
     int rc = gemm(x, false, false, false, p, x->cfg.n_agents, st); if (rc) return rc;
     A = p.C; lda = p.ldc; sAa = p.sCa; sAn = p.sCn;
   }
@@ -529,31 +553,31 @@ static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long l
   const NetD& n = ps.n;
   const int rows = ps.rows;
   int row0 = 0;
-  if (n.planes && x->fuse_fwd && mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) {
+  if (n.planes && x->fuse_fwd && n.two_hidden() && mlp_fwd_ws_eligible(n.N(0), n.N(1), n.out, n.in, n.theta, n.sa, n.sn)) {
     // warp-specialised kernel on the TMA-fed weight planes: every row (partial tiles are masked)
     FwdW f{};
     f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
     f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
-    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr; f.sHa = ps.sHa(n.h1); f.sHn = ps.sHn(n.h1);
+    f.H1 = save_h ? ps.H[0] : nullptr; f.H2 = save_h ? ps.H[1] : nullptr; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
     f.H1p = save_h ? ps.H1p : nullptr; f.sQa = ps.sQa; f.sQn = ps.sQn;
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
-    f.rows = rows; f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1;
+    f.rows = rows; f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1);
     f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
     if (mlp_fwd_ws_launch(f, x->cfg.n_agents, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused forward launch failed");
     count_launch(x, "k_mlp_fwd_ws", st);
     return 0;
   }
-  if (x->fuse_fwd && mlp_fwd_tc_eligible(n.h1, n.h2, n.out, rows, n.theta, n.sa, n.sn, n.in)) {
+  if (x->fuse_fwd && n.two_hidden() && mlp_fwd_tc_eligible(n.N(0), n.N(1), n.out, rows, n.theta, n.sa, n.sn, n.in)) {
     int tiles = rows / TC_BM;
     if (rows % TC_BM >= 16) tiles += 1;
     FwdP f{};
     f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
     f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
-    f.H1 = save_h ? ps.H1 : nullptr; f.H2 = save_h ? ps.H2 : nullptr; f.sHa = ps.sHa(n.h1); f.sHn = ps.sHn(n.h1);
+    f.H1 = save_h ? ps.H[0] : nullptr; f.H2 = save_h ? ps.H[1] : nullptr; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
     f.rows = tiles * TC_BM < rows ? tiles * TC_BM : rows;
-    f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1; f.dbg = g_tc_dbg;
+    f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1); f.dbg = g_tc_dbg;
     dim3 grid(tiles, x->cfg.n_agents * n.nnet);
     k_mlp_fwd_tc<<<grid, FW_NT, FW_BYTES, st>>>(f);
     count_launch(x, "k_mlp_fwd_tc", st);
@@ -577,31 +601,36 @@ struct BwdFused {
   bool dw0_planes = false;   // dH1 left as planes only: dW0 from the dH1 plane image (k_dw0_planes)
 };
 
-// Backward through the layers, from layer 2 down to layer 0, of whatever the fused chain left: per layer the weight
-// gradient (grads) and, without the fused chain, the input gradient (dH2, dH1, then the dXa columns).
+// Backward through the layers, from the output layer down to layer 0, of whatever the fused chain left: per layer the
+// weight gradient (grads) and, without the fused chain, the input gradient (the hidden layers' dH, then the dXa columns).
 static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd, long long sDa, long long sDn,
-                               float* dH2, float* dH1, float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN,
-                               const BwdFused& fz, cudaStream_t st) {
+                               float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN, const BwdFused& fz,
+                               cudaStream_t st) {
   const NetD& n = ps.n;
-  const int na = x->cfg.n_agents;
+  const int na = x->cfg.n_agents, nh = n.nh;
   const int krows = (ps.kpad && rup(ps.rows, 32) <= ps.rowsAllocH) ? (int)rup(ps.rows, 32) : ps.rows;
-  // activation i (X, H1, H2) and its gradient D[i] (dH1, dH2, dOut for i = 1, 2, 3); H_i and dH_i share ld and strides
-  const float* Act[3] = {ps.X, ps.H1, ps.H2};
-  const float* D[4] = {nullptr, dH1, dH2, dOut};
-  float* const dH[3] = {nullptr, dH1, dH2};
-  const int ld[4] = {ps.ldx, n.h1, n.h2, ldd};
-  const long long sa[4] = {ps.sXa, ps.sHa(n.h1), ps.sHa(n.h2), sDa}, sn[4] = {ps.sXn, ps.sHn(n.h1), ps.sHn(n.h2), sDn};
+  // activation i (X, then the hidden layers' H) and its gradient D[i] (the hidden layers' dH, then dOut for i = nh + 1);
+  // H_i and dH_i share ld and strides
+  const float* Act[MAXH + 1]; const float* D[MAXH + 2]; float* dH[MAXH + 1];
+  int ld[MAXH + 2]; long long sa[MAXH + 2], sn[MAXH + 2];
+  Act[0] = ps.X; D[0] = nullptr; dH[0] = nullptr; ld[0] = ps.ldx; sa[0] = ps.sXa; sn[0] = ps.sXn;
+  for (int i = 1; i <= nh; ++i) {
+    Act[i] = ps.H[i - 1]; D[i] = dH[i] = ps.dH[i - 1];
+    ld[i] = n.N(i - 1); sa[i] = ps.sHa(ld[i]); sn[i] = ps.sHn(ld[i]);
+  }
+  D[nh + 1] = dOut; ld[nh + 1] = ldd; sa[nh + 1] = sDa; sn[nh + 1] = sDn;
   // the three weight-gradient GEMMs are independent of each other: with the fused chain they fan out over three streams
   // (captured into the graph as parallel branches) - at small populations each is one under-filled, latency-bound wave
   const bool fan = fz.chain && grads && x->fork && !x->prof && x->s3 && x->s4;
-  cudaStream_t wst[3] = {st, st, st};    // streams of dW0, dW1, dW2
-  if (fan) {
+  cudaStream_t wst[MAXH + 1];            // stream of each layer's dW
+  for (int l = 0; l <= nh; ++l) wst[l] = st;
+  if (fan) {                             // fz.chain: two hidden layers
     CU(cudaEventRecord(x->ev_g, st));
     CU(cudaStreamWaitEvent(x->s3, x->ev_g, 0)); CU(cudaStreamWaitEvent(x->s4, x->ev_g, 0));
     wst[2] = x->s3; wst[0] = x->s4;
   }
   int rc;
-  for (int l = 2; l >= 0; --l) {
+  for (int l = nh; l >= 0; --l) {
     if (grads && l == 1 && fz.dw1_planes) {   // dW1 = H1^T . dH2 from the plane images
       DwP d{};
       d.Ap = ps.H1p; d.sAa = ps.sQa; d.sAn = ps.sQn; d.Bp = ps.dH2p; d.sBa = ps.sQa; d.sBn = ps.sQn;
@@ -615,7 +644,7 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
       k_dw0_planes<<<na * n.nnet, WS_NT, DW0_BYTES, wst[0]>>>(d);
       count_launch(x, "k_dw0_planes", wst[0]);
     } else if (grads) {   // [dW_l; db_l] = [Act_l, 1]^T . D_l+1, without the ones row where the fused kernel formed db_l
-      const bool ones = l == 2 || !fz.bias;
+      const bool ones = l == nh || !fz.bias;
       GemmP p{}; p.nnet = n.nnet;
       p.A = Act[l]; p.lda = ld[l]; p.sAa = sa[l]; p.sAn = sn[l];
       p.B = D[l + 1]; p.ldb = ld[l + 1]; p.sBa = sa[l + 1]; p.sBn = sn[l + 1];
@@ -628,7 +657,7 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
       CU(cudaStreamWaitEvent(st, x->ev_g3, 0)); CU(cudaStreamWaitEvent(st, x->ev_g4, 0));
     }
     if (fz.chain || (l == 0 && !dXa)) continue;
-    // l > 0: dH_l = (D_l+1 . W_l^T) * act_l-1'(H_l);  l = 0: dX[:, S:S+A] = dH1 . W0[S:S+A, :]^T
+    // l > 0: dH_l = (D_l+1 . W_l^T) * act_l-1'(H_l);  l = 0: dX[:, S:S+A] = D_1 . W0[S:S+A, :]^T
     GemmP p{}; p.nnet = n.nnet;
     p.A = D[l + 1]; p.lda = ld[l + 1]; p.sAa = sa[l + 1]; p.sAn = sn[l + 1];
     p.B = n.theta + n.oW(l); p.ldb = n.N(l); p.sBa = n.sa; p.sBn = n.sn;
@@ -636,10 +665,10 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
       p.C = dH[l]; p.ldc = ld[l]; p.sCa = sa[l]; p.sCn = sn[l]; p.aux = Act[l];
       p.N = n.K(l); p.epi = EPI_MUL_DACT; p.act = n.act(l - 1);
     } else {
-      p.B += (long long)(n.in - A_cols) * n.h1;
+      p.B += (long long)(n.in - A_cols) * n.N(0);
       p.C = dXa; p.ldc = A_cols; p.sCa = sXaA; p.sCn = sXaN; p.N = A_cols; p.epi = EPI_NONE;
     }
-    p.M = ps.rows; p.K = l == 2 ? ps.kout() : n.N(l);
+    p.M = ps.rows; p.K = l == nh ? ps.kout() : n.N(l);
     rc = gemm(x, false, true, false, p, na, st); if (rc) return rc;
   }
   return 0;
@@ -650,22 +679,22 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
 // The fused gradient chain (dH2, dH1, dXa) runs on tensor cores with the tile resident in TMEM where a kernel takes the
 // pass; the per-layer loop does the rest.
 static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd, long long sDa, long long sDn,
-                        float* dH2, float* dH1, float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN,
-                        cudaStream_t st) {
+                        float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN, cudaStream_t st) {
   const NetD& n = ps.n;
   const int na = x->cfg.n_agents, rows = ps.rows, tiles = cdiv(rows, TC_BM);
   BwdFused fz;
-  const bool ws = n.planes && x->fuse_bwd &&
-                  mlp_bwd_ws_eligible(n.h1, n.h2, ps.kout(), n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn);
-  if (ws || (x->fuse_bwd && mlp_bwd_tc_eligible(n.h1, n.h2, n.out, rows, dXa != nullptr, A_cols, n.theta, n.sa, n.sn))) {
+  const bool ws = n.planes && x->fuse_bwd && n.two_hidden() &&
+                  mlp_bwd_ws_eligible(n.N(0), n.N(1), ps.kout(), n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn);
+  if (ws || (x->fuse_bwd && n.two_hidden() &&
+             mlp_bwd_tc_eligible(n.N(0), n.N(1), n.out, rows, dXa != nullptr, A_cols, n.theta, n.sa, n.sn))) {
     float* dbpart = grads && dbpart_fits(x, n, rows) ? x->dbpart : nullptr;
     auto chain = [&](auto& f) {    // the fields BwdW and BwdP share
       f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = ps.kout();
       f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
-      f.H1 = ps.H1; f.H2 = ps.H2; f.sHa = ps.sHa(n.h1); f.sHn = ps.sHn(n.h1);
-      f.dH2 = grads ? dH2 : nullptr; f.dH1 = grads ? dH1 : nullptr;
+      f.H1 = ps.H[0]; f.H2 = ps.H[1]; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
+      f.dH2 = grads ? ps.dH[1] : nullptr; f.dH1 = grads ? ps.dH[0] : nullptr;
       f.dXa = dXa; f.s_cols = n.in - A_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
-      f.rows = rows; f.nnet = n.nnet; f.act0 = n.act0; f.act1 = n.act1; f.dbpart = dbpart;
+      f.rows = rows; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1); f.dbpart = dbpart;
     };
     if (ws) {
       BwdW f{}; chain(f);
@@ -691,27 +720,27 @@ static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd
       fz.bias = true;
     }
   }
-  return mlp_backward_layers(x, ps, dOut, ldd, sDa, sDn, dH2, dH1, grads, dXa, A_cols, sXaA, sXaN, fz, st);
+  return mlp_backward_layers(x, ps, dOut, ldd, sDa, sDn, grads, dXa, A_cols, sXaA, sXaN, fz, st);
 }
 
 static NetD actor_net(const saceo_ctx* x) {
   const saceo_config& c = x->cfg;
-  NetD d{x->k.T.actor, x->L.na_stride, 0, 1, c.S, c.actor_hidden[0], c.actor_hidden[1], x->L.Ao,
-         c.actor_act[0], c.actor_act[1]};
+  NetD d = net_desc(x->k.T.actor, x->L.na_stride, 0, 1, c.S, x->L.Ao, 2, c.actor_hidden, c.actor_act);
   d.planes = x->pl_actor; d.pa = ws_image_bytes(c.S, x->L.Ao); d.pn = 0;
   return d;
 }
 static NetD critic_net(const saceo_ctx* x, bool target) {
   const saceo_config& c = x->cfg;
-  NetD d{target ? x->k.T.qt : x->k.T.q, 2 * x->L.nc_stride, x->L.nc_stride, 2, c.S + c.A,
-         c.critic_hidden[0], c.critic_hidden[1], 1, c.critic_act[0], c.critic_act[1]};
+  NetD d = net_desc(target ? x->k.T.qt : x->k.T.q, 2 * x->L.nc_stride, x->L.nc_stride, 2, c.S + c.A, 1, 2, c.critic_hidden,
+                    c.critic_act);
   d.planes = target ? x->pl_qt : x->pl_q; d.pn = ws_image_bytes(c.S + c.A, 1); d.pa = 2 * d.pn;
   return d;
 }
-static NetD model_net(const saceo_ctx* x, int nnet) {
+// the dynamics models (model_layers hidden layers) with parameters theta: the bound table, or the one being fitted
+static NetD model_net(const saceo_ctx* x, const float* theta, int nnet) {
   const saceo_config& c = x->cfg;
-  return NetD{x->k.T.model, 2 * x->L.nm_stride, x->L.nm_stride, nnet, c.S + c.A, c.model_hidden[0],
-              c.model_hidden[1], x->L.model_out, c.model_act[0], c.model_act[1]};
+  return net_desc(theta, 2 * x->L.nm_stride, x->L.nm_stride, nnet, c.S + c.A, x->L.model_out, c.model_layers,
+                  c.model_hidden, c.model_act);
 }
 
 // Gives a pass the plane images if mlp_backward(grads) of it takes the plane path (fused chain + column-sum biases +
@@ -719,15 +748,15 @@ static NetD model_net(const saceo_ctx* x, int nnet) {
 static void plane_path(const saceo_ctx* x, Pass& ps, uint8_t* H1p, uint8_t* dH2p, uint8_t* dH1p, long long sQa, long long sQn) {
   const NetD& n = ps.n;
   if (!n.planes || !x->fuse_bwd || !x->fuse_fwd || !H1p || !dH2p || !dbpart_fits(x, n, ps.rows)) return;
-  if (!mlp_bwd_ws_eligible(n.h1, n.h2, ps.kout(), n.out, false, 0, n.theta, n.sa, n.sn)) return;
-  if (!mlp_fwd_ws_eligible(n.h1, n.h2, n.out, n.in, n.theta, n.sa, n.sn)) return;
+  if (!n.two_hidden() || !mlp_bwd_ws_eligible(n.N(0), n.N(1), ps.kout(), n.out, false, 0, n.theta, n.sa, n.sn)) return;
+  if (!mlp_fwd_ws_eligible(n.N(0), n.N(1), n.out, n.in, n.theta, n.sa, n.sn)) return;
   ps.H1p = H1p; ps.dH2p = dH2p; ps.dH1p = dH1p; ps.sQa = sQa; ps.sQn = sQn;
 }
 
 // the actor on the staged observation rows Xpi of view k: <= B rows (TD target, temperature, acting) or the E expert
 // rows of the on-policy expert gradient
 static Pass actor_pass(const saceo_ctx* x, const KCtx& k, int rows) {
-  return Pass{actor_net(x), k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, rows, k.Rs, k.aH1, k.aH2};
+  return Pass{actor_net(x), k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, rows, k.Rs, {k.aH1, k.aH2}, {k.daH1, k.daH2}};
 }
 // the actor update over its R = B + E rows
 static Pass actor_update_pass(const saceo_ctx* x, const KCtx& k) {
@@ -739,7 +768,7 @@ static Pass actor_update_pass(const saceo_ctx* x, const KCtx& k) {
 // twin critics (or their targets) on the first `rows` of B critic input rows X (Xc, Xc2 or Xc3)
 static Pass critic_pass(const saceo_ctx* x, bool target, const float* X, int rows) {
   const KCtx& k = x->k;
-  return Pass{critic_net(x, target), X, k.ldXc, (long long)k.B * k.ldXc, 0, rows, k.B, k.cH1, k.cH2};
+  return Pass{critic_net(x, target), X, k.ldXc, (long long)k.B * k.ldXc, 0, rows, k.B, {k.cH1, k.cH2}, {k.cdH1, k.cdH2}};
 }
 // the critic update over the B minibatch rows
 static Pass critic_update_pass(const saceo_ctx* x) {
@@ -750,26 +779,34 @@ static Pass critic_update_pass(const saceo_ctx* x) {
 // the actor on the fvp_rows states (Fisher-vector product, CG, TRPO / PPO surrogate)
 static Pass fvp_pass(const saceo_ctx* x) {
   const KCtx& k = x->k; const FvpWs& f = x->f;
-  return Pass{actor_net(x), f.X, k.S, (long long)f.N * k.S, 0, f.N, f.N, f.H1, f.H2};
+  return Pass{actor_net(x), f.X, k.S, (long long)f.N * k.S, 0, f.N, f.N, {f.H1, f.H2}, {f.dH1, f.dH2}};
+}
+// a pass of the models over the staged rows X with the per-layer activation buffers H, dH
+static Pass model_pass(const NetD& n, const float* X, long long sXa, long long sXn, int rows, long long rowsAllocH,
+                       float* const* H, float* const* dH) {
+  Pass ps{n, X, n.in, sXa, sXn, rows, rowsAllocH, {}, {}};
+  for (int l = 0; l < n.nh; ++l) { ps.H[l] = H[l]; ps.dH[l] = dH[l]; }
+  return ps;
 }
 // the models on the first `rows` of the E staged rows of Xm; every model reads net 0's block (zero net stride)
 static Pass model_eval_pass(const saceo_ctx* x, int rows) {
   const KCtx& k = x->k; const int SA = k.S + k.A;
-  return Pass{model_net(x, k.nmod), k.Xm, SA, 2LL * k.E * SA, 0, rows, k.E, k.mH1, k.mH2};
+  return model_pass(model_net(x, k.T.model, k.nmod), k.Xm, 2LL * k.E * SA, 0, rows, k.E, x->mH, x->mdH);
 }
 // the k.nmod frozen models of view k, each on its share of the E staged expert rows of Xm (expert-observation term)
 static Pass model_term_pass(const saceo_ctx* x, const KCtx& k) {
   const int SA = k.S + k.A;
-  Pass ps{model_net(x, k.nmod), k.Xm, SA, 2LL * k.E * SA, (long long)k.E * SA, k.nmod == 2 ? k.E / 2 : k.E, k.E, k.mH1, k.mH2};
+  Pass ps = model_pass(model_net(x, k.T.model, k.nmod), k.Xm, 2LL * k.E * SA, (long long)k.E * SA,
+                       k.nmod == 2 ? k.E / 2 : k.E, k.E, x->mH, x->mdH);
   ps.hnets = 2;         // the model buffers are carved [agent][2][E rows] whatever nmod, as k_model_loss reads mOut / mdOut
   ps.dout_cols = k.S;   // k_model_loss writes the S state columns of mdOut: the reward output column gets no gradient
   ps.fwd_f16 = false;   // the expert term's forward keeps the bf16 planes it has always used and been tested with
   return ps;
 }
 // a model or reward net being fitted on the staged minibatch rows
-static Pass fit_pass(const saceo_ctx* x, const NetD& n, float* H1, float* H2) {
+static Pass fit_pass(const saceo_ctx* x, const NetD& n, float* const* H, float* const* dH) {
   const FitCtx& f = x->fit; const int SA = x->cfg.S + x->cfg.A;
-  return Pass{n, f.X, SA, 2LL * f.mbs * SA, (long long)f.mbs * SA, f.mb, f.mbs, H1, H2};
+  return model_pass(n, f.X, 2LL * f.mbs * SA, (long long)f.mbs * SA, f.mb, f.mbs, H, dH);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -801,7 +838,7 @@ static int phase_critic_grads(saceo_ctx* x, cudaStream_t st) {
   const Pass qp = critic_update_pass(x);
   rc = mlp_forward(x, qp, k.cQ, 1, 2LL * B, B, st); if (rc) return rc;
   LAUNCH(x, k_critic_loss, dim3(2, n), 256, 0, st, k);
-  rc = mlp_backward(x, qp, k.cdQ, 1, 2LL * B, B, k.cdH2, k.cdH1, k.g_q, nullptr, 0, 0, 0, st);
+  rc = mlp_backward(x, qp, k.cdQ, 1, 2LL * B, B, k.g_q, nullptr, 0, 0, 0, st);
   if (rc) return rc;
   return check_launch();
 }
@@ -840,7 +877,7 @@ static int model_term_phase(saceo_ctx* x, const KCtx& k, cudaStream_t st) {
   int rc = mlp_forward_unfused(x, mp, 0, k.mOut, mo, 2LL * E * mo, (long long)E * mo, st); if (rc) return rc;
   LAUNCH(x, k_model_loss, dim3(n), 256, 0, st, k);
   // backward to the action columns (weights frozen)
-  return mlp_backward_layers(x, mp, k.mdOut, S, 2LL * E * S, (long long)E * S, k.mdH2, k.mdH1, nullptr, k.mdXa, A,
+  return mlp_backward_layers(x, mp, k.mdOut, S, 2LL * E * S, (long long)E * S, nullptr, k.mdXa, A,
                              2LL * E * A, (long long)E * A, BwdFused{}, st);
 }
 
@@ -868,14 +905,14 @@ static int phase_actor_post(saceo_ctx* x, cudaStream_t st, bool bc = false) {
     const Pass qp = critic_pass(x, false, k.Xc2, B);
     rc = mlp_forward(x, qp, k.cQ, 1, 2LL * B, B, st); if (rc) return rc;
     LAUNCH(x, k_actor_q, dim3(n), 256, 0, st, k);
-    rc = mlp_backward(x, qp, k.cdQ, 1, 2LL * B, B, k.cdH2, k.cdH1, nullptr, k.cdXa, A, 2LL * B * A, (long long)B * A, st);
+    rc = mlp_backward(x, qp, k.cdQ, 1, 2LL * B, B, nullptr, k.cdXa, A, 2LL * B * A, (long long)B * A, st);
     if (rc) return rc;
   } else {
     CU(cudaMemsetAsync(k.cdXa, 0, sizeof(float) * (size_t)n * 2 * B * A, st));
   }
   LAUNCH(x, k_head_bwd, dim3(cdiv(R, 128), n), 128, 0, st, k, R);
-  rc = mlp_backward(x, actor_update_pass(x, k), k.daOut, k.Ao, (long long)k.Rs * k.Ao, 0, k.daH2, k.daH1, k.g_actor,
-                    nullptr, 0, 0, 0, st);
+  rc = mlp_backward(x, actor_update_pass(x, k), k.daOut, k.Ao, (long long)k.Rs * k.Ao, 0, k.g_actor, nullptr, 0, 0, 0,
+                    st);
   if (rc) return rc;
   if (!k.per_state_std) LAUNCH(x, k_lsv_reduce, dim3(n), 32 * cdiv(A, 32), 0, st, k, R);
   return check_launch();
@@ -1250,9 +1287,14 @@ extern "C" int saceo_fit_bind(saceo_ctx* x, const saceo_fit_tables* t, int32_t m
   for (int pass = 0; pass < 2; ++pass) {
     Bump b{pass ? (char*)x->fit_ws : nullptr, 0, pass ? &x->names : nullptr};
     f.X = b.get<float>("fit_X", n2 * mb * SA);        f.T = b.get<float>("fit_T", n2 * mb * (c.S + 1));
-    f.H1 = b.get<float>("fit_H1", n2 * mb * c.model_hidden[0]); f.H2 = b.get<float>("fit_H2", n2 * mb * c.model_hidden[1]);
+    char nm[24];
+    for (int l = 0; l < c.model_layers; ++l) {
+      snprintf(nm, sizeof(nm), "fit_H%d", l + 1); f.H[l] = b.get<float>(nm, n2 * mb * c.model_hidden[l]);
+    }
     f.Out = b.get<float>("fit_Out", n2 * mb * mo);    f.dOut = b.get<float>("fit_dOut", n2 * mb * mo);
-    f.dH2 = b.get<float>("fit_dH2", n2 * mb * c.model_hidden[1]); f.dH1 = b.get<float>("fit_dH1", n2 * mb * c.model_hidden[0]);
+    for (int l = c.model_layers - 1; l >= 0; --l) {
+      snprintf(nm, sizeof(nm), "fit_dH%d", l + 1); f.dH[l] = b.get<float>(nm, n2 * mb * c.model_hidden[l]);
+    }
     f.g = b.get<float>("g_model", n2 * x->L.nm_stride);
     f.loss_part = b.get<float>("fit_loss", n2);
     f.g_ls = b.get<float>("g_model_logstd", n2 * c.S);
@@ -1286,10 +1328,11 @@ extern "C" int saceo_model_fit(saceo_ctx* x, int32_t n_steps, const int64_t* idx
   cudaStream_t st = (cudaStream_t)stream;
   const KCtx& k = x->k; const FitCtx& f = x->fit;
   const int n = k.n_agents, mb = f.mb, ms = f.mbs, SA = k.S + k.A, mo = x->L.model_out;
-  const Pass mp = fit_pass(x, NetD{f.model, 2 * x->L.nm_stride, x->L.nm_stride, f.nmod, SA, x->cfg.model_hidden[0],
-                                   x->cfg.model_hidden[1], mo, x->cfg.model_act[0], x->cfg.model_act[1]}, f.H1, f.H2);
-  const Pass rp = fit_pass(x, NetD{f.rw, 2 * f.nr_stride, f.nr_stride, f.nmod, SA, f.rh1, f.rh2, 1, f.ract0, f.ract1},
-                           f.rH1, f.rH2);
+  const Pass mp = fit_pass(x, model_net(x, f.model, f.nmod), f.H, f.dH);
+  const int rh[2] = {f.rh1, f.rh2}, ra[2] = {f.ract0, f.ract1};
+  float* const rH[2] = {f.rH1, f.rH2};
+  float* const rdH[2] = {f.rdH1, f.rdH2};
+  const Pass rp = fit_pass(x, net_desc(f.rw, 2 * f.nr_stride, f.nr_stride, f.nmod, SA, 1, 2, rh, ra), rH, rdH);
   for (int s = 0; s < n_steps; ++s) {
     const long long* ix = reinterpret_cast<const long long*>(idx) + (long long)s * n * f.nmod * mb;
     LAUNCH(x, k_fit_begin, cdiv(n, 128), 128, 0, st, f, n);
@@ -1303,10 +1346,10 @@ extern "C" int saceo_model_fit(saceo_ctx* x, int32_t n_steps, const int64_t* idx
     LAUNCH(x, k_fit_loss, dim3(f.nmod, n), 256, 0, st, k, f,
            losses_out ? losses_out + (long long)s * n * f.nmod : (float*)nullptr);
     // no kpad: K = 200 on the register-staged kernel beats K = 224 streamed (measured)
-    rc = mlp_backward(x, mp, f.dOut, mo, 2LL * ms * mo, (long long)ms * mo, f.dH2, f.dH1, f.g, nullptr, 0, 0, 0, st);
+    rc = mlp_backward(x, mp, f.dOut, mo, 2LL * ms * mo, (long long)ms * mo, f.g, nullptr, 0, 0, 0, st);
     if (rc) return rc;
     if (f.rw) {
-      rc = mlp_backward(x, rp, f.rdOut, 1, 2LL * ms, (long long)ms, f.rdH2, f.rdH1, f.g_r, nullptr, 0, 0, 0, st);
+      rc = mlp_backward(x, rp, f.rdOut, 1, 2LL * ms, (long long)ms, f.g_r, nullptr, 0, 0, 0, st);
       if (rc) return rc;
     }
     if (f.use_clip) LAUNCH(x, k_fit_gnorm, n, 1024, 0, st, f);
@@ -1332,33 +1375,33 @@ static int fvp_apply(saceo_ctx* x, const float* xin, float damp, float* Fx, cuda
   const KCtx& k = x->k; const FvpWs& f = x->f; const int n = k.n_agents, N = f.N;
   NetD an = actor_net(x);
   NetD tn = an; tn.theta = xin;                       // tangent "network": same flat layout
-  const long long sH1 = (long long)N * an.h1, sH2 = (long long)N * an.h2, sO = (long long)N * k.Ao;
+  const long long sH1 = (long long)N * an.N(0), sH2 = (long long)N * an.N(1), sO = (long long)N * k.Ao;
   int rc; GemmP p{};
   // T1 = (X.P0 + c0) * act0'(H1)
   p = GemmP{}; p.nnet = 1; p.A = f.X; p.lda = k.S; p.sAa = (long long)N * k.S;
-  p.B = tn.theta + tn.oW(0); p.ldb = an.h1; p.sBa = an.sa; p.bias = tn.theta + tn.ob(0); p.sba = an.sa;
-  p.C = f.T1; p.ldc = an.h1; p.sCa = sH1; p.aux = f.H1; p.M = N; p.N = an.h1; p.K = k.S; p.epi = EPI_MUL_DACT; p.act = an.act0;
+  p.B = tn.theta + tn.oW(0); p.ldb = an.N(0); p.sBa = an.sa; p.bias = tn.theta + tn.ob(0); p.sba = an.sa;
+  p.C = f.T1; p.ldc = an.N(0); p.sCa = sH1; p.aux = f.H1; p.M = N; p.N = an.N(0); p.K = k.S; p.epi = EPI_MUL_DACT; p.act = an.act(0);
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
   // Tmp = T1.W1 ;  T2 = (H1.P1 + c1 + Tmp) * act1'(H2)
-  p = GemmP{}; p.nnet = 1; p.A = f.T1; p.lda = an.h1; p.sAa = sH1; p.B = an.theta + an.oW(1); p.ldb = an.h2; p.sBa = an.sa;
-  p.C = f.Tmp; p.ldc = an.h2; p.sCa = sH2; p.M = N; p.N = an.h2; p.K = an.h1; p.epi = EPI_NONE;
+  p = GemmP{}; p.nnet = 1; p.A = f.T1; p.lda = an.N(0); p.sAa = sH1; p.B = an.theta + an.oW(1); p.ldb = an.N(1); p.sBa = an.sa;
+  p.C = f.Tmp; p.ldc = an.N(1); p.sCa = sH2; p.M = N; p.N = an.N(1); p.K = an.N(0); p.epi = EPI_NONE;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  p = GemmP{}; p.nnet = 1; p.A = f.H1; p.lda = an.h1; p.sAa = sH1; p.B = tn.theta + tn.oW(1); p.ldb = an.h2; p.sBa = an.sa;
+  p = GemmP{}; p.nnet = 1; p.A = f.H1; p.lda = an.N(0); p.sAa = sH1; p.B = tn.theta + tn.oW(1); p.ldb = an.N(1); p.sBa = an.sa;
   p.bias = tn.theta + tn.ob(1); p.sba = an.sa; p.addend = f.Tmp; p.aux = f.H2;
-  p.C = f.T2; p.ldc = an.h2; p.sCa = sH2; p.M = N; p.N = an.h2; p.K = an.h1; p.epi = EPI_MUL_DACT; p.act = an.act1;
+  p.C = f.T2; p.ldc = an.N(1); p.sCa = sH2; p.M = N; p.N = an.N(1); p.K = an.N(0); p.epi = EPI_MUL_DACT; p.act = an.act(1);
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
   // Tmp = T2.W2 ; TOut = H2.P2 + c2 + Tmp
-  p = GemmP{}; p.nnet = 1; p.A = f.T2; p.lda = an.h2; p.sAa = sH2; p.B = an.theta + an.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
-  p.C = f.Tmp; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.h2; p.epi = EPI_NONE;
+  p = GemmP{}; p.nnet = 1; p.A = f.T2; p.lda = an.N(1); p.sAa = sH2; p.B = an.theta + an.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
+  p.C = f.Tmp; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.N(1); p.epi = EPI_NONE;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  p = GemmP{}; p.nnet = 1; p.A = f.H2; p.lda = an.h2; p.sAa = sH2; p.B = tn.theta + tn.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
+  p = GemmP{}; p.nnet = 1; p.A = f.H2; p.lda = an.N(1); p.sAa = sH2; p.B = tn.theta + tn.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
   p.bias = tn.theta + tn.ob(2); p.sba = an.sa; p.addend = f.Tmp;
-  p.C = f.TOut; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.h2; p.epi = EPI_NONE;
+  p.C = f.TOut; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.N(1); p.epi = EPI_NONE;
   rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
   // metric: G = M . J x / N   (per row), plus per-row logstd_var contribution
   LAUNCH(x, k_fvp_metric, dim3(cdiv(N, 128), n), 128, 0, st, k, f, xin, x->cfg.std_mult);
   // J^T G  -> Fx (flat layout), then + damp x
-  rc = mlp_backward(x, fvp_pass(x), f.G, k.Ao, sO, 0, f.dH2, f.dH1, Fx, nullptr, 0, 0, 0, st); if (rc) return rc;
+  rc = mlp_backward(x, fvp_pass(x), f.G, k.Ao, sO, 0, Fx, nullptr, 0, 0, 0, st); if (rc) return rc;
   LAUNCH(x, k_fvp_finish, dim3(cdiv(x->L.na, 256), n), 256, 0, st, k, f, xin, damp, Fx);
   return check_launch();
 }
@@ -1411,7 +1454,7 @@ static int surrogate_grad(saceo_ctx* x, const float* act, const float* adv, cons
   LAUNCH(x, k_trpo_rows, dim3(cdiv(N, 128), n), 128, 0, st, k, f, act, adv, nlp_old, (const float*)nullptr, alpha,
          x->cfg.std_mult, 1, clip_eps, (float*)nullptr, (float*)nullptr);
   if (stats_out) LAUNCH(x, k_trpo_reduce, dim3(n), 256, 0, st, f, stats_out);
-  rc = mlp_backward(x, fvp_pass(x), f.G, k.Ao, (long long)N * k.Ao, 0, f.dH2, f.dH1, grad_out, nullptr, 0, 0, 0, st);
+  rc = mlp_backward(x, fvp_pass(x), f.G, k.Ao, (long long)N * k.Ao, 0, grad_out, nullptr, 0, 0, 0, st);
   if (rc) return rc;
   // logstd-variable entries = fixed-order column sums of the per-row terms (damp 0: the x operand is only a finite filler)
   LAUNCH(x, k_fvp_finish, dim3(cdiv(x->L.na, 256), n), 256, 0, st, k, f, (const float*)k.T.actor, 0.f, grad_out);
@@ -1454,7 +1497,7 @@ extern "C" int saceo_onpolicy_expert_grad(saceo_ctx* x, int32_t n_models, int32_
   LAUNCH(x, k_ghead, dim3(cdiv(E, 128), n), 128, 0, st, k, x->cfg.std_mult, clip_actions, 0);
   rc = model_term_phase(x, k, st); if (rc) return rc;
   LAUNCH(x, k_ghead, dim3(cdiv(E, 128), n), 128, 0, st, k, x->cfg.std_mult, clip_actions, 1);
-  rc = mlp_backward(x, ap, k.daOut, k.Ao, (long long)Rs * k.Ao, 0, k.daH2, k.daH1, grad_out, nullptr, 0, 0, 0, st);
+  rc = mlp_backward(x, ap, k.daOut, k.Ao, (long long)Rs * k.Ao, 0, grad_out, nullptr, 0, 0, 0, st);
   if (rc) return rc;
   if (!k.per_state_std) LAUNCH(x, k_lsv_reduce, dim3(n), 32 * cdiv(k.A, 32), 0, st, k, E);
   if (stats_out) LAUNCH(x, k_exp_stats, dim3(cdiv(n, 128)), 128, 0, st, k, stats_out);

@@ -13,7 +13,8 @@ from typing import Optional
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SACEO_LIB") or os.path.join(_HERE, "libsaceo.so")     # SACEO_LIB: alternative build (experiments)
 
-ABI_VERSION = 1
+ABI_VERSION = 2
+POLICY_MAX_HIDDEN = 8       # SACEO_POLICY_MAX_HIDDEN: most hidden layers of a dynamics model or an acted policy
 ACT_IDS = {"relu": 0, "tanh": 1, "elu": 2}
 GEMM_FP32_SIMT = 0
 GEMM_TCGEN05_BF16X3 = 1
@@ -27,8 +28,10 @@ class Config(C.Structure):
     _fields_ = [
         ("abi_version", C.c_int32), ("device", C.c_int32), ("n_agents", C.c_int32),
         ("S", C.c_int32), ("A", C.c_int32),
-        ("actor_hidden", C.c_int32 * 2), ("critic_hidden", C.c_int32 * 2), ("model_hidden", C.c_int32 * 2),
-        ("actor_act", C.c_int32 * 2), ("critic_act", C.c_int32 * 2), ("model_act", C.c_int32 * 2),
+        ("actor_hidden", C.c_int32 * 2), ("critic_hidden", C.c_int32 * 2),
+        ("actor_act", C.c_int32 * 2), ("critic_act", C.c_int32 * 2),
+        ("model_layers", C.c_int32), ("model_hidden", C.c_int32 * POLICY_MAX_HIDDEN),
+        ("model_act", C.c_int32 * POLICY_MAX_HIDDEN),
         ("per_state_std", C.c_int32), ("separate_reward_nn", C.c_int32), ("num_models", C.c_int32),
         ("delta_clip_pred", C.c_float),
         ("B", C.c_int32), ("E", C.c_int32), ("target_update_int", C.c_int32),
@@ -69,9 +72,6 @@ class FitTables(C.Structure):
                [("reward_hidden", C.c_int32 * 2), ("reward_act", C.c_int32 * 2), ("reward_stride", C.c_int64)]
     POINTERS = ("model", "model_m", "model_v", "model_t", "fit_hyper", "model_logstd", "model_logstd_m", "model_logstd_v",
                 "reward", "reward_m", "reward_v")
-
-
-POLICY_MAX_HIDDEN = 8
 
 
 class PolicyConfig(C.Structure):

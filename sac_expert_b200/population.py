@@ -30,13 +30,14 @@ class PopulationSpec:
     A: int
     actor_hidden: Tuple[int, int] = (256, 256)
     critic_hidden: Tuple[int, int] = (256, 256)
-    model_hidden: Tuple[int, int] = (512, 512)
+    model_hidden: Tuple[int, ...] = (512, 512)     # 1 to 8 hidden layers (lib.POLICY_MAX_HIDDEN)
     actor_acts: Tuple[str, str] = ("relu", "relu")
     critic_acts: Tuple[str, str] = ("relu", "relu")
-    model_acts: Tuple[str, str] = ("relu", "relu")
+    model_acts: Tuple[str, ...] = ("relu", "relu")  # one per entry of model_hidden
     per_state_std: bool = True
     separate_reward_nn: bool = False
-    reward_hidden: Optional[Tuple[int, int]] = None     # separate_reward_nn: the reward network (default: model_hidden / model_acts)
+    # separate_reward_nn: the reward network, two hidden layers (default: model_hidden / model_acts, which then must have two)
+    reward_hidden: Optional[Tuple[int, int]] = None
     reward_acts: Optional[Tuple[str, str]] = None
     num_models: int = 2            # 0 = plain SAC
     delta_clip_pred: float = 0.0
@@ -64,12 +65,16 @@ class PopulationSpec:
         for i in range(2):
             c.actor_hidden[i] = self.actor_hidden[i]
             c.critic_hidden[i] = self.critic_hidden[i]
+            for dst, src in ((c.actor_act, self.actor_acts), (c.critic_act, self.critic_acts)):
+                dst[i] = _act_id(src[i])
+        nh = len(self.model_hidden)
+        if not 1 <= nh <= _l.POLICY_MAX_HIDDEN or len(self.model_acts) != nh:
+            raise ValueError(f"model_hidden needs 1 to {_l.POLICY_MAX_HIDDEN} widths and model_acts one activation per "
+                             f"width (got {tuple(self.model_hidden)}, {tuple(self.model_acts)})")
+        c.model_layers = nh
+        for i in range(nh):
             c.model_hidden[i] = self.model_hidden[i]
-            for dst, src in ((c.actor_act, self.actor_acts), (c.critic_act, self.critic_acts),
-                             (c.model_act, self.model_acts)):
-                if src[i] not in _l.ACT_IDS:
-                    raise ValueError("activations must be tanh, relu or elu")   # nn_utils.py:18
-                dst[i] = _l.ACT_IDS[src[i]]
+            c.model_act[i] = _act_id(self.model_acts[i])
         c.per_state_std = int(self.per_state_std)
         c.separate_reward_nn = int(self.separate_reward_nn)
         c.num_models = self.num_models
@@ -88,10 +93,28 @@ class PopulationSpec:
         c.reserved[6] = 0 if self.fork_actor else 1
         return c
 
+    def reward_net(self) -> Tuple[Tuple[int, int], Tuple[str, str]]:
+        """(hidden, acts) of the separate reward network: ``reward_hidden`` / ``reward_acts``, else those of the model.
+        The reward network always has two hidden layers, so a model of another depth needs an explicit reward_hidden."""
+        rh = tuple(self.reward_hidden or self.model_hidden)
+        ra = tuple(self.reward_acts or self.model_acts)
+        if len(rh) != 2 or len(ra) != 2:
+            raise ValueError(f"the reward network of separate_reward_nn has two hidden layers: give two-entry "
+                             f"reward_hidden and reward_acts (got {rh}, {ra})")
+        return rh, ra
+
+
+def _act_id(name: str) -> int:
+    if name not in _l.ACT_IDS:
+        raise ValueError("activations must be tanh, relu or elu")   # nn_utils.py:18
+    return _l.ACT_IDS[name]
+
 
 def net_shapes(n_in: int, hidden: Sequence[int], n_out: int) -> List[Tuple[int, ...]]:
-    """Keras ``get_weights()`` shapes ``[W0,b0,W1,b1,W2,b2]`` (nn_utils.py:86-138)."""
-    return [(n_in, hidden[0]), (hidden[0],), (hidden[0], hidden[1]), (hidden[1],), (hidden[1], n_out), (n_out,)]
+    """Keras ``get_weights()`` shapes ``[W0,b0,W1,b1,...,Wn,bn]`` of a net with ``len(hidden)`` hidden layers
+    (nn_utils.py:86-138)."""
+    dims = [n_in] + list(hidden) + [n_out]
+    return [sh for k, n in zip(dims[:-1], dims[1:]) for sh in ((k, n), (n,))]
 
 
 def pack_flat(ws: Sequence[np.ndarray]) -> np.ndarray:
@@ -198,8 +221,9 @@ class Population:
             actor=net_shapes(spec.S, spec.actor_hidden, L.Ao) + ([] if spec.per_state_std else [(1, spec.A)]),
             q=net_shapes(spec.S + spec.A, spec.critic_hidden, 1),
             model=net_shapes(spec.S + spec.A, spec.model_hidden, L.model_out),
-            reward=net_shapes(spec.S + spec.A, tuple(spec.reward_hidden or spec.model_hidden), 1),
         )
+        if spec.separate_reward_nn and spec.num_models > 0:
+            self.shapes["reward"] = net_shapes(spec.S + spec.A, spec.reward_net()[0], 1)
         self._host_size = np.zeros(n, np.int64)
         self._host_start = np.zeros(n, np.int64)
         if spec.separate_reward_nn and spec.num_models > 0:      # reward networks: fitted by model_fit, unused by the update
@@ -580,12 +604,9 @@ class Population:
         for name in _l.FitTables.POINTERS:
             setattr(ft, name, self.t[name].data_ptr() if name in self.t else None)
         if self.spec.separate_reward_nn:
-            rh = tuple(self.spec.reward_hidden or self.spec.model_hidden)
-            ra = tuple(self.spec.reward_acts or self.spec.model_acts)
+            rh, ra = self.spec.reward_net()
             for i in range(2):
-                if ra[i] not in _l.ACT_IDS:
-                    raise ValueError("activations must be relu, tanh, or elu")
-                ft.reward_hidden[i] = int(rh[i]); ft.reward_act[i] = _l.ACT_IDS[ra[i]]
+                ft.reward_hidden[i] = int(rh[i]); ft.reward_act[i] = _act_id(ra[i])
             ft.reward_stride = self.nr_stride
         torch.cuda.synchronize(self.dev)
         _l.check(self.lib.saceo_fit_bind(self.ctx, C.byref(ft), int(model_batch), int(bool(use_grad_clip))))

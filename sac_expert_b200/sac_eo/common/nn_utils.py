@@ -1,8 +1,8 @@
 """Weight-list conventions of the reference networks (``/root/reference/sac_eo/common/nn_utils.py``):
 Keras ``Sequential`` of ``Dense`` layers, ``y = x @ W + b``, ``W: [in, out]``, ``get_weights()`` order
 ``[W0, b0, W1, b1, W2, b2]``; orthogonal(sqrt 2) hidden / orthogonal(gain) final initialisation, zero biases.
-The networks this project trains have two hidden layers (every BASELINE config is 2x256 / 2x512); weight lists of any
-depth are built for actors that are only acted (expert policies)."""
+Actors, critics and reward networks the project trains have two hidden layers (every BASELINE config is 2x256 / 2x512);
+dynamics models have 1 to 8, and weight lists of any depth are built for actors that are only acted (expert policies)."""
 import math
 
 import numpy as np
@@ -27,6 +27,23 @@ def check_two_hidden(layers):
     if len(layers) != 2:
         raise ValueError("sac_expert_b200 supports exactly two hidden layers per network (got %r)" % (layers,))
     return tuple(int(h) for h in layers)
+
+
+MODEL_MAX_HIDDEN = 8     # include/saceo.h SACEO_POLICY_MAX_HIDDEN
+
+
+def check_model_hidden(layers):
+    """Hidden widths of a dynamics model: 1 to MODEL_MAX_HIDDEN layers, each at least 1 wide."""
+    hidden = tuple(int(h) for h in layers)
+    if not 1 <= len(hidden) <= MODEL_MAX_HIDDEN or min(hidden) < 1:
+        raise ValueError("sac_expert_b200 dynamics models have 1 to %d hidden layers of width >= 1 (got %r)"
+                         % (MODEL_MAX_HIDDEN, layers))
+    return hidden
+
+
+def trainable_names(n_hidden):
+    """Keras variable order of a Sequential of n_hidden + 1 Dense layers: W0, b0, ..., Wn, bn."""
+    return ["%s%d" % (k, l) for l in range(n_hidden + 1) for k in ("W", "b")]
 
 
 def _orthogonal(rng, rows, cols, gain):

@@ -25,7 +25,8 @@ class _DeviceF:
         if models:
             m0 = models[0]
             mkw = dict(num_models=len(models), E=len(expert[0]), model_hidden=m0.layers, model_acts=m0.activations,
-                       separate_reward_nn=m0.separate_reward_nn, delta_clip_pred=float(m0.delta_clip_pred or 0.0))
+                       separate_reward_nn=m0.separate_reward_nn, reward_hidden=m0.reward_layers,
+                       reward_acts=m0.reward_activations, delta_clip_pred=float(m0.delta_clip_pred or 0.0))
         else:
             mkw = dict(num_models=0, E=0)
         spec = PopulationSpec(n_agents=1, S=actor.s_dim, A=actor.a_dim, actor_hidden=actor.layers,
@@ -38,7 +39,7 @@ class _DeviceF:
             self.pop.set_norm(0, s_mean=actor.s_rms.mean, s_std=actor.s_rms.std)
         if models:
             for i, m in enumerate(models):
-                self.pop.set_net(0, "m%d" % (i + 1), m.get_weights()[:6])
+                self.pop.set_net(0, "m%d" % (i + 1), m.get_weights()[:2 * len(m.layers) + 2])     # without a Gaussian logstd
             m0 = models[0]
             if getattr(m0, "s_rms", None) is not None:        # the models' own normaliser set (SAC_expert.py:139-144)
                 self.pop.set_norm(0, m_s_mean=m0.s_rms.mean, m_s_std=m0.s_rms.std, m_a_mean=m0.a_rms.mean,

@@ -8,7 +8,7 @@ import torch
 
 from ..common.device_net import DeviceNet
 from ..common.lockstep import Request, inline
-from ..common.nn_utils import broadcast_activations, check_two_hidden, create_nn_weights
+from ..common.nn_utils import broadcast_activations, check_model_hidden, check_two_hidden, create_nn_weights, trainable_names
 from ..envs.synthetic import flatdim
 
 
@@ -19,7 +19,7 @@ class MSEModel(DeviceNet):
                  reward_gain, model_setup_kwargs, std_mult=1.0):
         super().__init__()
         self.s_dim, self.a_dim = flatdim(env.observation_space), flatdim(env.action_space)
-        self.layers = check_two_hidden(model_layers)
+        self.layers = check_model_hidden(model_layers)
         self.activations = broadcast_activations(model_layers, model_activations)
         self.separate_reward_nn = bool(model_setup_kwargs.get("separate_reward_nn", False))
         self.delta_clip_pred = model_setup_kwargs.get("delta_clip_pred", None)
@@ -35,7 +35,7 @@ class MSEModel(DeviceNet):
         self._reward_weights = (create_nn_weights(self.s_dim + self.a_dim, 1, self.reward_layers, reward_gain)
                                 if self.separate_reward_nn else None)
         self._logstd = np.ones((1, self.s_dim), np.float32) * np.log(std_mult) if self.gaussian else None
-        self.trainable = ["W0", "b0", "W1", "b1", "W2", "b2"] + (["logstd"] if self.gaussian else [])
+        self.trainable = trainable_names(len(self.layers)) + (["logstd"] if self.gaussian else [])
 
     def set_rms(self, normalizer):
         self._rms = normalizer.get_rms()

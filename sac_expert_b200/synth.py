@@ -31,10 +31,10 @@ def _orthogonal(gen, n, rows, cols, gain, dev):
 def _init_nets(gen, tab, n_in, hidden, n_out, gain, dev):
     """tab: [n, stride] flat tables; fills W blocks, leaves biases zero."""
     n = tab.shape[0]
-    dims = [n_in, hidden[0], hidden[1], n_out]
+    dims = [n_in] + list(hidden) + [n_out]
     o = 0
-    for l in range(3):
-        g = math.sqrt(2.0) if l < 2 else gain
+    for l in range(len(hidden) + 1):
+        g = math.sqrt(2.0) if l < len(hidden) else gain
         w = _orthogonal(gen, n, dims[l], dims[l + 1], g, dev)
         tab[:, o:o + dims[l] * dims[l + 1]] = w.reshape(n, -1)
         o += dims[l] * dims[l + 1] + dims[l + 1]
@@ -107,14 +107,16 @@ def fill_synthetic(pop: Population, seed: int = 0, replay_rows: int | None = Non
 def algorithmic_flops(sp) -> float:
     """Matmul FLOPs per agent-update (SURVEY.md §8d formula)."""
     S, A, B, E = sp.S, sp.A, sp.B, (sp.E if sp.num_models > 0 else 0)
-    H, Hm = sp.actor_hidden[0], sp.model_hidden[0]
+    H, hm = sp.actor_hidden[0], list(sp.model_hidden)
     Ao = 2 * A if sp.per_state_std else A
     Pa = S * H + H * H + H * Ao
     Pc = (S + A) * H + H * H + H
-    Pm = (S + A) * Hm + Hm * Hm + Hm * (S + 1)
+    dm = [S + A] + hm + [S + 1]
+    Pm = sum(k * n for k, n in zip(dm[:-1], dm[1:]))                        # model forward
+    Bm = hm[-1] * S + sum(k * n for k, n in zip(hm[:-1], hm[1:])) + A * hm[0]   # model backward to the action columns
     f = 2 * B * (4 * Pa + 8 * Pc + 5 * H * H + H * Ao + 2 * A * H + 4 * H)
     if E:
-        f += 2 * E * (2 * Pa + H * Ao + H * H + Pm + Hm * S + Hm * Hm + A * Hm)
+        f += 2 * E * (2 * Pa + H * Ao + H * H + Pm + Bm)
     return float(f)
 
 
