@@ -387,6 +387,31 @@ int saceo_test_gemm(int32_t gemm_mode, int32_t batch, int32_t M, int32_t N, int3
                     int32_t transA, int32_t transB, const float *A, const float *Bm, float *C,
                     void *stream);
 
+/* Test surface over the whole GEMM dispatch the MLP passes use:
+ *   C[z] = epi(op(A[z]) . op(B[z]) + bias[z] + addend[z]),  z = (agent, net),  element (m, n) at C + m * ldc + n.
+ * ones: op(A) = [X^T; 1], A holds X[K, M-1] (transA = 1), row M-1 of op(A) is all ones ([dW; db] products).
+ * bias (indexed by n), addend and aux (C's shape and strides) may be NULL; epi / act as in the library's epilogue
+ * (0 none, 1 act(v), 2 v * act'(aux) from the post-activation aux).  f16: the tcgen05 engine splits operands into fp16
+ * instead of bf16 planes.  The route taken is written to *route. */
+typedef struct {
+  int32_t gemm_mode;              /* SACEO_GEMM_*; the tcgen05 tile variant in bits 8..15 */
+  int32_t n_agents, nnet;
+  int32_t transA, transB, ones;
+  int32_t M, N, K, lda, ldb, ldc;
+  int64_t sAa, sAn, sBa, sBn, sCa, sCn, sba, sbn;   /* agent / net strides in floats */
+  const float *A, *B;
+  float *C;
+  const float *bias, *addend, *aux;
+  int32_t epi, act, f16;
+} saceo_gemm_args;
+typedef struct {
+  int32_t n_tc, n_skinny, n_simt;  /* launches of k_gemm_tc* / k_gemm_skinny / k_gemm_simt */
+  int32_t tc_rows;                 /* rows [0, tc_rows) went to the tensor-core launch (0: none) */
+  int32_t tc_stream;               /* 1: streaming kernel <tc_akc, tc_bkc>; 0: register-staged <tc_bn, tc_stages, tc_threads> */
+  int32_t tc_akc, tc_bkc, tc_bn, tc_stages, tc_threads;
+} saceo_gemm_route;
+int saceo_test_gemm_ex(const saceo_gemm_args *args, saceo_gemm_route *route, void *stream);
+
 const char *saceo_last_error(void);
 int saceo_abi_version(void);
 

@@ -1686,3 +1686,35 @@ extern "C" int saceo_test_gemm(int32_t gemm_mode, int32_t batch, int32_t M, int3
   int rc = gemm(&tmp, transA != 0, transB != 0, false, p, batch, (cudaStream_t)stream); if (rc) return rc;
   return check_launch();
 }
+
+extern "C" int saceo_test_gemm_ex(const saceo_gemm_args* a, saceo_gemm_route* route, void* stream) {
+  if (!a || !route || !a->A || !a->B || !a->C || a->n_agents < 1 || a->nnet < 1) return fail(SACEO_E_INVALID, "bad argument");
+  if (a->ones && !a->transA) return fail(SACEO_E_INVALID, "the ones row needs transA");
+  const bool TA = a->transA != 0, TB = a->transB != 0, ONES = a->ones != 0;
+  GemmP p{};
+  p.A = a->A; p.B = a->B; p.C = a->C; p.bias = a->bias; p.addend = a->addend; p.aux = a->aux;
+  p.M = a->M; p.N = a->N; p.K = a->K; p.lda = a->lda; p.ldb = a->ldb; p.ldc = a->ldc;
+  p.sAa = a->sAa; p.sAn = a->sAn; p.sBa = a->sBa; p.sBn = a->sBn; p.sCa = a->sCa; p.sCn = a->sCn; p.sba = a->sba; p.sbn = a->sbn;
+  p.nnet = a->nnet; p.epi = a->epi; p.act = a->act; p.f16 = a->f16;
+  saceo_ctx tmp; tmp.tc = (a->gemm_mode & 0xff) == SACEO_GEMM_TCGEN05_BF16X3; tmp.tc_variant = (a->gemm_mode >> 8) & 0xff;
+  tmp.prof = true;        // count_launch records each launch's name: the route report
+  if (tmp.tc) CU(tc_gemm_init());
+  *route = saceo_gemm_route{};
+  const bool tc = tmp.tc && p.M > 0 && p.N > 0 && p.K > 0 && tc_gemm_eligible(TA, TB, ONES, p);
+  if (tc) {
+    const TcRoute r = tc_route(TA, TB, p, tmp.tc_variant);
+    route->tc_rows = tc_rows(ONES, p);
+    route->tc_stream = r.stream; route->tc_akc = r.akc; route->tc_bkc = r.bkc;
+    route->tc_bn = r.bn; route->tc_stages = r.stages; route->tc_threads = r.threads;
+  }
+  int rc = gemm(&tmp, TA, TB, ONES, p, a->n_agents, (cudaStream_t)stream);
+  for (size_t i = 0; i < tmp.prof_n; ++i) {
+    const std::string name = tmp.prof_name[i];
+    if (name == "k_gemm_tc") route->n_tc++;
+    else if (name == "k_gemm_skinny") route->n_skinny++;
+    else if (name == "k_gemm_simt") route->n_simt++;
+  }
+  for (cudaEvent_t e : tmp.prof_ev) cudaEventDestroy(e);
+  if (rc) return rc;
+  return check_launch();
+}

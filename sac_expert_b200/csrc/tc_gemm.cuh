@@ -595,6 +595,28 @@ static inline bool tc_gemm_eligible(bool TA, bool TB, bool ONES, const GemmP& p)
   return p.m_off == 0 && p.N > 32 && p.K >= 8 && (r >= 96 || (r >= 16 && (long long)p.N * p.K >= 128 * 128));
 }
 
+// Which tensor-core kernel takes a GEMM: the streaming kernel k_gemm_tc_stream<akc, bkc>, or the register-staged
+// k_gemm_tc<bn, stages, threads, ...>.
+struct TcRoute {
+  bool stream;
+  bool akc, bkc;               // streaming: op(A) / op(B) storage contiguous along k
+  int bn, stages, threads;     // register-staged tile
+};
+static inline TcRoute tc_route(bool TA, bool TB, const GemmP& p, int variant) {
+  TcRoute r{};
+  r.akc = (TA ? p.lda : 1) == 1; r.bkc = (TB ? 1 : p.ldb) == 1;
+  const bool aligned = ((p.lda & 3) == 0) && ((p.ldb & 3) == 0) && (((p.sAa | p.sAn | p.sBa | p.sBn) & 3) == 0) &&
+                       ((reinterpret_cast<uintptr_t>(p.A) & 15) == 0) && ((reinterpret_cast<uintptr_t>(p.B) & 15) == 0);
+  // both operands contiguous along k (dX = dY . W^T): the register-staged 64-k kernel reads whole 256-byte rows and wins
+  // (134 vs 160 us on 256^3 x 512, tools/gemm_bench.py); every other orientation streams
+  const bool both_kc = r.akc && r.bkc;
+  r.stream = variant != 2 && aligned && !both_kc && (p.K % TS_BK) == 0 && (p.N % TS_BN) == 0;
+  if (r.stream) return r;
+  if (variant == 1) { r.bn = p.N > 64 ? 128 : 64; r.stages = 1; r.threads = 256; }
+  else { r.bn = p.N > 128 ? 256 : p.N > 64 ? 128 : 64; r.stages = r.bn == 256 ? 2 : r.bn == 128 ? 3 : 4; r.threads = 512; }
+  return r;
+}
+
 static unsigned long long* g_tc_dbg = nullptr;   // set by saceo_test_gemm_timed only
 // launches the tensor-core part (rows [0, tc_rows)); the caller finishes rows [tc_rows, M). <0 on a launch error
 static inline int tc_gemm_launch(bool TA, bool TB, bool ONES, const GemmP& p, int nagents, int variant, cudaStream_t st) {
@@ -605,21 +627,16 @@ static inline int tc_gemm_launch(bool TA, bool TB, bool ONES, const GemmP& p, in
   const int mt = (q.m_rows + TC_BM - 1) / TC_BM;
 #define TC_GO(BN_, NS_, NT_, MB_) do { dim3 grid((p.N + BN_ - 1) / BN_, mt, nagents * p.nnet); \
     k_gemm_tc<BN_, NS_, NT_, MB_><<<grid, NT_, TcSmem<BN_, NS_, NT_>::BYTES, st>>>(q); } while (0)
-  const bool aligned = ((p.lda & 3) == 0) && ((p.ldb & 3) == 0) && (((p.sAa | p.sAn | p.sBa | p.sBn) & 3) == 0) &&
-                       ((reinterpret_cast<uintptr_t>(p.A) & 15) == 0) && ((reinterpret_cast<uintptr_t>(p.B) & 15) == 0);
-  // both operands contiguous along k (dX = dY . W^T): the register-staged 64-k kernel reads whole 256-byte rows and wins
-  // (134 vs 160 us on 256^3 x 512, tools/gemm_bench.py); every other orientation streams
-  const bool both_kc = (q.a_sk == 1) && (q.b_sk == 1);
-  if (variant != 2 && aligned && !both_kc && (p.K % TS_BK) == 0 && (p.N % TS_BN) == 0) {
+  const TcRoute r = tc_route(TA, TB, p, variant);
+  if (r.stream) {
     dim3 grid(p.N / TS_BN, mt, nagents * p.nnet);
-    const bool akc = (q.a_sk == 1), bkc = (q.b_sk == 1);
-    if (akc) k_gemm_tc_stream<true, false><<<grid, TS_NT, TS_BYTES, st>>>(q);
-    else if (bkc) k_gemm_tc_stream<false, true><<<grid, TS_NT, TS_BYTES, st>>>(q);
+    if (r.akc) k_gemm_tc_stream<true, false><<<grid, TS_NT, TS_BYTES, st>>>(q);
+    else if (r.bkc) k_gemm_tc_stream<false, true><<<grid, TS_NT, TS_BYTES, st>>>(q);
     else k_gemm_tc_stream<false, false><<<grid, TS_NT, TS_BYTES, st>>>(q);
-  } else if (variant == 1) {
-    if (p.N > 64) TC_GO(128, 1, 256, 2); else TC_GO(64, 1, 256, 2);
+  } else if (r.threads == 256) {
+    if (r.bn == 128) TC_GO(128, 1, 256, 2); else TC_GO(64, 1, 256, 2);
   } else {
-    if (p.N > 128) TC_GO(256, 2, 512, 1); else if (p.N > 64) TC_GO(128, 3, 512, 1); else TC_GO(64, 4, 512, 1);
+    if (r.bn == 256) TC_GO(256, 2, 512, 1); else if (r.bn == 128) TC_GO(128, 3, 512, 1); else TC_GO(64, 4, 512, 1);
   }
 #undef TC_GO
   if (cudaPeekAtLastError() != cudaSuccess) return -1;

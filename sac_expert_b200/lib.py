@@ -83,6 +83,21 @@ class PolicyConfig(C.Structure):
     ]
 
 
+class GemmArgs(C.Structure):
+    """saceo_gemm_args (include/saceo.h): one call of the GEMM dispatch, for saceo_test_gemm_ex."""
+    _fields_ = [(n, C.c_int32) for n in ("gemm_mode", "n_agents", "nnet", "transA", "transB", "ones",
+                                         "M", "N", "K", "lda", "ldb", "ldc")] + \
+               [(n, C.c_int64) for n in ("sAa", "sAn", "sBa", "sBn", "sCa", "sCn", "sba", "sbn")] + \
+               [(n, C.c_void_p) for n in ("A", "B", "C", "bias", "addend", "aux")] + \
+               [(n, C.c_int32) for n in ("epi", "act", "f16")]
+
+
+class GemmRoute(C.Structure):
+    """saceo_gemm_route (include/saceo.h): which kernels a saceo_test_gemm_ex call launched."""
+    _fields_ = [(n, C.c_int32) for n in ("n_tc", "n_skinny", "n_simt", "tc_rows", "tc_stream", "tc_akc", "tc_bkc",
+                                         "tc_bn", "tc_stages", "tc_threads")]
+
+
 FIT_HYPER = 8
 FIT_HYPER_NAMES = ("model_lr", "reward_loss_coef", "delta_clip_loss", "reward_clip_loss", "model_max_grad_norm",
                    "r_mean", "r_std", "scale_model_loss")
@@ -96,7 +111,7 @@ EXPORTS = [
     "saceo_actor_forward", "saceo_critic_forward", "saceo_model_eval", "saceo_fvp", "saceo_cg_solve",
     "saceo_fit_bind", "saceo_model_fit", "saceo_trpo_grad", "saceo_trpo_eval", "saceo_actor_step", "saceo_ppo_grad", "saceo_actor_adam", "saceo_onpolicy_expert_grad", "saceo_grad_blend",
     "saceo_policy_layout", "saceo_policy_act",
-    "saceo_debug_ptr", "saceo_launch_count", "saceo_test_gemm", "saceo_last_error", "saceo_abi_version",
+    "saceo_debug_ptr", "saceo_launch_count", "saceo_test_gemm", "saceo_test_gemm_ex", "saceo_last_error", "saceo_abi_version",
 ]
 
 
@@ -145,6 +160,7 @@ def load() -> C.CDLL:
         "saceo_debug_ptr": (vp, [vp, C.c_char_p, C.POINTER(i64)]),
         "saceo_launch_count": (i64, [vp]),
         "saceo_test_gemm": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp]),
+        "saceo_test_gemm_ex": (C.c_int, [C.POINTER(GemmArgs), C.POINTER(GemmRoute), vp]),
         "saceo_last_error": (C.c_char_p, []),
         "saceo_abi_version": (C.c_int, []),
     }
