@@ -17,8 +17,7 @@ struct KCtx {
   float eps_force;   // >= 0: expert weight used instead of hyper[5] (behaviour cloning = 1), < 0: per-agent table value
   int ldXc, ldXp;    // leading dimensions of Xc (S+A -> multiple of 4) and Xpi (S -> multiple of 4): 16-byte aligned rows, pad columns stay zero
   int Rs;   // row stride of the per-agent [R rows] actor buffers (R rounded up to 32; the pad rows stay zero)
-  int ah1, ah2, ch1, ch2, mh1, mh2;
-  int aact0, aact1, cact0, cact1, mact0, mact1;
+  int mh1, mh2, mact0, mact1;
   int mnh;           // hidden layers of the models; mh1 / mh2 / mact0 / mact1 describe them only when mnh == 2
   float delta_clip;
   int cap;
@@ -27,8 +26,8 @@ struct KCtx {
   // workspace (per-agent arrays; strides derive from the dims above)
   long long* idx; float* noise; int* perm;
   float *mb_s, *mb_a, *mb_sp, *mb_r, *mb_omd;
-  float *Xpi, *aH1, *aH2, *aOut, *daOut, *daH2, *daH1, *dls;
-  float *Xc, *cH1, *cH2, *cQ, *cdQ, *cdH2, *cdH1, *cdXa;
+  float *Xpi, *aOut, *daOut, *dls;
+  float *Xc, *cQ, *cdQ, *cdXa;
   float *Xc2;        // live-critic input [N_s(s) | N_a(a)] (Xc holds the target-critic input [N_s(sp) | N_a(a')])
   float *Xc3;        // actor-phase critic input [N_s(s) | N_a(pi(s))]: state columns written by the gather, action columns by the head
   float *Xm, *mOut, *mdOut, *mdXa;

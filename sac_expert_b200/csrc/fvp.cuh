@@ -12,7 +12,7 @@ namespace saceo {
 
 struct FvpWs {
   int N;
-  float *X, *H1, *H2, *Out, *T1, *T2, *Tmp, *TOut, *G, *dH2, *dH1, *gls;
+  float *Out, *Tmp, *TOut, *G, *gls;
   float *p, *r, *z, *x, *sc;   // CG vectors [n, na_stride]; sc[agent*8 + {0: rr, 1: active}]
 };
 

@@ -20,7 +20,6 @@ struct FitCtx {
   float *g_ls;               // workspace: gradient of logstd [n_agents, 2, S]
   // workspace, all [n_agents, 2, ...]
   float *X, *T, *Out, *dOut, *g;
-  float *H[SACEO_POLICY_MAX_HIDDEN], *dH[SACEO_POLICY_MAX_HIDDEN];   // per hidden layer of the model: activation, gradient
   float *loss_part;      // [n_agents, 2]
   float *gscale;         // [n_agents] gradient scale of clip_by_global_norm (1 when clipping is off)
   float *gnorm;          // [n_agents] global gradient norm (diagnostic)
@@ -29,8 +28,7 @@ struct FitCtx {
   long long nm, nm_stride;
   // separate_reward_nn: the reward network of every model (caller tables + workspace), NULL otherwise
   float *rw, *rw_m, *rw_v, *g_r;
-  float *rH1, *rH2, *rOut, *rdOut, *rdH2, *rdH1;
-  int rh1, rh2, ract0, ract1;
+  float *rOut, *rdOut;
   long long nr, nr_stride;
 };
 

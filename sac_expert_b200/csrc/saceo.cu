@@ -8,6 +8,7 @@
 #include <string>
 #include <vector>
 #include <map>
+#include <algorithm>
 
 #include "../../include/saceo.h"
 #include "gemm_simt.cuh"
@@ -53,6 +54,8 @@ struct NetD {            // one (population of) MLP(s) in the flat Keras layout:
   int act(int l) const { return l == nh ? ACT_LINEAR : ha[l]; }
   long long oW(int l) const { return l == 0 ? 0 : ob(l - 1) + N(l - 1); }
   long long ob(int l) const { return oW(l) + (long long)K(l) * N(l); }
+  long long n() const { return ob(nh) + N(nh); }                                      // parameters
+  int widest(int l0) const { return l0 == nh ? N(nh) : std::max(N(l0), widest(l0 + 1)); }   // of layers l0 ... nh
   // the fused kernels (mlp_ws.cuh, k_mlp_fwd_tc / k_mlp_bwd_tc, k_bias_finish) take only nets of two hidden layers
   bool two_hidden() const { return nh == 2; }
 };
@@ -62,6 +65,19 @@ static NetD net_desc(const float* theta, long long sa, long long sn, int nnet, i
   for (int l = 0; l < nh; ++l) { d.hw[l] = hw[l]; d.ha[l] = ha[l]; }
   return d;
 }
+// The nets of a config, shape only: fill_layout and carve size from them, actor_net / critic_net / model_net bind them.
+static NetD actor_desc(const saceo_config& c) {
+  return net_desc(nullptr, 0, 0, 1, c.S, c.per_state_std ? 2 * c.A : c.A, 2, c.actor_hidden, c.actor_act);
+}
+static NetD critic_desc(const saceo_config& c) {
+  return net_desc(nullptr, 0, 0, 2, c.S + c.A, 1, 2, c.critic_hidden, c.critic_act);
+}
+static NetD model_desc(const saceo_config& c) {
+  return net_desc(nullptr, 0, 0, c.num_models, c.S + c.A, c.separate_reward_nn ? c.S : c.S + 1, c.model_layers,
+                  c.model_hidden, c.model_act);
+}
+// an actor's parameters: its layers, then without a per-state std its logstd variable (continuous_actors.py:56-57)
+static long long actor_params(const NetD& d, bool per_state_std) { return d.n() + (per_state_std ? 0 : d.out); }
 
 struct saceo_ctx {
   saceo_config cfg;
@@ -90,8 +106,10 @@ struct saceo_ctx {
   // bf16 hi/lo plane images of h1 / dH2 (actor: Rs rows, critics: B rows per net): operands of k_dw_planes
   uint8_t *aH1p = nullptr, *adH2p = nullptr, *cH1p = nullptr, *cdH2p = nullptr, *adH1p = nullptr, *cdH1p = nullptr;
   long long a_img = 0, c_img = 0;      // bytes per (agent, net) image
-  // model activations of each hidden layer and their gradients, [agent][2][E rows][width] (evaluation, expert term)
-  float *mH[MAXH] = {}, *mdH[MAXH] = {};
+  // activations of each hidden layer and their gradients, [agent][net][rows][width]: actor, critics, models (evaluation,
+  // expert term) and the actor on the fvp_rows states (with its input fX and the tangent fT of J x)
+  float *aH[MAXH] = {}, *daH[MAXH] = {}, *cH[MAXH] = {}, *cdH[MAXH] = {}, *mH[MAXH] = {}, *mdH[MAXH] = {};
+  float *fX = nullptr, *fH[MAXH] = {}, *fdH[MAXH] = {}, *fT[MAXH] = {};
   cudaStream_t s2 = nullptr, s3 = nullptr, s4 = nullptr;      // s3 / s4: the three independent weight-gradient GEMMs of a backward pass side by side
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_g = nullptr, ev_g3 = nullptr, ev_g4 = nullptr;
   // saceo_update_host_async: the H2D copies of step t+1 ride a copy stream into one of two device staging sets while step
@@ -102,6 +120,8 @@ struct saceo_ctx {
   bool hstage_used[2] = {false, false};
   int hslot = 0;
   FitCtx fit;             // dynamics-model fitting (saceo_fit_bind)
+  NetD fit_rnet{};        // its reward nets (separate_reward_nn)
+  float *fit_H[MAXH] = {}, *fit_dH[MAXH] = {}, *fit_rH[MAXH] = {}, *fit_rdH[MAXH] = {};   // per-layer H / dH of both
   bool fit_bound = false;
   void* fit_ws = nullptr;
   long long launches = 0;
@@ -171,23 +191,26 @@ struct Bump {   // workspace carver (also used dry to size it)
     off += bytes;
     return p;
   }
+  // one buffer of `rows` rows per hidden layer l of net n, named <name><l+1>; down: from the last layer to the first
+  void layers(float** H, const char* name, const NetD& n, long long rows, bool down = false) {
+    char nm[24];
+    for (int i = 0; i < n.nh; ++i) {
+      const int l = down ? n.nh - 1 - i : i;
+      snprintf(nm, sizeof(nm), "%s%d", name, l + 1);
+      H[l] = get<float>(nm, rows * n.N(l));
+    }
+  }
 };
 
 static void fill_layout(const saceo_config* c, saceo_layout* L) {
   memset(L, 0, sizeof(*L));
   const int S = c->S, A = c->A;
-  L->Ao = c->per_state_std ? 2 * A : A;
-  L->model_out = c->separate_reward_nn ? S : S + 1;
-  auto cnt = [](long long in, long long h1, long long h2, long long out) {
-    return in * h1 + h1 + h1 * h2 + h2 + h2 * out + out; };
-  L->na = cnt(S, c->actor_hidden[0], c->actor_hidden[1], L->Ao) + (c->per_state_std ? 0 : A);
-  L->nc = cnt(S + A, c->critic_hidden[0], c->critic_hidden[1], 1);
-  L->nm = 0;
-  for (int l = 0, in = S + A; c->num_models > 0 && l <= c->model_layers; ++l) {
-    const int w = l < c->model_layers ? c->model_hidden[l] : L->model_out;
-    L->nm += (long long)in * w + w;
-    in = w;
-  }
+  const NetD an = actor_desc(*c), mn = model_desc(*c);
+  L->Ao = an.out;
+  L->model_out = mn.out;
+  L->na = actor_params(an, c->per_state_std);
+  L->nc = critic_desc(*c).n();
+  L->nm = c->num_models > 0 ? mn.n() : 0;
   L->na_stride = rup(L->na + 1, 32);   // last padded word carries g_alpha in the grad buffer
   L->nc_stride = rup(L->nc, 32);
   L->nm_stride = rup(L->nm > 0 ? L->nm : 1, 32);
@@ -224,6 +247,9 @@ static void carve(saceo_ctx* x, char* base) {
   const long long n = c.n_agents;
   const int S = c.S, A = c.A, B = c.B, E = c.num_models > 0 ? c.E : 0, R = (int)rup(B + E, 32);   // padded row stride
   const int SA = S + A;
+  const NetD an = actor_desc(c), cn = critic_desc(c);
+  NetD mn = model_desc(c);
+  if (c.num_models == 0) for (int l = 0; l < mn.nh; ++l) mn.hw[l] = 1;   // no models: one-float placeholders
   k.idx = b.get<long long>("idx", n * B);
   k.noise = b.get<float>("noise", n * (3LL * B + E) * A);
   k.perm = b.get<int>("perm", n * (E > 0 ? E : 1));
@@ -231,9 +257,9 @@ static void carve(saceo_ctx* x, char* base) {
   k.mb_sp = b.get<float>("mb_sp", n * B * S); k.mb_r = b.get<float>("mb_r", n * B);
   k.mb_omd = b.get<float>("mb_omd", n * B);
   k.Xpi = b.get<float>("Xpi", n * R * rup(S, 4));
-  k.aH1 = b.get<float>("aH1", n * R * c.actor_hidden[0]);  k.aH2 = b.get<float>("aH2", n * R * c.actor_hidden[1]);
+  b.layers(x->aH, "aH", an, n * R);
   k.aOut = b.get<float>("aOut", n * R * L.Ao);             k.daOut = b.get<float>("daOut", n * R * L.Ao);
-  k.daH2 = b.get<float>("daH2", n * R * c.actor_hidden[1]); k.daH1 = b.get<float>("daH1", n * R * c.actor_hidden[0]);
+  b.layers(x->daH, "daH", an, n * R, true);
   k.dls = b.get<float>("dls", n * R * A);
   k.Xc = b.get<float>("Xc", n * B * rup(SA, 4));
   k.Xc2 = b.get<float>("Xc2", n * B * rup(SA, 4));
@@ -241,18 +267,15 @@ static void carve(saceo_ctx* x, char* base) {
   x->Xpi2 = b.get<float>("Xpi2", n * R * rup(S, 4));
   x->aOut2 = b.get<float>("aOut2", n * R * L.Ao);
   x->nlp2 = b.get<float>("nlp2", n * R);
-  k.cH1 = b.get<float>("cH1", n * 2 * B * c.critic_hidden[0]);  k.cH2 = b.get<float>("cH2", n * 2 * B * c.critic_hidden[1]);
+  b.layers(x->cH, "cH", cn, n * 2 * B);
   k.cQ = b.get<float>("cQ", n * 2 * B);                          k.cdQ = b.get<float>("cdQ", n * 2 * B);
-  k.cdH2 = b.get<float>("cdH2", n * 2 * B * c.critic_hidden[1]); k.cdH1 = b.get<float>("cdH1", n * 2 * B * c.critic_hidden[0]);
+  b.layers(x->cdH, "cdH", cn, n * 2 * B, true);
   k.cdXa = b.get<float>("cdXa", n * 2 * B * A);
   const long long e1 = E > 0 ? E : 1;
-  const int mnh = c.model_layers;
-  auto mh = [&](int l) -> long long { return c.num_models > 0 ? c.model_hidden[l] : 1; };
-  char nm[24];
   k.Xm = b.get<float>("Xm", n * 2 * e1 * SA);
-  for (int l = 0; l < mnh; ++l) { snprintf(nm, sizeof(nm), "mH%d", l + 1); x->mH[l] = b.get<float>(nm, n * 2 * e1 * mh(l)); }
+  b.layers(x->mH, "mH", mn, n * 2 * e1);
   k.mOut = b.get<float>("mOut", n * 2 * e1 * L.model_out); k.mdOut = b.get<float>("mdOut", n * 2 * e1 * S);
-  for (int l = mnh - 1; l >= 0; --l) { snprintf(nm, sizeof(nm), "mdH%d", l + 1); x->mdH[l] = b.get<float>(nm, n * 2 * e1 * mh(l)); }
+  b.layers(x->mdH, "mdH", mn, n * 2 * e1, true);
   k.mdXa = b.get<float>("mdXa", n * 2 * e1 * A);
   k.y = b.get<float>("y", n * B);  k.nlp = b.get<float>("nlp", n * R);
   k.g_q = b.get<float>("g_q", n * 2 * L.nc_stride);
@@ -289,14 +312,14 @@ static void carve(saceo_ctx* x, char* base) {
   const long long N = c.fvp_rows;
   f.N = (int)N;
   if (N > 0) {
-    f.X = b.get<float>("fX", n * N * S);
-    f.H1 = b.get<float>("fH1", n * N * c.actor_hidden[0]); f.H2 = b.get<float>("fH2", n * N * c.actor_hidden[1]);
+    x->fX = b.get<float>("fX", n * N * S);
+    b.layers(x->fH, "fH", an, n * N);
     f.Out = b.get<float>("fOut", n * N * L.Ao);
-    f.T1 = b.get<float>("fT1", n * N * c.actor_hidden[0]); f.T2 = b.get<float>("fT2", n * N * c.actor_hidden[1]);
-    f.Tmp = b.get<float>("fTmp", n * N * (long long)(c.actor_hidden[1] > L.Ao ? c.actor_hidden[1] : L.Ao));
+    b.layers(x->fT, "fT", an, n * N);
+    f.Tmp = b.get<float>("fTmp", n * N * an.widest(1));   // T[l-1].W_l of every layer l >= 1 (fvp_apply)
     f.TOut = b.get<float>("fTOut", n * N * L.Ao);
     f.G = b.get<float>("fG", n * N * L.Ao);
-    f.dH2 = b.get<float>("fdH2", n * N * c.actor_hidden[1]); f.dH1 = b.get<float>("fdH1", n * N * c.actor_hidden[0]);
+    b.layers(x->fdH, "fdH", an, n * N, true);
     f.gls = b.get<float>("fgls", n * N * A);
     f.p = b.get<float>("cg_p", n * L.na_stride); f.r = b.get<float>("cg_r", n * L.na_stride);
     f.z = b.get<float>("cg_z", n * L.na_stride); f.x = b.get<float>("cg_x", n * L.na_stride);
@@ -360,11 +383,7 @@ static int create_fill(saceo_ctx* x, const saceo_config* cfg) {
   k.B = cfg->B; k.E = cfg->num_models > 0 ? cfg->E : 0; k.R = k.B + k.E; k.Rs = (int)rup(k.R, 32); k.nmod = cfg->num_models;
   k.ldXc = (int)rup(cfg->S + cfg->A, 4); k.ldXp = (int)rup(cfg->S, 4);
   k.per_state_std = cfg->per_state_std; k.sep_reward = cfg->separate_reward_nn;
-  k.ah1 = cfg->actor_hidden[0]; k.ah2 = cfg->actor_hidden[1];
-  k.ch1 = cfg->critic_hidden[0]; k.ch2 = cfg->critic_hidden[1];
   k.mnh = cfg->model_layers; k.mh1 = cfg->model_hidden[0]; k.mh2 = cfg->model_hidden[1];
-  k.aact0 = cfg->actor_act[0]; k.aact1 = cfg->actor_act[1];
-  k.cact0 = cfg->critic_act[0]; k.cact1 = cfg->critic_act[1];
   k.mact0 = cfg->model_act[0]; k.mact1 = cfg->model_act[1];
   k.delta_clip = cfg->delta_clip_pred; k.cap = cfg->replay_capacity; k.L = x->L; k.eps_force = -1.f;
   // identity expert permutation until draws are injected / generated
@@ -511,8 +530,8 @@ struct Pass {
   NetD n;
   const float* X; int ldx; long long sXa, sXn;        // input rows
   int rows; long long rowsAllocH;                      // rows of the pass / rows per net allocated in H, dH
-  float* H[MAXH];                                      // saved activation of each hidden layer
-  float* dH[MAXH];                                     // its gradient (backward)
+  float* const* H;                                     // saved activation of each hidden layer
+  float* const* dH;                                    // its gradient (backward)
   uint8_t *H1p = nullptr, *dH2p = nullptr, *dH1p = nullptr;   // bf16 hi/lo plane images of h1 / dH2 / dH1
   long long sQa = 0, sQn = 0;                          // their bytes per agent / net
   // the caller guarantees that rows [rows, rowsAllocH) of X, H, dOut, dH are zero, so the
@@ -634,13 +653,13 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
     if (grads && l == 1 && fz.dw1_planes) {   // dW1 = H1^T . dH2 from the plane images
       DwP d{};
       d.Ap = ps.H1p; d.sAa = ps.sQa; d.sAn = ps.sQn; d.Bp = ps.dH2p; d.sBa = ps.sQa; d.sBn = ps.sQn;
-      d.G = grads + n.oW(1); d.sGa = n.sa; d.sGn = n.sn; d.rows = ps.rows; d.nnet = n.nnet;
+      d.G = grads + n.oW(l); d.sGa = n.sa; d.sGn = n.sn; d.rows = ps.rows; d.nnet = n.nnet;
       k_dw_planes<<<na * n.nnet, WS_NT, DW_BYTES, wst[1]>>>(d);
       count_launch(x, "k_dw_planes", wst[1]);
     } else if (grads && l == 0 && fz.dw0_planes) {   // dW0 = X^T . dH1 from the plane image
       Dw0P d{};
       d.X = ps.X; d.ldx = ps.ldx; d.sXa = ps.sXa; d.sXn = ps.sXn; d.Bp = ps.dH1p; d.sBa = ps.sQa; d.sBn = ps.sQn;
-      d.G = grads + n.oW(0); d.sGa = n.sa; d.sGn = n.sn; d.rows = ps.rows; d.in = n.in; d.nnet = n.nnet;
+      d.G = grads + n.oW(l); d.sGa = n.sa; d.sGn = n.sn; d.rows = ps.rows; d.in = n.in; d.nnet = n.nnet;
       k_dw0_planes<<<na * n.nnet, WS_NT, DW0_BYTES, wst[0]>>>(d);
       count_launch(x, "k_dw0_planes", wst[0]);
     } else if (grads) {   // [dW_l; db_l] = [Act_l, 1]^T . D_l+1, without the ones row where the fused kernel formed db_l
@@ -665,7 +684,7 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
       p.C = dH[l]; p.ldc = ld[l]; p.sCa = sa[l]; p.sCn = sn[l]; p.aux = Act[l];
       p.N = n.K(l); p.epi = EPI_MUL_DACT; p.act = n.act(l - 1);
     } else {
-      p.B += (long long)(n.in - A_cols) * n.N(0);
+      p.B += (long long)(n.in - A_cols) * n.N(l);
       p.C = dXa; p.ldc = A_cols; p.sCa = sXaA; p.sCn = sXaN; p.N = A_cols; p.epi = EPI_NONE;
     }
     p.M = ps.rows; p.K = l == nh ? ps.kout() : n.N(l);
@@ -724,23 +743,22 @@ static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd
 }
 
 static NetD actor_net(const saceo_ctx* x) {
-  const saceo_config& c = x->cfg;
-  NetD d = net_desc(x->k.T.actor, x->L.na_stride, 0, 1, c.S, x->L.Ao, 2, c.actor_hidden, c.actor_act);
-  d.planes = x->pl_actor; d.pa = ws_image_bytes(c.S, x->L.Ao); d.pn = 0;
+  NetD d = actor_desc(x->cfg);
+  d.theta = x->k.T.actor; d.sa = x->L.na_stride;
+  d.planes = x->pl_actor; d.pa = ws_image_bytes(d.in, d.out);
   return d;
 }
 static NetD critic_net(const saceo_ctx* x, bool target) {
-  const saceo_config& c = x->cfg;
-  NetD d = net_desc(target ? x->k.T.qt : x->k.T.q, 2 * x->L.nc_stride, x->L.nc_stride, 2, c.S + c.A, 1, 2, c.critic_hidden,
-                    c.critic_act);
-  d.planes = target ? x->pl_qt : x->pl_q; d.pn = ws_image_bytes(c.S + c.A, 1); d.pa = 2 * d.pn;
+  NetD d = critic_desc(x->cfg);
+  d.theta = target ? x->k.T.qt : x->k.T.q; d.sa = 2 * x->L.nc_stride; d.sn = x->L.nc_stride;
+  d.planes = target ? x->pl_qt : x->pl_q; d.pn = ws_image_bytes(d.in, 1); d.pa = 2 * d.pn;
   return d;
 }
 // the dynamics models (model_layers hidden layers) with parameters theta: the bound table, or the one being fitted
 static NetD model_net(const saceo_ctx* x, const float* theta, int nnet) {
-  const saceo_config& c = x->cfg;
-  return net_desc(theta, 2 * x->L.nm_stride, x->L.nm_stride, nnet, c.S + c.A, x->L.model_out, c.model_layers,
-                  c.model_hidden, c.model_act);
+  NetD d = model_desc(x->cfg);
+  d.theta = theta; d.sa = 2 * x->L.nm_stride; d.sn = x->L.nm_stride; d.nnet = nnet;
+  return d;
 }
 
 // Gives a pass the plane images if mlp_backward(grads) of it takes the plane path (fused chain + column-sum biases +
@@ -756,7 +774,7 @@ static void plane_path(const saceo_ctx* x, Pass& ps, uint8_t* H1p, uint8_t* dH2p
 // the actor on the staged observation rows Xpi of view k: <= B rows (TD target, temperature, acting) or the E expert
 // rows of the on-policy expert gradient
 static Pass actor_pass(const saceo_ctx* x, const KCtx& k, int rows) {
-  return Pass{actor_net(x), k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, rows, k.Rs, {k.aH1, k.aH2}, {k.daH1, k.daH2}};
+  return Pass{actor_net(x), k.Xpi, k.ldXp, (long long)k.Rs * k.ldXp, 0, rows, k.Rs, x->aH, x->daH};
 }
 // the actor update over its R = B + E rows
 static Pass actor_update_pass(const saceo_ctx* x, const KCtx& k) {
@@ -768,7 +786,7 @@ static Pass actor_update_pass(const saceo_ctx* x, const KCtx& k) {
 // twin critics (or their targets) on the first `rows` of B critic input rows X (Xc, Xc2 or Xc3)
 static Pass critic_pass(const saceo_ctx* x, bool target, const float* X, int rows) {
   const KCtx& k = x->k;
-  return Pass{critic_net(x, target), X, k.ldXc, (long long)k.B * k.ldXc, 0, rows, k.B, {k.cH1, k.cH2}, {k.cdH1, k.cdH2}};
+  return Pass{critic_net(x, target), X, k.ldXc, (long long)k.B * k.ldXc, 0, rows, k.B, x->cH, x->cdH};
 }
 // the critic update over the B minibatch rows
 static Pass critic_update_pass(const saceo_ctx* x) {
@@ -779,25 +797,18 @@ static Pass critic_update_pass(const saceo_ctx* x) {
 // the actor on the fvp_rows states (Fisher-vector product, CG, TRPO / PPO surrogate)
 static Pass fvp_pass(const saceo_ctx* x) {
   const KCtx& k = x->k; const FvpWs& f = x->f;
-  return Pass{actor_net(x), f.X, k.S, (long long)f.N * k.S, 0, f.N, f.N, {f.H1, f.H2}, {f.dH1, f.dH2}};
-}
-// a pass of the models over the staged rows X with the per-layer activation buffers H, dH
-static Pass model_pass(const NetD& n, const float* X, long long sXa, long long sXn, int rows, long long rowsAllocH,
-                       float* const* H, float* const* dH) {
-  Pass ps{n, X, n.in, sXa, sXn, rows, rowsAllocH, {}, {}};
-  for (int l = 0; l < n.nh; ++l) { ps.H[l] = H[l]; ps.dH[l] = dH[l]; }
-  return ps;
+  return Pass{actor_net(x), x->fX, k.S, (long long)f.N * k.S, 0, f.N, f.N, x->fH, x->fdH};
 }
 // the models on the first `rows` of the E staged rows of Xm; every model reads net 0's block (zero net stride)
 static Pass model_eval_pass(const saceo_ctx* x, int rows) {
   const KCtx& k = x->k; const int SA = k.S + k.A;
-  return model_pass(model_net(x, k.T.model, k.nmod), k.Xm, 2LL * k.E * SA, 0, rows, k.E, x->mH, x->mdH);
+  return Pass{model_net(x, k.T.model, k.nmod), k.Xm, SA, 2LL * k.E * SA, 0, rows, k.E, x->mH, x->mdH};
 }
 // the k.nmod frozen models of view k, each on its share of the E staged expert rows of Xm (expert-observation term)
 static Pass model_term_pass(const saceo_ctx* x, const KCtx& k) {
   const int SA = k.S + k.A;
-  Pass ps = model_pass(model_net(x, k.T.model, k.nmod), k.Xm, 2LL * k.E * SA, (long long)k.E * SA,
-                       k.nmod == 2 ? k.E / 2 : k.E, k.E, x->mH, x->mdH);
+  Pass ps{model_net(x, k.T.model, k.nmod), k.Xm, SA, 2LL * k.E * SA, (long long)k.E * SA, k.nmod == 2 ? k.E / 2 : k.E, k.E,
+          x->mH, x->mdH};
   ps.hnets = 2;         // the model buffers are carved [agent][2][E rows] whatever nmod, as k_model_loss reads mOut / mdOut
   ps.dout_cols = k.S;   // k_model_loss writes the S state columns of mdOut: the reward output column gets no gradient
   ps.fwd_f16 = false;   // the expert term's forward keeps the bf16 planes it has always used and been tested with
@@ -806,7 +817,7 @@ static Pass model_term_pass(const saceo_ctx* x, const KCtx& k) {
 // a model or reward net being fitted on the staged minibatch rows
 static Pass fit_pass(const saceo_ctx* x, const NetD& n, float* const* H, float* const* dH) {
   const FitCtx& f = x->fit; const int SA = x->cfg.S + x->cfg.A;
-  return model_pass(n, f.X, 2LL * f.mbs * SA, (long long)f.mbs * SA, f.mb, f.mbs, H, dH);
+  return Pass{n, f.X, SA, 2LL * f.mbs * SA, (long long)f.mbs * SA, f.mb, f.mbs, H, dH};
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1253,14 +1264,15 @@ extern "C" int saceo_fit_bind(saceo_ctx* x, const saceo_fit_tables* t, int32_t m
   if (!x || !t) return fail(SACEO_E_INVALID, "null argument");
   if (x->cfg.num_models < 1) return fail(SACEO_E_INVALID, "model fitting needs num_models >= 1");
   const bool sep = x->cfg.separate_reward_nn != 0;
+  NetD rn{};             // the reward nets
   if (sep) {
     if (!t->reward || !t->reward_m || !t->reward_v) return fail(SACEO_E_INVALID, "separate_reward_nn: the reward tables of saceo_fit_tables are required");
     if (t->reward_hidden[0] < 1 || t->reward_hidden[1] < 1) return fail(SACEO_E_INVALID, "reward_hidden must be positive");
     for (int i = 0; i < 2; ++i)
       if (t->reward_act[i] < 0 || t->reward_act[i] > SACEO_ACT_ELU) return fail(SACEO_E_INVALID, "bad reward activation");
-    const long long nr_ = (long long)(x->cfg.S + x->cfg.A) * t->reward_hidden[0] + t->reward_hidden[0] +
-                          (long long)t->reward_hidden[0] * t->reward_hidden[1] + t->reward_hidden[1] + t->reward_hidden[1] + 1;
-    if (t->reward_stride < nr_ || (t->reward_stride % 32) != 0) return fail(SACEO_E_INVALID, "reward_stride must be a multiple of 32 and >= %lld", nr_);
+    rn = net_desc(t->reward, 2 * t->reward_stride, t->reward_stride, x->cfg.num_models, x->cfg.S + x->cfg.A, 1, 2,
+                  t->reward_hidden, t->reward_act);
+    if (t->reward_stride < rn.n() || (t->reward_stride % 32) != 0) return fail(SACEO_E_INVALID, "reward_stride must be a multiple of 32 and >= %lld", rn.n());
   }
   if (model_batch < 1) return fail(SACEO_E_INVALID, "model_batch must be >= 1");
   if (!t->model || !t->model_m || !t->model_v || !t->model_t || !t->fit_hyper)
@@ -1279,31 +1291,26 @@ extern "C" int saceo_fit_bind(saceo_ctx* x, const saceo_fit_tables* t, int32_t m
   f.nm = x->L.nm; f.nm_stride = x->L.nm_stride;
   if (sep) {
     f.rw = t->reward; f.rw_m = t->reward_m; f.rw_v = t->reward_v;
-    f.rh1 = t->reward_hidden[0]; f.rh2 = t->reward_hidden[1]; f.ract0 = t->reward_act[0]; f.ract1 = t->reward_act[1];
-    f.nr_stride = t->reward_stride;
-    f.nr = (long long)(c.S + c.A) * f.rh1 + f.rh1 + (long long)f.rh1 * f.rh2 + f.rh2 + f.rh2 + 1;
+    f.nr_stride = t->reward_stride; f.nr = rn.n();
   }
+  x->fit_rnet = rn;
+  const NetD mn = model_desc(c);
   const long long n2 = 2LL * c.n_agents, mb = f.mbs, SA = c.S + c.A, mo = x->L.model_out;
   for (int pass = 0; pass < 2; ++pass) {
     Bump b{pass ? (char*)x->fit_ws : nullptr, 0, pass ? &x->names : nullptr};
     f.X = b.get<float>("fit_X", n2 * mb * SA);        f.T = b.get<float>("fit_T", n2 * mb * (c.S + 1));
-    char nm[24];
-    for (int l = 0; l < c.model_layers; ++l) {
-      snprintf(nm, sizeof(nm), "fit_H%d", l + 1); f.H[l] = b.get<float>(nm, n2 * mb * c.model_hidden[l]);
-    }
+    b.layers(x->fit_H, "fit_H", mn, n2 * mb);
     f.Out = b.get<float>("fit_Out", n2 * mb * mo);    f.dOut = b.get<float>("fit_dOut", n2 * mb * mo);
-    for (int l = c.model_layers - 1; l >= 0; --l) {
-      snprintf(nm, sizeof(nm), "fit_dH%d", l + 1); f.dH[l] = b.get<float>(nm, n2 * mb * c.model_hidden[l]);
-    }
+    b.layers(x->fit_dH, "fit_dH", mn, n2 * mb, true);
     f.g = b.get<float>("g_model", n2 * x->L.nm_stride);
     f.loss_part = b.get<float>("fit_loss", n2);
     f.g_ls = b.get<float>("g_model_logstd", n2 * c.S);
     f.gscale = b.get<float>("fit_gscale", c.n_agents); f.gnorm = b.get<float>("fit_gnorm", c.n_agents);
     f.lrt = b.get<float>("fit_lrt", c.n_agents);
     if (sep) {
-      f.rH1 = b.get<float>("fit_rH1", n2 * mb * f.rh1); f.rH2 = b.get<float>("fit_rH2", n2 * mb * f.rh2);
+      b.layers(x->fit_rH, "fit_rH", rn, n2 * mb);
       f.rOut = b.get<float>("fit_rOut", n2 * mb);       f.rdOut = b.get<float>("fit_rdOut", n2 * mb);
-      f.rdH2 = b.get<float>("fit_rdH2", n2 * mb * f.rh2); f.rdH1 = b.get<float>("fit_rdH1", n2 * mb * f.rh1);
+      b.layers(x->fit_rdH, "fit_rdH", rn, n2 * mb, true);
       f.g_r = b.get<float>("g_reward", n2 * f.nr_stride);
     }
     if (!pass) {
@@ -1328,11 +1335,8 @@ extern "C" int saceo_model_fit(saceo_ctx* x, int32_t n_steps, const int64_t* idx
   cudaStream_t st = (cudaStream_t)stream;
   const KCtx& k = x->k; const FitCtx& f = x->fit;
   const int n = k.n_agents, mb = f.mb, ms = f.mbs, SA = k.S + k.A, mo = x->L.model_out;
-  const Pass mp = fit_pass(x, model_net(x, f.model, f.nmod), f.H, f.dH);
-  const int rh[2] = {f.rh1, f.rh2}, ra[2] = {f.ract0, f.ract1};
-  float* const rH[2] = {f.rH1, f.rH2};
-  float* const rdH[2] = {f.rdH1, f.rdH2};
-  const Pass rp = fit_pass(x, net_desc(f.rw, 2 * f.nr_stride, f.nr_stride, f.nmod, SA, 1, 2, rh, ra), rH, rdH);
+  const Pass mp = fit_pass(x, model_net(x, f.model, f.nmod), x->fit_H, x->fit_dH);
+  const Pass rp = fit_pass(x, x->fit_rnet, x->fit_rH, x->fit_rdH);
   for (int s = 0; s < n_steps; ++s) {
     const long long* ix = reinterpret_cast<const long long*>(idx) + (long long)s * n * f.nmod * mb;
     LAUNCH(x, k_fit_begin, cdiv(n, 128), 128, 0, st, f, n);
@@ -1365,7 +1369,7 @@ extern "C" int saceo_model_fit(saceo_ctx* x, int32_t n_steps, const int64_t* idx
 static int fvp_prepare(saceo_ctx* x, cudaStream_t st) {
   { int rcp = ensure_planes(x, st); if (rcp) return rcp; }
   const KCtx& k = x->k; const FvpWs& f = x->f; const int n = k.n_agents, N = f.N;
-  LAUNCH(x, k_stage_obs, dim3(cdiv((long long)N * k.S, 256), n), 256, 0, st, k, k.T.fvp_states, N, 0, N, f.X, k.S,
+  LAUNCH(x, k_stage_obs, dim3(cdiv((long long)N * k.S, 256), n), 256, 0, st, k, k.T.fvp_states, N, 0, N, x->fX, k.S,
          (long long)N * k.S, 0);
   return mlp_forward(x, fvp_pass(x), f.Out, k.Ao, (long long)N * k.Ao, 0, st);
 }
@@ -1375,29 +1379,26 @@ static int fvp_apply(saceo_ctx* x, const float* xin, float damp, float* Fx, cuda
   const KCtx& k = x->k; const FvpWs& f = x->f; const int n = k.n_agents, N = f.N;
   NetD an = actor_net(x);
   NetD tn = an; tn.theta = xin;                       // tangent "network": same flat layout
-  const long long sH1 = (long long)N * an.N(0), sH2 = (long long)N * an.N(1), sO = (long long)N * k.Ao;
-  int rc; GemmP p{};
-  // T1 = (X.P0 + c0) * act0'(H1)
-  p = GemmP{}; p.nnet = 1; p.A = f.X; p.lda = k.S; p.sAa = (long long)N * k.S;
-  p.B = tn.theta + tn.oW(0); p.ldb = an.N(0); p.sBa = an.sa; p.bias = tn.theta + tn.ob(0); p.sba = an.sa;
-  p.C = f.T1; p.ldc = an.N(0); p.sCa = sH1; p.aux = f.H1; p.M = N; p.N = an.N(0); p.K = k.S; p.epi = EPI_MUL_DACT; p.act = an.act(0);
-  rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  // Tmp = T1.W1 ;  T2 = (H1.P1 + c1 + Tmp) * act1'(H2)
-  p = GemmP{}; p.nnet = 1; p.A = f.T1; p.lda = an.N(0); p.sAa = sH1; p.B = an.theta + an.oW(1); p.ldb = an.N(1); p.sBa = an.sa;
-  p.C = f.Tmp; p.ldc = an.N(1); p.sCa = sH2; p.M = N; p.N = an.N(1); p.K = an.N(0); p.epi = EPI_NONE;
-  rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  p = GemmP{}; p.nnet = 1; p.A = f.H1; p.lda = an.N(0); p.sAa = sH1; p.B = tn.theta + tn.oW(1); p.ldb = an.N(1); p.sBa = an.sa;
-  p.bias = tn.theta + tn.ob(1); p.sba = an.sa; p.addend = f.Tmp; p.aux = f.H2;
-  p.C = f.T2; p.ldc = an.N(1); p.sCa = sH2; p.M = N; p.N = an.N(1); p.K = an.N(0); p.epi = EPI_MUL_DACT; p.act = an.act(1);
-  rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  // Tmp = T2.W2 ; TOut = H2.P2 + c2 + Tmp
-  p = GemmP{}; p.nnet = 1; p.A = f.T2; p.lda = an.N(1); p.sAa = sH2; p.B = an.theta + an.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
-  p.C = f.Tmp; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.N(1); p.epi = EPI_NONE;
-  rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
-  p = GemmP{}; p.nnet = 1; p.A = f.H2; p.lda = an.N(1); p.sAa = sH2; p.B = tn.theta + tn.oW(2); p.ldb = k.Ao; p.sBa = an.sa;
-  p.bias = tn.theta + tn.ob(2); p.sba = an.sa; p.addend = f.Tmp;
-  p.C = f.TOut; p.ldc = k.Ao; p.sCa = sO; p.M = N; p.N = k.Ao; p.K = an.N(1); p.epi = EPI_NONE;
-  rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
+  const long long sO = (long long)N * k.Ao;
+  int rc;
+  // J x layer by layer: T[0] = (X.P0 + c0) * act0'(H[0]);  T[l] = (H[l-1].P_l + c_l + Tmp) * act_l'(H[l]) with
+  // Tmp = T[l-1].W_l;  the output layer writes TOut, without the activation factor
+  for (int l = 0; l <= an.nh; ++l) {
+    const int K = an.K(l), W = an.N(l);
+    const long long sK = (long long)N * K, sW = (long long)N * W;
+    GemmP p{};
+    if (l > 0) {
+      p.nnet = 1; p.A = x->fT[l - 1]; p.lda = K; p.sAa = sK; p.B = an.theta + an.oW(l); p.ldb = W; p.sBa = an.sa;
+      p.C = f.Tmp; p.ldc = W; p.sCa = sW; p.M = N; p.N = W; p.K = K; p.epi = EPI_NONE;
+      rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
+      p = GemmP{}; p.addend = f.Tmp;
+    }
+    p.nnet = 1; p.A = l > 0 ? x->fH[l - 1] : x->fX; p.lda = K; p.sAa = sK; p.B = tn.theta + tn.oW(l); p.ldb = W; p.sBa = an.sa;
+    p.bias = tn.theta + tn.ob(l); p.sba = an.sa;
+    p.C = l < an.nh ? x->fT[l] : f.TOut; p.ldc = W; p.sCa = sW; p.M = N; p.N = W; p.K = K; p.epi = EPI_NONE;
+    if (l < an.nh) { p.aux = x->fH[l]; p.epi = EPI_MUL_DACT; p.act = an.act(l); }
+    rc = gemm(x, false, false, false, p, n, st); if (rc) return rc;
+  }
   // metric: G = M . J x / N   (per row), plus per-row logstd_var contribution
   LAUNCH(x, k_fvp_metric, dim3(cdiv(N, 128), n), 128, 0, st, k, f, xin, x->cfg.std_mult);
   // J^T G  -> Fx (flat layout), then + damp x
@@ -1439,8 +1440,8 @@ extern "C" int saceo_cg_solve(saceo_ctx* x, const float* b, int32_t iters, float
 static int trpo_check(saceo_ctx* x) {
   if (!x) return fail(SACEO_E_INVALID, "null ctx");
   if (!x->bound || !x->k.T.fvp_states || x->f.N < 1) return fail(SACEO_E_UNBOUND, "fvp_states not bound / fvp_rows == 0");
-  // the four per-row statistics live in the [N, max(h2, Ao)] scratch of the Fisher-vector workspace
-  if (x->cfg.actor_hidden[1] < 4 && x->L.Ao < 4) return fail(SACEO_E_INVALID, "TRPO / PPO entry points need actor_hidden[1] >= 4");
+  // the four per-row statistics live in the Tmp scratch of the Fisher-vector workspace, [N, widest layer past the first]
+  if (actor_net(x).widest(1) < 4) return fail(SACEO_E_INVALID, "TRPO / PPO entry points need actor_hidden[1] >= 4");
   return 0;
 }
 
@@ -1510,11 +1511,11 @@ extern "C" int saceo_grad_blend(saceo_ctx* x, const float* neg_pg, const float* 
                                 float* out, float* stats_out, void* stream) {
   if (!x || !neg_pg || !mse_grad || !eps || !out) return fail(SACEO_E_INVALID, "null argument");
   cudaStream_t st = (cudaStream_t)stream; const KCtx& k = x->k;
-  NetD an = actor_net(x);
-  BlendSeg sg{};
-  const long long bnd[8] = {0, an.ob(0), an.oW(1), an.ob(1), an.oW(2), an.ob(2), an.ob(2) + an.out, x->L.na};
-  sg.nseg = (x->L.na > bnd[6]) ? 7 : 6;           // + the state-independent logstd variable
-  for (int i = 0; i < 8; ++i) sg.b[i] = bnd[i];
+  const NetD an = actor_net(x);
+  BlendSeg sg{};                                   // the bounds of every weight and bias tensor
+  for (int l = 0; l <= an.nh; ++l) { sg.b[sg.nseg++] = an.oW(l); sg.b[sg.nseg++] = an.ob(l); }
+  sg.b[sg.nseg] = an.n();
+  if (x->L.na > an.n()) sg.b[++sg.nseg] = x->L.na;  // + the state-independent logstd variable
   LAUNCH(x, k_grad_blend, dim3(k.n_agents), 256, 0, st, k, sg, neg_pg, mse_grad, eps, out, stats_out);
   if (max_grad_norm > 0.f || stats_out) LAUNCH(x, k_grad_clip, dim3(k.n_agents), 256, 0, st, k, out, max_grad_norm, stats_out);
   return check_launch();
@@ -1573,17 +1574,12 @@ static int policy_validate(const saceo_policy_config* c) {
 }
 
 static void policy_layout(const saceo_policy_config* c, long long* n, long long* stride, int* nstride, long long* off) {
-  const int Ao = c->per_state_std ? 2 * c->A : c->A;
-  long long o = 0; int in = c->S;
-  for (int l = 0; l <= c->n_hidden; ++l) {
-    const int outw = l < c->n_hidden ? c->hidden[l] : Ao;
-    if (off) off[l] = o;
-    o += (long long)in * outw + outw;
-    in = outw;
+  const NetD d = net_desc(nullptr, 0, 0, 1, c->S, c->per_state_std ? 2 * c->A : c->A, c->n_hidden, c->hidden, c->act);
+  if (off) {
+    for (int l = 0; l <= d.nh; ++l) off[l] = d.oW(l);
+    off[d.nh + 1] = d.n();
   }
-  if (off) off[c->n_hidden + 1] = o;
-  if (!c->per_state_std) o += c->A;          // logstd variable (continuous_actors.py:56-57)
-  *n = o; *stride = rup(o, 32); *nstride = (int)rup(2LL * c->S + c->A, 4);
+  *n = actor_params(d, c->per_state_std); *stride = rup(*n, 32); *nstride = (int)rup(2LL * c->S + c->A, 4);
 }
 
 extern "C" int saceo_policy_layout(const saceo_policy_config* cfg, int64_t* n_params, int64_t* param_stride,
