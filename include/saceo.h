@@ -93,8 +93,8 @@ typedef struct saceo_config {
   int32_t reserved[8];        /* tuning switches, 0 = default: [0] tcgen05 tile variant (0: 128x256 tile, 1: 128x128 2 CTAs/SM,
                                  2: force the register-staged kernel); [1] != 0 disables the fused 3-layer forward kernel;
                                  [2] != 0 disables the fused backward-chain kernel;
-                                 [5] != 0 disables the warp-specialised TMA-fed fused kernels and their weight planes
-                                 (round-1 fused kernels are used instead); [6] != 0 keeps the whole update on one stream (no
+                                 [5] != 0 disables the weight planes and with them the warp-specialised TMA-fed fused
+                                 kernels: every MLP pass runs on the per-layer GEMM chain; [6] != 0 keeps the whole update on one stream (no
                                  concurrent actor-phase branch); [3], [4], [7] must be 0 (SACEO_E_INVALID otherwise) */
 } saceo_config;
 

@@ -1,6 +1,7 @@
 // Warp-specialised fused forward / backward chains of the 2x256 MLPs (actor, twin critics, twin targets), round 2.
 //
-// What changed against the round-1 kernels (tc_gemm.cuh::k_mlp_fwd_tc / k_mlp_bwd_tc, kept as the fallback engine):
+// What changed against the round-1 fused kernels (in-kernel operand conversion; since retired: nets these kernels do not
+// take run on the per-layer GEMM chain):
 //   * WEIGHT PLANES.  The fp32 -> fp16 hi/lo operand split of W0 and W1 is no longer done by every CTA for every
 //     128-row tile of every pass (the convert -> fence -> barrier chain that bounded the W1 loop, 7.05 us against
 //     3.25 us of pure streaming).  The optimiser owns it: k_adam (and its Polyak line) emits the split planes of
@@ -37,6 +38,7 @@
 
 namespace saceo {
 
+constexpr int FW_H = 256;                     // hidden width of the nets these kernels take
 constexpr int WS_NEW = 16;                    // conversion / epilogue warps: 4 TMEM lane quarters x 4 column groups of 64
 constexpr int WS_NEPI = WS_NEW * 32, WS_NT = WS_NEPI + 64;    // + TMA producer warp + MMA / TMEM-allocator warp
 constexpr int WS_NST = 3, WS_RING = WS_NST * WS_STAGE;
@@ -68,6 +70,22 @@ __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 512;" ::: 
 __device__ __forceinline__ uint64_t umma_desc_mn(uint32_t saddr, uint32_t lbo = 4096) {
   return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) |
          ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
+}
+__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t db, uint32_t idesc, uint32_t acc) {
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+               "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+               ::"r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(acc) : "memory");
+}
+__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+               "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
+               "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                 "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
+                 "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
+                 "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+               : "r"(taddr) : "memory");
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 constexpr uint32_t WS_IDESC_FWD = (1u << 4) | (1u << 16) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);  // fp16, B MN-major, N 256
 constexpr uint32_t WS_IDESC_BWD = (1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);              // fp16, K-major, N 128
@@ -1048,6 +1066,17 @@ __global__ void __launch_bounds__(WS_NT, 1) k_mlp_bwd_ws(BwdW f) {
   if (warp == WS_NEW + 1) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512) : "memory");
   }
+}
+
+// g[ob1 + c] = sum_tiles dbpart[.][tile][0][c],  g[ob0 + c] = sum_tiles dbpart[.][tile][1][c]   (fixed tile order)
+// grid: (n_agents * nnet), block 512
+__global__ void k_bias_finish(const float* __restrict__ dbpart, int ntiles, float* __restrict__ g, long long sGa, long long sGn,
+                              int nnet, long long ob1, long long ob0) {
+  const int z = blockIdx.x, agent = z / nnet, net = z - agent * nnet;
+  const int t = threadIdx.x & (FW_H - 1), which = threadIdx.x >> 8;
+  float acc = 0.f;
+  for (int tile = 0; tile < ntiles; ++tile) acc += dbpart[(((long long)z * ntiles + tile) * 2 + which) * FW_H + t];
+  g[agent * sGa + net * sGn + (which ? ob0 : ob1) + t] = acc;
 }
 
 // ==========================================================================================

@@ -56,8 +56,12 @@ struct NetD {            // one (population of) MLP(s) in the flat Keras layout:
   long long ob(int l) const { return oW(l) + (long long)K(l) * N(l); }
   long long n() const { return ob(nh) + N(nh); }                                      // parameters
   int widest(int l0) const { return l0 == nh ? N(nh) : std::max(N(l0), widest(l0 + 1)); }   // of layers l0 ... nh
-  // the fused kernels (mlp_ws.cuh, k_mlp_fwd_tc / k_mlp_bwd_tc, k_bias_finish) take only nets of two hidden layers
-  bool two_hidden() const { return nh == 2; }
+  // the warp-specialised fused kernels (mlp_ws.cuh) take this net in both directions: two FW_H-wide hidden layers,
+  // 1 to WS_MAXOUT outputs, 16-byte aligned parameters.  Every other net runs on the per-layer GEMM chain.
+  bool ws() const {
+    return nh == 2 && mlp_fwd_ws_eligible(N(0), N(1), out, in, theta, sa, sn) &&
+           mlp_bwd_ws_eligible(N(0), N(1), out, out, false, 0, theta, sa, sn);
+  }
 };
 static NetD net_desc(const float* theta, long long sa, long long sn, int nnet, int in, int out, int nh, const int* hw,
                      const int* ha) {
@@ -84,8 +88,8 @@ struct saceo_ctx {
   // engine switches, decoded once from cfg.gemm_mode and the cfg.reserved tuning switches (include/saceo.h)
   bool tc = false;                     // tcgen05 bf16x3 GEMM engine
   int tc_variant = 0;                  // its tile variant
-  bool fuse_fwd = false, fuse_bwd = false;   // fused 3-layer forward / backward-chain kernels (tcgen05 engine only)
-  bool ws_kernels = false;             // warp-specialised TMA-fed fused kernels and their weight planes (tcgen05 engine only)
+  bool fuse_fwd = false, fuse_bwd = false;   // fused forward / backward-chain kernel (needs ws_kernels)
+  bool ws_kernels = false;             // weight-plane images for the warp-specialised fused kernels (tcgen05 engine only)
   bool fork = false;                   // side streams: the concurrent actor-phase branch and the weight-gradient fan-out
   saceo_layout L;
   KCtx k;                 // device-visible view (tables + workspace)
@@ -293,13 +297,13 @@ static void carve(saceo_ctx* x, char* base) {
   x->pl_actor = x->pl_q = x->pl_qt = nullptr;
   x->aH1p = x->adH2p = x->cH1p = x->cdH2p = x->adH1p = x->cdH1p = nullptr;
   x->a_img = (long long)(R / 32) * WS_STAGE; x->c_img = (long long)(rup(B, 32) / 32) * WS_STAGE;
-  if (x->ws_kernels) {
-    if (c.actor_hidden[0] == FW_H && c.actor_hidden[1] == FW_H) {
+  if (x->ws_kernels) {   // plane images only for the nets the fused kernels take
+    if (an.ws()) {
       x->pl_actor = b.get<uint8_t>("pl_actor", n * ws_image_bytes(S, L.Ao));
       x->aH1p = b.get<uint8_t>("aH1p", n * x->a_img); x->adH2p = b.get<uint8_t>("adH2p", n * x->a_img);
       x->adH1p = b.get<uint8_t>("adH1p", n * x->a_img);
     }
-    if (c.critic_hidden[0] == FW_H && c.critic_hidden[1] == FW_H) {
+    if (cn.ws()) {
       x->pl_q = b.get<uint8_t>("pl_q", n * 2 * ws_image_bytes(SA, 1));
       x->pl_qt = b.get<uint8_t>("pl_qt", n * 2 * ws_image_bytes(SA, 1));
       x->cH1p = b.get<uint8_t>("cH1p", n * 2 * x->c_img); x->cdH2p = b.get<uint8_t>("cdH2p", n * 2 * x->c_img);
@@ -401,7 +405,6 @@ static int create_fill(saceo_ctx* x, const saceo_config* cfg) {
   CU(cudaEventCreateWithFlags(&x->ev_g3, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&x->ev_g4, cudaEventDisableTiming));
   CU(tc_gemm_init());
-  CU(mlp_fwd_tc_init());
   CU(mlp_ws_init());
   CU(model_term_init());
   return 0;
@@ -545,11 +548,10 @@ struct Pass {
   int kout() const { return dout_cols ? dout_cols : n.out; }
 };
 
-// forward through one population of MLPs (nn_utils.py:101-136), rows [row0, rows), unfused: one GEMM per layer
-static int mlp_forward_unfused(saceo_ctx* x, const Pass& ps, int row0, float* Out, int ldo, long long sOa, long long sOn,
-                               cudaStream_t st) {
+// forward through one population of MLPs (nn_utils.py:101-136), unfused: one GEMM per layer
+static int mlp_forward_unfused(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long long sOa, long long sOn, cudaStream_t st) {
   const NetD& n = ps.n;
-  const float* A = ps.X + (long long)row0 * ps.ldx; int lda = ps.ldx; long long sAa = ps.sXa, sAn = ps.sXn;
+  const float* A = ps.X; int lda = ps.ldx; long long sAa = ps.sXa, sAn = ps.sXn;
   for (int l = 0; l <= n.nh; ++l) {
     GemmP p{}; p.nnet = n.nnet; p.f16 = ps.fwd_f16;
     p.A = A; p.lda = lda; p.sAa = sAa; p.sAn = sAn;
@@ -557,22 +559,22 @@ static int mlp_forward_unfused(saceo_ctx* x, const Pass& ps, int row0, float* Ou
     p.bias = n.theta + n.ob(l); p.sba = n.sa; p.sbn = n.sn;
     if (l < n.nh) { p.C = ps.H[l]; p.ldc = n.N(l); p.sCa = ps.sHa(n.N(l)); p.sCn = ps.sHn(n.N(l)); }
     else { p.C = Out; p.ldc = ldo; p.sCa = sOa; p.sCn = sOn; }
-    p.C += (long long)row0 * p.ldc;
-    p.M = ps.rows - row0; p.N = n.N(l); p.K = n.K(l); p.epi = l < n.nh ? EPI_ACT : EPI_NONE; p.act = n.act(l);
+    p.M = ps.rows; p.N = n.N(l); p.K = n.K(l); p.epi = l < n.nh ? EPI_ACT : EPI_NONE; p.act = n.act(l);
     int rc = gemm(x, false, false, false, p, x->cfg.n_agents, st); if (rc) return rc;
     A = p.C; lda = p.ldc; sAa = p.sCa; sAn = p.sCn;
   }
   return 0;
 }
 
-// Forward pass dispatcher: full 128-row tiles of 2x256 nets go through the fused tcgen05 kernel (activations
-// stay in TMEM between layers; h1/h2 reach HBM only when save_h), leftover rows through the GEMM chain.
+// whether mlp_forward runs net n in k_mlp_fwd_ws, which writes no hidden activation unless asked to (save_h)
+static bool fwd_ws(const saceo_ctx* x, const NetD& n) { return n.planes && x->fuse_fwd && n.ws(); }
+
+// Forward pass dispatcher: nets with a weight-plane image go through the warp-specialised fused kernel (activations
+// stay in TMEM between layers; h1/h2 reach HBM only when save_h), every other net through the GEMM chain.
 static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long long sOa, long long sOn, cudaStream_t st,
                        bool save_h = true) {
   const NetD& n = ps.n;
-  const int rows = ps.rows;
-  int row0 = 0;
-  if (n.planes && x->fuse_fwd && n.two_hidden() && mlp_fwd_ws_eligible(n.N(0), n.N(1), n.out, n.in, n.theta, n.sa, n.sn)) {
+  if (fwd_ws(x, n)) {
     // warp-specialised kernel on the TMA-fed weight planes: every row (partial tiles are masked)
     FwdW f{};
     f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
@@ -581,29 +583,13 @@ static int mlp_forward(saceo_ctx* x, const Pass& ps, float* Out, int ldo, long l
     f.H1 = save_h ? ps.H[0] : nullptr; f.H2 = save_h ? ps.H[1] : nullptr; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
     f.H1p = save_h ? ps.H1p : nullptr; f.sQa = ps.sQa; f.sQn = ps.sQn;
     f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
-    f.rows = rows; f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1);
+    f.rows = ps.rows; f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1);
     f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
     if (mlp_fwd_ws_launch(f, x->cfg.n_agents, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused forward launch failed");
     count_launch(x, "k_mlp_fwd_ws", st);
     return 0;
   }
-  if (x->fuse_fwd && n.two_hidden() && mlp_fwd_tc_eligible(n.N(0), n.N(1), n.out, rows, n.theta, n.sa, n.sn, n.in)) {
-    int tiles = rows / TC_BM;
-    if (rows % TC_BM >= 16) tiles += 1;
-    FwdP f{};
-    f.X = ps.X; f.ldx = ps.ldx; f.sXa = ps.sXa; f.sXn = ps.sXn;
-    f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn;
-    f.H1 = save_h ? ps.H[0] : nullptr; f.H2 = save_h ? ps.H[1] : nullptr; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
-    f.Out = Out; f.ldo = ldo; f.sOa = sOa; f.sOn = sOn;
-    f.rows = tiles * TC_BM < rows ? tiles * TC_BM : rows;
-    f.K0 = n.in; f.nout = n.out; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1); f.dbg = g_tc_dbg;
-    dim3 grid(tiles, x->cfg.n_agents * n.nnet);
-    k_mlp_fwd_tc<<<grid, FW_NT, FW_BYTES, st>>>(f);
-    count_launch(x, "k_mlp_fwd_tc", st);
-    row0 = f.rows;
-    if (row0 >= rows) return 0;
-  }
-  return mlp_forward_unfused(x, ps, row0, Out, ldo, sOa, sOn, st);
+  return mlp_forward_unfused(x, ps, Out, ldo, sOa, sOn, st);
 }
 
 // The fused backward kernels index dbpart as [agent*nnet+net][tile][2][256]: callers with more row tiles than the
@@ -695,43 +681,33 @@ static int mlp_backward_layers(saceo_ctx* x, const Pass& ps, const float* dOut, 
 
 // backward through the same MLPs.  grads (nullable): flat [W|b] blocks in the layout of theta, via the ones-row trick.
 // dXa (nullable): gradient w.r.t. the last A_cols (action) columns of the input only (their rows of W0).
-// The fused gradient chain (dH2, dH1, dXa) runs on tensor cores with the tile resident in TMEM where a kernel takes the
-// pass; the per-layer loop does the rest.
+// The fused gradient chain (dH2, dH1, dXa) runs on tensor cores with the tile resident in TMEM where the warp-specialised
+// kernel takes the pass; the per-layer loop does the rest.
 static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd, long long sDa, long long sDn,
                         float* grads, float* dXa, int A_cols, long long sXaA, long long sXaN, cudaStream_t st) {
   const NetD& n = ps.n;
   const int na = x->cfg.n_agents, rows = ps.rows, tiles = cdiv(rows, TC_BM);
   BwdFused fz;
-  const bool ws = n.planes && x->fuse_bwd && n.two_hidden() &&
-                  mlp_bwd_ws_eligible(n.N(0), n.N(1), ps.kout(), n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn);
-  if (ws || (x->fuse_bwd && n.two_hidden() &&
-             mlp_bwd_tc_eligible(n.N(0), n.N(1), n.out, rows, dXa != nullptr, A_cols, n.theta, n.sa, n.sn))) {
+  if (n.planes && x->fuse_bwd && n.ws() &&   // and the kernel has a variant for this pass's dOut width and dXa columns
+      mlp_bwd_ws_eligible(n.N(0), n.N(1), ps.kout(), n.out, dXa != nullptr, A_cols, n.theta, n.sa, n.sn)) {
     float* dbpart = grads && dbpart_fits(x, n, rows) ? x->dbpart : nullptr;
-    auto chain = [&](auto& f) {    // the fields BwdW and BwdP share
-      f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = ps.kout();
-      f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
-      f.H1 = ps.H[0]; f.H2 = ps.H[1]; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
-      f.dH2 = grads ? ps.dH[1] : nullptr; f.dH1 = grads ? ps.dH[0] : nullptr;
-      f.dXa = dXa; f.s_cols = n.in - A_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
-      f.rows = rows; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1); f.dbpart = dbpart;
-    };
-    if (ws) {
-      BwdW f{}; chain(f);
-      f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
-      // hidden-to-hidden weight gradient from bf16 plane images (k_dw_planes): dH2 then leaves the kernel as planes only
-      fz.dw1_planes = dbpart && ps.H1p;
-      if (fz.dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
-      // first-layer weight gradient from the dH1 plane image (k_dw0_planes): dH1 then leaves the kernel as planes only
-      fz.dw0_planes = fz.dw1_planes && ps.dH1p && dw0_planes_eligible(n.in, rows, ps.ldx, ps.X, ps.sXa, ps.sXn);
-      if (fz.dw0_planes) { f.dH1 = nullptr; f.dH1p = ps.dH1p; }
-      f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
-      if (mlp_bwd_ws_launch(f, na, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused backward launch failed");
-      count_launch(x, "k_mlp_bwd_ws", st);
-    } else {
-      BwdP f{}; chain(f);
-      k_mlp_bwd_tc<<<dim3(tiles, na * n.nnet), FW_NT, FW_BYTES, st>>>(f);
-      count_launch(x, "k_mlp_bwd_tc", st);
-    }
+    BwdW f{};
+    f.dOut = dOut; f.ldd = ldd; f.sDa = sDa; f.sDn = sDn; f.kout = ps.kout();
+    f.theta = n.theta; f.sTa = n.sa; f.sTn = n.sn; f.K0 = n.in; f.nout = n.out;
+    f.planes = n.planes; f.sPa = n.pa; f.sPn = n.pn;
+    f.H1 = ps.H[0]; f.H2 = ps.H[1]; f.sHa = ps.sHa(n.N(0)); f.sHn = ps.sHn(n.N(0));
+    f.dH2 = grads ? ps.dH[1] : nullptr; f.dH1 = grads ? ps.dH[0] : nullptr;
+    f.dXa = dXa; f.s_cols = n.in - A_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
+    f.rows = rows; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1); f.dbpart = dbpart;
+    // hidden-to-hidden weight gradient from bf16 plane images (k_dw_planes): dH2 then leaves the kernel as planes only
+    fz.dw1_planes = dbpart && ps.H1p;
+    if (fz.dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
+    // first-layer weight gradient from the dH1 plane image (k_dw0_planes): dH1 then leaves the kernel as planes only
+    fz.dw0_planes = fz.dw1_planes && ps.dH1p && dw0_planes_eligible(n.in, rows, ps.ldx, ps.X, ps.sXa, ps.sXn);
+    if (fz.dw0_planes) { f.dH1 = nullptr; f.dH1p = ps.dH1p; }
+    f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
+    if (mlp_bwd_ws_launch(f, na, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused backward launch failed");
+    count_launch(x, "k_mlp_bwd_ws", st);
     fz.chain = true;
     if (dbpart) {     // bias gradients of the two hidden layers come from the kernel's column sums
       k_bias_finish<<<na * n.nnet, 2 * FW_H, 0, st>>>(dbpart, tiles, grads, n.sa, n.sn, n.nnet, n.ob(1), n.ob(0));
@@ -765,9 +741,7 @@ static NetD model_net(const saceo_ctx* x, const float* theta, int nnet) {
 // k_dw_planes); decided once, so that its forward and backward calls cannot disagree.
 static void plane_path(const saceo_ctx* x, Pass& ps, uint8_t* H1p, uint8_t* dH2p, uint8_t* dH1p, long long sQa, long long sQn) {
   const NetD& n = ps.n;
-  if (!n.planes || !x->fuse_bwd || !x->fuse_fwd || !H1p || !dH2p || !dbpart_fits(x, n, ps.rows)) return;
-  if (!n.two_hidden() || !mlp_bwd_ws_eligible(n.N(0), n.N(1), ps.kout(), n.out, false, 0, n.theta, n.sa, n.sn)) return;
-  if (!mlp_fwd_ws_eligible(n.N(0), n.N(1), n.out, n.in, n.theta, n.sa, n.sn)) return;
+  if (!n.planes || !x->fuse_bwd || !x->fuse_fwd || !H1p || !dH2p || !dbpart_fits(x, n, ps.rows) || !n.ws()) return;
   ps.H1p = H1p; ps.dH2p = dH2p; ps.dH1p = dH1p; ps.sQa = sQa; ps.sQn = sQn;
 }
 
@@ -882,10 +856,9 @@ static int model_term_phase(saceo_ctx* x, const KCtx& k, cudaStream_t st) {
     count_launch(x, "k_model_term", st);
     return 0;
   }
-  // the GEMM chain directly, not the mlp_forward / mlp_backward dispatchers: 256-wide models with >= 128 rows per
-  // model would take the fused MLP kernels, which this term has never run on
+  // the GEMM chain: the models have no weight-plane image
   const Pass mp = model_term_pass(x, k);
-  int rc = mlp_forward_unfused(x, mp, 0, k.mOut, mo, 2LL * E * mo, (long long)E * mo, st); if (rc) return rc;
+  int rc = mlp_forward_unfused(x, mp, k.mOut, mo, 2LL * E * mo, (long long)E * mo, st); if (rc) return rc;
   LAUNCH(x, k_model_loss, dim3(n), 256, 0, st, k);
   // backward to the action columns (weights frozen)
   return mlp_backward_layers(x, mp, k.mdOut, S, 2LL * E * S, (long long)E * S, nullptr, k.mdXa, A,
@@ -964,9 +937,9 @@ static int step_once(saceo_ctx* x, int use_rng, int do_polyak, cudaStream_t st) 
   if ((rc = phase_gather(x, st))) return rc;
   // fork: the critic-independent half of the actor phase on the second stream (captured into the same graph).
   // Off on a single-stream context and in the per-kernel profile.
-  // Only with the warp-specialised fused kernels: the fallback engines write their hidden activations of the
-  // TD-target actor pass into the buffers the actor phase saves into.
-  const bool fork = x->fork && !x->prof && x->s2 != nullptr && x->pl_actor != nullptr && x->pl_q != nullptr && x->fuse_fwd;
+  // Only when the TD-target actor pass runs in k_mlp_fwd_ws, which then writes no hidden activation: the GEMM chain
+  // would write them into the buffers the actor phase saves into.
+  const bool fork = x->fork && !x->prof && x->s2 != nullptr && fwd_ws(x, actor_net(x)) && x->pl_q != nullptr;
   if (fork) {
     CU(cudaEventRecord(x->ev_fork, st));
     CU(cudaStreamWaitEvent(x->s2, x->ev_fork, 0));

@@ -644,600 +644,3 @@ static inline int tc_gemm_launch(bool TA, bool TB, bool ONES, const GemmP& p, in
 }
 
 }  // namespace saceo
-
-// ==========================================================================================
-// Fused three-layer MLP forward for one (agent, net, 128-row tile):
-//     h1 = act0(X W0 + b0);  h2 = act1(h1 W1 + b1);  out = h2 W2 + b2          (nn_utils.py:101-136)
-// The activation tile never leaves the SM between layers: the fp32 accumulator (TMEM columns [0,256)) is read
-// back with tcgen05.ld, bias + activation are applied, the result is split into bf16 hi/lo and written with
-// tcgen05.st into TMEM columns [256,512) where the next layer's tcgen05.mma reads it as its A operand
-// (A-from-TMEM form).  W1 (the 256 KB that dominates traffic) streams through the cp.async ring; its first two
-// slabs are already in flight while layer 0 runs.  h1 / h2 are written to global memory only when the caller
-// needs them for the backward pass.  Requires hidden = (256, 256), out <= 64.
-// ==========================================================================================
-namespace saceo {
-
-struct FwdP {
-  const float* X; int ldx; long long sXa, sXn;      // input rows [rows, K0]
-  const float* theta; long long sTa, sTn;           // flat nets
-  float* H1; float* H2; long long sHa, sHn;         // optional [rows, 256] outputs (nullable)
-  float* Out; int ldo; long long sOa, sOn;          // [rows, nout]
-  int rows, K0, nout, nnet, act0, act1;
-  unsigned long long* dbg;
-};
-#define FW_STAMP(i) do { if (f.dbg && threadIdx.x == 0) f.dbg[(size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 8 + (i)] = gtime(); } while (0)
-
-constexpr int FW_H = 256, FW_NT = 512;
-constexpr int FW_R1 = 98304;                         // L0 stage / B stage + patches
-constexpr int FW_R2 = 3 * FW_H * TS_BK * 4;          // raw ring: 3 x 32 KB (slab j+2 is issued before slab j is consumed)
-constexpr int FW_MAIN = FW_R1 + FW_R2;
-constexpr int FW_BYTES = FW_MAIN + 1024 + 64;
-
-__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t db, uint32_t idesc, uint32_t acc) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-               "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-               ::"r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-               "{%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
-                 "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-               "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-               "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                 "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-                 "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-                 "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-               : "r"(taddr) : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// element-wise part of the hidden epilogues, specialised on the activation so the inner loops are branch-free
-//   FWD: x = act(acc + bias)        BWD: x = acc * act'(h_saved)
-template <int ACT, bool BWD>
-__device__ __forceinline__ void hidden_math(uint32_t (&v)[32], const float (&aux)[32], uint32_t (&hi)[16], uint32_t (&lo)[16]) {
-#pragma unroll
-  for (int j = 0; j < 16; ++j) {
-    float x0 = __uint_as_float(v[2 * j]), x1 = __uint_as_float(v[2 * j + 1]);
-    if (BWD) { x0 *= dact_from_out(ACT, aux[2 * j]); x1 *= dact_from_out(ACT, aux[2 * j + 1]); }
-    else { x0 = apply_act(ACT, x0 + aux[2 * j]); x1 = apply_act(ACT, x1 + aux[2 * j + 1]); }
-    v[2 * j] = __float_as_uint(x0); v[2 * j + 1] = __float_as_uint(x1);
-    if (!BWD) {       // forward activations: fp16 hi/lo (see split8)
-      asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi[j]) : "f"(x1), "f"(x0));
-      const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hi[j]));
-      asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo[j]) : "f"(x1 - hf.y), "f"(x0 - hf.x));
-    } else {          // gradients: bf16 hi/lo (range)
-      const __nv_bfloat162 hp = __floats2bfloat162_rn(x0, x1);
-      hi[j] = *reinterpret_cast<const uint32_t*>(&hp);
-      const float f0 = __uint_as_float(hi[j] << 16), f1 = __uint_as_float(hi[j] & 0xFFFF0000u);
-      const __nv_bfloat162 lp = __floats2bfloat162_rn(x0 - f0, x1 - f1);
-      lo[j] = *reinterpret_cast<const uint32_t*>(&lp);
-    }
-  }
-}
-template <bool BWD>
-__device__ __forceinline__ void hidden_math_dispatch(int act, uint32_t (&v)[32], const float (&aux)[32], uint32_t (&hi)[16],
-                                                     uint32_t (&lo)[16]) {
-  if (act == ACT_RELU) hidden_math<ACT_RELU, BWD>(v, aux, hi, lo);
-  else if (act == ACT_TANH) hidden_math<ACT_TANH, BWD>(v, aux, hi, lo);
-  else hidden_math<ACT_ELU, BWD>(v, aux, hi, lo);
-}
-
-// hidden epilogue (forward and backward): D (TMEM cols [0,256)) -> element-wise op -> [global tile] + bf16 hi/lo A
-// operand (TMEM cols 256.., 384..).  FWD: aux = bias[col..col+31] (same for every row); BWD: aux = saved H[row][col..].
-//   outer_w != null (critic backward, single output): the incoming tile is the outer product outer_s[row] * outer_w[col]
-//                    (dq . W2^T has K = 1), formed in registers instead of by an MMA.
-//   qdot_w  != null (critic forward, single output): q[row] = h2[row,:] . qdot_w is accumulated here on CUDA cores
-//                    (returned per thread, partial over this warp's 64 columns); the tile is then NOT written to TMEM.
-template <bool BWD>
-__device__ __forceinline__ float hidden_epilogue(uint32_t tmem, uint32_t patch_base, const float* __restrict__ auxp, int act,
-                                                 float* __restrict__ Gout, int row0, int rows, int warp, int lane,
-                                                 const float* __restrict__ outer_w = nullptr, float outer_s = 0.f,
-                                                 const float* __restrict__ qdot_w = nullptr, uint32_t cs_base = 0) {
-  // cs_base != 0 (needs Gout): column sums of the tile over this warp's 32 rows go to smem [4 quarters][256] (floats) -
-  // the bias gradients of the layer below, so that no separate pass has to re-read the tile from global memory.
-  const int q = warp & 3, grp = warp >> 2;                 // lane quarter, 64-column group
-  constexpr int PSTR = 36;
-  const uint32_t patch = patch_base + (uint32_t)warp * 32 * PSTR * 4;
-  const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-  const int grow_own = row0 + q * 32 + lane;
-  float qacc = 0.f;
-#pragma unroll 1
-  for (int c0 = 0; c0 < 64; c0 += 32) {
-    const int col = grp * 64 + c0;
-    float aux[32];
-    if (!BWD) {
-      const float4* ap = reinterpret_cast<const float4*>(auxp + col);          // bias: the same 32 values for every row
-#pragma unroll
-      for (int j = 0; j < 8; ++j) { const float4 t4 = __ldg(ap + j); aux[4 * j] = t4.x; aux[4 * j + 1] = t4.y; aux[4 * j + 2] = t4.z; aux[4 * j + 3] = t4.w; }
-    } else {
-      // saved activations [32 rows x 32 cols] of this warp: read row-wise (8 lanes = one 128-byte row segment, whole
-      // lines per request) into the warp's patch, then every lane picks up ITS row - a lane-per-row global read would
-      // touch 32 different lines per request
-      const int lr = lane >> 3, lc = (lane & 7) * 4;
-#pragma unroll
-      for (int rr = 0; rr < 32; rr += 4) {
-        const int r = rr + lr;
-        const int grow = row0 + q * 32 + r;
-        float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (grow < rows) t4 = __ldg(reinterpret_cast<const float4*>(auxp + (long long)grow * FW_H + col + lc));
-        sts128(patch + (uint32_t)(r * PSTR + lc) * 4, make_uint4(__float_as_uint(t4.x), __float_as_uint(t4.y), __float_as_uint(t4.z), __float_as_uint(t4.w)));
-      }
-      __syncwarp();
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float4 t4 = lds128(patch + (uint32_t)(lane * PSTR + 4 * j) * 4);
-        aux[4 * j] = t4.x; aux[4 * j + 1] = t4.y; aux[4 * j + 2] = t4.z; aux[4 * j + 3] = t4.w;
-      }
-      __syncwarp();                                                             // the patch is reused for the output tile below
-    }
-    uint32_t v[32];
-    if (outer_w) {
-      const float4* wp = reinterpret_cast<const float4*>(outer_w + col);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float4 t4 = __ldg(wp + j);
-        v[4 * j] = __float_as_uint(outer_s * t4.x); v[4 * j + 1] = __float_as_uint(outer_s * t4.y);
-        v[4 * j + 2] = __float_as_uint(outer_s * t4.z); v[4 * j + 3] = __float_as_uint(outer_s * t4.w);
-      }
-    } else {
-      tmem_ld32(tmem + lane_addr + (uint32_t)col, v);
-    }
-    uint32_t hi[16], lo[16];
-    hidden_math_dispatch<BWD>(act, v, aux, hi, lo);
-    if (qdot_w) {
-      const float4* wp = reinterpret_cast<const float4*>(qdot_w + col);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float4 t4 = __ldg(wp + j);
-        qacc = fmaf(__uint_as_float(v[4 * j]), t4.x, qacc); qacc = fmaf(__uint_as_float(v[4 * j + 1]), t4.y, qacc);
-        qacc = fmaf(__uint_as_float(v[4 * j + 2]), t4.z, qacc); qacc = fmaf(__uint_as_float(v[4 * j + 3]), t4.w, qacc);
-      }
-    } else {
-      tmem_st16(tmem + lane_addr + (uint32_t)(256 + (col >> 1)), hi);
-      tmem_st16(tmem + lane_addr + (uint32_t)(384 + (col >> 1)), lo);
-    }
-    if (Gout) {      // coalesced global write through the warp-private patch
-#pragma unroll
-      for (int j = 0; j < 8; ++j) sts128(patch + (uint32_t)(lane * PSTR + 4 * j) * 4, make_uint4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]));
-      __syncwarp();
-      const int lr = lane >> 3, lc = (lane & 7) * 4;
-#pragma unroll
-      for (int rr = 0; rr < 32; rr += 4) {
-        const int r = rr + lr;
-        const int grow = row0 + q * 32 + r;
-        if (grow < rows) {
-          const float4 t4 = lds128(patch + (uint32_t)(r * PSTR + lc) * 4);
-          *reinterpret_cast<float4*>(Gout + (long long)grow * FW_H + col + lc) = t4;
-        }
-      }
-      if (cs_base) {
-        const int nvalid = rows - (row0 + q * 32);
-        float cs = 0.f;
-#pragma unroll 8
-        for (int r = 0; r < 32; ++r) { const float t = lds32(patch + (uint32_t)(r * PSTR + lane) * 4); cs += r < nvalid ? t : 0.f; }
-        asm volatile("st.shared.f32 [%0], %1;" ::"r"(cs_base + (uint32_t)(q * FW_H + col + lane) * 4), "f"(cs) : "memory");
-      }
-      __syncwarp();
-    }
-  }
-  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-  return qacc;
-}
-
-__global__ void __launch_bounds__(FW_NT, 1) k_mlp_fwd_tc(FwdP f) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t sb = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t r1 = sb, r2 = sb + FW_R1;
-  const uint32_t bars = sb + FW_MAIN;                  // [0],[1] half free, [2] layer0, [3] layer1, [4] layer2
-  const uint32_t tmem_slot = bars + 40;
-  FW_STAMP(0);
-  const int z = blockIdx.y;
-  const int agent = z / f.nnet, net = z - agent * f.nnet;
-  const int row0 = blockIdx.x * TC_BM;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const float* __restrict__ X = f.X + agent * f.sXa + net * f.sXn;
-  const float* __restrict__ th = f.theta + agent * f.sTa + net * f.sTn;
-  const long long oW0 = 0, ob0 = (long long)f.K0 * FW_H, oW1 = ob0 + FW_H, ob1 = oW1 + (long long)FW_H * FW_H,
-                  oW2 = ob1 + FW_H, ob2 = oW2 + (long long)FW_H * f.nout;
-  float* H1 = f.H1 ? f.H1 + agent * f.sHa + net * f.sHn : nullptr;
-  float* H2 = f.H2 ? f.H2 + agent * f.sHa + net * f.sHn : nullptr;
-  float* Out = f.Out + agent * f.sOa + net * f.sOn;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < 5; ++s) mbar_init(bars + 8 * s, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  // W1 slabs 0 and 1 start flying now (ring r2), they are consumed after layer 0 and its epilogue
-  TsPlan<FW_H, false> pw1;
-  pw1.init(th + oW1, 1, FW_H, 0);
-  pw1.issue(r2);
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  pw1.issue(r2 + FW_H * TS_BK * 4);
-  asm volatile("cp.async.commit_group;" ::: "memory");
-
-  // ---------------- layer 0: D = X . W0   (register-staged slabs, SS MMAs) ----------------
-  Slab<TC_BM, FW_NT> sx;
-  Slab<FW_H, FW_NT> sw;
-  sx.init(X, f.ldx, 1, row0, f.rows);
-  sw.init(th + oW0, 1, FW_H, 0, FW_H);
-  const int nk0 = (f.K0 + TC_BK - 1) / TC_BK;
-  sx.ld(0, f.K0); sw.ld(0, f.K0);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem = lds_u32(tmem_slot);
-  constexpr uint32_t IDESC = umma_idesc(TC_BM, FW_H, 0u);      // fp16 operands
-  {
-    const uint32_t a_hi = r1, a_lo = r1 + 16384, b_hi = r1 + 32768, b_lo = r1 + 65536;
-    for (int kc = 0; kc < nk0; ++kc) {
-      if (kc > 0) mbar_wait(bars + 16, (uint32_t)((kc - 1) & 1));
-      sx.st<true>(a_hi, a_lo); sw.st<true>(b_hi, b_lo);
-      if (kc + 1 < nk0) { sx.ld((kc + 1) * TC_BK, f.K0); sw.ld((kc + 1) * TC_BK, f.K0); }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk) {
-          const uint32_t ko = kk * 32;
-          umma_f16(tmem, umma_desc(a_hi + ko), umma_desc(b_hi + ko), IDESC, (kc | kk) ? 1u : 0u);
-          umma_f16(tmem, umma_desc(a_hi + ko), umma_desc(b_lo + ko), IDESC, 1u);
-          umma_f16(tmem, umma_desc(a_lo + ko), umma_desc(b_hi + ko), IDESC, 1u);
-        }
-        umma_commit(bars + 16);
-      }
-    }
-    mbar_wait(bars + 16, (uint32_t)((nk0 - 1) & 1));
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  }
-  FW_STAMP(1);
-  // W2 (tiny, nout <= 64): four 64-k slabs, loaded into registers before epilogue 1 and staged to smem after it
-  Slab<64, FW_NT> sw2[4];
-#pragma unroll
-  for (int kc = 0; kc < 4; ++kc) sw2[kc].init(th + oW2, 1, f.nout, 0, f.nout);
-
-  // ---------------- epilogue 0: h1 ----------------
-  hidden_epilogue<false>(tmem, r1, th + ob0, f.act0, H1, row0, f.rows, warp, lane);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-
-  FW_STAMP(2);
-  // ---------------- layer 1: D = h1 . W1   (A from TMEM, W1 streamed) ----------------
-  const uint32_t b_hi = r1, b_lo = r1 + TS_BPLANE;
-  constexpr int NS1 = FW_H / TS_BK;    // 8 slabs
-  // One block barrier per slab: it publishes slab j's raw data AND the planes of slab j-1, whose MMAs the elected
-  // thread then issues while everybody converts slab j (the issue cost is off the convert -> barrier chain).
-  auto issue_l1 = [&](int js) {
-    const int hs = js & 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) {
-      const int ks = js * 2 + kk;                             // k16 step inside K = 256
-      const uint32_t ko = (uint32_t)(hs * 2 + kk) * 32;
-      const uint32_t ta_hi = tmem + 256 + ks * 8, ta_lo = tmem + 384 + ks * 8;
-      umma_f16_ts(tmem, ta_hi, umma_desc(b_hi + ko), IDESC, ks ? 1u : 0u);
-      umma_f16_ts(tmem, ta_hi, umma_desc(b_lo + ko), IDESC, 1u);
-      umma_f16_ts(tmem, ta_lo, umma_desc(b_hi + ko), IDESC, 1u);
-    }
-    umma_commit(bars + 8 * hs);
-  };
-  for (int j = 0; j < NS1; ++j) {
-    const int h = j & 1;
-    const uint32_t raw = r2 + (j % 3) * (FW_H * TS_BK * 4);
-    asm volatile("cp.async.wait_group 1;" ::: "memory");       // this thread's pieces of slab j have landed
-    __syncthreads();                                            // ... everybody's; planes of slab j-1 are complete
-    if (j + 2 < NS1) pw1.issue(r2 + ((j + 2) % 3) * (FW_H * TS_BK * 4));   // raw buffer of slab j-1 is free now
-    asm volatile("cp.async.commit_group;" ::: "memory");       // (possibly empty) keeps the group count uniform
-    if (threadIdx.x == 0 && j >= 1) issue_l1(j - 1);
-    if (j >= 2) mbar_wait(bars + 8 * h, (uint32_t)((j / 2 - 1) & 1));      // MMAs of slab j-2 released plane half h
-    pw1.convert<true>(raw, h, b_hi, b_lo);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) { issue_l1(NS1 - 1); umma_commit(bars + 24); }
-  mbar_wait(bars + 24, 0);
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-
-  FW_STAMP(3);
-  // ---------------- epilogue 1: h2 ; stage W2 ----------------
-  if (f.nout == 1) {
-    // single output (critics): q = h2 . w2 + b2 on CUDA cores inside the epilogue - no MMA, no TMEM round trip
-    const float qp = hidden_epilogue<false>(tmem, r1, th + ob1, f.act1, H2, row0, f.rows, warp, lane, nullptr, 0.f, th + oW2);
-    __syncthreads();                                          // patches (r1) no longer read
-    float* qs = reinterpret_cast<float*>(smem_raw) + ((sb - smem_u32(smem_raw)) >> 2);     // [4 groups][128 rows] in r1
-    qs[(warp >> 2) * TC_BM + (warp & 3) * 32 + lane] = qp;
-    __syncthreads();
-    if (warp < 4) {
-      const int r = warp * 32 + lane, grow = row0 + r;
-      if (grow < f.rows) Out[(long long)grow * f.ldo] = ((qs[r] + qs[TC_BM + r]) + (qs[2 * TC_BM + r] + qs[3 * TC_BM + r])) + __ldg(th + ob2);
-    }
-    FW_STAMP(6);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) {
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512) : "memory");
-    }
-    return;
-  }
-#pragma unroll
-  for (int kc = 0; kc < 4; ++kc) sw2[kc].ld(kc * TC_BK, FW_H);      // in flight during the epilogue
-  hidden_epilogue<false>(tmem, r1, th + ob1, f.act1, H2, row0, f.rows, warp, lane);
-  __syncthreads();                                            // patches (r1) no longer read
-  // W2 as B operand: 4 chunks of 64 k, each [64 rows x 128 B] hi plane + lo plane (16 KB per chunk)
-  const uint32_t w2s = r1;
-#pragma unroll
-  for (int kc = 0; kc < 4; ++kc) sw2[kc].st<true>(w2s + kc * 16384, w2s + kc * 16384 + 8192);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-
-  FW_STAMP(4);
-  // ---------------- layer 2: D[:, :npad] = h2 . W2 ----------------
-  const int npad = f.nout <= 16 ? 16 : (f.nout <= 32 ? 32 : 64);
-  if (threadIdx.x == 0) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t idesc2 = umma_idesc(TC_BM, npad, 0u);
-    for (int ks = 0; ks < 16; ++ks) {
-      const uint32_t cb = w2s + (ks >> 2) * 16384 + (ks & 3) * 32;
-      const uint32_t ta_hi = tmem + 256 + ks * 8, ta_lo = tmem + 384 + ks * 8;
-      umma_f16_ts(tmem, ta_hi, umma_desc(cb), idesc2, ks ? 1u : 0u);
-      umma_f16_ts(tmem, ta_hi, umma_desc(cb + 8192), idesc2, 1u);
-      umma_f16_ts(tmem, ta_lo, umma_desc(cb), idesc2, 1u);
-    }
-    umma_commit(bars + 32);
-  }
-  mbar_wait(bars + 32, 0);
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  FW_STAMP(5);
-  if (warp < 4) {                                             // one warp per lane quarter reads the output columns
-    const int grow = row0 + warp * 32 + lane;
-    for (int c0 = 0; c0 < npad; c0 += 32) {
-      uint32_t v[32];
-      tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, v);
-      if (grow < f.rows) {
-#pragma unroll
-        for (int n = 0; n < 32; ++n) if (c0 + n < f.nout) Out[(long long)grow * f.ldo + c0 + n] = __uint_as_float(v[n]) + __ldg(th + ob2 + c0 + n);
-      }
-    }
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  FW_STAMP(6);
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512) : "memory");
-  }
-}
-
-// ==========================================================================================
-// Fused backward chain through one (agent, net, 128-row tile) of a 2x256 MLP (weights fixed):
-//     dH2 = (dOut W2[:, :kout]^T) * act1'(H2);  dH1 = (dH2 W1^T) * act0'(H1);  dXa = dH1 W0[S:S+A, :]^T
-// Same structure as the fused forward: the gradient tile stays in TMEM between layers (fp32 accumulator ->
-// tcgen05.ld -> multiply by the activation derivative taken from the SAVED post-activation tile -> bf16 hi/lo
-// -> tcgen05.st -> A operand of the next MMA); W1 streams through the cp.async ring, read K-contiguously
-// (B(n=i, k=j) = W1[i, j]), so no transposed copy of the weights is ever made.  dH2 / dH1 are written to
-// global memory only when the weight-gradient GEMMs need them; for the actor-phase critics (gradient to the
-// action only) nothing but dXa [rows, A] leaves the SM.
-// ==========================================================================================
-struct BwdP {
-  const float* dOut; int ldd; long long sDa, sDn; int kout;   // upstream gradient [rows, >=kout]
-  const float* theta; long long sTa, sTn; int K0, nout;       // flat nets (W2 leading dim = nout)
-  const float* H1; const float* H2; long long sHa, sHn;       // saved activations [rows, 256]
-  float* dH2; float* dH1;                                      // optional outputs, strides as H
-  float* dXa; int s_cols, a_cols; long long sXa, sXn;         // optional [rows, a_cols]
-  int rows, nnet, act0, act1;
-  float* dbpart;      // optional [agent*nnet+net][tile][2][256]: column sums of dH2 (slot 0) and dH1 (slot 1) per row tile
-};
-
-__global__ void __launch_bounds__(FW_NT, 1) k_mlp_bwd_tc(BwdP f) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t sb = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t r1 = sb, r2 = sb + FW_R1;
-  const uint32_t bars = sb + FW_MAIN;                  // [0],[1] half free, [2] layer2^T, [3] layer1^T, [4] layer0^T
-  const uint32_t tmem_slot = bars + 40;
-  const uint32_t cs2 = r1 + 80 * 1024, cs1 = cs2 + 4096;    // column-sum scratch, beyond the patches / planes / W0 stage
-  const int z = blockIdx.y;
-  const int agent = z / f.nnet, net = z - agent * f.nnet;
-  const int row0 = blockIdx.x * TC_BM;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const float* __restrict__ dOut = f.dOut + agent * f.sDa + net * f.sDn;
-  const float* __restrict__ th = f.theta + agent * f.sTa + net * f.sTn;
-  const long long oW0 = 0, ob0 = (long long)f.K0 * FW_H, oW1 = ob0 + FW_H, ob1 = oW1 + (long long)FW_H * FW_H, oW2 = ob1 + FW_H;
-  const float* H1 = f.H1 + agent * f.sHa + net * f.sHn;
-  const float* H2 = f.H2 + agent * f.sHa + net * f.sHn;
-  float* dH1 = f.dH1 ? f.dH1 + agent * f.sHa + net * f.sHn : nullptr;
-  float* dH2 = f.dH2 ? f.dH2 + agent * f.sHa + net * f.sHn : nullptr;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < 5; ++s) mbar_init(bars + 8 * s, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  // W1 read K-contiguously as B(n = input index i, k = output index j): first two slabs in flight now
-  TsPlan<FW_H, true> pw1;
-  pw1.init(th + oW1, FW_H, 1, 0);
-  pw1.issue(r2);
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  pw1.issue(r2 + FW_H * TS_BK * 4);
-  asm volatile("cp.async.commit_group;" ::: "memory");
-
-  // ---------------- layer 2 transposed: D = dOut[:, :kout] . W2[:, :kout]^T  (one 64-wide slab, kout <= 64) ----------------
-  const bool outer = (f.kout == 1 && f.nout == 1);     // critics: K = 1, the "GEMM" is an outer product formed in the epilogue
-  Slab<TC_BM, FW_NT> sx;
-  Slab<FW_H, FW_NT> sw;
-  if (!outer) {
-    sx.init(dOut, f.ldd, 1, row0, f.rows);
-    sw.init(th + oW2, f.nout, 1, 0, FW_H);            // B(n = hidden j, k = out c) = W2[j*nout + c]
-    sx.ld(0, f.kout); sw.ld(0, f.kout);
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem = lds_u32(tmem_slot);
-  constexpr uint32_t IDESC = umma_idesc(TC_BM, FW_H);
-  if (!outer) {
-    const uint32_t a_hi = r1, a_lo = r1 + 16384, b_hi = r1 + 32768, b_lo = r1 + 65536;
-    sx.st(a_hi, a_lo); sw.st(b_hi, b_lo);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const int nks = (f.kout + 15) >> 4;
-      for (int kk = 0; kk < nks; ++kk) {
-        const uint32_t ko = kk * 32;
-        umma_f16(tmem, umma_desc(a_hi + ko), umma_desc(b_hi + ko), IDESC, kk ? 1u : 0u);
-        umma_f16(tmem, umma_desc(a_hi + ko), umma_desc(b_lo + ko), IDESC, 1u);
-        umma_f16(tmem, umma_desc(a_lo + ko), umma_desc(b_hi + ko), IDESC, 1u);
-      }
-      umma_commit(bars + 16);
-    }
-    mbar_wait(bars + 16, 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  }
-  // action rows of W0 (tiny) into registers now, staged after layer 1^T
-  Slab<32, FW_NT> sw0[4];
-  if (f.dXa) {
-#pragma unroll
-    for (int kc = 0; kc < 4; ++kc) sw0[kc].init(th + oW0 + (long long)f.s_cols * FW_H, FW_H, 1, 0, f.a_cols);   // B(n = a, k = j) = W0[(S+a)*256 + j]
-  }
-
-  {
-    const int grow = row0 + (warp & 3) * 32 + lane;
-    const float dq = (outer && grow < f.rows) ? __ldg(dOut + (long long)grow * f.ldd) : 0.f;
-    hidden_epilogue<true>(tmem, r1, H2, f.act1, dH2, row0, f.rows, warp, lane, outer ? th + oW2 : nullptr, dq, nullptr,
-                          (f.dbpart && dH2) ? cs2 : 0u);
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-
-  // ---------------- layer 1 transposed: D = dH2 . W1^T ----------------
-  const uint32_t b_hi = r1, b_lo = r1 + TS_BPLANE;
-  constexpr int NS1 = FW_H / TS_BK;
-  // one block barrier per slab (see k_mlp_fwd_tc): it publishes raw slab j and the planes of slab j-1
-  auto issue_l1 = [&](int js) {
-    const int hs = js & 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) {
-      const int ks = js * 2 + kk;
-      const uint32_t ko = (uint32_t)(hs * 2 + kk) * 32;
-      const uint32_t ta_hi = tmem + 256 + ks * 8, ta_lo = tmem + 384 + ks * 8;
-      umma_f16_ts(tmem, ta_hi, umma_desc(b_hi + ko), IDESC, ks ? 1u : 0u);
-      umma_f16_ts(tmem, ta_hi, umma_desc(b_lo + ko), IDESC, 1u);
-      umma_f16_ts(tmem, ta_lo, umma_desc(b_hi + ko), IDESC, 1u);
-    }
-    umma_commit(bars + 8 * hs);
-  };
-  for (int j = 0; j < NS1; ++j) {
-    const int h = j & 1;
-    const uint32_t raw = r2 + (j % 3) * (FW_H * TS_BK * 4);
-    asm volatile("cp.async.wait_group 1;" ::: "memory");       // this thread's pieces of slab j have landed
-    __syncthreads();                                            // ... everybody's; planes of slab j-1 are complete
-    if (j + 2 < NS1) pw1.issue(r2 + ((j + 2) % 3) * (FW_H * TS_BK * 4));   // raw buffer of slab j-1 is free now
-    asm volatile("cp.async.commit_group;" ::: "memory");       // (possibly empty) keeps the group count uniform
-    if (threadIdx.x == 0 && j >= 1) issue_l1(j - 1);
-    if (j >= 2) mbar_wait(bars + 8 * h, (uint32_t)((j / 2 - 1) & 1));
-    pw1.convert(raw, h, b_hi, b_lo);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) { issue_l1(NS1 - 1); umma_commit(bars + 24); }
-  mbar_wait(bars + 24, 0);
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-
-  if (f.dXa) {
-#pragma unroll
-    for (int kc = 0; kc < 4; ++kc) sw0[kc].ld(kc * TC_BK, FW_H);
-  }
-  hidden_epilogue<true>(tmem, r1, H1, f.act0, dH1, row0, f.rows, warp, lane, nullptr, 0.f, nullptr, (f.dbpart && dH1) ? cs1 : 0u);
-  if (f.dXa) {
-    __syncthreads();
-    const uint32_t w0s = r1;
-#pragma unroll
-    for (int kc = 0; kc < 4; ++kc) sw0[kc].st(w0s + kc * 8192, w0s + kc * 8192 + 4096);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    const int npad = f.a_cols <= 16 ? 16 : 32;
-    if (threadIdx.x == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const uint32_t idesc2 = umma_idesc(TC_BM, npad);
-      for (int ks = 0; ks < 16; ++ks) {
-        const uint32_t cb = w0s + (ks >> 2) * 8192 + (ks & 3) * 32;
-        const uint32_t ta_hi = tmem + 256 + ks * 8, ta_lo = tmem + 384 + ks * 8;
-        umma_f16_ts(tmem, ta_hi, umma_desc(cb), idesc2, ks ? 1u : 0u);
-        umma_f16_ts(tmem, ta_hi, umma_desc(cb + 4096), idesc2, 1u);
-        umma_f16_ts(tmem, ta_lo, umma_desc(cb), idesc2, 1u);
-      }
-      umma_commit(bars + 32);
-    }
-    mbar_wait(bars + 32, 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (warp < 4) {
-      uint32_t v[32];
-      tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16), v);
-      const int grow = row0 + warp * 32 + lane;
-      if (grow < f.rows) {
-        float* o = f.dXa + agent * f.sXa + net * f.sXn + (long long)grow * f.a_cols;
-#pragma unroll
-        for (int n = 0; n < 32; ++n) if (n < f.a_cols) o[n] = __uint_as_float(v[n]);
-      }
-    }
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (f.dbpart && f.dH2 && f.dH1) {      // fixed-order sum of the four row quarters -> per-tile bias-gradient partials
-    const int t = threadIdx.x & (FW_H - 1), which = threadIdx.x >> 8;
-    const uint32_t b = (which ? cs1 : cs2) + (uint32_t)t * 4;
-    const float v = ((lds32(b) + lds32(b + FW_H * 4)) + lds32(b + 2 * FW_H * 4)) + lds32(b + 3 * FW_H * 4);
-    f.dbpart[(((long long)z * gridDim.x + blockIdx.x) * 2 + which) * FW_H + t] = v;
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512) : "memory");
-  }
-}
-
-// g[ob1 + c] = sum_tiles dbpart[.][tile][0][c],  g[ob0 + c] = sum_tiles dbpart[.][tile][1][c]   (fixed tile order)
-// grid: (n_agents * nnet), block 512
-__global__ void k_bias_finish(const float* __restrict__ dbpart, int ntiles, float* __restrict__ g, long long sGa, long long sGn,
-                              int nnet, long long ob1, long long ob0) {
-  const int z = blockIdx.x, agent = z / nnet, net = z - agent * nnet;
-  const int t = threadIdx.x & (FW_H - 1), which = threadIdx.x >> 8;
-  float acc = 0.f;
-  for (int tile = 0; tile < ntiles; ++tile) acc += dbpart[(((long long)z * ntiles + tile) * 2 + which) * FW_H + t];
-  g[agent * sGa + net * sGn + (which ? ob0 : ob1) + t] = acc;
-}
-
-static inline bool mlp_fwd_tc_eligible(int h1, int h2, int nout, int rows, const float* theta, long long sTa, long long sTn, int K0) {
-  return h1 == FW_H && h2 == FW_H && nout >= 1 && nout <= 64 && rows >= TC_BM && K0 >= 1 &&
-         ((reinterpret_cast<uintptr_t>(theta) & 15) == 0) && ((sTa & 3) == 0) && ((sTn & 3) == 0);
-}
-static inline bool mlp_bwd_tc_eligible(int h1, int h2, int kout, int rows, bool want_dxa, int a_cols, const float* theta,
-                                       long long sTa, long long sTn) {
-  return h1 == FW_H && h2 == FW_H && kout >= 1 && kout <= 64 && rows >= TC_BM && (rows % TC_BM == 0 || rows % TC_BM >= 16) &&
-         (!want_dxa || a_cols <= 32) && ((reinterpret_cast<uintptr_t>(theta) & 15) == 0) && ((sTa & 3) == 0) && ((sTn & 3) == 0);
-}
-static inline cudaError_t mlp_fwd_tc_init() {
-  static bool done_dev[64] = {};
-  int dev_ = 0; cudaGetDevice(&dev_);
-  bool& done = done_dev[dev_ & 63];       // cudaFuncSetAttribute is per device
-  if (done) return cudaSuccess;
-  cudaError_t e = cudaFuncSetAttribute(k_mlp_fwd_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, FW_BYTES);
-  if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(k_mlp_bwd_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, FW_BYTES);
-  if (e == cudaSuccess) done = true;
-  return e;
-}
-
-}  // namespace saceo

@@ -52,7 +52,8 @@ class PopulationSpec:
     fuse_forward: bool = True      # fused 3-layer tcgen05 forward (activations resident in TMEM)
     fuse_backward: bool = True     # fused tcgen05 gradient chain dOut -> dH2 -> dH1 -> dXa
     use_graph: bool = True         # one update = one CUDA-graph replay
-    ws_kernels: bool = True        # warp-specialised TMA-fed fused kernels on optimiser-maintained weight planes (round 2)
+    ws_kernels: bool = True        # warp-specialised TMA-fed fused kernels on optimiser-maintained weight planes (round 2);
+                                   # off: every MLP pass runs on the per-layer GEMM chain
     fork_actor: bool = True        # critic-independent half of the actor phase on a second stream (needs ws_kernels)
     device: int = 0
 

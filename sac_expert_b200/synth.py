@@ -160,8 +160,7 @@ def kernel_design_bytes(sp, L) -> dict:
         + (L.na + 2 * R * sp.actor_hidden[0] + 2 * R * sp.actor_hidden[0] + R * Ao))
     dw = (2 * (B * SA + 4 * B * H + L.nc)) + (R * S + 4 * R * sp.actor_hidden[0] + R * Ao + L.na)   # activations in, gradients out
     return {
-        "k_mlp_fwd_tc": float(w * fwd), "k_mlp_fwd_ws": float(w * fwd),
-        "k_mlp_bwd_tc": float(w * bwd), "k_mlp_bwd_ws": float(w * bwd),
+        "k_mlp_fwd_ws": float(w * fwd), "k_mlp_bwd_ws": float(w * bwd),
         "k_model_term": float(w * (sp.num_models * L.nm + E * (2 * S + A))) if sp.num_models > 0 else 0.0,
         "k_adam": float(w * (2 * 11 * L.nc + 8 * L.na)),        # + the fp16 hi/lo weight planes of theta and of the targets
         "k_dw_planes+k_dw0_planes+k_gemm": float(w * dw), "k_gemm_tc+k_gemm_skinny": float(w * dw),

@@ -41,6 +41,31 @@ def test_fused_vs_unfused_mlp_vs_fp32_engine():
     assert rel(fused["g_q"], plain["g_q"]) < 2e-4 and rel(fused["g_a"][:, :-1], plain["g_a"][:, :-1]) < TOL
 
 
+@pytest.mark.parametrize("B", [256, 260])
+def test_wide_head_actor_fork_matches_one_stream(B):
+    """A 2x256 actor with more outputs than the warp-specialised kernels take (per-state std, A = 20: 40 outputs) runs
+    on the GEMM chain, which writes the hidden activations of every pass, the TD-target pass included.  The actor phase
+    must then not run on a second stream next to it: graphed updates with and without fork_actor agree bit for bit, and
+    the first one agrees with the oracle.  B = 260 leaves 4 rows past the last full 128-row tile."""
+    cfg = NetCfg(S=17, A=20, model_acts=("tanh", "tanh"))
+    outs = []
+    for fork in (True, False):
+        pop, probs = build(cfg, n_agents=2, B=B, E=20, N=1500, seed=23, gemm_mode=L.GEMM_TCGEN05_BF16X3,
+                           use_graph=True, fork_actor=fork)
+        worst = compare_update(pop, cfg, probs)
+        bad = {k: v for k, v in worst.items() if v > TOL and not k.startswith("oracle32")}
+        assert not bad, (fork, bad)
+        for step in range(1, 4):
+            pop.update(1, num_timesteps=step, use_device_rng=False)
+        torch.cuda.synchronize()
+        out = {k: pop.t[k].cpu().numpy().copy() for k in ("actor", "q", "qt", "alpha")}
+        out["losses"] = pop.losses.cpu().numpy().copy()
+        outs.append(out)
+        pop.close()
+    for k in outs[0]:
+        assert np.array_equal(outs[0][k], outs[1][k]), k
+
+
 def test_humanoid_shaped_batch_1024():
     """BASELINE configs[3]: obs 376, act 17, batch 1024 - multi-slab first layer in the fused kernels, 8 row tiles."""
     cfg = NetCfg(S=376, A=17)
