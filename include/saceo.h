@@ -412,6 +412,50 @@ typedef struct {
 } saceo_gemm_route;
 int saceo_test_gemm_ex(const saceo_gemm_args *args, saceo_gemm_route *route, void *stream);
 
+/* Test surface over the MLP pass dispatch (mlp_forward / mlp_backward) of one population of 2-hidden-layer nets in
+ * the flat Keras layout [W0|b0|W1|b1|W2|b2], with the tcgen05 engine and the fused kernels on:
+ *   out = act1(act0(X W0 + b0) W1 + b1) W2 + b2            (out != NULL)
+ *   backward of dout[:, :kout] through the same nets     (dout != NULL): grads in theta's layout (NULL: none), dXa =
+ *   the gradient w.r.t. the last A_cols input columns (NULL: none); H / dH: [agent][hnets][rowsAllocH][hidden].
+ * planes: room for n_agents * nnet weight-plane images (NULL: no image, the GEMM chain), built here from theta as the
+ * library builds its own when the fused kernels take the net (otherwise left untouched).  H1p / dH2p / dH1p: bf16 activation plane images of rup(rows, 32) rows (sQa / sQn bytes per
+ * agent / net), rows [rows, rup(rows, 32)) zero; used where the library would give the pass its images (a backward
+ * of such a pass that the fused kernel does not take is refused).  dbpart:
+ * per-tile bias partials of dbpart_cap floats.  Strides are in floats unless stated.  The kernels launched and the
+ * fused backward instantiation are written to *route. */
+typedef struct {
+  int32_t n_agents, nnet, hnets;
+  int32_t in, nout, kout, hidden[2], act[2];
+  int32_t rows;
+  int64_t rowsAllocH;
+  const float *theta;
+  int64_t sTa, sTn;
+  const float *X;
+  int32_t ldx;
+  int64_t sXa, sXn;
+  float *out;
+  int32_t ldo;
+  int64_t sOa, sOn;
+  const float *dout;
+  int32_t ldd;
+  int64_t sDa, sDn;
+  float *H[2], *dH[2];
+  uint8_t *planes, *H1p, *dH2p, *dH1p;
+  int64_t sQa, sQn;
+  float *dbpart;
+  int64_t dbpart_cap;
+  float *grads, *dXa;
+  int32_t A_cols;
+  int64_t sXaA, sXaN;
+  int32_t save_h;
+} saceo_mlp_ws_args;
+typedef struct {
+  int32_t plane_path;              /* the pass was given the activation plane images */
+  int32_t n_fwd_ws, n_bwd_ws, n_dw_planes, n_dw0_planes, n_bias_finish, n_tc, n_skinny, n_simt;   /* launches */
+  int32_t bwd_ng, bwd_na, bwd_mode;   /* k_mlp_bwd_ws<NG, NA, MODE> of the fused backward launch (-1: none) */
+} saceo_mlp_ws_route;
+int saceo_test_mlp_ws(const saceo_mlp_ws_args *args, saceo_mlp_ws_route *route, void *stream);
+
 const char *saceo_last_error(void);
 int saceo_abi_version(void);
 

@@ -1339,19 +1339,29 @@ static inline bool mlp_bwd_ws_eligible(int h1, int h2, int kout, int nout, bool 
   if (want_dxa && (kout != 1 || a_cols < 1 || a_cols > 32)) return false;
   return ((reinterpret_cast<uintptr_t>(theta) & 15) == 0) && ((sTa & 3) == 0) && ((sTn & 3) == 0);
 }
-static inline cudaError_t mlp_bwd_ws_launch(const BwdW& f, int nagents, cudaStream_t st) {
-  dim3 grid((f.rows + TC_BM - 1) / TC_BM, nagents * f.nnet);
+// the k_mlp_bwd_ws<NG, NA, MODE> instantiation a launch with arguments f takes
+struct BwdVariant { int ng, na, mode; };
+static inline BwdVariant mlp_bwd_ws_variant(const BwdW& f) {
   const int ng = f.kout == 1 ? 0 : (f.kout + 15) / 16, na = f.dXa ? (f.a_cols + 15) / 16 : 0;
   // the shapes of the SAC / SAC-EO step get compile-time specialised forms (MODE 1 / 2)
   const bool m1 = f.H1p && f.dH2p && f.dH1p && !f.dH2 && !f.dH1, m2 = f.H1p && !f.dH2p && !f.dH1p && !f.dH2 && !f.dH1;
-  if (ng == 0 && na == 0 && m1) k_mlp_bwd_ws<0, 0, 1><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 1 && na == 0 && m1) k_mlp_bwd_ws<1, 0, 1><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 0 && na == 1 && m2) k_mlp_bwd_ws<0, 1, 2><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 0 && na == 0) k_mlp_bwd_ws<0, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 0 && na == 1) k_mlp_bwd_ws<0, 1, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 0) k_mlp_bwd_ws<0, 2, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 1) k_mlp_bwd_ws<1, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
-  else if (ng == 2) k_mlp_bwd_ws<2, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  if (ng == 0 && na == 0 && m1) return {0, 0, 1};
+  if (ng == 1 && na == 0 && m1) return {1, 0, 1};
+  if (ng == 0 && na == 1 && m2) return {0, 1, 2};
+  if (ng == 0) return {0, na, 0};
+  return {ng, 0, 0};
+}
+static inline cudaError_t mlp_bwd_ws_launch(const BwdW& f, int nagents, cudaStream_t st) {
+  dim3 grid((f.rows + TC_BM - 1) / TC_BM, nagents * f.nnet);
+  const BwdVariant v = mlp_bwd_ws_variant(f);
+  if (v.mode == 1 && v.ng == 0) k_mlp_bwd_ws<0, 0, 1><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.mode == 1) k_mlp_bwd_ws<1, 0, 1><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.mode == 2) k_mlp_bwd_ws<0, 1, 2><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.ng == 0 && v.na == 0) k_mlp_bwd_ws<0, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.ng == 0 && v.na == 1) k_mlp_bwd_ws<0, 1, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.ng == 0) k_mlp_bwd_ws<0, 2, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.ng == 1) k_mlp_bwd_ws<1, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
+  else if (v.ng == 2) k_mlp_bwd_ws<2, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
   else k_mlp_bwd_ws<3, 0, 0><<<grid, WS_NT, WS_BYTES, st>>>(f);
   return cudaPeekAtLastError();
 }

@@ -134,6 +134,7 @@ struct saceo_ctx {
   std::vector<cudaEvent_t> prof_ev;
   std::vector<const char*> prof_name;
   size_t prof_n = 0;
+  BwdVariant bwd_variant{-1, -1, -1};   // profiling mode: the k_mlp_bwd_ws instantiation of the last fused backward launch
   cudaGraphExec_t graph[3][2] = {{nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}};   // [rng mode][polyak]
   long long graph_nodes[3][2] = {{0, 0}, {0, 0}, {0, 0}};
 };
@@ -464,16 +465,19 @@ extern "C" int saceo_weights_changed(saceo_ctx* x) {
   x->planes_dirty = 3;
   return 0;
 }
+// the images of `nets` consecutive nets with K0 inputs and nout outputs, net i's fp32 table at theta + i * stride
+// (maintenance: not counted as a launch of the step)
+static void planes_build(const float* theta, long long stride, uint8_t* img, int K0, int nout, int nets, cudaStream_t st) {
+  const int items = (((K0 + 31) / 32) * 32 + 256 + ws_w2_rows(nout)) * 32;
+  k_planes_build<<<dim3(cdiv(items, 256), nets), 256, 0, st>>>(theta, stride, img, K0, nout);
+}
 static int ensure_planes(saceo_ctx* x, cudaStream_t st) {
   if (!x->planes_dirty || !x->bound) return 0;
   const saceo_config& c = x->cfg; const int n = c.n_agents;
-  auto items = [](int K0, int nout) { return (((K0 + 31) / 32) * 32 + 256 + ws_w2_rows(nout)) * 32; };
-  if (x->pl_actor && (x->planes_dirty & 1)) {
-    k_planes_build<<<dim3(cdiv(items(c.S, x->L.Ao), 256), n), 256, 0, st>>>(x->k.T.actor, x->L.na_stride, x->pl_actor, c.S, x->L.Ao);   // maintenance: not counted as a launch of the step
-  }
+  if (x->pl_actor && (x->planes_dirty & 1)) planes_build(x->k.T.actor, x->L.na_stride, x->pl_actor, c.S, x->L.Ao, n, st);
   if (x->pl_q && (x->planes_dirty & 2)) {
-    k_planes_build<<<dim3(cdiv(items(c.S + c.A, 1), 256), 2 * n), 256, 0, st>>>(x->k.T.q, x->L.nc_stride, x->pl_q, c.S + c.A, 1);
-    k_planes_build<<<dim3(cdiv(items(c.S + c.A, 1), 256), 2 * n), 256, 0, st>>>(x->k.T.qt, x->L.nc_stride, x->pl_qt, c.S + c.A, 1);
+    planes_build(x->k.T.q, x->L.nc_stride, x->pl_q, c.S + c.A, 1, 2 * n, st);
+    planes_build(x->k.T.qt, x->L.nc_stride, x->pl_qt, c.S + c.A, 1, 2 * n, st);
   }
   x->planes_dirty = 0;
   cudaError_t e = cudaPeekAtLastError();
@@ -535,7 +539,11 @@ struct Pass {
   int rows; long long rowsAllocH;                      // rows of the pass / rows per net allocated in H, dH
   float* const* H;                                     // saved activation of each hidden layer
   float* const* dH;                                    // its gradient (backward)
-  uint8_t *H1p = nullptr, *dH2p = nullptr, *dH1p = nullptr;   // bf16 hi/lo plane images of h1 / dH2 / dH1
+  // bf16 hi/lo plane images of h1 / dH2 / dH1, rup(rows, 32) rows each.  The kernels write rows [0, rows) only, while
+  // k_dw_planes / k_dw0_planes contract over whole 32-row slabs: rows [rows, rup(rows, 32)) must hold zeros (the
+  // workspace is cleared at creation and nothing writes those rows afterwards).  A pass with images keeps h1 only as
+  // its image, so its backward must be one the fused kernel takes: mlp_backward refuses any other
+  uint8_t *H1p = nullptr, *dH2p = nullptr, *dH1p = nullptr;
   long long sQa = 0, sQn = 0;                          // their bytes per agent / net
   // the caller guarantees that rows [rows, rowsAllocH) of X, H, dOut, dH are zero, so the
   // weight-gradient contractions may run over a row count rounded up to the 32-row slabs of the streaming kernel
@@ -699,15 +707,18 @@ static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd
     f.dH2 = grads ? ps.dH[1] : nullptr; f.dH1 = grads ? ps.dH[0] : nullptr;
     f.dXa = dXa; f.s_cols = n.in - A_cols; f.a_cols = A_cols; f.sXa = sXaA; f.sXn = sXaN;
     f.rows = rows; f.nnet = n.nnet; f.act0 = n.act(0); f.act1 = n.act(1); f.dbpart = dbpart;
+    // on the plane path mlp_forward left h1 as its plane image only: read it there, with or without grads
+    if (ps.H1p) { f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
     // hidden-to-hidden weight gradient from bf16 plane images (k_dw_planes): dH2 then leaves the kernel as planes only
     fz.dw1_planes = dbpart && ps.H1p;
-    if (fz.dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; f.H1p = ps.H1p; f.sQa = ps.sQa; f.sQn = ps.sQn; }
+    if (fz.dw1_planes) { f.dH2 = nullptr; f.dH2p = ps.dH2p; }
     // first-layer weight gradient from the dH1 plane image (k_dw0_planes): dH1 then leaves the kernel as planes only
     fz.dw0_planes = fz.dw1_planes && ps.dH1p && dw0_planes_eligible(n.in, rows, ps.ldx, ps.X, ps.sXa, ps.sXn);
     if (fz.dw0_planes) { f.dH1 = nullptr; f.dH1p = ps.dH1p; }
     f.dbg = (g_ws_dbg && g_ws_count++ == g_ws_sel) ? g_ws_dbg : nullptr;
     if (mlp_bwd_ws_launch(f, na, st) != cudaSuccess) return fail(SACEO_E_CUDA, "fused backward launch failed");
     count_launch(x, "k_mlp_bwd_ws", st);
+    if (x->prof) x->bwd_variant = mlp_bwd_ws_variant(f);
     fz.chain = true;
     if (dbpart) {     // bias gradients of the two hidden layers come from the kernel's column sums
       k_bias_finish<<<na * n.nnet, 2 * FW_H, 0, st>>>(dbpart, tiles, grads, n.sa, n.sn, n.nnet, n.ob(1), n.ob(0));
@@ -715,6 +726,8 @@ static int mlp_backward(saceo_ctx* x, const Pass& ps, const float* dOut, int ldd
       fz.bias = true;
     }
   }
+  if (ps.H1p && !fz.chain)
+    return fail(SACEO_E_INVALID, "pass on the plane path needs the fused backward (the GEMM chain cannot read the h1 image)");
   return mlp_backward_layers(x, ps, dOut, ldd, sDa, sDn, grads, dXa, A_cols, sXaA, sXaN, fz, st);
 }
 
@@ -738,7 +751,8 @@ static NetD model_net(const saceo_ctx* x, const float* theta, int nnet) {
 }
 
 // Gives a pass the plane images if mlp_backward(grads) of it takes the plane path (fused chain + column-sum biases +
-// k_dw_planes); decided once, so that its forward and backward calls cannot disagree.
+// k_dw_planes); decided once, so that its forward and backward calls cannot disagree.  The images' rows
+// [ps.rows, rup(ps.rows, 32)) must be zero (see Pass::H1p).
 static void plane_path(const saceo_ctx* x, Pass& ps, uint8_t* H1p, uint8_t* dH2p, uint8_t* dH1p, long long sQa, long long sQn) {
   const NetD& n = ps.n;
   if (!n.planes || !x->fuse_bwd || !x->fuse_fwd || !H1p || !dH2p || !dbpart_fits(x, n, ps.rows) || !n.ws()) return;
@@ -1680,6 +1694,57 @@ extern "C" int saceo_test_gemm_ex(const saceo_gemm_args* a, saceo_gemm_route* ro
   for (size_t i = 0; i < tmp.prof_n; ++i) {
     const std::string name = tmp.prof_name[i];
     if (name == "k_gemm_tc") route->n_tc++;
+    else if (name == "k_gemm_skinny") route->n_skinny++;
+    else if (name == "k_gemm_simt") route->n_simt++;
+  }
+  for (cudaEvent_t e : tmp.prof_ev) cudaEventDestroy(e);
+  if (rc) return rc;
+  return check_launch();
+}
+
+extern "C" int saceo_test_mlp_ws(const saceo_mlp_ws_args* a, saceo_mlp_ws_route* route, void* stream) {
+  if (!a || !route || !a->theta || !a->X || !a->H[0] || !a->H[1] || a->n_agents < 1 || a->nnet < 1 || a->rows < 1 ||
+      a->rowsAllocH < a->rows || a->hnets < a->nnet || a->in < 1 || a->nout < 1 || (!a->out && !a->dout))
+    return fail(SACEO_E_INVALID, "bad argument");
+  for (int l = 0; l < 2; ++l)
+    if (a->hidden[l] < 1 || a->act[l] < 0 || a->act[l] > 2) return fail(SACEO_E_INVALID, "bad hidden layer %d", l);
+  if (a->dout && (!a->dH[0] || !a->dH[1] || a->kout < 1 || a->kout > a->nout || (a->dXa && (a->A_cols < 1 || a->A_cols > a->in))))
+    return fail(SACEO_E_INVALID, "bad backward argument");
+  if (a->planes && a->nnet > 1 && a->sTa != a->nnet * a->sTn)
+    return fail(SACEO_E_INVALID, "the plane image needs the nets of an agent at consecutive theta strides");
+  const cudaStream_t st = (cudaStream_t)stream;
+  saceo_ctx tmp;
+  tmp.cfg.n_agents = a->n_agents;
+  tmp.tc = tmp.fuse_fwd = tmp.fuse_bwd = tmp.ws_kernels = true;
+  tmp.prof = true;        // count_launch records each launch's name: the route report
+  tmp.dbpart = a->dbpart; tmp.dbpart_cap = a->dbpart_cap;
+  CU(tc_gemm_init());
+  CU(mlp_ws_init());
+  NetD n = net_desc(a->theta, a->sTa, a->sTn, a->nnet, a->in, a->nout, 2, a->hidden, a->act);
+  if (a->planes && n.ws()) {   // the image, built by the launch ensure_planes uses, for nets the fused kernels take
+    n.planes = a->planes; n.pn = ws_image_bytes(a->in, a->nout); n.pa = a->nnet * n.pn;
+    planes_build(a->theta, a->nnet > 1 ? a->sTn : a->sTa, a->planes, a->in, a->nout, a->n_agents * a->nnet, st);
+  }
+  float* H[2] = {a->H[0], a->H[1]};
+  float* dH[2] = {a->dH[0], a->dH[1]};
+  Pass ps{n, a->X, a->ldx, a->sXa, a->sXn, a->rows, a->rowsAllocH, H, dH};
+  ps.hnets = a->hnets; ps.dout_cols = a->kout;
+  plane_path(&tmp, ps, a->H1p, a->dH2p, a->dH1p, a->sQa, a->sQn);
+  *route = saceo_mlp_ws_route{};
+  route->plane_path = ps.H1p != nullptr;
+  int rc = 0;
+  if (a->out) rc = mlp_forward(&tmp, ps, a->out, a->ldo, a->sOa, a->sOn, st, a->save_h != 0);
+  if (!rc && a->dout)
+    rc = mlp_backward(&tmp, ps, a->dout, a->ldd, a->sDa, a->sDn, a->grads, a->dXa, a->A_cols, a->sXaA, a->sXaN, st);
+  route->bwd_ng = tmp.bwd_variant.ng; route->bwd_na = tmp.bwd_variant.na; route->bwd_mode = tmp.bwd_variant.mode;
+  for (size_t i = 0; i < tmp.prof_n; ++i) {
+    const std::string name = tmp.prof_name[i];
+    if (name == "k_mlp_fwd_ws") route->n_fwd_ws++;
+    else if (name == "k_mlp_bwd_ws") route->n_bwd_ws++;
+    else if (name == "k_dw_planes") route->n_dw_planes++;
+    else if (name == "k_dw0_planes") route->n_dw0_planes++;
+    else if (name == "k_bias_finish") route->n_bias_finish++;
+    else if (name == "k_gemm_tc") route->n_tc++;
     else if (name == "k_gemm_skinny") route->n_skinny++;
     else if (name == "k_gemm_simt") route->n_simt++;
   }

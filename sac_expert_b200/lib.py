@@ -98,6 +98,27 @@ class GemmRoute(C.Structure):
                                          "tc_bn", "tc_stages", "tc_threads")]
 
 
+class MlpWsArgs(C.Structure):
+    """saceo_mlp_ws_args (include/saceo.h): one pass of the MLP dispatch, for saceo_test_mlp_ws."""
+    _fields_ = [(n, C.c_int32) for n in ("n_agents", "nnet", "hnets", "in_", "nout", "kout")] + \
+               [("hidden", C.c_int32 * 2), ("act", C.c_int32 * 2), ("rows", C.c_int32), ("rowsAllocH", C.c_int64),
+                ("theta", C.c_void_p), ("sTa", C.c_int64), ("sTn", C.c_int64),
+                ("X", C.c_void_p), ("ldx", C.c_int32), ("sXa", C.c_int64), ("sXn", C.c_int64),
+                ("out", C.c_void_p), ("ldo", C.c_int32), ("sOa", C.c_int64), ("sOn", C.c_int64),
+                ("dout", C.c_void_p), ("ldd", C.c_int32), ("sDa", C.c_int64), ("sDn", C.c_int64),
+                ("H", C.c_void_p * 2), ("dH", C.c_void_p * 2)] + \
+               [(n, C.c_void_p) for n in ("planes", "H1p", "dH2p", "dH1p")] + \
+               [("sQa", C.c_int64), ("sQn", C.c_int64), ("dbpart", C.c_void_p), ("dbpart_cap", C.c_int64),
+                ("grads", C.c_void_p), ("dXa", C.c_void_p), ("A_cols", C.c_int32), ("sXaA", C.c_int64),
+                ("sXaN", C.c_int64), ("save_h", C.c_int32)]
+
+
+class MlpWsRoute(C.Structure):
+    """saceo_mlp_ws_route (include/saceo.h): which kernels a saceo_test_mlp_ws call launched."""
+    _fields_ = [(n, C.c_int32) for n in ("plane_path", "n_fwd_ws", "n_bwd_ws", "n_dw_planes", "n_dw0_planes",
+                                         "n_bias_finish", "n_tc", "n_skinny", "n_simt", "bwd_ng", "bwd_na", "bwd_mode")]
+
+
 FIT_HYPER = 8
 FIT_HYPER_NAMES = ("model_lr", "reward_loss_coef", "delta_clip_loss", "reward_clip_loss", "model_max_grad_norm",
                    "r_mean", "r_std", "scale_model_loss")
@@ -111,7 +132,7 @@ EXPORTS = [
     "saceo_actor_forward", "saceo_critic_forward", "saceo_model_eval", "saceo_fvp", "saceo_cg_solve",
     "saceo_fit_bind", "saceo_model_fit", "saceo_trpo_grad", "saceo_trpo_eval", "saceo_actor_step", "saceo_ppo_grad", "saceo_actor_adam", "saceo_onpolicy_expert_grad", "saceo_grad_blend",
     "saceo_policy_layout", "saceo_policy_act",
-    "saceo_debug_ptr", "saceo_launch_count", "saceo_test_gemm", "saceo_test_gemm_ex", "saceo_last_error", "saceo_abi_version",
+    "saceo_debug_ptr", "saceo_launch_count", "saceo_test_gemm", "saceo_test_gemm_ex", "saceo_test_mlp_ws", "saceo_last_error", "saceo_abi_version",
 ]
 
 
@@ -161,6 +182,7 @@ def load() -> C.CDLL:
         "saceo_launch_count": (i64, [vp]),
         "saceo_test_gemm": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp]),
         "saceo_test_gemm_ex": (C.c_int, [C.POINTER(GemmArgs), C.POINTER(GemmRoute), vp]),
+        "saceo_test_mlp_ws": (C.c_int, [C.POINTER(MlpWsArgs), C.POINTER(MlpWsRoute), vp]),
         "saceo_last_error": (C.c_char_p, []),
         "saceo_abi_version": (C.c_int, []),
     }
